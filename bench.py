@@ -2,6 +2,7 @@
 """bench.py -- megapixels/s of the JPEG encode hot path on N B200s (BASELINE.json `metric`).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c1|c2|c4a|c4b|c5] [--impl reference]
+                    [--dump-outputs DIR]
 
 A step = one pass of the whole encode path (colour -> DCT -> quant -> entropy -> stuffed JFIF bytes)
 over one batch of synthetic frames. Default workload: BASELINE config 3, a batch of 1920x1080 RGB
@@ -78,6 +79,30 @@ def resolve_cfg(cfg):
 def frames_for(width, height, color, n_distinct):
     import images
     return [images.synth_frame(width, height, BPP[color], seed=s) for s in range(n_distinct)]
+
+
+DUMP_WINDOW = 1 << 15  # bytes per window of a sampled dump
+DUMP_BUDGET = 8 << 20  # bytes of the timed path's stream per dump (x4 as float32); the config-5 leg of the default line adds half
+
+
+def dump_outputs(out_dir, name, d_bytes, offsets, budget):
+    """--dump-outputs: what a caller of the timed path receives from one step -- the JPEG files back to back in
+    device memory (`d_bytes`, uint8) and the file offsets -- written as <name>_offsets.npy (float64, every file) and
+    <name>_bytes.npy (float32). A stream longer than `budget` bytes is sampled: budget / DUMP_WINDOW windows of
+    DUMP_WINDOW contiguous bytes at starts drawn from a fixed seed (<name>_window_starts.npy, float64), so two builds
+    that produce the same stream dump the same arrays."""
+    import torch
+    n = int(offsets[-1])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + "_offsets.npy"), np.asarray(offsets, dtype=np.float64))
+    if n <= budget:
+        data = d_bytes[:n]
+    else:
+        starts = np.sort(np.random.default_rng(20261020).integers(0, n - DUMP_WINDOW + 1, budget // DUMP_WINDOW))
+        np.save(os.path.join(out_dir, name + "_window_starts.npy"), starts.astype(np.float64))
+        idx = torch.from_numpy(starts[:, None] + np.arange(DUMP_WINDOW)).to(d_bytes.device)
+        data = d_bytes[idx]
+    np.save(os.path.join(out_dir, name + "_bytes.npy"), data.cpu().numpy().astype(np.float32))
 
 
 def stage_a_bytes(width, height, color, cfg):
@@ -288,10 +313,11 @@ def run_product(args):
 
     rank_ms = []
 
-    def timed_device(n_frames, stage_timers=False):
+    def timed_device(n_frames, stage_timers=False, dump=False):
         """K timed steps of the device-resident path over the first n_frames resident frames: (ms per step max over
         ranks, per-stage ms, launches). With stage_timers the library brackets every stage with CUDA events (and
-        launches kernel by kernel instead of replaying its CUDA graph): used for the breakdown, not for `value`."""
+        launches kernel by kernel instead of replaying its CUDA graph): used for the breakdown, not for `value`.
+        With dump and --dump-outputs, rank 0 writes the files of the last timed step."""
         device.set_timing(stage_timers)
         for _ in range(args.warmup):
             enc.encode_batch_device(d_in.data_ptr(), stride, n_frames, width, height, ct)
@@ -300,12 +326,14 @@ def run_product(args):
         stage_ms_, launches_ = {}, 0
         e0.record(stream)
         for _ in range(args.steps):
-            enc.encode_batch_device(d_in.data_ptr(), stride, n_frames, width, height, ct)
+            d_files_, offs_ = enc.encode_batch_device(d_in.data_ptr(), stride, n_frames, width, height, ct)
             launches_ += device.last_launch_count()
             for k, v in (device.last_timing() or {}).items():
                 stage_ms_[k] = stage_ms_.get(k, 0.0) + v
         e1.record(stream)
         barrier()
+        if dump and args.dump_outputs and rank == 0:  # before the next call on the context reuses its output buffer
+            dump_outputs(args.dump_outputs, "files", _as_tensor(d_files_, offs_[-1], dev_t), offs_, DUMP_BUDGET)
         ms_ = e0.elapsed_time(e1)
         if world > 1:
             t_ = torch.tensor([ms_], device=dev_t)
@@ -322,7 +350,7 @@ def run_product(args):
     if rank == 0:
         sampler.start()
         time.sleep(0.3)
-    ms_per_step, _, launches = timed_device(batch)
+    ms_per_step, _, launches = timed_device(batch, dump=True)
     rank_ms_value = list(rank_ms)
     _, stage_ms, _ = timed_device(batch, stage_timers=True)  # second pass: per-stage breakdown and the roofline numerator
     device.set_timing(False)
@@ -437,8 +465,7 @@ def run_product(args):
         torch.cuda.empty_cache()
         c5_args = argparse.Namespace(**vars(args))
         c5_args.workload, c5_args.size, c5_args.skip_parity = "c5", args.c5_size, False
-        c5_args.steps, c5_args.warmup = max(3, min(args.steps, 10)), max(3, min(args.warmup, 5))
-        c5_line = run_strips(c5_args, rank, world, local, dev_t, extra=True)
+        c5_line = run_strips(c5_args, rank, world, local, dev_t, extra=True, dump_name="c5_file")
         if rank == 0:
             c5 = {k: c5_line[k] for k in ("value", "unit", "ms_per_step", "steps", "warmup", "scaling", "gpu_launches", "stage_ms_per_step", "gather_ms_per_step")}
             c5.update(parity=True, workload=c5_line["config"]["workload"], strips=c5_line["config"]["strips"], bytes_out=c5_line["config"]["bytes_out"],
@@ -523,7 +550,7 @@ def run_product(args):
 
 
 # ---- one very large image, strips across the GPUs (BASELINE config 5) ---------------------------
-def run_strips(args, rank, world, local, dev_t, extra=False):
+def run_strips(args, rank, world, local, dev_t, extra=False, dump_name="file"):
     import torch
     import torch.distributed as dist
     import images
@@ -623,10 +650,13 @@ def run_strips(args, rank, world, local, dev_t, extra=False):
     launches = 0
     e0.record(stream)
     for _ in range(args.steps):
-        _, l, _ = step(timed=True)
+        out, l, _ = step(timed=True)
         launches += l
     e1.record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:  # the last timed step's file, before the next step overwrites it
+        f = fetch(out)
+        dump_outputs(args.dump_outputs, dump_name, f, [0, f.numel()], DUMP_BUDGET // 2 if extra else DUMP_BUDGET)
     # second pass with the library's per-stage events (kernel-by-kernel launches instead of the graph replay): breakdown only
     device.set_timing(True)
     stage_ms = {}
@@ -798,7 +828,11 @@ def main():
     ap.add_argument("--no-c5", action="store_true", help="default workload only: skip the config-5 (strips + gather) leg")
     ap.add_argument("--no-weak", action="store_true", help="default workload only: skip the weak-scaling leg at N > 1")
     ap.add_argument("--skip-parity", action="store_true", help="c5 only: skip the whole-image oracle comparison")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's outputs of the last timed step as .npy files "
+                    "(JPEG bytes as float32, a fixed sample of long streams; offsets as float64) for comparing builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)

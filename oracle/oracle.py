@@ -3,9 +3,12 @@
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs import
 this module. The product package (jpeg_encoder_b200) never does.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -33,9 +36,27 @@ class _Params(C.Structure):
     ]
 
 
+_native_dir = None
+
+
+def _native_path():
+    """The -march=native build suits only the machine that runs it, and its users (bench.py) may run from a read-only
+    tree: it goes to a temporary directory of this process, removed at exit."""
+    global _native_dir
+    if _native_dir is None:
+        _native_dir = tempfile.mkdtemp(prefix="jpeg_oracle_native_")
+        atexit.register(shutil.rmtree, _native_dir, True)
+    return os.path.join(_native_dir, "liborc_native.so")
+
+
 def build(native=False, force=False):
     """Compile the oracle with gcc (oracle/Makefile). Returns the path of the shared object."""
-    target = "liborc_native.so" if native else "liborc.so"
+    if native:
+        path = _native_path()
+        if force or not os.path.exists(path):
+            subprocess.check_call(["make", "-C", _DIR, "NATIVE_SO=" + path, path], stdout=subprocess.DEVNULL)
+        return path
+    target = "liborc.so"
     path = os.path.join(_DIR, target)
     src = os.path.join(_DIR, "jpeg_oracle.c")
     stale = (not os.path.exists(path)) or os.path.getmtime(path) < max(

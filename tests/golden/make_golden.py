@@ -4,6 +4,8 @@ exist on the GPU box):  python tests/golden/make_golden.py
 * rgb_to_ycbcr_kat.json, fdct_kat.json: the literal known-answer vectors of the reference's own unit tests,
   read out of its sources (test_rgb_to_ycbcr, /root/reference/src/image_buffer.rs:324-421; test_fdct_libjpeg,
   /root/reference/src/fdct.rs:249-300).
+* reference_constants.json: the reference's constant data, read out of its sources: the 9 + 9 quantization table
+  families (src/quantization.rs), the four K.3 Huffman tables (src/huffman.rs) and ZIGZAG (src/writer.rs).
 * oracle_jpegs.json: SHA-256 and length of the oracle's file bytes for a fixed matrix of configurations over
   deterministic images. It guards the oracle against regressions (tests/test_oracle.py) and gives the GPU
   tests a committed target that does not depend on the oracle being built (tests/test_gpu_parity.py).
@@ -75,8 +77,42 @@ def kat_fdct():
     return out
 
 
+def reference_constants():
+    def families(src, name):
+        body = re.search(r"static " + name + r"[^=]*=\s*\[(.*?)\n\];", src, re.S).group(1)
+        out = []
+        for a in re.findall(r"\[([^\[\]]*?)\]", body, re.S):
+            nums = ints(re.sub(r"//.*", "", a))
+            if len(nums) == 64:
+                out.append(nums)
+        assert len(out) == 9, name
+        return out
+
+    def hex_array(src, name):
+        return [int(x, 16) for x in re.findall(r"0x[0-9A-Fa-f]+", re.search(r"static " + name + r"[^=]*=\s*\[(.*?)\];", src, re.S).group(1))]
+
+    quant = open(os.path.join(REF, "quantization.rs")).read()
+    huff = open(os.path.join(REF, "huffman.rs")).read()
+    writer = open(os.path.join(REF, "writer.rs")).read()
+    return {
+        "quantization_luma": families(quant, "DEFAULT_LUMA_TABLES"),
+        "quantization_chroma": families(quant, "DEFAULT_CHROMA_TABLES"),
+        "huffman": {k: {"counts": hex_array(huff, "DEFAULT_%s_CODE_LENGTHS" % k.upper()), "values": hex_array(huff, "DEFAULT_%s_VALUES" % k.upper())}
+                    for k in ("luma_dc", "luma_ac", "chroma_dc", "chroma_ac")},
+        "zigzag": ints(re.search(r"ZIGZAG[^=]*=\s*\[(.*?)\];", writer, re.S).group(1)),
+    }
+
+
+def write_reference_constants(consts):
+    """one table per line"""
+    s = json.dumps(consts, separators=(",", ":"))
+    s = s.replace("],[", "],\n[").replace('{"', '{\n"').replace(',"', ',\n"')
+    open(os.path.join(HERE, "reference_constants.json"), "w").write(s + "\n")
+
+
 def main():
     if os.path.isdir(REF):
+        write_reference_constants(reference_constants())
         rgb = kat_rgb()
         assert len(rgb) > 50
         json.dump(rgb, open(os.path.join(HERE, "rgb_to_ycbcr_kat.json"), "w"))

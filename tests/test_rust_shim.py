@@ -28,15 +28,6 @@ def api():
     return json.load(open(GOLD))
 
 
-def test_golden_is_current_with_the_reference(api):
-    if not os.path.isdir("/root/reference/src"):
-        pytest.skip("reference sources are only present in the build container")
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import make_rust_api
-    assert make_rust_api.extract() == api, "re-run tests/golden/make_rust_api.py"
-
-
 def _enum_body(shim, name):
     m = re.search(r"pub enum %s \{" % re.escape(name), shim)
     assert m, "enum %s missing" % name
