@@ -22,6 +22,14 @@ using namespace jpgb;
 
 namespace {
 
+// test hook (JPGB_POISON_ALLOC=1): every buffer a context allocates starts out as all ones, so a read of memory that no
+// call has written shows the same way every time instead of depending on what the allocator hands back. Read only when
+// a buffer is (re)allocated: steady-state calls never get here.
+bool poison_alloc() {
+    const char *e = std::getenv("JPGB_POISON_ALLOC");
+    return e && e[0] == '1';
+}
+
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
@@ -34,6 +42,10 @@ struct DevBuf {
         want = (want + 255) & ~(size_t)255;
         cudaError_t e = cudaMalloc(&p, want);
         if (e == cudaSuccess) cap = want;
+        if (e == cudaSuccess && poison_alloc()) { // filled before the caller can enqueue work on another stream
+            e = cudaMemset(p, 0xFF, want);
+            if (e == cudaSuccess) e = cudaDeviceSynchronize();
+        }
         return e;
     }
     template <typename T>
@@ -55,7 +67,10 @@ struct PinnedBuf {
         cap = 0;
         const size_t want = bytes + bytes / 8 + 256;
         cudaError_t e = cudaMallocHost(&p, want);
-        if (e == cudaSuccess) cap = want;
+        if (e == cudaSuccess) {
+            cap = want;
+            if (poison_alloc()) std::memset(p, 0xFF, want);
+        }
         return e;
     }
     template <typename T>
@@ -405,6 +420,15 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, 
         ocap = enc->caps[1];
         pool_units = enc->caps[2];
     }
+    // test hook (JPGB_TIGHT_CAPS, a comma list of pool, stream, out): attempt 0 starts from the floor of each named
+    // capacity, so the retry branch that capacity leads to (recode, tail with a larger stream, tail with a larger output)
+    // runs on purpose
+    if (const char *tight = std::getenv("JPGB_TIGHT_CAPS")) {
+        const std::string t = std::string(",") + tight + ",";
+        if (t.find(",pool,") != std::string::npos) pool_units = 1;
+        if (t.find(",stream,") != std::string::npos) ucap = kStuffChunk;
+        if (t.find(",out,") != std::string::npos) ocap = 4096;
+    }
     bool coded = false;
     const char *poison_env = std::getenv("JPGB_POISON_STREAM");
     const bool poison = poison_env && poison_env[0] == '1';
@@ -440,10 +464,10 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, 
         b.out_cap = ocap;
         const bool with_tables = optimized && attempt == 0, with_coder = !coded;
         auto enqueue = [&]() -> int {
-            // status words of the coder (all, or all but the pool cursor when only the tail is repeated) and of the table build
+            // status words of the coder and of the table build (only the words the tail writes when only the tail is repeated)
             if (with_coder) {
                 CK(cudaMemsetAsync(b.status, 0, 2 * kStatusWords * 8 + mask_bytes, st), "clear status and raw mask");
-            } else { // the pool cursor (and the table status) stay
+            } else { // the pool cursor and the table status are not read again (see below)
                 CK(cudaMemsetAsync(b.status, 0, 4 * 8, st), "clear status");
                 CK(cudaMemsetAsync(b.raw_mask, 0, mask_bytes, st), "clear raw mask");
             }
@@ -550,9 +574,12 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, 
         const uint64_t *status = enc->h_small.as<uint64_t>() + (n + 1);
         if (status[3]) return fail(enc, JPGB_ERR_CUDA, "internal: prefix-sum look-back timed out");
         if (status[2] & 8) return fail(enc, JPGB_ERR_BAD_PARAMS, "a scan segment exceeds 4 GiB (use a restart interval)");
-        if (optimized && (status[kStatusWords + 2] & 16)) return fail(enc, JPGB_ERR_HUFFMAN, "an optimized Huffman code does not fit (longer than 32 bits, or code plus value bits beyond 31)");
+        // What survives a tail-only attempt is the device buffers the coder wrote (pool, chunk and segment positions), not
+        // the status block: it grows with the raw mask, so a larger stream reallocates it. The table flag is read on the
+        // attempt that built the tables, the pool cursor on an attempt that ran the coder.
+        if (with_tables && (status[kStatusWords + 2] & 16)) return fail(enc, JPGB_ERR_HUFFMAN, "an optimized Huffman code does not fit (longer than 32 bits, or code plus value bits beyond 31)");
         ubytes = status[0];
-        pool_used = status[5];
+        if (with_coder) pool_used = status[5];
         if (status[2] == 0) {
             total = ubytes + status[1];
             break;

@@ -721,6 +721,15 @@ def _random_cases(n=None, seed=None):
     return out
 
 
+def _sweep_image(i, color, w, h, kind):
+    rng = np.random.default_rng(1000 + i)
+    if kind == "photo":
+        return _img(color, w, h, seed=i)
+    if kind == "noise":
+        return rng.integers(0, 256, (h, w, BPP[color]), dtype=np.uint8)
+    return np.full((h, w, BPP[color]), int(rng.integers(0, 256)), np.uint8)
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("chunk", range(8))
 def test_random_settings_sweep(chunk):
@@ -729,13 +738,7 @@ def test_random_settings_sweep(chunk):
     file must equal the oracle's byte for byte."""
     failures = []
     for i, color, w, h, cfg, kind in _random_cases()[chunk::8]:
-        rng = np.random.default_rng(1000 + i)
-        if kind == "photo":
-            img = _img(color, w, h, seed=i)
-        elif kind == "noise":
-            img = rng.integers(0, 256, (h, w, BPP[color]), dtype=np.uint8)
-        else:
-            img = np.full((h, w, BPP[color]), int(rng.integers(0, 256)), np.uint8)
+        img = _sweep_image(i, color, w, h, kind)
         got = gpu_encode(img, w, h, color, cfg)
         want = oracle_encode(img, w, h, color, cfg)
         if got != want:
