@@ -196,7 +196,8 @@ int jpgb_gather_target_open(jpgb_encoder *enc, const uint8_t ipc_handle[64], voi
 int jpgb_gather_target_close(jpgb_encoder *enc, void *d_target, int opened_from_handle);
 int jpgb_last_piece_offsets_device(jpgb_encoder *enc, const uint64_t **d_offsets, uint32_t *n_scans);
 /* d_table: world * (n_scans + 1) piece offsets in rank order (device memory). d_total (optional, device): receives the
- * size of the assembled file. Pieces are read from the output of the last jpgb_encode_strip_device* call. */
+ * size of the assembled file. Pieces are read from the output of the last jpgb_encode_strip_device* call. A piece that
+ * would overrun target_capacity is not written; *d_total > target_capacity reports it. */
 int jpgb_gather_place_pieces(jpgb_encoder *enc, void *d_target, size_t target_capacity, const uint64_t *d_table, uint32_t world,
                              uint32_t rank, uint64_t *d_total);
 

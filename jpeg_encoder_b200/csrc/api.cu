@@ -11,6 +11,7 @@
 #include <condition_variable>
 #include <mutex>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/jpegenc_b200.h"
@@ -30,61 +31,39 @@ bool poison_alloc() {
     return e && e[0] == '1';
 }
 
-struct DevBuf {
+// A device (cudaMalloc) or pinned host (cudaMallocHost) buffer, freed with its owner
+template <bool kPinned>
+struct Buf {
     void *p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(Buf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    Buf &operator=(Buf o) noexcept { // the old buffer leaves with `o`
+        std::swap(p, o.p);
+        std::swap(cap, o.cap);
+        return *this;
+    }
+    ~Buf() { if (p) kPinned ? cudaFreeHost(p) : cudaFree(p); }
     cudaError_t reserve(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
+        *this = Buf();
         size_t want = bytes + bytes / 8 + 256; // grow-only with slack: steady-state calls never allocate
-        want = (want + 255) & ~(size_t)255;
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e == cudaSuccess) cap = want;
-        if (e == cudaSuccess && poison_alloc()) { // filled before the caller can enqueue work on another stream
-            e = cudaMemset(p, 0xFF, want);
-            if (e == cudaSuccess) e = cudaDeviceSynchronize();
+        if (!kPinned) want = (want + 255) & ~(size_t)255;
+        cudaError_t e = kPinned ? cudaMallocHost(&p, want) : cudaMalloc(&p, want);
+        if (e != cudaSuccess) return p = nullptr, e;
+        cap = want;
+        if (poison_alloc()) { // device memory is filled before the caller can enqueue work on another stream
+            if (kPinned) std::memset(p, 0xFF, want);
+            else if ((e = cudaMemset(p, 0xFF, want)) == cudaSuccess) e = cudaDeviceSynchronize();
         }
         return e;
     }
     template <typename T>
     T *as() const { return static_cast<T *>(p); }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
 };
+using DevBuf = Buf<false>;
+using PinnedBuf = Buf<true>;
 
-struct PinnedBuf {
-    void *p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        const size_t want = bytes + bytes / 8 + 256;
-        cudaError_t e = cudaMallocHost(&p, want);
-        if (e == cudaSuccess) {
-            cap = want;
-            if (poison_alloc()) std::memset(p, 0xFF, want);
-        }
-        return e;
-    }
-    template <typename T>
-    T *as() const { return static_cast<T *>(p); }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
-
-} // namespace
-
-namespace {
 // What the device plan is a function of: the caller's settings without the APPn payloads (they only change header
 // bytes, which are uploaded, not baked into launches), the strip and the input kind.
 struct PlanSig {
@@ -123,13 +102,67 @@ struct CapKey {
     uint64_t raw_bytes;
     uint32_t n, pad;
 };
+
+// Capacities of one attempt: unstuffed stream and output in bytes, chunk pool in 16-byte units
+struct Caps { uint64_t ustream, out, pool_units; };
+
+// What a captured launch sequence bakes in (graph_key), word by word: no padding of the caller's structs takes part
 struct GraphKey {
-    EntropyBuffers b;
-    CoderLaunch coder;
     PlanSig sig;
-    uint64_t misc[8];
-    uint32_t n, flags;
+    uint64_t words[39];
 };
+
+// Replay of the launch sequence behind stage A as a CUDA graph (same settings, batch size and buffers)
+struct GraphCache {
+    struct Slot {
+        cudaGraphExec_t exec = nullptr;
+        GraphKey key{};
+        uint32_t launches = 0;
+        uint64_t used = 0;
+    } slots[4]; // the pipelined host path alternates between two pixel / output buffers and ends on a shorter chunk
+    uint64_t clock = 0;
+    bool ok = true; // false once a capture failed (e.g. on the legacy default stream): launches go direct from then on
+    ~GraphCache() {
+        for (Slot &s : slots)
+            if (s.exec) cudaGraphExecDestroy(s.exec);
+    }
+    // Launches the graph of `key`, first capturing it from `enqueue` (which counts its launches in `launches`) when no
+    // slot holds it; the least recently used slot makes room. `replayed` stays false when capture failed: the caller
+    // then enqueues directly.
+    template <typename Enqueue>
+    cudaError_t replay(const GraphKey &key, cudaStream_t st, uint32_t &launches, Enqueue &&enqueue, bool &replayed) {
+        Slot *slot = nullptr, *victim = &slots[0];
+        for (Slot &g : slots) {
+            if (g.exec && std::memcmp(&g.key, &key, sizeof(key)) == 0) slot = &g;
+            if (!g.exec || (victim->exec && g.used < victim->used)) victim = &g;
+        }
+        if (!slot) {
+            if (victim->exec) cudaGraphExecDestroy(victim->exec), victim->exec = nullptr;
+            const uint32_t launches_before = launches;
+            cudaGraph_t graph = nullptr;
+            const bool capturing = cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
+            const int rc = capturing ? enqueue() : JPGB_ERR_CUDA;
+            if (capturing && cudaStreamEndCapture(st, &graph) == cudaSuccess && rc == JPGB_OK && graph &&
+                cudaGraphInstantiate(&victim->exec, graph, 0) == cudaSuccess) {
+                victim->key = key;
+                victim->launches = launches - launches_before;
+                slot = victim;
+            } else {
+                victim->exec = nullptr;
+                ok = false;
+            }
+            if (graph) cudaGraphDestroy(graph);
+            launches = launches_before;
+            cudaGetLastError();
+        }
+        if (!slot) return cudaSuccess;
+        slot->used = ++clock;
+        const cudaError_t e = cudaGraphLaunch(slot->exec, st);
+        if (e == cudaSuccess) launches += slot->launches, replayed = true;
+        return e;
+    }
+};
+
 } // namespace
 
 struct jpgb_encoder {
@@ -138,7 +171,7 @@ struct jpgb_encoder {
     bool own_stream = false;
     std::string err;
     DevBuf pixels, coef, huff, hdr, hdr_len, scratch, pool, chunk_bits, chunk_pool, chunk_bitpos, seglen, segpos, ustream, ffcount, ffpos,
-        out, scan_tmp, hist, piece_off, out2, pixels2, status, aux_status, hdr_parts;
+        out, scan_tmp, hist, piece_off, out2, pixels2, status, hdr_parts;
     std::vector<uint8_t> last_tables; // what the device currently holds
     double ucap_ratio = 0; // unstuffed-stream bytes to provision per raw pixel byte, learnt from earlier calls
     double pool_ratio = 0; // the same for the chunk pool (code bytes incl. per-chunk alignment)
@@ -146,7 +179,6 @@ struct jpgb_encoder {
     cudaEvent_t ev_stage[2] = {};
     bool stage_busy[2] = {};
     CopyPool copy_pool;
-    int out_slot = 0; // which of out / out2 the next encode_device writes
     cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
     std::vector<cudaEvent_t> ev_slice;
     cudaEvent_t ev_in[2] = {}, ev_out[2] = {}, ev_enc[2] = {};
@@ -164,20 +196,12 @@ struct jpgb_encoder {
     const void *coef_pixels = nullptr;
     uint64_t coef_stride = 0;
     float coef_ms[2] = {0.f, 0.f}; // with timing on: what the colour+DCT kernel and the histogram of that call took (added to the reusing call's stages)
-    // replay of the launch sequence behind stage A as a CUDA graph (same settings, batch size and buffers)
-    bool graphs_ok = true;
-    struct CachedGraph {
-        cudaGraphExec_t exec = nullptr;
-        GraphKey key{};
-        uint32_t launches = 0;
-        uint64_t used = 0;
-    } graphs[4]; // the pipelined host path alternates between two pixel / output buffers and ends on a shorter chunk
-    uint64_t graph_clock = 0;
+    GraphCache graphs;
+    // Capacities are sticky per (settings, batch size): steady-state calls provision exactly what the last successful
+    // call settled on, so the launch sequence has identical parameters call after call and is replayed as a CUDA graph.
     bool have_caps = false;
     CapKey cap_key{};
-    uint64_t caps[3] = {};
-    // result of the last device batch
-    uint64_t out_total = 0;
+    Caps caps{};
 };
 
 namespace {
@@ -240,78 +264,42 @@ int validate_and_plan(jpgb_encoder *enc, const jpgb_params *p, size_t len_each, 
     return JPGB_OK;
 }
 
-// The whole device pipeline for `n` device-resident images. On success the files lie back to back
-// in enc->out and `offsets` (host, n + 1) delimits them.
-// `given_hist` (strips with optimized tables): the symbol histogram of the *whole* image, [table][dc|ac][257],
-// used instead of the one of these pixels.
-int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, size_t image_stride, uint32_t n,
-                  std::vector<uint64_t> &offsets, std::vector<uint64_t> *piece_offsets = nullptr, const uint32_t *given_hist = nullptr,
-                  bool coef_ready = false) {
+// Where the launches find the file headers in enc->hdr
+struct HeaderLayout {
+    size_t hdr_stride = 0;               // bytes between the headers of two images
+    uint32_t head_len = 0, tail_len = 0; // optimized tables: header bytes in front of / behind the DHT segments
+    int n_tables = 0;                    // optimized tables: tables per class and image (1 or 2)
+};
+
+// Huffman tables and the file header (SOI/APPn prefix, SOF/DQT/DHT/DRI, first SOS -- Q21).
+// Default tables (Annex K.3): built on the host once per settings, shared by all images.
+// Optimized tables: per image on the device, from its symbol histogram (tables.cu) -- no host round trip. Here only
+// the header parts around the DHT segments, and for strips the whole image's histogram `given_hist`.
+int setup_header(jpgb_encoder *enc, const Plan &plan, uint32_t n, const uint32_t *given_hist, HeaderLayout &hl) {
     cudaStream_t st = enc->stream;
-    DevPlan hp;
-    plan.fill_device_plan(hp);
-    StageAParams ap;
-    plan.fill_stage_a(ap);
-
-    const uint64_t n_blocks = plan.blocks_per_image * n;
-    const uint64_t n_segs = (uint64_t)plan.segs_per_image * n;
-
-    CK(enc->coef.reserve(n_blocks * 128), "alloc coefficients");
-    if (!coef_ready) enc->coef_tagged = false;
-    // ---- stage A (unless the caller has already run it slice by slice behind the upload) ----
-    if (!coef_ready) {
-        StageTimer t(enc, 0);
-        ap.pixels = d_pixels;
-        ap.coef = enc->coef.as<int16_t>();
-        ap.image_stride = image_stride;
-        CK(launch_stage_a(ap, n, st), "stage A launch");
-        enc->launches += 1;
-    }
-
-    // One device buffer (allocated below, next to the stream it describes): [n + 1 file offsets][8 status words of the
-    // entropy stage (word 3: look-back scan error)][8 status words of the table build][raw-byte mask of the stream].
-    // The first three parts are read back with one copy; the last three are cleared with one memset.
-    unsigned long long *aux_status = nullptr, *scan_err = nullptr;
-
-    // ---- Huffman tables and the file header (SOI/APPn prefix, SOF/DQT/DHT/DRI, first SOS -- Q21) ----
-    // Default tables (Annex K.3): built on the host once per settings, shared by all images.
-    // Optimized tables: per image on the device, from its symbol histogram (tables.cu) -- no host round trip.
     const bool optimized = plan.p.optimize_huffman != 0;
     const uint32_t n_huff = optimized ? n : 1;
-    HuffTable tables[4];
-    default_huffman_tables(reinterpret_cast<HuffTable(*)[2]>(tables));
-    size_t hdr_stride = 0;
-    uint32_t opt_head_len = 0, opt_tail_len = 0;
-    int opt_tables = 0;
-    CK(enc->huff.reserve((size_t)n_huff * kHuffWordsPerImage * 4), "alloc huffman tables");
+    const size_t tab_bytes = kHuffWordsPerImage * 4;
+    CK(enc->huff.reserve((size_t)n_huff * tab_bytes), "alloc huffman tables");
     CK(enc->hdr_len.reserve((size_t)n_huff * 4), "alloc header lengths");
-    if (!optimized) {
+    std::vector<uint8_t> fresh; // what the device is to hold
+    if (!optimized) { // [kernel words of the four tables][header, padded to hdr_stride][header length]
+        HuffTable tables[4];
+        default_huffman_tables(reinterpret_cast<HuffTable(*)[2]>(tables));
         std::vector<uint8_t> h = plan.prefix;
         plan.frame_header(reinterpret_cast<const HuffTable(*)[2]>(tables), h);
         h.insert(h.end(), plan.scans[0].sos.begin(), plan.scans[0].sos.end());
-        hdr_stride = (h.size() + 15) & ~(size_t)15;
-        const size_t tab_bytes = kHuffWordsPerImage * 4, blob = tab_bytes + hdr_stride + 4;
-        CK(enc->h_tables.reserve(blob), "alloc tables (host)");
-        uint8_t *hb = enc->h_tables.as<uint8_t>();
-        std::vector<uint8_t> fresh(blob, 0);
+        hl.hdr_stride = (h.size() + 15) & ~(size_t)15;
+        fresh.assign(tab_bytes + hl.hdr_stride + 4, 0);
+        CK(enc->h_tables.reserve(fresh.size()), "alloc tables (host)");
         for (int t = 0; t < 4; ++t) // [table][dc, ac]
             if (!tables[t].device_words(t & 1, reinterpret_cast<uint32_t *>(fresh.data() + (size_t)t * 1024)))
                 return fail(enc, JPGB_ERR_HUFFMAN, "a Huffman code plus its value bits exceeds 31 bits");
         std::memcpy(fresh.data() + tab_bytes, h.data(), h.size());
-        const uint32_t hl = (uint32_t)h.size();
-        std::memcpy(fresh.data() + tab_bytes + hdr_stride, &hl, 4);
-        CK(enc->hdr.reserve(hdr_stride), "alloc headers");
-        if (enc->last_tables != fresh) { // repeated calls with the same settings skip the upload (the device copy is still valid)
-            CK(cudaStreamSynchronize(enc->stream), "staging reuse sync"); // an earlier upload may still read h_tables
-            enc->last_tables = fresh;
-            std::memcpy(hb, fresh.data(), blob);
-            CK(cudaMemcpyAsync(enc->huff.p, hb, tab_bytes, cudaMemcpyHostToDevice, st), "upload huffman tables");
-            CK(cudaMemcpyAsync(enc->hdr.p, hb + tab_bytes, hdr_stride, cudaMemcpyHostToDevice, st), "upload headers");
-            CK(cudaMemcpyAsync(enc->hdr_len.p, hb + tab_bytes + hdr_stride, 4, cudaMemcpyHostToDevice, st), "upload header lengths");
-        }
-    } else {
-        // head = everything in front of the DHT segments, tail = what follows them (writer.rs:390-422, encoder.rs:633-667)
-        std::vector<uint8_t> with, without;
+        const uint32_t len = (uint32_t)h.size();
+        std::memcpy(fresh.data() + tab_bytes + hl.hdr_stride, &len, 4);
+    } else { // [head][tail][0xA5]: head = everything in front of the DHT segments, tail = what follows them (writer.rs:390-422, encoder.rs:633-667)
+        std::vector<uint8_t> with;
         {
             HuffTable empty[2][2];
             const uint8_t none[16] = {0};
@@ -320,60 +308,225 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, 
             with = plan.prefix;
             plan.frame_header(empty, with); // DHT segments with no values: 21 bytes each
         }
-        const int n_tables = plan.ncomp >= 3 ? 2 : 1; // encoder.rs:648-660, 1089
+        hl.n_tables = plan.ncomp >= 3 ? 2 : 1; // encoder.rs:648-660, 1089
         size_t dht_at = plan.prefix.size(); // first DHT marker: behind SOF and the two DQT
         while (dht_at + 3 < with.size() && !(with[dht_at] == 0xFF && with[dht_at + 1] == 0xC4))
             dht_at += 2 + ((size_t)with[dht_at + 2] << 8 | with[dht_at + 3]);
-        std::vector<uint8_t> head(with.begin(), with.begin() + dht_at);
-        std::vector<uint8_t> tail(with.begin() + dht_at + (size_t)n_tables * 2 * 21, with.end());
-        tail.insert(tail.end(), plan.scans[0].sos.begin(), plan.scans[0].sos.end());
-        hdr_stride = (head.size() + (size_t)n_tables * 2 * (21 + 256) + tail.size() + 15) & ~(size_t)15;
-        const size_t blob = head.size() + tail.size();
-        CK(enc->h_tables.reserve(blob + 16), "alloc header parts (host)");
-        CK(enc->hdr_parts.reserve(blob + 16), "alloc header parts");
-        std::vector<uint8_t> fresh(head);
-        fresh.insert(fresh.end(), tail.begin(), tail.end());
+        fresh.assign(with.begin(), with.begin() + dht_at);
+        fresh.insert(fresh.end(), with.begin() + dht_at + (size_t)hl.n_tables * 2 * 21, with.end());
+        fresh.insert(fresh.end(), plan.scans[0].sos.begin(), plan.scans[0].sos.end());
+        hl.head_len = (uint32_t)dht_at;
+        hl.tail_len = (uint32_t)(fresh.size() - dht_at);
+        hl.hdr_stride = (fresh.size() + (size_t)hl.n_tables * 2 * (21 + 256) + 15) & ~(size_t)15;
+        CK(enc->h_tables.reserve(fresh.size() + 16), "alloc header parts (host)");
+        CK(enc->hdr_parts.reserve(fresh.size() + 16), "alloc header parts");
         fresh.push_back(0xA5); // never equal to the blob of the default-table path
-        if (enc->last_tables != fresh) {
-            CK(cudaStreamSynchronize(enc->stream), "staging reuse sync");
-            enc->last_tables = fresh;
-            std::memcpy(enc->h_tables.p, fresh.data(), blob);
-            CK(cudaMemcpyAsync(enc->hdr_parts.p, enc->h_tables.p, blob, cudaMemcpyHostToDevice, st), "upload header parts");
-        }
         const size_t hist_words = (size_t)n * 2 * 2 * 257;
         CK(enc->hist.reserve(hist_words * 4), "alloc histogram");
         if (given_hist) { // strips: the whole image's histogram comes from the caller (n == 1)
             CK(enc->h_hist.reserve(hist_words * 4), "alloc histogram (host)");
-            CK(cudaStreamSynchronize(enc->stream), "staging reuse sync");
+            CK(cudaStreamSynchronize(st), "staging reuse sync");
             std::memcpy(enc->h_hist.p, given_hist, hist_words * 4);
             CK(cudaMemcpyAsync(enc->hist.p, enc->h_hist.p, hist_words * 4, cudaMemcpyHostToDevice, st), "upload histogram");
         }
-        CK(enc->hdr.reserve((size_t)n * hdr_stride), "alloc headers");
-        opt_head_len = (uint32_t)head.size();
-        opt_tail_len = (uint32_t)tail.size();
-        opt_tables = n_tables;
     }
-    // histogram + Annex K.2 on the device (part of the replayable launch sequence below)
-    auto enqueue_tables = [&]() -> int {
+    CK(enc->hdr.reserve((size_t)n_huff * hl.hdr_stride), "alloc headers");
+    if (enc->last_tables != fresh) { // repeated calls with the same settings skip the upload (the device copy is still valid)
+        CK(cudaStreamSynchronize(st), "staging reuse sync"); // an earlier upload may still read h_tables
+        enc->last_tables = fresh;
+        const uint8_t *hb = enc->h_tables.as<uint8_t>();
+        std::memcpy(enc->h_tables.p, fresh.data(), fresh.size());
+        if (!optimized) {
+            CK(cudaMemcpyAsync(enc->huff.p, hb, tab_bytes, cudaMemcpyHostToDevice, st), "upload huffman tables");
+            CK(cudaMemcpyAsync(enc->hdr.p, hb + tab_bytes, hl.hdr_stride, cudaMemcpyHostToDevice, st), "upload headers");
+            CK(cudaMemcpyAsync(enc->hdr_len.p, hb + tab_bytes + hl.hdr_stride, 4, cudaMemcpyHostToDevice, st), "upload header lengths");
+        } else {
+            CK(cudaMemcpyAsync(enc->hdr_parts.p, hb, hl.head_len + hl.tail_len, cudaMemcpyHostToDevice, st), "upload header parts");
+        }
+    }
+    return JPGB_OK;
+}
+
+// ---- Capacities. No host round trip inside the pipeline: the pool, the unstuffed stream and the output are sized
+// from what this context has seen before; the kernels read the real sizes on the device and raise a flag instead of
+// overrunning, and the part of the pipeline that did not fit is repeated with room to spare.
+
+// Attempt 0: what the last call with the same settings and batch size settled on, else the bytes per raw byte learnt
+// from earlier calls (first call: a third of the raw size)
+Caps first_caps(const jpgb_encoder *enc, const CapKey &ck, uint64_t n_chunks) {
+    const uint64_t raw_bytes = ck.raw_bytes;
+    Caps c;
+    c.ustream = (enc->ucap_ratio > 0 ? (uint64_t)(raw_bytes * enc->ucap_ratio) : raw_bytes / 3) + (uint64_t)ck.n * 4096 + 65536;
+    c.out = c.ustream + c.ustream / 32 + 4096;
+    // every chunk is rounded up to 16 bytes in the pool
+    c.pool_units = (enc->pool_ratio > 0 ? (uint64_t)(raw_bytes * enc->pool_ratio) : raw_bytes / 3) / 16 + n_chunks + 4096;
+    if (enc->have_caps && std::memcmp(&enc->cap_key, &ck, sizeof(ck)) == 0) c = enc->caps;
+    // test hook (JPGB_TIGHT_CAPS, a comma list of pool, stream, out): attempt 0 starts from the floor of each named
+    // capacity, so the retry branch that capacity leads to (recode, tail with a larger stream, tail with a larger output)
+    // runs on purpose
+    if (const char *tight = std::getenv("JPGB_TIGHT_CAPS")) {
+        const std::string t = std::string(",") + tight + ",";
+        if (t.find(",pool,") != std::string::npos) c.pool_units = 1;
+        if (t.find(",stream,") != std::string::npos) c.ustream = kStuffChunk;
+        if (t.find(",out,") != std::string::npos) c.out = 4096;
+    }
+    return c;
+}
+
+// After an overflow, from the read-back entropy status of the attempt: room to spare for what did not fit.
+// What survives a tail-only attempt is the device buffers the coder wrote (pool, chunk and segment positions), not
+// the status block: it grows with the raw mask, so a larger stream reallocates it. Hence the pool cursor `pool_used`
+// is read only from an attempt that ran the coder, and the table flag only from the attempt that built the tables.
+void grow_caps(Caps &c, const unsigned long long *status, uint64_t pool_used) {
+    const uint64_t ubytes = status[kStatUnstuffed];
+    // the pool: code again (the cursor counted every request, so the exact need is known)
+    if (status[kStatFlags] & kFlagPool) c.pool_units = pool_used + pool_used / 64 + 4096;
+    if (status[kStatFlags] & kFlagStream) {
+        c.ustream = ubytes + ubytes / 16 + 65536;
+        c.out = c.ustream + c.ustream / 8 + 4096; // the 0xFF count is not known yet: generous
+    } else if (status[kStatFlags] & kFlagOut) {
+        c.out = ubytes + status[kStatDataFF] + 4096;
+    }
+}
+
+// Next call with these settings: what this one needed plus 15 %, unless the present capacities are already within
+// 5 .. 40 % of the need (then they stay, and with them the captured graph)
+void settle_caps(jpgb_encoder *enc, const CapKey &ck, const Caps &c, uint64_t ubytes, uint64_t total, uint64_t pool_used, uint64_t n_chunks) {
+    auto settle = [](uint64_t cap, uint64_t need, uint64_t slack) {
+        const uint64_t lo = need + need / 20 + slack / 2, hi = need + need * 2 / 5 + 2 * slack;
+        return (cap >= lo && cap <= hi) ? cap : need + need * 3 / 20 + slack;
+    };
+    enc->cap_key = ck;
+    enc->caps.ustream = settle(c.ustream, ubytes, (uint64_t)ck.n * 4096 + 65536);
+    enc->caps.out = std::max(settle(c.out, total, 4096), enc->caps.ustream + enc->caps.ustream / 64);
+    enc->caps.pool_units = settle(c.pool_units, pool_used, 4096);
+    enc->have_caps = true;
+    const double raw = (double)std::max<uint64_t>(ck.raw_bytes, 1);
+    enc->pool_ratio = std::max(enc->pool_ratio * 0.98, 1.1 * (double)((pool_used > n_chunks ? pool_used - n_chunks : 0) * 16) / raw);
+    enc->ucap_ratio = std::max(enc->ucap_ratio * 0.98, 1.15 * (double)ubytes / raw);
+}
+
+// What one attempt's launch sequence runs: the optimized tables (first attempt only; with given_hist from the caller's
+// histogram), the coder (else only the tail is repeated), the JPGB_POISON_STREAM hook, the read-back of strip pieces
+struct SequenceFlags { bool tables, given_hist, coder, poison, pieces; };
+
+// Everything behind stage A, for one attempt: tables, coding and positions, placement, stuffing, and the copy of the
+// file offsets and status words to enc->h_small. Every launch counts itself in enc->launches.
+int enqueue_sequence(jpgb_encoder *enc, const Plan &plan, const DevPlan &hp, const EntropyBuffers &b, uint32_t n, const CoderLaunch &coder,
+                     const HeaderLayout &hl, const SequenceFlags &f) {
+    cudaStream_t st = enc->stream;
+    const uint64_t n_chunks = (uint64_t)plan.chunks_per_image * n, n_segs = b.n_segs_total, n_pieces = b.ustream_cap / kStuffChunk;
+    const StatusBlock sb = status_block(n, b.ustream_cap);
+    unsigned long long *scan_err = b.status + kStatScanError;
+    // status words of the coder and of the table build (only the words the tail writes when only the tail is repeated)
+    if (f.coder) {
+        CK(cudaMemsetAsync(b.status, 0, 2 * kStatusWords * 8 + sb.mask_bytes, st), "clear status and raw mask");
+    } else { // the pool cursor and the table status are not read again (grow_caps)
+        CK(cudaMemsetAsync(b.status, 0, (kStatScanError + 1) * 8, st), "clear status");
+        CK(cudaMemsetAsync(b.raw_mask, 0, sb.mask_bytes, st), "clear raw mask");
+    }
+    if (f.tables) { // histogram + Annex K.2 on the device
         StageTimer t(enc, 1);
-        if (!given_hist) {
+        if (!f.given_hist) {
             CK(cudaMemsetAsync(enc->hist.p, 0, (size_t)n * 2 * 2 * 257 * 4, st), "clear histogram");
-            CK(launch_histogram(hp, enc->coef.as<int16_t>(), n, enc->hist.as<uint32_t>(), st), "histogram launch");
+            CK(launch_histogram(hp, b.coef, n, enc->hist.as<uint32_t>(), st), "histogram launch");
             enc->launches += 1;
         }
-        CK(launch_build_tables(enc->hist.as<uint32_t>(), 1, opt_tables, n, enc->huff.as<uint32_t>(), enc->hdr_parts.as<uint8_t>(), opt_head_len,
-                               enc->hdr_parts.as<uint8_t>() + opt_head_len, opt_tail_len, enc->hdr.as<uint8_t>(), (uint32_t)hdr_stride,
-                               enc->hdr_len.as<uint32_t>(), aux_status, st),
+        CK(launch_build_tables(enc->hist.as<uint32_t>(), 1, hl.n_tables, n, enc->huff.as<uint32_t>(), enc->hdr_parts.as<uint8_t>(), hl.head_len,
+                               enc->hdr_parts.as<uint8_t>() + hl.head_len, hl.tail_len, enc->hdr.as<uint8_t>(), (uint32_t)hl.hdr_stride,
+                               enc->hdr_len.as<uint32_t>(), sb.table_status(b.file_off), st),
            "table build launch");
         enc->launches += 1;
-        return JPGB_OK;
-    };
+    }
+    if (f.coder) {
+        StageTimer t(enc, 2);
+        CK(launch_encode_chunks(b, hp, n, coder, st), "coding launch");
+        enc->launches += 1;
+        const bool few_chunks = n_chunks <= 4096, few_segs = n_segs <= 4096;
+        if (!few_chunks) CK(launch_exclusive_scan(b.chunk_bits, b.chunk_bitpos, n_chunks, b.scan_tmp, st, &enc->launches, scan_err), "chunk position scan");
+        if (few_segs) { // chunk positions (when few), segment lengths and positions in one single-CTA launch
+            CK(launch_positions(b, hp, n, few_chunks, st), "positions launch");
+            enc->launches += 1;
+        } else {
+            if (few_chunks) CK(launch_exclusive_scan(b.chunk_bits, b.chunk_bitpos, n_chunks, b.scan_tmp, st, &enc->launches, scan_err), "chunk position scan");
+            CK(launch_segment_lengths(b, hp, n, st), "segment length launch");
+            CK(launch_exclusive_scan(b.seglen, b.segpos, n_segs, b.scan_tmp, st, &enc->launches, scan_err), "segment position scan");
+            enc->launches += 1;
+        }
+    }
+    {
+        StageTimer t(enc, 3);
+        // test hook: the stream starts out as all ones, so a byte that the kernels neither store nor zero shows in the output
+        if (f.poison) CK(cudaMemsetAsync(b.ustream, 0xFF, b.ustream_cap + 64, st), "poison stream");
+        CK(launch_segment_leads(b, hp, n, st), "segment lead launch");
+        CK(launch_place_chunks(b, hp, n, st), "placement launch");
+        enc->launches += 2;
+    }
+    {
+        StageTimer t(enc, 4);
+        CK(launch_count_ff(b, st), "count ff launch");
+        if (ff_scan_needed(b)) CK(launch_exclusive_scan(b.ffcount, b.ffpos, n_pieces, b.scan_tmp, st, &enc->launches, scan_err), "ff scan");
+        // ... and the file offsets (for a strip also where each scan's bytes start) by extra CTAs of the same launch
+        CK(launch_stuff_scatter(b, hp, n, f.pieces ? enc->piece_off.as<unsigned long long>() : nullptr, st), "scatter launch");
+        enc->launches += 2;
+        if (f.pieces)
+            CK(cudaMemcpyAsync(enc->h_pieces.p, enc->piece_off.p, (plan.scans.size() + 1) * 8, cudaMemcpyDeviceToHost, st), "read piece offsets");
+        CK(cudaMemcpyAsync(enc->h_small.p, b.file_off, sb.readback_bytes(), cudaMemcpyDeviceToHost, st), "read file offsets and status");
+    }
+    return JPGB_OK;
+}
 
-    // ---- entropy coding: chunks -> pool, two small prefix sums, placement, stuffing. No host round trip: the pool,
-    // the unstuffed stream and the output are sized from what this context has seen before (first call: a fraction
-    // of the raw pixels); the kernels read the real sizes on the device and raise a flag instead of overrunning, in
-    // which case the affected part of the pipeline is repeated once with exact sizes.
+// Every value enqueue_sequence bakes into the launches, with the plan through its signature
+GraphKey graph_key(const jpgb_encoder *enc, const PlanSig &sig, const EntropyBuffers &b, uint32_t n, const CoderLaunch &coder,
+                   const HeaderLayout &hl, const SequenceFlags &f) {
+    static_assert(sizeof(EntropyBuffers) == 26 * 8, "every field of EntropyBuffers takes part in the graph key");
+    GraphKey k{{}, {
+        (uint64_t)b.coef, (uint64_t)b.huff, (uint64_t)b.huff_per_image, (uint64_t)b.scratch, (uint64_t)b.pool, b.pool_cap,
+        (uint64_t)b.chunk_bits, (uint64_t)b.chunk_pool, (uint64_t)b.chunk_bitpos, (uint64_t)b.seglen, (uint64_t)b.segpos,
+        (uint64_t)b.hdr_len, (uint64_t)b.hdr, b.hdr_stride, (uint64_t)b.ustream, (uint64_t)b.raw_mask, (uint64_t)b.ffcount,
+        (uint64_t)b.ffpos, (uint64_t)b.out, (uint64_t)b.file_off, (uint64_t)b.scan_tmp, b.ustream_cap, b.out_cap, b.n_segs_total,
+        (uint64_t)b.status, b.scan_tmp_bytes,
+        coder.grid, coder.smem, coder.scratch_bytes, n,
+        (uint64_t)f.tables | (uint64_t)f.given_hist << 1 | (uint64_t)f.coder << 2 | (uint64_t)f.poison << 3 | (uint64_t)f.pieces << 4,
+        hl.head_len, hl.tail_len, (uint64_t)hl.n_tables,
+        (uint64_t)enc->hist.p, (uint64_t)enc->hdr_parts.p, (uint64_t)enc->piece_off.p, (uint64_t)enc->h_small.p, (uint64_t)enc->h_pieces.p}};
+    std::memcpy(&k.sig, &sig, sizeof(sig));
+    return k;
+}
+
+// The whole device pipeline for `n` device-resident images. On success the files lie back to back
+// in `out` and `offsets` (host, n + 1) delimits them.
+// `given_hist` (strips with optimized tables): the symbol histogram of the *whole* image, [table][dc|ac][257],
+// used instead of the one of these pixels.
+int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, size_t image_stride, uint32_t n, DevBuf &out,
+                  std::vector<uint64_t> &offsets, std::vector<uint64_t> *piece_offsets = nullptr, const uint32_t *given_hist = nullptr,
+                  bool coef_ready = false) {
+    cudaStream_t st = enc->stream;
+    DevPlan hp;
+    plan.fill_device_plan(hp);
+
+    const uint64_t n_segs = (uint64_t)plan.segs_per_image * n;
     const uint64_t n_chunks = (uint64_t)plan.chunks_per_image * n;
+
+    CK(enc->coef.reserve(plan.blocks_per_image * n * 128), "alloc coefficients");
+    // ---- stage A (unless the caller has already run it slice by slice behind the upload) ----
+    if (!coef_ready) {
+        enc->coef_tagged = false;
+        StageAParams ap;
+        plan.fill_stage_a(ap);
+        ap.pixels = d_pixels;
+        ap.coef = enc->coef.as<int16_t>();
+        ap.image_stride = image_stride;
+        StageTimer t(enc, 0);
+        CK(launch_stage_a(ap, n, st), "stage A launch");
+        enc->launches += 1;
+    }
+
+    HeaderLayout hl;
+    int rc = setup_header(enc, plan, n, given_hist, hl);
+    if (rc != JPGB_OK) return rc;
+
+    // ---- entropy coding: chunks -> pool, two small prefix sums, placement, stuffing ----
     CK(enc->chunk_bits.reserve(n_chunks * 4), "alloc chunk sizes");
     CK(enc->chunk_pool.reserve(n_chunks * 4), "alloc chunk places");
     CK(enc->chunk_bitpos.reserve((n_chunks + 1) * 8), "alloc chunk positions");
@@ -382,11 +535,16 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, 
     CoderLaunch coder{};
     CK(coder_launch_config(hp, n, coder), "coder configuration");
     CK(enc->scratch.reserve(coder.scratch_bytes), "alloc coder scratch");
+    CK(enc->h_small.reserve(status_block(n, 0).readback_bytes()), "alloc readback");
+    if (piece_offsets) {
+        CK(enc->piece_off.reserve((plan.scans.size() + 1) * 8), "alloc piece offsets");
+        CK(enc->h_pieces.reserve((plan.scans.size() + 1) * 8), "alloc piece offsets (host)");
+    }
 
     EntropyBuffers b{};
     b.coef = enc->coef.as<int16_t>();
     b.huff = enc->huff.as<uint32_t>();
-    b.huff_per_image = optimized ? 1 : 0;
+    b.huff_per_image = plan.p.optimize_huffman != 0 ? 1 : 0;
     b.scratch = enc->scratch.as<uint32_t>();
     b.chunk_bits = enc->chunk_bits.as<uint32_t>();
     b.chunk_pool = enc->chunk_pool.as<uint32_t>();
@@ -395,231 +553,76 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, 
     b.segpos = enc->segpos.as<unsigned long long>();
     b.hdr_len = enc->hdr_len.as<uint32_t>();
     b.hdr = enc->hdr.as<uint8_t>();
-    b.hdr_stride = (uint32_t)hdr_stride;
-
-
-    const uint64_t raw_bytes = (uint64_t)plan.p.width * plan.p.height * plan.bpp * n;
-    // learnt bytes per raw byte from earlier calls on this context, else a third of the raw size
-    uint64_t ucap = enc->ucap_ratio > 0 ? (uint64_t)(raw_bytes * enc->ucap_ratio) + (uint64_t)n * 4096 + 65536
-                                        : raw_bytes / 3 + (uint64_t)n * 4096 + 65536;
-    uint64_t ocap = ucap + ucap / 32 + 4096;
-    // every chunk is rounded up to 16 bytes in the pool
-    uint64_t pool_units = (enc->pool_ratio > 0 ? (uint64_t)(raw_bytes * enc->pool_ratio) : raw_bytes / 3) / 16 + n_chunks + 4096;
-    uint64_t ubytes = 0, total = 0, pool_used = 0;
-    CK(enc->h_small.reserve((size_t)(2 * kStatusWords + n + 1) * 8), "alloc readback");
+    b.hdr_stride = (uint32_t)hl.hdr_stride;
     b.n_segs_total = n_segs;
-    // Capacities are sticky per (settings, batch size): steady-state calls provision exactly what the last successful
-    // call used, so the launch sequence below has identical parameters call after call and is replayed as a CUDA graph.
+
     CapKey ck;
     std::memset(&ck, 0, sizeof(ck));
     ck.sig = plan_sig(plan);
-    ck.raw_bytes = raw_bytes;
+    ck.raw_bytes = (uint64_t)plan.p.width * plan.p.height * plan.bpp * n;
     ck.n = n;
-    if (enc->have_caps && std::memcmp(&enc->cap_key, &ck, sizeof(ck)) == 0) {
-        ucap = enc->caps[0];
-        ocap = enc->caps[1];
-        pool_units = enc->caps[2];
-    }
-    // test hook (JPGB_TIGHT_CAPS, a comma list of pool, stream, out): attempt 0 starts from the floor of each named
-    // capacity, so the retry branch that capacity leads to (recode, tail with a larger stream, tail with a larger output)
-    // runs on purpose
-    if (const char *tight = std::getenv("JPGB_TIGHT_CAPS")) {
-        const std::string t = std::string(",") + tight + ",";
-        if (t.find(",pool,") != std::string::npos) pool_units = 1;
-        if (t.find(",stream,") != std::string::npos) ucap = kStuffChunk;
-        if (t.find(",out,") != std::string::npos) ocap = 4096;
-    }
-    bool coded = false;
+    Caps caps = first_caps(enc, ck, n_chunks);
     const char *poison_env = std::getenv("JPGB_POISON_STREAM");
-    const bool poison = poison_env && poison_env[0] == '1';
+    uint64_t ubytes = 0, total = 0, pool_used = 0;
+    bool coded = false;
     for (int attempt = 0;; ++attempt) {
-        ucap = (ucap + kStuffChunk - 1) / kStuffChunk * kStuffChunk;
-        const uint64_t n_pieces = ucap / kStuffChunk;
-        CK(enc->ustream.reserve(ucap + 64), "alloc unstuffed stream");
-        const size_t mask_bytes = (size_t)(ucap / 32 + 2) * 4;
-        CK(enc->status.reserve((size_t)(n + 1 + 2 * kStatusWords) * 8 + mask_bytes), "alloc status and raw mask");
+        caps.ustream = (caps.ustream + kStuffChunk - 1) / kStuffChunk * kStuffChunk;
+        const uint64_t n_pieces = caps.ustream / kStuffChunk;
+        const StatusBlock sb = status_block(n, caps.ustream);
+        CK(enc->ustream.reserve(caps.ustream + 64), "alloc unstuffed stream");
+        CK(enc->status.reserve(sb.bytes()), "alloc status and raw mask");
         CK(enc->ffcount.reserve((n_pieces + 1) * 4), "alloc ff counts");
         CK(enc->ffpos.reserve((n_pieces + 2) * 8), "alloc ff positions");
         CK(enc->scan_tmp.reserve(scan_tmp_bytes(std::max<uint64_t>(n_pieces, std::max(n_chunks, n_segs)))), "alloc scan scratch");
-        CK(enc->pool.reserve(pool_units * 16), "alloc chunk pool");
-        DevBuf &outb = enc->out_slot ? enc->out2 : enc->out;
-        CK(outb.reserve(ocap + 64), "alloc output");
-        if (piece_offsets) {
-            CK(enc->piece_off.reserve((plan.scans.size() + 1) * 8), "alloc piece offsets");
-            CK(enc->h_pieces.reserve((plan.scans.size() + 1) * 8), "alloc piece offsets (host)");
-        }
+        CK(enc->pool.reserve(caps.pool_units * 16), "alloc chunk pool");
+        CK(out.reserve(caps.out + 64), "alloc output");
         b.pool = enc->pool.as<uint32_t>();
-        b.pool_cap = pool_units;
+        b.pool_cap = caps.pool_units;
         b.ustream = enc->ustream.as<uint8_t>();
-        b.file_off = enc->status.as<unsigned long long>();
-        b.status = b.file_off + (n + 1);
-        aux_status = b.status + kStatusWords;
-        scan_err = b.status + 3;
-        b.raw_mask = reinterpret_cast<uint32_t *>(b.status + 2 * kStatusWords);
+        b.file_off = sb.file_off(enc->status.p);
+        b.status = sb.status(enc->status.p);
+        b.raw_mask = sb.raw_mask(enc->status.p);
         b.ffcount = enc->ffcount.as<uint32_t>();
         b.ffpos = enc->ffpos.as<unsigned long long>();
         b.scan_tmp = enc->scan_tmp.p;
-        b.out = outb.as<uint8_t>();
-        b.ustream_cap = ucap;
-        b.out_cap = ocap;
-        const bool with_tables = optimized && attempt == 0, with_coder = !coded;
-        auto enqueue = [&]() -> int {
-            // status words of the coder and of the table build (only the words the tail writes when only the tail is repeated)
-            if (with_coder) {
-                CK(cudaMemsetAsync(b.status, 0, 2 * kStatusWords * 8 + mask_bytes, st), "clear status and raw mask");
-            } else { // the pool cursor and the table status are not read again (see below)
-                CK(cudaMemsetAsync(b.status, 0, 4 * 8, st), "clear status");
-                CK(cudaMemsetAsync(b.raw_mask, 0, mask_bytes, st), "clear raw mask");
-            }
-            if (with_tables) {
-                const int rc = enqueue_tables();
-                if (rc != JPGB_OK) return rc;
-            }
-            if (with_coder) {
-                StageTimer t(enc, 2);
-                CK(launch_encode_chunks(b, hp, n, coder, st), "coding launch");
-                enc->launches += 1;
-                const bool few_chunks = n_chunks <= 4096, few_segs = n_segs <= 4096;
-                if (!few_chunks) CK(launch_exclusive_scan(b.chunk_bits, b.chunk_bitpos, n_chunks, b.scan_tmp, st, &enc->launches, scan_err), "chunk position scan");
-                if (few_segs) { // chunk positions (when few), segment lengths and positions in one single-CTA launch
-                    CK(launch_positions(b, hp, n, few_chunks, st), "positions launch");
-                    enc->launches += 1;
-                } else {
-                    if (few_chunks) CK(launch_exclusive_scan(b.chunk_bits, b.chunk_bitpos, n_chunks, b.scan_tmp, st, &enc->launches, scan_err), "chunk position scan");
-                    CK(launch_segment_lengths(b, hp, n, st), "segment length launch");
-                    CK(launch_exclusive_scan(b.seglen, b.segpos, n_segs, b.scan_tmp, st, &enc->launches, scan_err), "segment position scan");
-                    enc->launches += 1;
-                }
-            }
-            {
-                StageTimer t(enc, 3);
-                // test hook: the stream starts out as all ones, so a byte that the kernels neither store nor zero shows in the output
-                if (poison) CK(cudaMemsetAsync(b.ustream, 0xFF, ucap + 64, st), "poison stream");
-                CK(launch_segment_leads(b, hp, n, st), "segment lead launch");
-                CK(launch_place_chunks(b, hp, n, st), "placement launch");
-                enc->launches += 2;
-            }
-            {
-                StageTimer t(enc, 4);
-                CK(launch_count_ff(b, st), "count ff launch");
-                if (ff_scan_needed(b)) CK(launch_exclusive_scan(b.ffcount, b.ffpos, n_pieces, b.scan_tmp, st, &enc->launches, scan_err), "ff scan");
-                // ... and the file offsets (for a strip also where each scan's bytes start) by extra CTAs of the same launch
-                CK(launch_stuff_scatter(b, hp, n, piece_offsets ? enc->piece_off.as<unsigned long long>() : nullptr, st), "scatter launch");
-                enc->launches += 2;
-                if (piece_offsets)
-                    CK(cudaMemcpyAsync(enc->h_pieces.p, enc->piece_off.p, (plan.scans.size() + 1) * 8, cudaMemcpyDeviceToHost, st), "read piece offsets");
-                CK(cudaMemcpyAsync(enc->h_small.p, b.file_off, (size_t)(n + 1 + 2 * kStatusWords) * 8, cudaMemcpyDeviceToHost, st), "read file offsets and status");
-            }
-            return JPGB_OK;
-        };
+        b.out = out.as<uint8_t>();
+        b.ustream_cap = caps.ustream;
+        b.out_cap = caps.out;
+        const SequenceFlags f{plan.p.optimize_huffman != 0 && attempt == 0, given_hist != nullptr, !coded, poison_env && poison_env[0] == '1',
+                              piece_offsets != nullptr};
+        auto enqueue = [&] { return enqueue_sequence(enc, plan, hp, b, n, coder, hl, f); };
         // Everything behind stage A is one fixed launch sequence per (settings, batch size, buffers): captured once,
         // replayed afterwards (a dozen launches cost ~10 us each from the host; a 1080p frame needs 70 us of kernels).
         bool replayed = false;
-        if (attempt == 0 && enc->graphs_ok && !enc->timing) {
-            GraphKey gk;
-            std::memset(&gk, 0, sizeof(gk));
-            gk.b = b;
-            gk.sig = ck.sig;
-            gk.n = n;
-            gk.coder = coder;
-            gk.flags = (optimized ? 1u : 0u) | (piece_offsets ? 2u : 0u) | (given_hist ? 4u : 0u) | (poison ? 8u : 0u) | (uint32_t)hdr_stride << 8;
-            gk.misc[0] = (uint64_t)enc->hist.p;
-            gk.misc[1] = (uint64_t)enc->huff.p;
-            gk.misc[2] = (uint64_t)enc->hdr_parts.p;
-            gk.misc[3] = (uint64_t)enc->piece_off.p;
-            gk.misc[4] = (uint64_t)enc->h_small.p;
-            gk.misc[5] = (uint64_t)enc->h_pieces.p;
-            gk.misc[6] = ((uint64_t)opt_head_len << 32) | opt_tail_len;
-            gk.misc[7] = (uint64_t)enc->coef.p;
-            jpgb_encoder::CachedGraph *slot = nullptr, *victim = &enc->graphs[0];
-            for (auto &g : enc->graphs) {
-                if (g.exec && std::memcmp(&gk, &g.key, sizeof(gk)) == 0) slot = &g;
-                if (!g.exec || (victim->exec && g.used < victim->used)) victim = &g;
-            }
-            if (!slot) {
-                if (victim->exec) cudaGraphExecDestroy(victim->exec), victim->exec = nullptr;
-                const uint32_t launches_before = enc->launches;
-                if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-                    const int rc = enqueue();
-                    cudaGraph_t graph = nullptr;
-                    const cudaError_t ce = cudaStreamEndCapture(st, &graph);
-                    if (rc == JPGB_OK && ce == cudaSuccess && graph && cudaGraphInstantiate(&victim->exec, graph, 0) == cudaSuccess) {
-                        victim->key = gk;
-                        victim->launches = enc->launches - launches_before;
-                        slot = victim;
-                    } else {
-                        victim->exec = nullptr;
-                        enc->graphs_ok = false; // e.g. the legacy default stream cannot be captured: launch directly from now on
-                    }
-                    if (graph) cudaGraphDestroy(graph);
-                    enc->launches = launches_before;
-                    cudaGetLastError();
-                } else {
-                    enc->graphs_ok = false;
-                    cudaGetLastError();
-                }
-            }
-            if (slot) {
-                slot->used = ++enc->graph_clock;
-                CK(cudaGraphLaunch(slot->exec, st), "graph launch");
-                enc->launches += slot->launches;
-                replayed = true;
-            }
-        }
+        if (attempt == 0 && enc->graphs.ok && !enc->timing)
+            CK(enc->graphs.replay(graph_key(enc, ck.sig, b, n, coder, hl, f), st, enc->launches, enqueue, replayed), "graph launch");
         if (!replayed) {
-            const int rc = enqueue();
+            rc = enqueue();
             if (rc != JPGB_OK) return rc;
         }
         CK(cudaStreamSynchronize(st), "final sync");
-        const uint64_t *status = enc->h_small.as<uint64_t>() + (n + 1);
-        if (status[3]) return fail(enc, JPGB_ERR_CUDA, "internal: prefix-sum look-back timed out");
-        if (status[2] & 8) return fail(enc, JPGB_ERR_BAD_PARAMS, "a scan segment exceeds 4 GiB (use a restart interval)");
-        // What survives a tail-only attempt is the device buffers the coder wrote (pool, chunk and segment positions), not
-        // the status block: it grows with the raw mask, so a larger stream reallocates it. The table flag is read on the
-        // attempt that built the tables, the pool cursor on an attempt that ran the coder.
-        if (with_tables && (status[kStatusWords + 2] & 16)) return fail(enc, JPGB_ERR_HUFFMAN, "an optimized Huffman code does not fit (longer than 32 bits, or code plus value bits beyond 31)");
-        ubytes = status[0];
-        if (with_coder) pool_used = status[5];
-        if (status[2] == 0) {
-            total = ubytes + status[1];
+        const unsigned long long *status = sb.status(enc->h_small.p);
+        if (status[kStatScanError]) return fail(enc, JPGB_ERR_CUDA, "internal: prefix-sum look-back timed out");
+        if (status[kStatFlags] & kFlagSegment4G) return fail(enc, JPGB_ERR_BAD_PARAMS, "a scan segment exceeds 4 GiB (use a restart interval)");
+        if (f.tables && (sb.table_status(enc->h_small.p)[kStatFlags] & kFlagHuffmanLong))
+            return fail(enc, JPGB_ERR_HUFFMAN, "an optimized Huffman code does not fit (longer than 32 bits, or code plus value bits beyond 31)");
+        ubytes = status[kStatUnstuffed];
+        if (f.coder) pool_used = status[kStatPoolCursor];
+        if (status[kStatFlags] == 0) {
+            total = ubytes + status[kStatDataFF];
             break;
         }
         if (attempt >= 3) return fail(enc, JPGB_ERR_CUDA, "internal: buffer capacity retry did not converge");
-        // overflow: the sizing results are still on the device; redo what did not fit with room to spare
-        if (status[2] & 4) { // the pool: code again (the cursor counted every request, so the exact need is known)
-            pool_units = pool_used + pool_used / 64 + 4096;
-            coded = false;
-        } else {
-            coded = true;
-        }
-        if (status[2] & 1) {
-            ucap = ubytes + ubytes / 16 + 65536;
-            ocap = ucap + ucap / 8 + 4096; // the 0xFF count is not known yet: generous
-        } else if (status[2] & 2) {
-            ocap = ubytes + status[1] + 4096;
-        }
+        // overflow: the sizing results are still on the device; a pool overflow codes again, the rest repeats the tail
+        coded = !(status[kStatFlags] & kFlagPool);
+        grow_caps(caps, status, pool_used);
     }
-    // next call with these settings: what this one needed plus 15 %, unless the present capacities are already within
-    // 5 .. 40 % of the need (then they stay, and with them the captured graph)
-    auto settle = [](uint64_t cap, uint64_t need, uint64_t slack) {
-        const uint64_t lo = need + need / 20 + slack / 2, hi = need + need * 2 / 5 + 2 * slack;
-        return (cap >= lo && cap <= hi) ? cap : need + need * 3 / 20 + slack;
-    };
-    enc->cap_key = ck;
-    enc->caps[0] = settle(ucap, ubytes, (uint64_t)n * 4096 + 65536);
-    enc->caps[1] = settle(ocap, total, 4096);
-    enc->caps[1] = std::max(enc->caps[1], enc->caps[0] + enc->caps[0] / 64);
-    enc->caps[2] = settle(pool_units, pool_used, 4096);
-    enc->have_caps = true;
-    enc->pool_ratio = std::max(enc->pool_ratio * 0.98, 1.1 * (double)((pool_used > n_chunks ? pool_used - n_chunks : 0) * 16) / (double)std::max<uint64_t>(raw_bytes, 1));
-    enc->ucap_ratio = std::max(enc->ucap_ratio * 0.98, 1.15 * (double)ubytes / (double)std::max<uint64_t>(raw_bytes, 1));
-    CK(cudaStreamSynchronize(st), "final sync");
+    settle_caps(enc, ck, caps, ubytes, total, pool_used, n_chunks);
     if (piece_offsets) {
         piece_offsets->assign(enc->h_pieces.as<uint64_t>(), enc->h_pieces.as<uint64_t>() + plan.scans.size() + 1);
         enc->last_piece_scans = (uint32_t)plan.scans.size();
     }
     offsets.assign(enc->h_small.as<uint64_t>(), enc->h_small.as<uint64_t>() + n + 1);
-    enc->out_total = total;
     if (offsets[n] != total) return fail(enc, JPGB_ERR_CUDA, "internal: file offsets disagree with stream size");
     return JPGB_OK;
 }
@@ -717,7 +720,7 @@ int encode_host_pipelined(jpgb_encoder *enc, const Plan &plan, const uint8_t *co
             enc->launches += 1;
         }
         std::vector<uint64_t> off;
-        const int rc = encode_device(enc, plan, enc->pixels.as<uint8_t>(), stride, 1, off, nullptr, nullptr, true);
+        const int rc = encode_device(enc, plan, enc->pixels.as<uint8_t>(), stride, 1, enc->out, off, nullptr, nullptr, true);
         if (rc != JPGB_OK) return rc;
         CK(enc->h_out.reserve(std::max<size_t>(off[1], 1 << 20)), "alloc pinned output");
         CK(cudaMemcpyAsync(enc->h_out.p, enc->out.p, off[1], cudaMemcpyDeviceToHost, st), "download file");
@@ -749,15 +752,12 @@ int encode_host_pipelined(jpgb_encoder *enc, const Plan &plan, const uint8_t *co
         const uint32_t lo = c * chunk, hi = std::min(n, lo + chunk), cn = hi - lo;
         if (c + 1 < n_chunks) CK(upload(c + 1), "upload pixels");
         DevBuf &px = (c & 1) ? enc->pixels2 : enc->pixels;
+        DevBuf &ob = (c & 1) ? enc->out2 : enc->out;
         CK(cudaStreamWaitEvent(st, enc->ev_in[c & 1], 0), "wait upload");
         if (c >= 2) CK(cudaStreamWaitEvent(st, enc->ev_out[c & 1], 0), "wait download"); // out slot reused
-        enc->out_slot = (int)(c & 1);
         std::vector<uint64_t> off;
-        const uint32_t launches_before = enc->launches;
-        const int rc = encode_device(enc, plan, px.as<uint8_t>(), stride, cn, off);
-        enc->out_slot = 0;
+        const int rc = encode_device(enc, plan, px.as<uint8_t>(), stride, cn, ob, off);
         if (rc != JPGB_OK) return rc;
-        (void)launches_before;
         CK(cudaEventRecord(enc->ev_enc[c & 1], st), "record encode");
         const uint64_t bytes = off[cn];
         if (total + bytes > enc->h_out.cap) { // grow the pinned buffer, keeping what is already there
@@ -765,10 +765,8 @@ int encode_host_pipelined(jpgb_encoder *enc, const Plan &plan, const uint8_t *co
             PinnedBuf bigger;
             CK(bigger.reserve((total + bytes) * 2), "grow pinned output");
             std::memcpy(bigger.p, enc->h_out.p, total);
-            enc->h_out.release();
-            enc->h_out = bigger;
+            std::swap(enc->h_out, bigger);
         }
-        DevBuf &ob = (c & 1) ? enc->out2 : enc->out;
         // encode_device has synchronised the context's stream: the files are complete in `ob`
         CK(cudaMemcpyAsync(enc->h_out.as<uint8_t>() + total, ob.p, bytes, cudaMemcpyDeviceToHost, enc->s_d2h), "download files");
         CK(cudaEventRecord(enc->ev_out[c & 1], enc->s_d2h), "record download");
@@ -869,16 +867,6 @@ void jpgb_encoder_destroy(jpgb_encoder *e) {
     if (!e) return;
     cudaSetDevice(e->device);
     cudaStreamSynchronize(e->stream);
-    DevBuf *bufs[] = {&e->pixels, &e->coef, &e->huff, &e->hdr, &e->hdr_len, &e->scratch, &e->pool, &e->chunk_bits, &e->chunk_pool, &e->chunk_bitpos, &e->seglen, &e->segpos,
-                      &e->ustream, &e->ffcount, &e->ffpos, &e->out, &e->scan_tmp, &e->hist, &e->piece_off, &e->out2, &e->pixels2, &e->status, &e->aux_status, &e->hdr_parts};
-    for (DevBuf *b : bufs) b->release();
-    e->h_small.release();
-    e->h_hist.release();
-    e->h_tables.release();
-    e->h_pieces.release();
-    e->h_out.release();
-    for (auto &g : e->graphs)
-        if (g.exec) cudaGraphExecDestroy(g.exec);
     if (e->s_h2d) cudaStreamDestroy(e->s_h2d);
     if (e->s_d2h) cudaStreamDestroy(e->s_d2h);
     for (cudaEvent_t ev : e->ev_slice) cudaEventDestroy(ev);
@@ -887,13 +875,12 @@ void jpgb_encoder_destroy(jpgb_encoder *e) {
         if (e->ev_out[i]) cudaEventDestroy(e->ev_out[i]);
         if (e->ev_enc[i]) cudaEventDestroy(e->ev_enc[i]);
         if (e->ev_stage[i]) cudaEventDestroy(e->ev_stage[i]);
-        e->h_stage[i].release();
     }
     for (int i = 0; i < JPGB_N_STAGES; ++i)
         for (int k = 0; k < 2; ++k)
             if (e->ev[i][k]) cudaEventDestroy(e->ev[i][k]);
     if (e->own_stream) cudaStreamDestroy(e->stream);
-    delete e;
+    delete e; // frees the buffers and graphs
 }
 
 const char *jpgb_last_error(const jpgb_encoder *e) { return e ? e->err.c_str() : "no encoder"; }
@@ -929,7 +916,7 @@ static int encode_planar_pinned(jpgb_encoder *enc, const jpgb_params *p, const u
         CK(upload_host(enc, enc->pixels.as<uint8_t>() + plane_bytes * c, planes[c], plane_bytes, enc->stream), "upload plane");
     }
     std::vector<uint64_t> off;
-    const int rc2 = encode_device(enc, plan, enc->pixels.as<uint8_t>(), stride, 1, off);
+    const int rc2 = encode_device(enc, plan, enc->pixels.as<uint8_t>(), stride, 1, enc->out, off);
     if (rc2 != JPGB_OK) return rc2;
     const size_t sz = (size_t)off[1];
     CK(enc->h_out.reserve(sz ? sz : 1), "alloc pinned output");
@@ -1004,7 +991,7 @@ int jpgb_encode_batch_device(jpgb_encoder *enc, const jpgb_params *p, const void
     CK(cudaSetDevice(enc->device), "cudaSetDevice");
     timing_begin(enc);
     std::vector<uint64_t> off;
-    rc = encode_device(enc, plan, static_cast<const uint8_t *>(d_pixels), image_stride, n, off);
+    rc = encode_device(enc, plan, static_cast<const uint8_t *>(d_pixels), image_stride, n, enc->out, off);
     if (rc != JPGB_OK) return rc;
     timing_end(enc);
     std::memcpy(offsets, off.data(), (size_t)(n + 1) * 8);
@@ -1074,7 +1061,7 @@ static int encode_strip(jpgb_encoder *enc, const jpgb_params *p, const jpgb_stri
         const PlanSig sig = plan_sig(plan);
         reuse = std::memcmp(&sig, &enc->coef_sig, sizeof(sig)) == 0;
     }
-    const int rc2 = encode_device(enc, plan, static_cast<const uint8_t *>(d_pixels), stride, 1, off, &pieces, hist_total, reuse);
+    const int rc2 = encode_device(enc, plan, static_cast<const uint8_t *>(d_pixels), stride, 1, enc->out, off, &pieces, hist_total, reuse);
     enc->coef_tagged = false;
     if (rc2 != JPGB_OK) return rc2;
     timing_end(enc);
@@ -1230,10 +1217,8 @@ int jpgb_gather_place_pieces(jpgb_encoder *enc, void *d_target, size_t target_ca
     if (!enc) return JPGB_ERR_BAD_PARAMS;
     if (!d_target || !d_table || world == 0 || rank >= world || enc->last_piece_scans == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "bad gather arguments");
     CK(cudaSetDevice(enc->device), "cudaSetDevice");
-    CK(enc->aux_status.reserve(kStatusWords * 8), "alloc status");
     CK(launch_place_pieces(enc->out.as<uint8_t>(), static_cast<uint8_t *>(d_target), target_capacity, reinterpret_cast<const unsigned long long *>(d_table),
-                           world, rank, enc->last_piece_scans, reinterpret_cast<unsigned long long *>(d_total),
-                           enc->aux_status.as<unsigned long long>() + 4, enc->stream),
+                           world, rank, enc->last_piece_scans, reinterpret_cast<unsigned long long *>(d_total), enc->stream),
        "piece placement launch");
     return JPGB_OK;
 }
@@ -1333,7 +1318,6 @@ int jpgb_optimized_huffman_tables_device(jpgb_encoder *enc, const uint32_t *freq
     CK(cudaSetDevice(enc->device), "cudaSetDevice");
     cudaStream_t st = enc->stream;
     DevBuf d_hist, d_words, d_dht, d_len, d_bad;
-    auto release = [&] { d_hist.release(); d_words.release(); d_dht.release(); d_len.release(); d_bad.release(); };
     std::vector<uint8_t> dht((size_t)n * 277);
     std::vector<uint32_t> len(n), bad(n);
     cudaError_t e = d_hist.reserve((size_t)n * 257 * 4);
@@ -1348,7 +1332,6 @@ int jpgb_optimized_huffman_tables_device(jpgb_encoder *enc, const uint32_t *freq
     if (e == cudaSuccess) e = cudaMemcpyAsync(len.data(), d_len.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(bad.data(), d_bad.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    release();
     if (e != cudaSuccess) return fail_cuda(enc, e, "device table build");
     for (uint32_t i = 0; i < n; ++i) {
         status[i] = bad[i] ? JPGB_ERR_HUFFMAN : JPGB_OK;

@@ -269,8 +269,8 @@ __global__ void __launch_bounds__(T, coder_min_ctas(T, FULL)) encode_chunks_kern
     };
     unsigned long long next_ticket = 0;
     if (tid == 0) {
-        decode(atomicAdd(b.status + 4, 1ull), items[0]);
-        next_ticket = atomicAdd(b.status + 4, 1ull);
+        decode(atomicAdd(b.status + kStatTicket, 1ull), items[0]);
+        next_ticket = atomicAdd(b.status + kStatTicket, 1ull);
     }
 
     for (unsigned round = 0;; ++round) {
@@ -279,7 +279,7 @@ __global__ void __launch_bounds__(T, coder_min_ctas(T, FULL)) encode_chunks_kern
         if (it.done) break;
         if (tid == 0) {
             decode(next_ticket, items[(round & 1) ^ 1]);
-            next_ticket = atomicAdd(b.status + 4, 1ull);
+            next_ticket = atomicAdd(b.status + kStatTicket, 1ull);
         }
         if (it.n_valid == 0) { // a chunk slot past the end of a short last segment: it exists only as an (empty) descriptor
             for (int j = tid; j < P.spg; j += T) {
@@ -453,7 +453,7 @@ __global__ void __launch_bounds__(T, coder_min_ctas(T, FULL)) encode_chunks_kern
             const unsigned pool_units = (total_words + 3) >> 2; // 16-byte units
             unsigned long long pool_at = 0;
             if (tid == 0) {
-                if (pool_units) pool_at = atomicAdd(b.status + 5, (unsigned long long)pool_units);
+                if (pool_units) pool_at = atomicAdd(b.status + kStatPoolCursor, (unsigned long long)pool_units);
                 b.chunk_bits[ci] = total;
             }
             for (unsigned wb = 0; wb < total_words; wb += L::kAsmWords) { // one pass unless the chunk is larger than the buffer
@@ -492,7 +492,7 @@ __global__ void __launch_bounds__(T, coder_min_ctas(T, FULL)) encode_chunks_kern
                 }
                 if (tid == 0 && wb == 0) {
                     if (pool_at + pool_units > b.pool_cap) {
-                        atomicOr(b.status + 2, 4ull);
+                        atomicOr(b.status + kStatFlags, kFlagPool);
                         pool_at = ~0ull;
                     }
                     wsum[8] = (uint32_t)pool_at;
@@ -535,11 +535,11 @@ __global__ void __launch_bounds__(256) segment_len_kernel(const __grid_constant_
     const unsigned long long bits = b.chunk_bitpos[c0 + cps] - b.chunk_bitpos[c0];
     const unsigned tail = (s == P.segs_per_image - 1 && P.has_eoi) ? 2u : 0u; // EOI, encoder.rs:564
     const unsigned long long bytes = lead_len(b, P, img, k, i) + ((bits + 7) >> 3) + tail;
-    if (bytes > 0xFFFFFFFFull) atomicOr(b.status + 2, 8ull); // seglen is 32-bit: reported, never wrapped silently
+    if (bytes > 0xFFFFFFFFull) atomicOr(b.status + kStatFlags, kFlagSegment4G); // seglen is 32-bit: reported, never wrapped silently
     b.seglen[g] = (unsigned)bytes;
 }
 
-// bytes of local segment g (lead + data + EOI); raises flag 8 beyond 4 GiB
+// bytes of local segment g (lead + data + EOI); the caller raises kFlagSegment4G beyond 4 GiB
 __device__ __forceinline__ unsigned long long segment_bytes(const EntropyBuffers &b, const DevPlan &P, unsigned long long g) {
     const unsigned long long img = g / P.segs_per_image;
     const unsigned s = (unsigned)(g - img * P.segs_per_image);
@@ -605,7 +605,7 @@ __global__ void __launch_bounds__(1024) positions_kernel(const __grid_constant__
         unsigned long long bytes = 0;
         if (g < n_segs) {
             bytes = segment_bytes(b, P, g);
-            if (bytes > 0xFFFFFFFFull) atomicOr(b.status + 2, 8ull);
+            if (bytes > 0xFFFFFFFFull) atomicOr(b.status + kStatFlags, kFlagSegment4G);
         }
         const unsigned long long ex = cta1024_exclusive(bytes, sm, total);
         if (g < n_segs) b.segpos[g] = carry + ex;
@@ -634,8 +634,8 @@ __global__ void __launch_bounds__(128) segment_lead_kernel(const __grid_constant
     const int lane = threadIdx.x & 31;
     if (blockIdx.x == 0 && threadIdx.x == 0) { // size of the unstuffed stream for the host; too large for the buffer: nothing is written
         const unsigned long long bytes = stream_bytes(b);
-        b.status[0] = bytes;
-        if (bytes > b.ustream_cap) atomicOr(b.status + 2, 1ull);
+        b.status[kStatUnstuffed] = bytes;
+        if (bytes > b.ustream_cap) atomicOr(b.status + kStatFlags, kFlagStream);
     }
     if (g >= n_segs || !stream_fits(b)) return;
     const unsigned long long img = g / P.segs_per_image;
@@ -702,7 +702,7 @@ __global__ void __launch_bounds__(128) segment_lead_kernel(const __grid_constant
 // pad bits of finalize_bit_buffer behind the segment's last bit (writer.rs:138-145: ones up to the byte boundary).
 __global__ void __launch_bounds__(256) place_chunks_kernel(const __grid_constant__ EntropyBuffers b, const __grid_constant__ DevPlan P, unsigned long long n_chunks,
                                                            const unsigned per_warp) {
-    if (!stream_fits(b) || (b.status[2] & 4ull)) return;
+    if (!stream_fits(b) || (b.status[kStatFlags] & kFlagPool)) return;
     const int lane = threadIdx.x & 31;
     const unsigned long long warps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
     uint32_t *stream = reinterpret_cast<uint32_t *>(b.ustream);
@@ -901,8 +901,8 @@ __global__ void __launch_bounds__(256) stuff_scatter_kernel(const __grid_constan
         ff_total = b.ffpos[n_pieces];
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) {
-        b.status[1] = ff_total;
-        if (bytes + ff_total > b.out_cap) atomicOr(b.status + 2, 2ull);
+        b.status[kStatDataFF] = ff_total;
+        if (bytes + ff_total > b.out_cap) atomicOr(b.status + kStatFlags, kFlagOut);
     }
     if (bytes + ff_total > b.out_cap) return;
     if ((unsigned long long)blockIdx.x * kStuffChunk >= bytes) return;

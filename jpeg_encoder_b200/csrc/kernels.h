@@ -43,13 +43,32 @@ struct EntropyBuffers {
     // capacities (bytes) of ustream / out and the status block the kernels report into: the host sizes the
     // buffers from the previous call and checks `status` once at the end instead of syncing mid-pipeline
     unsigned long long ustream_cap, out_cap, n_segs_total;
-    // [0] unstuffed bytes, [1] data 0xFF bytes, [2] flags (1: ustream, 2: out, 4: pool overflow; 8: a segment over 4 GiB;
-    // 16: an optimized Huffman code does not fit),
-    // [3] scan error, [4] work-item ticket of the coding kernel, [5] pool cursor (16-byte units)
-    unsigned long long *status;
+    unsigned long long *status;    // kStatusWords entropy status words (kStat* below)
     size_t scan_tmp_bytes;
 };
+
+// The status block of one encode call, one device buffer: [n + 1 file offsets][kStatusWords entropy status words]
+// [kStatusWords table-build status words][raw mask]. The first three parts are read back with one copy.
 constexpr int kStatusWords = 8;
+// Words of a status part: unstuffed bytes, 0xFF bytes of the coded data, flags, look-back scan error, work-item ticket
+// of the coding kernel, pool cursor (16-byte units; it counts every request, also beyond the capacity).
+constexpr int kStatUnstuffed = 0, kStatDataFF = 1, kStatFlags = 2, kStatScanError = 3, kStatTicket = 4, kStatPoolCursor = 5;
+// Flag bits: overflow of the unstuffed stream, the output, the chunk pool; a scan segment over 4 GiB; an optimized
+// Huffman code that does not fit (longer than 32 bits, or code plus value bits beyond 31; table-build part)
+constexpr unsigned long long kFlagStream = 1, kFlagOut = 2, kFlagPool = 4, kFlagSegment4G = 8, kFlagHuffmanLong = 16;
+
+struct StatusBlock {
+    uint32_t n;        // images
+    size_t mask_bytes; // raw mask: one bit per byte of the unstuffed stream
+    size_t readback_bytes() const { return (size_t)(n + 1 + 2 * kStatusWords) * 8; }
+    size_t bytes() const { return readback_bytes() + mask_bytes; }
+    // the parts inside a block (device) or its read-back copy (host) at `base`
+    unsigned long long *file_off(void *base) const { return static_cast<unsigned long long *>(base); }
+    unsigned long long *status(void *base) const { return file_off(base) + n + 1; }
+    unsigned long long *table_status(void *base) const { return status(base) + kStatusWords; }
+    uint32_t *raw_mask(void *base) const { return reinterpret_cast<uint32_t *>(table_status(base) + kStatusWords); }
+};
+inline StatusBlock status_block(uint32_t n, unsigned long long ustream_cap) { return {n, (size_t)(ustream_cap / 32 + 2) * 4}; }
 
 // A visit codes at most 1 + 63 symbols of <= 16 code + 11 value bits = 1728 bits = 54 words.
 constexpr int kSlotWords = 56;
@@ -88,7 +107,7 @@ cudaError_t launch_build_single_tables(const uint32_t *hist, uint32_t n, int ac,
 
 // gather.cu -- a rank's pieces stored at their place in the assembled file (possibly in a peer GPU's memory)
 cudaError_t launch_place_pieces(const uint8_t *src, uint8_t *dst, unsigned long long dst_cap, const unsigned long long *table, unsigned world,
-                                unsigned rank, unsigned n_scans, unsigned long long *total_out, unsigned long long *status, cudaStream_t stream);
+                                unsigned rank, unsigned n_scans, unsigned long long *total_out, cudaStream_t stream);
 
 // scan.cu -- device-wide exclusive prefix sum of u32 into u64; out has n + 1 entries (out[n] = total)
 size_t scan_tmp_bytes(uint64_t n);

@@ -228,7 +228,7 @@ __global__ void __launch_bounds__(128) build_tables_kernel(const uint32_t *__res
     if (t < n_tables) {
         const uint32_t *f = hist + (hist_per_image ? img : 0) * (2 * 2 * 257) + (size_t)(t * 2 + cls) * 257;
         const bool ok = build_one(S[warp], f, cls == 1, t, words[warp], dht[warp], dht_len[warp]);
-        if (!ok && lane == 0) atomicOr(status + 2, 16ull);
+        if (!ok && lane == 0) atomicOr(status + kStatFlags, kFlagHuffmanLong);
         uint32_t *dst = huff + img * kHuffWordsPerImage + (size_t)(t * 2 + cls) * 256;
         for (int i = lane; i < 256; i += 32) dst[i] = words[warp][i];
     }
