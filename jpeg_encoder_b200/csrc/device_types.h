@@ -46,6 +46,7 @@ struct StageAParams {
     int width, height, bpp, color_type, ncomp;
     int hmax, vmax;
     int mcu_cols, mcu_rows;
+    // groups .. tile_pitch and task_*: the CTA tiling of the generic kernel, filled by its launcher
     int groups;            // 32-MCU groups per CTA tile
     int tiles_per_row;
     int tasks_per_group;   // warp tasks per group = sum over components of H_c*V_c
@@ -53,7 +54,7 @@ struct StageAParams {
     int n_images;
     int planar;            // 1: pixels = ncomp full-resolution planes of width*height bytes (plane_stride apart)
     unsigned long long plane_stride;
-    int use_fast;          // 1: stage_a_warp_kernel
+    int use_fast;          // 1: stage_a_warp_kernel / stage_a_plane_kernel, 0: stage_a_kernel
     // Coefficient layout (DESIGN.md section 3). mcu_order = 1 (interleaved scan): blocks in the order the scan codes
     // them, block = (mcu * bpu + slot). mcu_order = 0: per component the raster of its TRUE grid (comp_tw x comp_th,
     // the one encode_blocks walks), components back to back; blocks of the MCU padding are not stored.
@@ -61,7 +62,7 @@ struct StageAParams {
     int mcu_row0;          // a horizontal slice of the image: its first MCU row inside the whole image (destination rows are global)
     int slot_base[4];      // first slot of the component inside the MCU (mcu_order)
     int comp_tw[4], comp_th[4];
-    // per warp task inside a group: component and block position inside the MCU
+    // per warp task inside a group of the generic kernel: component and block position inside the MCU
     int8_t task_comp[kMaxSlots], task_v[kMaxSlots], task_h[kMaxSlots];
     int comp_h[4], comp_v[4], comp_qt[4], comp_pw[4];
     unsigned long long comp_off[4];

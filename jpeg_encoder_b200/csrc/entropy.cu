@@ -31,7 +31,6 @@
 //   stuff_scatter_kernel copies every byte to its final place, inserting 0x00 after data 0xFF; extra CTAs work out
 //                        the file offsets and a strip's piece offsets
 //   histogram_kernel     optimized tables: symbol statistics of every image (same walk as the coder)
-#include <mutex>
 
 #include "kernels.h"
 
@@ -1066,39 +1065,11 @@ cudaError_t launch_histogram(const DevPlan &hp, const int16_t *coef, uint32_t n_
 }
 
 namespace {
-constexpr int kMaxDevices = 64;
-struct CoderInfo {
-    bool ready = false;
-    int n_sms = 0, ctas_per_sm = 0;
-};
-template <int T, bool FULL>
-cudaError_t coder_info(CoderInfo &out) {
-    static std::mutex mu;
-    static CoderInfo cache[kMaxDevices];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    std::lock_guard<std::mutex> lock(mu);
-    CoderInfo &c = cache[dev < kMaxDevices ? dev : kMaxDevices - 1];
-    if (!c.ready) {
-        auto kernel = encode_chunks_kernel<T, FULL>;
-        const int smem = CoderSmem<T, FULL>::kBytes;
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-        cudaDeviceGetAttribute(&c.n_sms, cudaDevAttrMultiProcessorCount, dev);
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.ctas_per_sm, kernel, T, smem);
-        if (e != cudaSuccess) return e;
-        if (c.ctas_per_sm < 1) c.ctas_per_sm = 1;
-        c.ready = true;
-    }
-    out = c;
-    return cudaSuccess;
-}
 template <int T, bool FULL>
 cudaError_t coder_config(unsigned long long n_items, CoderLaunch &cfg) {
-    CoderInfo info;
-    cudaError_t e = coder_info<T, FULL>(info);
+    unsigned long long grid = 0;
+    cudaError_t e = resident_ctas<encode_chunks_kernel<T, FULL>>(T, CoderSmem<T, FULL>::kBytes, grid);
     if (e != cudaSuccess) return e;
-    unsigned long long grid = (unsigned long long)info.n_sms * info.ctas_per_sm;
     if (grid > n_items) grid = n_items;
     if (grid < 1) grid = 1;
     cfg.grid = (unsigned)grid;

@@ -573,8 +573,6 @@ void Plan::fill_device_plan(DevPlan &d) const {
     }
 }
 
-bool force_generic_stage_a = false; // test hook: route every format through the generic kernel
-
 void Plan::fill_stage_a(StageAParams &a) const {
     std::memset(&a, 0, sizeof(a));
     a.blocks_per_image = blocks_per_image;
@@ -589,7 +587,6 @@ void Plan::fill_stage_a(StageAParams &a) const {
     a.mcu_rows = (int)mcu_rows;
     a.mcu_order = mode == Mode::Interleaved;
     a.bpu = (int)bpu_interleaved;
-    int n = 0;
     for (int c = 0; c < ncomp; ++c) {
         a.comp_h[c] = comps[c].h;
         a.comp_v[c] = comps[c].v;
@@ -599,32 +596,14 @@ void Plan::fill_stage_a(StageAParams &a) const {
         a.comp_tw[c] = (int)true_w[c];
         a.comp_th[c] = (int)true_h[c];
         a.slot_base[c] = (int)slot_base[c];
-        for (int v = 0; v < comps[c].v; ++v)
-            for (int h = 0; h < comps[c].h; ++h) {
-                a.task_comp[n] = (int8_t)c;
-                a.task_v[n] = (int8_t)v;
-                a.task_h[n] = (int8_t)h;
-                ++n;
-            }
     }
-    a.tasks_per_group = n;
-    // Warp kernel: every packed ColorType with luma factors in {1,2}; a task is (component, v, run of 32 consecutive blocks).
-    const bool fast_ct = true; // every ColorType, every sampling factor and planar input have a warp-kernel instantiation
-    const char *fg = std::getenv("JPGB_FORCE_GENERIC_STAGE_A"); // test hook
-    a.use_fast = fast_ct && !force_generic_stage_a && !(fg && fg[0] == '1');
-    // CTA tile: `groups` x 32 MCUs wide, one MCU row high; aim for ~24 KB of pixels in shared memory
+    // every ColorType, sampling factor and planar input has a warp-kernel instantiation; the generic kernel stays as
+    // the cross-check of the tests
+    const char *fg = std::getenv("JPGB_FORCE_GENERIC_STAGE_A");
+    a.use_fast = !(fg && fg[0] == '1');
     a.planar = planar ? 1 : 0;
     a.plane_stride = (unsigned long long)p.width * p.height;
     if (planar) a.bpp = 1;
-    const int group_bytes = 32 * 8 * hmax * 8 * vmax * (planar ? ncomp : bpp);
-    int g = std::max(1, 24576 / group_bytes);
-    g = std::min(g, 8);
-    g = std::min<int>(g, (int)((mcu_cols + 31) / 32));
-    a.groups = g;
-    a.tiles_per_row = (int)((mcu_cols + 32 * g - 1) / (32 * g));
-    a.tile_w_px = 32 * g * 8 * hmax;
-    a.tile_h_px = 8 * vmax;
-    a.tile_pitch = a.tile_w_px * (planar ? 1 : bpp);
     for (int t = 0; t < 2; ++t)
         for (int i = 0; i < 64; ++i) {
             const int32_t c = q[t].corr[i] * q[t].recip[i];

@@ -98,6 +98,5 @@ void default_huffman_tables(HuffTable huff[2][2]); // Annex K.3, src/huffman.rs:
 int bytes_per_pixel(uint8_t color_type);
 int num_components(uint8_t color_type);
 extern const uint8_t kZigzag[64];
-extern bool force_generic_stage_a;
 
 } // namespace jpgb

@@ -3,11 +3,42 @@
 #include <cuda_runtime.h>
 
 #include <cstdint>
+#include <mutex>
 
 #include "../../include/jpegenc_b200.h"
 #include "device_types.h"
 
 namespace jpgb {
+
+// CTAs of a persistent `Kernel` that fit on the current device at once (SMs x resident CTAs per SM) at `threads`
+// threads and `smem` bytes of dynamic shared memory, after opting the kernel in to that much shared memory. Each
+// kernel launches with one block size and one shared-memory size, so the answer is computed once per device.
+// Contexts on several host threads (and devices) launch concurrently: the table is guarded.
+template <auto Kernel>
+cudaError_t resident_ctas(int threads, size_t smem, unsigned long long &ctas) {
+    constexpr int kMaxDevices = 64;
+    static std::mutex mu;
+    static struct {
+        int dev = -1;
+        unsigned long long ctas = 0;
+    } cache[kMaxDevices];
+    int dev = 0;
+    cudaGetDevice(&dev);
+    std::lock_guard<std::mutex> lock(mu);
+    auto &c = cache[dev < kMaxDevices ? dev : kMaxDevices - 1];
+    if (c.dev != dev) {
+        cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        int n_sms = 0, per_sm = 0;
+        cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, dev);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, Kernel, threads, smem);
+        if (e != cudaSuccess) return e;
+        c.ctas = (unsigned long long)n_sms * (per_sm < 1 ? 1 : per_sm);
+        c.dev = dev;
+    }
+    ctas = c.ctas;
+    return cudaSuccess;
+}
 
 // stage_a.cu -- colour + decimate + level shift + fDCT + quantize -> zig-zag i16 coefficients
 cudaError_t launch_stage_a(const StageAParams &p, uint32_t n_images, cudaStream_t stream);

@@ -19,9 +19,9 @@
 // All arithmetic is 32-bit integer; tensor cores are not used (the DCT must be bit-exact).
 #include <cuda.h>
 
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
-#include <mutex>
 #include <utility>
 
 #include "kernels.h"
@@ -96,6 +96,16 @@ __device__ __forceinline__ void dct8(int &d0, int &d1, int &d2, int &d3, int &d4
     d1 = (tmp7 * (12299 - 7373) + (tmp4 * -7373 + z4m)) >> N;
 }
 
+// 2-D DCT of one block in registers, natural order: the rows (pass 1), then the columns (pass 2)
+__device__ __forceinline__ void dct_2d(int (&v)[64]) {
+#pragma unroll
+    for (int y = 0; y < 8; ++y)
+        dct8<1>(v[y * 8 + 0], v[y * 8 + 1], v[y * 8 + 2], v[y * 8 + 3], v[y * 8 + 4], v[y * 8 + 5], v[y * 8 + 6], v[y * 8 + 7]);
+#pragma unroll
+    for (int x = 0; x < 8; ++x)
+        dct8<2>(v[x], v[8 + x], v[16 + x], v[24 + x], v[32 + x], v[40 + x], v[48 + x], v[56 + x]);
+}
+
 struct ZZ {
     int v[64];
 };
@@ -113,21 +123,38 @@ __device__ __forceinline__ int quant32(const StageAParams &p, int v, int n) {
     return v * p.q[T].mul[n] + add;
 }
 
+__device__ __forceinline__ void store256(void *dst, uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t a4,
+                                         uint32_t a5, uint32_t a6, uint32_t a7) {
+    asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(dst), "r"(a0), "r"(a1), "r"(a2), "r"(a3),
+                 "r"(a4), "r"(a5), "r"(a6), "r"(a7)
+                 : "memory");
+}
+
+// the quantized block in zig-zag order -> its 128 bytes at `dst` (32-byte aligned), four 256-bit stores
 template <int T>
-__device__ __forceinline__ void quantize_store(const StageAParams &p, const int (&v)[64], int16_t *dst) {
+__device__ __forceinline__ void quantize_store256(const StageAParams &p, const int (&v)[64], int16_t *dst) {
     constexpr ZZ zz = make_zz();
-    uint4 *out = reinterpret_cast<uint4 *>(dst);
 #pragma unroll
-    for (int w = 0; w < 8; ++w) {
-        uint32_t r[4];
+    for (int w = 0; w < 4; ++w) {
+        uint32_t r[8];
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int i0 = w * 8 + k * 2, i1 = i0 + 1;
+        for (int k = 0; k < 8; ++k) {
+            const int i0 = w * 16 + k * 2, i1 = i0 + 1;
             const int a = quant32<T>(p, v[zz.v[i0]], zz.v[i0]);
             const int b = quant32<T>(p, v[zz.v[i1]], zz.v[i1]);
             r[k] = __byte_perm((uint32_t)a, (uint32_t)b, 0x7632); // {hi16(a), hi16(b)}
         }
-        out[w] = make_uint4(r[0], r[1], r[2], r[3]);
+        store256(dst + w * 16, r[0], r[1], r[2], r[3], r[4], r[5], r[6], r[7]);
+    }
+}
+
+// Byte-wise fill of one 16-byte chunk with the row's last pixel replicated (Q4). Cold path, kept out of line.
+template <int BPP>
+__device__ __noinline__ void stage_edge_chunk(uint8_t *dst, const uint8_t *row, int cb, int valid_px) {
+    for (int b = 0; b < 16; ++b) {
+        const int byte = cb + b;
+        const int px = byte / BPP, ch = byte - px * BPP;
+        dst[cb + b] = row[min(px, valid_px - 1) * BPP + ch];
     }
 }
 
@@ -155,17 +182,10 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
         const int ry = cc / chunks_per_row, cb = (cc - ry * chunks_per_row) * 16;
         const int sy = min(py0 + ry, p.height - 1);
         const uint8_t *row = src + (size_t)plane * p.plane_stride + (size_t)sy * row_bytes + (size_t)px0 * BPP;
-        uint8_t *dst = tile + plane * plane_tile + ry * p.tile_pitch + cb;
-        if (cb + 16 <= valid_bytes && ((reinterpret_cast<uintptr_t>(row + cb) & 15) == 0)) {
-            *reinterpret_cast<uint4 *>(dst) = __ldg(reinterpret_cast<const uint4 *>(row + cb));
-        } else {
-#pragma unroll 4
-            for (int b = 0; b < 16; ++b) {
-                const int byte = cb + b;
-                const int px = byte / BPP, ch = byte - px * BPP;
-                dst[b] = row[min(px, valid_px - 1) * BPP + ch];
-            }
-        }
+        uint8_t *dst = tile + plane * plane_tile + ry * p.tile_pitch;
+        if (cb + 16 <= valid_bytes && ((reinterpret_cast<uintptr_t>(row + cb) & 15) == 0))
+            *reinterpret_cast<uint4 *>(dst + cb) = __ldg(reinterpret_cast<const uint4 *>(row + cb));
+        else stage_edge_chunk<BPP>(dst, row, cb, valid_px);
     }
     __syncthreads();
 
@@ -189,13 +209,7 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
         for (int y = 0; y < 8; ++y)
 #pragma unroll
             for (int x = 0; x < 8; ++x) v[y * 8 + x] = sample<CT>(base + y * step_y + x * step_x, comp);
-
-#pragma unroll
-        for (int y = 0; y < 8; ++y)
-            dct8<1>(v[y * 8 + 0], v[y * 8 + 1], v[y * 8 + 2], v[y * 8 + 3], v[y * 8 + 4], v[y * 8 + 5], v[y * 8 + 6], v[y * 8 + 7]);
-#pragma unroll
-        for (int x = 0; x < 8; ++x)
-            dct8<2>(v[x], v[8 + x], v[16 + x], v[24 + x], v[32 + x], v[40 + x], v[48 + x], v[56 + x]);
+        dct_2d(v);
 
         size_t blk = (size_t)img * p.blocks_per_image;
         const int gy = mcu_y + p.mcu_row0; // MCU row inside the whole image (this launch may cover a slice of it)
@@ -207,8 +221,8 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
             blk += p.comp_off[comp] + (size_t)by * p.comp_tw[comp] + bx;
         }
         int16_t *dst = p.coef + blk * 64;
-        if (p.comp_qt[comp] == 0) quantize_store<0>(p, v, dst);
-        else quantize_store<1>(p, v, dst);
+        if (p.comp_qt[comp] == 0) quantize_store256<0>(p, v, dst);
+        else quantize_store256<1>(p, v, dst);
     }
 }
 
@@ -360,26 +374,26 @@ __device__ __forceinline__ void chroma_row(const uint32_t (&w)[NW], int *s, cons
     ((s[Is] = chroma_at<Is * SX * Fmt<CT>::BPP, NW>(w, c)), ...);
 }
 
-// 8 samples (unshifted, 0..255) of one block row. `row` points at the first pixel of the row in the
-// shared tile; the pixels used are 0, SX, 2*SX, ... (point decimation, encoder.rs:1222-1242).
-template <int CT, int ROLE, int SX>
-__device__ __forceinline__ void load_row(const uint8_t *row, int *s, const ChromaConsts *cc = nullptr) {
-    constexpr int BPP = Fmt<CT>::BPP;
-    constexpr int NW = (((7 * SX + 1) * BPP) + 3) / 4; // words spanned
-    uint32_t w[NW];
-    if constexpr (BPP == 1) {
-        const uint2 a = *reinterpret_cast<const uint2 *>(row);
-        w[0] = a.x;
-        w[1] = a.y;
-    } else if constexpr (BPP == 3 && SX == 1) {
+// The pixel words of one block row: the 8 * SX pixels from `row` (shared tile) on, as few wide loads as the
+// alignment allows. With 4 bytes per pixel and SX > 1 only every SX-th pixel is read; the words between are 0.
+template <int BPP, int SX>
+__host__ __device__ constexpr int row_words() { return (((7 * SX + 1) * BPP) + 3) / 4; }
+template <int BPP, int SX, int NW>
+__device__ __forceinline__ void load_words(const uint8_t *row, uint32_t (&w)[NW]) {
+    static_assert(NW == row_words<BPP, SX>(), "words spanned by the block row");
+    if constexpr (BPP == 4 && SX > 1) {
+        const uint32_t *r = reinterpret_cast<const uint32_t *>(row);
+#pragma unroll
+        for (int i = 0; i < NW; ++i) w[i] = (i % SX) ? 0u : r[i];
+    } else if constexpr ((SX * BPP) % 2 != 0) { // a block is 8 or 24 bytes wide: 8-byte aligned
         const uint2 *r = reinterpret_cast<const uint2 *>(row);
 #pragma unroll
-        for (int i = 0; i < 3; ++i) {
+        for (int i = 0; i < NW / 2; ++i) {
             const uint2 a = r[i];
             w[2 * i] = a.x;
             w[2 * i + 1] = a.y;
         }
-    } else if constexpr (BPP == 3) { // SX 2 or 4: the block's 8 * SX pixels are 48 / 96 bytes, 16-byte aligned
+    } else { // a block is a multiple of 16 bytes wide: 16-byte aligned
         const uint4 *r = reinterpret_cast<const uint4 *>(row);
 #pragma unroll
         for (int i = 0; i < (NW + 3) / 4; ++i) {
@@ -389,21 +403,16 @@ __device__ __forceinline__ void load_row(const uint8_t *row, int *s, const Chrom
             if (4 * i + 2 < NW) w[4 * i + 2] = a.z;
             if (4 * i + 3 < NW) w[4 * i + 3] = a.w;
         }
-    } else if constexpr (BPP == 4 && SX == 1) {
-        const uint4 *r = reinterpret_cast<const uint4 *>(row);
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-            const uint4 a = r[i];
-            w[4 * i] = a.x;
-            w[4 * i + 1] = a.y;
-            w[4 * i + 2] = a.z;
-            w[4 * i + 3] = a.w;
-        }
-    } else { // BPP == 4, SX 2 or 4: every SX-th pixel word
-        const uint32_t *r = reinterpret_cast<const uint32_t *>(row);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) w[SX * i] = r[SX * i];
     }
+}
+
+// 8 samples (unshifted, 0..255) of one block row. `row` points at the first pixel of the row in the
+// shared tile; the pixels used are 0, SX, 2*SX, ... (point decimation, encoder.rs:1222-1242).
+template <int CT, int ROLE, int SX>
+__device__ __forceinline__ void load_row(const uint8_t *row, int *s, const ChromaConsts *cc = nullptr) {
+    constexpr int NW = row_words<Fmt<CT>::BPP, SX>();
+    uint32_t w[NW];
+    load_words<Fmt<CT>::BPP, SX>(row, w);
     if constexpr (ROLE == ROLE_CBCR) chroma_row<CT, SX, NW>(w, s, *cc, std::make_integer_sequence<int, 8>{});
     else sample_row<CT, ROLE, SX, NW>(w, s, std::make_integer_sequence<int, 8>{});
 }
@@ -423,41 +432,9 @@ __device__ __forceinline__ void byte_row(const uint32_t (&w)[NW], int *s, unsign
 }
 template <int BPP, int SX>
 __device__ __forceinline__ void load_row_bytes(const uint8_t *row, int *s, unsigned coff, unsigned xorv) {
-    constexpr int NW = (((7 * SX + 1) * BPP) + 3) / 4;
+    constexpr int NW = row_words<BPP, SX>();
     uint32_t w[NW];
-    if constexpr (BPP == 3 && SX == 1) {
-        const uint2 *r = reinterpret_cast<const uint2 *>(row);
-#pragma unroll
-        for (int i = 0; i < 3; ++i) {
-            const uint2 a = r[i];
-            w[2 * i] = a.x;
-            w[2 * i + 1] = a.y;
-        }
-    } else if constexpr (BPP == 3) {
-        const uint4 *r = reinterpret_cast<const uint4 *>(row);
-#pragma unroll
-        for (int i = 0; i < (NW + 3) / 4; ++i) {
-            const uint4 a = r[i];
-            w[4 * i] = a.x;
-            if (4 * i + 1 < NW) w[4 * i + 1] = a.y;
-            if (4 * i + 2 < NW) w[4 * i + 2] = a.z;
-            if (4 * i + 3 < NW) w[4 * i + 3] = a.w;
-        }
-    } else if constexpr (SX == 1) {
-        const uint4 *r = reinterpret_cast<const uint4 *>(row);
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-            const uint4 a = r[i];
-            w[4 * i] = a.x;
-            w[4 * i + 1] = a.y;
-            w[4 * i + 2] = a.z;
-            w[4 * i + 3] = a.w;
-        }
-    } else { // 4 bytes per pixel, every SX-th pixel
-        const uint32_t *r = reinterpret_cast<const uint32_t *>(row);
-#pragma unroll
-        for (int i = 0; i < NW; ++i) w[i] = (i % SX) ? 0u : r[i];
-    }
+    load_words<BPP, SX>(row, w);
     byte_row<BPP, SX, NW>(w, s, coff, xorv, std::make_integer_sequence<int, 8>{});
 }
 template <int BPP, int SX, int SY>
@@ -472,30 +449,6 @@ __device__ __forceinline__ void load_block(const uint8_t *base, int pitch, int (
     for (int y = 0; y < 8; ++y) load_row<CT, ROLE, SX>(base + y * SY * pitch, &v[y * 8], cc);
 }
 
-__device__ __forceinline__ void store256(void *dst, uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t a4,
-                                         uint32_t a5, uint32_t a6, uint32_t a7) {
-    asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(dst), "r"(a0), "r"(a1), "r"(a2), "r"(a3),
-                 "r"(a4), "r"(a5), "r"(a6), "r"(a7)
-                 : "memory");
-}
-
-template <int T>
-__device__ __forceinline__ void quantize_store256(const StageAParams &p, const int (&v)[64], int16_t *dst) {
-    constexpr ZZ zz = make_zz();
-#pragma unroll
-    for (int w = 0; w < 4; ++w) {
-        uint32_t r[8];
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            const int i0 = w * 16 + k * 2, i1 = i0 + 1;
-            const int a = quant32<T>(p, v[zz.v[i0]], zz.v[i0]);
-            const int b = quant32<T>(p, v[zz.v[i1]], zz.v[i1]);
-            r[k] = __byte_perm((uint32_t)a, (uint32_t)b, 0x7632);
-        }
-        store256(dst + w * 16, r[0], r[1], r[2], r[3], r[4], r[5], r[6], r[7]);
-    }
-}
-
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
@@ -503,16 +456,6 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src)
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-// Byte-wise fill of one 16-byte chunk with the row's last pixel replicated (Q4). Cold path, kept out of line.
-template <int BPP>
-__device__ __noinline__ void stage_edge_chunk(uint8_t *dst, const uint8_t *row, int cb, int valid_px) {
-    for (int b = 0; b < 16; ++b) {
-        const int byte = cb + b;
-        const int px = byte / BPP, ch = byte - px * BPP;
-        dst[cb + b] = row[min(px, valid_px - 1) * BPP + ch];
-    }
-}
 
 // ---- TMA (cp.async.bulk.tensor) + mbarrier, one barrier per warp --------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t *bar, unsigned count) {
@@ -697,12 +640,7 @@ __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_const
                 else if (NCOMP == 3 || comp == 2) load_block<CT, ROLE_CR, SUB ? HS : 1, SUB ? VS : 1>(base, PITCH, v);
                 else load_block<CT, ROLE_K, 1, 1>(base, PITCH, v);
             }
-#pragma unroll
-            for (int y = 0; y < 8; ++y)
-                dct8<1>(v[y * 8 + 0], v[y * 8 + 1], v[y * 8 + 2], v[y * 8 + 3], v[y * 8 + 4], v[y * 8 + 5], v[y * 8 + 6], v[y * 8 + 7]);
-#pragma unroll
-            for (int x = 0; x < 8; ++x)
-                dct8<2>(v[x], v[8 + x], v[16 + x], v[24 + x], v[32 + x], v[40 + x], v[48 + x], v[56 + x]);
+            dct_2d(v);
 
             size_t blk = (size_t)img * p.blocks_per_image;
             if (p.mcu_order) { // H, V are 1 or 2 here: bx = mcu_x * H + bh
@@ -724,28 +662,6 @@ __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_const
 // (SX, SY = the component's decimation, point sampling as everywhere). Same warp-autonomous scheme as above:
 // a warp tile is 32 blocks of the component x MR block rows; only the sampled rows are staged (cp.async).
 // =================================================================================================
-template <int SX>
-__device__ __forceinline__ void load_row_plane(const uint8_t *row, int *s) {
-    constexpr int NW = ((7 * SX + 1) + 3) / 4;
-    uint32_t w[NW];
-    if constexpr (SX == 1) {
-        const uint2 a = *reinterpret_cast<const uint2 *>(row);
-        w[0] = a.x;
-        w[1] = a.y;
-    } else {
-        const uint4 *r = reinterpret_cast<const uint4 *>(row);
-#pragma unroll
-        for (int i = 0; i < NW / 4; ++i) {
-            const uint4 a = r[i];
-            w[4 * i] = a.x;
-            w[4 * i + 1] = a.y;
-            w[4 * i + 2] = a.z;
-            w[4 * i + 3] = a.w;
-        }
-    }
-    sample_row<JPGB_LUMA, ROLE_RAW, SX, NW>(w, s, std::make_integer_sequence<int, 8>{});
-}
-
 template <int SX>
 __host__ __device__ constexpr int plane_tile_block_rows() { return SX == 1 ? 4 : (SX == 2 ? 2 : 1); } // 8 KB per warp tile
 
@@ -814,14 +730,8 @@ __global__ void __launch_bounds__(128, 4) stage_a_plane_kernel(const __grid_cons
             if (bx >= tw) continue;
             const uint8_t *base = tile + mr * 8 * PITCH + lane * 8 * SX;
             int v[64];
-#pragma unroll
-            for (int y = 0; y < 8; ++y) load_row_plane<SX>(base + y * PITCH, &v[y * 8]);
-#pragma unroll
-            for (int y = 0; y < 8; ++y)
-                dct8<1>(v[y * 8 + 0], v[y * 8 + 1], v[y * 8 + 2], v[y * 8 + 3], v[y * 8 + 4], v[y * 8 + 5], v[y * 8 + 6], v[y * 8 + 7]);
-#pragma unroll
-            for (int x = 0; x < 8; ++x)
-                dct8<2>(v[x], v[8 + x], v[16 + x], v[24 + x], v[32 + x], v[40 + x], v[48 + x], v[56 + x]);
+            load_block<JPGB_LUMA, ROLE_RAW, SX, 1>(base, PITCH, v);
+            dct_2d(v);
             const int gby = by + p.mcu_row0 * V; // block row inside the whole image
             size_t blk = (size_t)img * p.blocks_per_image;
             if (p.mcu_order) {
@@ -866,98 +776,53 @@ inline bool make_pixel_tensor_map(CUtensorMap &map, const StageAParams &p, int b
               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-constexpr int kMaxDevices = 64;
-struct LaunchInfo {
-    bool ready = false;
-    int dev = -1, n_sms = 0, ctas_per_sm = 0;
-};
-
 template <int CT, int HS, int VS>
 cudaError_t launch_warp_variant(const StageAParams &p, cudaStream_t stream) {
     constexpr int BPP = Fmt<CT>::BPP;
     constexpr int MR = warp_tile_mcu_rows<CT, HS, VS>();
     constexpr int TILE = 256 * BPP * 8 * VS * MR;
-    const size_t smem = (size_t)4 * TILE + 4 * sizeof(uint64_t); // 4 warps per CTA: one private tile and one mbarrier each
-    auto kernel = stage_a_warp_kernel<CT, HS, VS>;
-    // per device, once: opt in to the dynamic shared memory and ask how many CTAs fit on an SM. Contexts on
-    // several host threads (and several devices) launch concurrently: the cache is per device and guarded.
-    static std::mutex mu;
-    static LaunchInfo cache[kMaxDevices];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    LaunchInfo info;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        LaunchInfo &c = cache[dev < kMaxDevices ? dev : kMaxDevices - 1];
-        if (!c.ready || c.dev != dev) {
-            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            cudaDeviceGetAttribute(&c.n_sms, cudaDevAttrMultiProcessorCount, dev);
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.ctas_per_sm, kernel, 128, smem);
-            if (e != cudaSuccess) return e;
-            if (c.ctas_per_sm < 1) c.ctas_per_sm = 1;
-            c.dev = dev;
-            c.ready = true;
-        }
-        info = c;
-    }
-    const int n_sms = info.n_sms, ctas_per_sm = info.ctas_per_sm;
+    constexpr size_t smem = (size_t)4 * TILE + 4 * sizeof(uint64_t); // 4 warps per CTA: one private tile and one mbarrier each
+    unsigned long long grid = 0;
+    const cudaError_t e = resident_ctas<stage_a_warp_kernel<CT, HS, VS>>(128, smem, grid);
+    if (e != cudaSuccess) return e;
     constexpr int MCUS = 32 / HS;
     const unsigned long long n_tiles = (unsigned long long)((p.mcu_cols + MCUS - 1) / MCUS) * ((p.mcu_rows + MR - 1) / MR) * p.n_images;
-    unsigned long long grid = (unsigned long long)n_sms * ctas_per_sm;
     if (grid * 4 > n_tiles) grid = (n_tiles + 3) / 4;
     CUtensorMap tmap;
     std::memset(&tmap, 0, sizeof(tmap));
     const int use_tma = make_pixel_tensor_map(tmap, p, BPP, 256 * BPP, 8 * VS * MR) ? 1 : 0;
-    kernel<<<(unsigned)grid, 128, smem, stream>>>(p, tmap, use_tma);
+    stage_a_warp_kernel<CT, HS, VS><<<(unsigned)grid, 128, smem, stream>>>(p, tmap, use_tma);
     return cudaGetLastError();
 }
 
-template <int CT, int HS, int VS>
-cudaError_t launch_fast(const StageAParams &p, dim3, size_t, cudaStream_t stream) {
-    return launch_warp_variant<CT, HS, VS>(p, stream);
-}
-
+// the warp kernel instantiated for the luma sampling factors (a single component is always sampled 1x1)
 template <int CT>
-cudaError_t launch_fast_ct(const StageAParams &p, dim3 block, size_t smem, cudaStream_t stream) {
-    if (p.hmax == 1 && p.vmax == 1) return launch_fast<CT, 1, 1>(p, block, smem, stream);
-    if (p.hmax == 2 && p.vmax == 1) return launch_fast<CT, 2, 1>(p, block, smem, stream);
-    if (p.hmax == 1 && p.vmax == 2) return launch_fast<CT, 1, 2>(p, block, smem, stream);
-    if (p.hmax == 2 && p.vmax == 2) return launch_fast<CT, 2, 2>(p, block, smem, stream);
-    if (p.hmax == 4 && p.vmax == 1) return launch_fast<CT, 4, 1>(p, block, smem, stream);
-    if (p.hmax == 4 && p.vmax == 2) return launch_fast<CT, 4, 2>(p, block, smem, stream);
-    if (p.hmax == 1 && p.vmax == 4) return launch_fast<CT, 1, 4>(p, block, smem, stream);
-    return launch_fast<CT, 2, 4>(p, block, smem, stream);
+cudaError_t launch_warp(const StageAParams &p, cudaStream_t stream) {
+    if constexpr (Fmt<CT>::NCOMP == 1) {
+        return launch_warp_variant<CT, 1, 1>(p, stream);
+    } else {
+        if (p.hmax == 1 && p.vmax == 1) return launch_warp_variant<CT, 1, 1>(p, stream);
+        if (p.hmax == 2 && p.vmax == 1) return launch_warp_variant<CT, 2, 1>(p, stream);
+        if (p.hmax == 1 && p.vmax == 2) return launch_warp_variant<CT, 1, 2>(p, stream);
+        if (p.hmax == 2 && p.vmax == 2) return launch_warp_variant<CT, 2, 2>(p, stream);
+        if (p.hmax == 4 && p.vmax == 1) return launch_warp_variant<CT, 4, 1>(p, stream);
+        if (p.hmax == 4 && p.vmax == 2) return launch_warp_variant<CT, 4, 2>(p, stream);
+        if (p.hmax == 1 && p.vmax == 4) return launch_warp_variant<CT, 1, 4>(p, stream);
+        return launch_warp_variant<CT, 2, 4>(p, stream);
+    }
 }
 
 template <int SX, int SY>
 cudaError_t launch_plane_variant(const StageAParams &p, int comp, cudaStream_t stream) {
     constexpr int MR = plane_tile_block_rows<SX>();
-    const size_t smem = (size_t)4 * 256 * SX * 8 * MR;
-    auto kernel = stage_a_plane_kernel<SX, SY>;
-    static std::mutex mu;
-    static LaunchInfo cache[kMaxDevices];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    LaunchInfo info;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        LaunchInfo &c = cache[dev < kMaxDevices ? dev : kMaxDevices - 1];
-        if (!c.ready || c.dev != dev) {
-            cudaDeviceGetAttribute(&c.n_sms, cudaDevAttrMultiProcessorCount, dev);
-            const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.ctas_per_sm, kernel, 128, smem);
-            if (e != cudaSuccess) return e;
-            if (c.ctas_per_sm < 1) c.ctas_per_sm = 1;
-            c.dev = dev;
-            c.ready = true;
-        }
-        info = c;
-    }
+    constexpr size_t smem = (size_t)4 * 256 * SX * 8 * MR;
+    unsigned long long grid = 0;
+    const cudaError_t e = resident_ctas<stage_a_plane_kernel<SX, SY>>(128, smem, grid);
+    if (e != cudaSuccess) return e;
     const int tw = p.mcu_order ? p.comp_pw[comp] : p.comp_tw[comp], th = p.mcu_rows * p.comp_v[comp];
     const unsigned long long n_tiles = (unsigned long long)((tw + 31) / 32) * ((th + MR - 1) / MR) * p.n_images;
-    unsigned long long grid = (unsigned long long)info.n_sms * info.ctas_per_sm;
     if (grid * 4 > n_tiles) grid = (n_tiles + 3) / 4;
-    kernel<<<(unsigned)grid, 128, smem, stream>>>(p, comp);
+    stage_a_plane_kernel<SX, SY><<<(unsigned)grid, 128, smem, stream>>>(p, comp);
     return cudaGetLastError();
 }
 
@@ -976,62 +841,68 @@ cudaError_t launch_planes(const StageAParams &p, cudaStream_t stream) {
     return cudaSuccess;
 }
 
+// The generic kernel's CTA tile: `groups` x 32 MCUs wide, one MCU row high, ~24 KB of pixels in shared memory. A warp
+// task is one block position of the MCU (component, v, h) in one group.
+template <int CT>
+cudaError_t launch_generic(StageAParams p, cudaStream_t stream) {
+    const int group_bytes = 32 * 8 * p.hmax * 8 * p.vmax * (p.planar ? p.ncomp : p.bpp);
+    const int g = std::min({std::max(1, 24576 / group_bytes), 8, (p.mcu_cols + 31) / 32});
+    p.groups = g;
+    p.tiles_per_row = (p.mcu_cols + 32 * g - 1) / (32 * g);
+    p.tile_w_px = 32 * g * 8 * p.hmax;
+    p.tile_h_px = 8 * p.vmax;
+    p.tile_pitch = p.tile_w_px * p.bpp; // planar input: one byte per sample
+    int n = 0;
+    for (int c = 0; c < p.ncomp; ++c)
+        for (int v = 0; v < p.comp_v[c]; ++v)
+            for (int h = 0; h < p.comp_h[c]; ++h, ++n) {
+                p.task_comp[n] = (int8_t)c;
+                p.task_v[n] = (int8_t)v;
+                p.task_h[n] = (int8_t)h;
+            }
+    p.tasks_per_group = n;
+    const size_t smem = (size_t)p.tile_pitch * p.tile_h_px * (p.planar ? p.ncomp : 1);
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(stage_a_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    const int warps = std::min(g * n, 8);
+    // grid.z carries the image index and is limited to 65535: larger batches go in several launches
+    const unsigned n_images = (unsigned)p.n_images;
+    for (unsigned i0 = 0; i0 < n_images; i0 += 65535) {
+        StageAParams q = p;
+        q.pixels = p.pixels + (size_t)i0 * p.image_stride;
+        q.coef = p.coef + (size_t)i0 * p.blocks_per_image * 64;
+        q.n_images = (int)std::min(n_images - i0, 65535u);
+        stage_a_kernel<CT><<<dim3(p.tiles_per_row, p.mcu_rows, q.n_images), warps * 32, smem, stream>>>(q);
+    }
+    return cudaGetLastError();
+}
+
+// packed pixels: the warp kernel, or the generic one when JPGB_FORCE_GENERIC_STAGE_A asks for the cross-check
+template <int CT>
+cudaError_t launch_packed(const StageAParams &p, cudaStream_t stream) {
+    return p.use_fast ? launch_warp<CT>(p, stream) : launch_generic<CT>(p, stream);
+}
+
 } // namespace
 
 cudaError_t launch_stage_a(const StageAParams &p_in, uint32_t n_images, cudaStream_t stream) {
     StageAParams p = p_in;
     p.n_images = (int)n_images;
-    const size_t smem = (size_t)p.tile_pitch * p.tile_h_px * (p.planar ? p.ncomp : 1);
-    const int n_tasks = p.groups * p.tasks_per_group;
-    const int warps = n_tasks < 8 ? n_tasks : 8;
-    dim3 grid(p.tiles_per_row, p.mcu_rows, 1), block(warps * 32);
-    if (p.use_fast && p.planar) return launch_planes(p, stream);
-    if (p.use_fast) {
-        switch (p.color_type) {
-        case JPGB_LUMA: return launch_fast<JPGB_LUMA, 1, 1>(p, block, smem, stream);
-        case JPGB_RGB: return launch_fast_ct<JPGB_RGB>(p, block, smem, stream);
-        case JPGB_RGBA: return launch_fast_ct<JPGB_RGBA>(p, block, smem, stream);
-        case JPGB_BGR: return launch_fast_ct<JPGB_BGR>(p, block, smem, stream);
-        case JPGB_BGRA: return launch_fast_ct<JPGB_BGRA>(p, block, smem, stream);
-        case JPGB_CMYK_AS_YCCK: return launch_fast_ct<JPGB_CMYK_AS_YCCK>(p, block, smem, stream);
-        case JPGB_YCBCR: return launch_fast_ct<JPGB_YCBCR>(p, block, smem, stream);
-        case JPGB_YCCK: return launch_fast_ct<JPGB_YCCK>(p, block, smem, stream);
-        case JPGB_CMYK: return launch_fast_ct<JPGB_CMYK>(p, block, smem, stream);
-        default: break;
-        }
-    }
-    // grid.z carries the image index and is limited to 65535: larger batches go in several launches
-#define JPGB_LAUNCH_A(CT)                                                                                        \
-    case CT: {                                                                                                   \
-        if (smem > 48 * 1024) {                                                                                  \
-            cudaError_t e = cudaFuncSetAttribute(stage_a_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-            if (e != cudaSuccess) return e;                                                                      \
-        }                                                                                                        \
-        for (uint32_t i0 = 0; i0 < n_images; i0 += 65535) {                                                      \
-            StageAParams q = p;                                                                                  \
-            q.pixels = p.pixels + (size_t)i0 * p.image_stride;                                                   \
-            q.coef = p.coef + (size_t)i0 * p.blocks_per_image * 64;                                              \
-            grid.z = n_images - i0 < 65535 ? n_images - i0 : 65535;                                              \
-            q.n_images = (int)grid.z;                                                                            \
-            stage_a_kernel<CT><<<grid, block, smem, stream>>>(q);                                                \
-        }                                                                                                        \
-        break;                                                                                                   \
-    }
-    switch (p.planar ? kPlanar : p.color_type) {
-        JPGB_LAUNCH_A(JPGB_LUMA)
-        JPGB_LAUNCH_A(JPGB_RGB)
-        JPGB_LAUNCH_A(JPGB_RGBA)
-        JPGB_LAUNCH_A(JPGB_BGR)
-        JPGB_LAUNCH_A(JPGB_BGRA)
-        JPGB_LAUNCH_A(JPGB_YCBCR)
-        JPGB_LAUNCH_A(JPGB_CMYK)
-        JPGB_LAUNCH_A(JPGB_CMYK_AS_YCCK)
-        JPGB_LAUNCH_A(JPGB_YCCK)
-        JPGB_LAUNCH_A(kPlanar)
+    if (p.planar) return p.use_fast ? launch_planes(p, stream) : launch_generic<kPlanar>(p, stream);
+    switch (p.color_type) {
+    case JPGB_LUMA: return launch_packed<JPGB_LUMA>(p, stream);
+    case JPGB_RGB: return launch_packed<JPGB_RGB>(p, stream);
+    case JPGB_RGBA: return launch_packed<JPGB_RGBA>(p, stream);
+    case JPGB_BGR: return launch_packed<JPGB_BGR>(p, stream);
+    case JPGB_BGRA: return launch_packed<JPGB_BGRA>(p, stream);
+    case JPGB_CMYK_AS_YCCK: return launch_packed<JPGB_CMYK_AS_YCCK>(p, stream);
+    case JPGB_YCBCR: return launch_packed<JPGB_YCBCR>(p, stream);
+    case JPGB_YCCK: return launch_packed<JPGB_YCCK>(p, stream);
+    case JPGB_CMYK: return launch_packed<JPGB_CMYK>(p, stream);
     default: return cudaErrorInvalidValue;
     }
-#undef JPGB_LAUNCH_A
-    return cudaGetLastError();
 }
 
 } // namespace jpgb
