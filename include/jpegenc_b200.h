@@ -132,6 +132,43 @@ int jpgb_encode_batch_pinned(jpgb_encoder *enc, const jpgb_params *p, const uint
 int jpgb_encode_batch_device(jpgb_encoder *enc, const jpgb_params *p, const void *d_pixels,
                              size_t image_stride, uint32_t n, const void **d_files, uint64_t *offsets);
 
+/* Device images in any row pitch, packed or channel-planar (crops and views of a tensor, pitched allocations,
+ * (N, C, H, W) tensors), read where they lie. Sample ch of pixel (x, y) of image i is at
+ *   packed (plane_stride == 0): data + i*image_stride + y*row_stride + x*bpp + ch
+ *   planar (plane_stride > 0):  data + i*image_stride + ch*plane_stride + y*row_stride + x
+ * with ch in the ColorType's byte order. */
+typedef struct jpgb_device_images {
+    const void *data;       /* device address of image 0's first sample (plane 0 when planar) */
+    uint64_t image_stride;  /* bytes between image i and image i + 1 (0: every image is the same pixels) */
+    uint64_t row_stride;    /* bytes between row y and row y + 1 of an image (of a plane when planar) */
+    uint64_t plane_stride;  /* 0: packed pixels, bpp bytes each in the ColorType's byte order;
+                               > 0: channel-planar, channel c of the ColorType's byte order at data + c * plane_stride */
+} jpgb_device_images;
+
+/* jpgb_encode_batch_device for a jpgb_device_images layout: the same output (files back to back in context-owned
+ * device memory, offsets[0..n]), and files byte-identical to those of the same pixels handed over packed. Per
+ * ColorType the samples mean what they mean packed: Rgb, Bgr, Rgba, Bgra planes come in that channel order, and the
+ * alpha plane of Rgba / Bgra is never read (it need not exist); Cmyk is inverted and CmykAsYcck converted; Ycbcr and
+ * Ycck are taken verbatim; Luma planar is Luma packed.
+ * Rejected before anything is enqueued (no launch), in this order, with JPGB_ERR_BAD_PARAMS unless noted:
+ *   null arguments or n == 0;
+ *   what jpgb_encode_batch_device rejects in `p` (same codes), except the BadImageData length check;
+ *   row_stride < width*bpp (packed) or < width (planar); plane_stride > 0 but < width;
+ *   an extent beyond 64-bit addresses;
+ *   data that is not device or managed memory usable on the context's device;
+ *   a last byte read outside the allocation that holds data: the byte at
+ *     (n-1)*image_stride + (height-1)*row_stride + width*bpp - 1                        (packed)
+ *     (n-1)*image_stride + c_max*plane_stride + (height-1)*row_stride + width - 1       (planar)
+ *   where c_max is the highest plane read (2 for Rgb, Bgr, Ycbcr, Rgba, Bgra; 3 for Cmyk, CmykAsYcck, Ycck; 0 for Luma).
+ * No kernel reads a byte outside the described samples. */
+int jpgb_encode_batch_device_strided(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_images *images,
+                                     uint32_t n, const void **d_files, uint64_t *offsets);
+
+/* Order the context's stream after all work queued so far on `stream` (an event wait; the host does not block).
+ * stream may be cudaStreamLegacy (1) or cudaStreamPerThread (2); the context's own stream is a no-op. Use it when
+ * the pixels of the next encode are produced on a stream of the caller's. */
+int jpgb_encoder_wait_stream(jpgb_encoder *enc, void *stream);
+
 /* ---- one very large image split into strips of whole MCU rows (BASELINE config 5) ---------------
  * No reference equivalent: the crate encodes an image on one thread. A strip boundary must fall on
  * a restart boundary of *every* scan (src/encoder.rs:748-757, 833-839: the DC predictors reset and

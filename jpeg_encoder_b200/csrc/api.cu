@@ -1,8 +1,11 @@
 // C ABI (include/jpegenc_b200.h) and the per-call orchestration of the device pipeline.
 // The product path has no CPU fallback: without a usable sm_100 device every entry point
 // returns JPGB_ERR_CUDA.
+#include <cuda.h>
 #include <cuda_runtime.h>
 
+#include <climits>
+#include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <algorithm>
@@ -182,6 +185,7 @@ struct jpgb_encoder {
     cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
     std::vector<cudaEvent_t> ev_slice;
     cudaEvent_t ev_in[2] = {}, ev_out[2] = {}, ev_enc[2] = {};
+    cudaEvent_t ev_wait = nullptr; // jpgb_encoder_wait_stream
     bool timing = false;
     cudaEvent_t ev[JPGB_N_STAGES + 1][2] = {};
     bool ev_used[JPGB_N_STAGES] = {};
@@ -261,6 +265,62 @@ int validate_and_plan(jpgb_encoder *enc, const jpgb_params *p, size_t len_each, 
     }
     const int rc = plan.build(*p);
     if (rc != JPGB_OK) return fail(enc, rc, rc == JPGB_ERR_ZERO_DIMENSIONS ? "Image dimensions must be non zero" : "invalid parameters");
+    return JPGB_OK;
+}
+
+typedef CUresult (*MemGetAddressRangeFn)(CUdeviceptr *, size_t *, CUdeviceptr);
+MemGetAddressRangeFn mem_get_address_range_fn() {
+    static MemGetAddressRangeFn fn = [] {
+        void *f = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &f, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) f = nullptr;
+        return reinterpret_cast<MemGetAddressRangeFn>(f);
+    }();
+    return fn;
+}
+
+// The checks of jpgb_encode_batch_device_strided on the layout, in the order the header lists them. Nothing is enqueued
+// before they pass, so no kernel reads a byte outside the allocation that holds `data`.
+int check_device_images(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images &im, uint32_t n) {
+    const uint64_t w = plan.p.width, h = plan.p.height;
+    const bool planes = im.plane_stride != 0;
+    const uint64_t row_bytes = planes ? w : w * (uint64_t)plan.bpp; // bytes of a row read (of one plane)
+    char m[192];
+    if (im.row_stride < row_bytes) {
+        snprintf(m, sizeof(m), "row_stride %llu is shorter than a row (%llu bytes)", (unsigned long long)im.row_stride, (unsigned long long)row_bytes);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    if (planes && im.plane_stride < w) {
+        snprintf(m, sizeof(m), "plane_stride %llu is shorter than a row (%llu bytes)", (unsigned long long)im.plane_stride, (unsigned long long)w);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    // the last byte read: (n-1)*image_stride + c_max*plane_stride + (h-1)*row_stride + row_bytes - 1 (alpha is not read)
+    const uint8_t ct = plan.p.color_type;
+    const uint64_t c_max = !planes ? 0 : (ct == JPGB_LUMA ? 0 : (plan.bpp == 3 || ct == JPGB_RGBA || ct == JPGB_BGRA) ? 2 : 3);
+    uint64_t last = 0, t = 0;
+    bool over = __builtin_mul_overflow((uint64_t)(n - 1), im.image_stride, &last);
+    over |= __builtin_mul_overflow(c_max, im.plane_stride, &t) || __builtin_add_overflow(last, t, &last);
+    over |= __builtin_mul_overflow(h - 1, im.row_stride, &t) || __builtin_add_overflow(last, t, &last);
+    over |= __builtin_add_overflow(last, row_bytes - 1, &last);
+    over |= __builtin_add_overflow((uint64_t)(uintptr_t)im.data, last, &t);
+    if (over) return fail(enc, JPGB_ERR_BAD_PARAMS, "the described pixels extend beyond 64-bit addresses");
+    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    cudaPointerAttributes attr{};
+    const bool known = cudaPointerGetAttributes(&attr, im.data) == cudaSuccess;
+    cudaGetLastError();
+    if (!known || !(attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == enc->device)))
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "data is not device or managed memory of the context's device");
+    MemGetAddressRangeFn range = mem_get_address_range_fn();
+    CUdeviceptr base = 0;
+    size_t size = 0;
+    if (!range || range(&base, &size, (CUdeviceptr)(uintptr_t)im.data) != CUDA_SUCCESS)
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "no allocation is found at data");
+    const uint64_t end = (uint64_t)(uintptr_t)im.data + last; // the last byte read
+    if (end >= (uint64_t)base + size) {
+        snprintf(m, sizeof(m), "the described pixels end %llu bytes past the end of the allocation that holds data",
+                 (unsigned long long)(end + 1 - ((uint64_t)base + size)));
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
     return JPGB_OK;
 }
 
@@ -494,11 +554,40 @@ GraphKey graph_key(const jpgb_encoder *enc, const PlanSig &sig, const EntropyBuf
     return k;
 }
 
+// Packed pixels, rows back to back, images `image_stride` apart; the ImageBuffer planes of a planar plan (one byte per
+// sample) back to back
+jpgb_device_images contiguous_images(const Plan &plan, const void *d_pixels, uint64_t image_stride) {
+    const uint64_t row = (uint64_t)plan.p.width * (plan.planar ? 1 : plan.bpp);
+    return {d_pixels, image_stride, row, plan.planar ? row * plan.p.height : 0};
+}
+
+// Where stage A finds the pixels (jpgb_device_images, include/jpegenc_b200.h). Channel-planar pixels of a packed
+// ColorType are staged by the kernels with byte k of a pixel taken from plane plane_of[k]: Bgr, Rgba and Bgra are the
+// Rgb kernels with their R, G, B planes in that order (the alpha plane is not read).
+void set_pixel_layout(StageAParams &ap, const Plan &plan, const jpgb_device_images &im) {
+    ap.pixels = static_cast<const uint8_t *>(im.data);
+    ap.image_stride = im.image_stride;
+    ap.row_stride = im.row_stride;
+    if (plan.planar) {
+        ap.plane_stride = im.plane_stride;
+    } else if (im.plane_stride && plan.ncomp > 1) {
+        const uint8_t ct = plan.p.color_type;
+        const bool bgr = ct == JPGB_BGR || ct == JPGB_BGRA;
+        ap.channel_planar = 1;
+        ap.plane_stride = im.plane_stride;
+        for (int k = 0; k < 4; ++k) ap.plane_of[k] = (bgr && k < 3) ? 2 - k : k;
+        if (ct == JPGB_BGR || ct == JPGB_RGBA || ct == JPGB_BGRA) {
+            ap.color_type = JPGB_RGB;
+            ap.bpp = 3;
+        }
+    }
+}
+
 // The whole device pipeline for `n` device-resident images. On success the files lie back to back
 // in `out` and `offsets` (host, n + 1) delimits them.
 // `given_hist` (strips with optimized tables): the symbol histogram of the *whole* image, [table][dc|ac][257],
 // used instead of the one of these pixels.
-int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, size_t image_stride, uint32_t n, DevBuf &out,
+int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images &images, uint32_t n, DevBuf &out,
                   std::vector<uint64_t> &offsets, std::vector<uint64_t> *piece_offsets = nullptr, const uint32_t *given_hist = nullptr,
                   bool coef_ready = false) {
     cudaStream_t st = enc->stream;
@@ -514,9 +603,8 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const uint8_t *d_pixels, 
         enc->coef_tagged = false;
         StageAParams ap;
         plan.fill_stage_a(ap);
-        ap.pixels = d_pixels;
+        set_pixel_layout(ap, plan, images);
         ap.coef = enc->coef.as<int16_t>();
-        ap.image_stride = image_stride;
         StageTimer t(enc, 0);
         CK(launch_stage_a(ap, n, st), "stage A launch");
         enc->launches += 1;
@@ -720,7 +808,7 @@ int encode_host_pipelined(jpgb_encoder *enc, const Plan &plan, const uint8_t *co
             enc->launches += 1;
         }
         std::vector<uint64_t> off;
-        const int rc = encode_device(enc, plan, enc->pixels.as<uint8_t>(), stride, 1, enc->out, off, nullptr, nullptr, true);
+        const int rc = encode_device(enc, plan, contiguous_images(plan, enc->pixels.p, stride), 1, enc->out, off, nullptr, nullptr, true);
         if (rc != JPGB_OK) return rc;
         CK(enc->h_out.reserve(std::max<size_t>(off[1], 1 << 20)), "alloc pinned output");
         CK(cudaMemcpyAsync(enc->h_out.p, enc->out.p, off[1], cudaMemcpyDeviceToHost, st), "download file");
@@ -756,7 +844,7 @@ int encode_host_pipelined(jpgb_encoder *enc, const Plan &plan, const uint8_t *co
         CK(cudaStreamWaitEvent(st, enc->ev_in[c & 1], 0), "wait upload");
         if (c >= 2) CK(cudaStreamWaitEvent(st, enc->ev_out[c & 1], 0), "wait download"); // out slot reused
         std::vector<uint64_t> off;
-        const int rc = encode_device(enc, plan, px.as<uint8_t>(), stride, cn, ob, off);
+        const int rc = encode_device(enc, plan, contiguous_images(plan, px.p, stride), cn, ob, off);
         if (rc != JPGB_OK) return rc;
         CK(cudaEventRecord(enc->ev_enc[c & 1], st), "record encode");
         const uint64_t bytes = off[cn];
@@ -859,6 +947,7 @@ int jpgb_encoder_create(int device, void *cuda_stream, jpgb_encoder **out) {
         cudaEventCreateWithFlags(&e->ev_enc[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&e->ev_stage[i], cudaEventDisableTiming);
     }
+    cudaEventCreateWithFlags(&e->ev_wait, cudaEventDisableTiming);
     *out = e;
     return JPGB_OK;
 }
@@ -876,6 +965,7 @@ void jpgb_encoder_destroy(jpgb_encoder *e) {
         if (e->ev_enc[i]) cudaEventDestroy(e->ev_enc[i]);
         if (e->ev_stage[i]) cudaEventDestroy(e->ev_stage[i]);
     }
+    if (e->ev_wait) cudaEventDestroy(e->ev_wait);
     for (int i = 0; i < JPGB_N_STAGES; ++i)
         for (int k = 0; k < 2; ++k)
             if (e->ev[i][k]) cudaEventDestroy(e->ev[i][k]);
@@ -916,7 +1006,7 @@ static int encode_planar_pinned(jpgb_encoder *enc, const jpgb_params *p, const u
         CK(upload_host(enc, enc->pixels.as<uint8_t>() + plane_bytes * c, planes[c], plane_bytes, enc->stream), "upload plane");
     }
     std::vector<uint64_t> off;
-    const int rc2 = encode_device(enc, plan, enc->pixels.as<uint8_t>(), stride, 1, enc->out, off);
+    const int rc2 = encode_device(enc, plan, contiguous_images(plan, enc->pixels.p, stride), 1, enc->out, off);
     if (rc2 != JPGB_OK) return rc2;
     const size_t sz = (size_t)off[1];
     CK(enc->h_out.reserve(sz ? sz : 1), "alloc pinned output");
@@ -991,11 +1081,43 @@ int jpgb_encode_batch_device(jpgb_encoder *enc, const jpgb_params *p, const void
     CK(cudaSetDevice(enc->device), "cudaSetDevice");
     timing_begin(enc);
     std::vector<uint64_t> off;
-    rc = encode_device(enc, plan, static_cast<const uint8_t *>(d_pixels), image_stride, n, enc->out, off);
+    rc = encode_device(enc, plan, contiguous_images(plan, d_pixels, image_stride), n, enc->out, off);
     if (rc != JPGB_OK) return rc;
     timing_end(enc);
     std::memcpy(offsets, off.data(), (size_t)(n + 1) * 8);
     *d_files = enc->out.p;
+    return JPGB_OK;
+}
+
+int jpgb_encode_batch_device_strided(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_images *images, uint32_t n,
+                                     const void **d_files, uint64_t *offsets) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    enc->launches = 0; // a rejected call reports no launches
+    if (!images || !images->data || !d_files || !offsets || n == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
+    Plan plan;
+    int rc = validate_and_plan(enc, p, SIZE_MAX, plan); // a strided layout has no length to check
+    if (rc != JPGB_OK) return rc;
+    rc = check_device_images(enc, plan, *images, n);
+    if (rc != JPGB_OK) return rc;
+    // Ycbcr and Ycck planes are the ImageBuffer planes: samples taken verbatim, one plane per component
+    plan.planar = images->plane_stride != 0 && (p->color_type == JPGB_YCBCR || p->color_type == JPGB_YCCK);
+    timing_begin(enc);
+    std::vector<uint64_t> off;
+    rc = encode_device(enc, plan, *images, n, enc->out, off);
+    if (rc != JPGB_OK) return rc;
+    timing_end(enc);
+    std::memcpy(offsets, off.data(), (size_t)(n + 1) * 8);
+    *d_files = enc->out.p;
+    return JPGB_OK;
+}
+
+int jpgb_encoder_wait_stream(jpgb_encoder *enc, void *stream) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (s == enc->stream) return JPGB_OK;
+    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    CK(cudaEventRecord(enc->ev_wait, s), "record the caller's stream");
+    CK(cudaStreamWaitEvent(enc->stream, enc->ev_wait, 0), "wait for the caller's stream");
     return JPGB_OK;
 }
 
@@ -1061,7 +1183,7 @@ static int encode_strip(jpgb_encoder *enc, const jpgb_params *p, const jpgb_stri
         const PlanSig sig = plan_sig(plan);
         reuse = std::memcmp(&sig, &enc->coef_sig, sizeof(sig)) == 0;
     }
-    const int rc2 = encode_device(enc, plan, static_cast<const uint8_t *>(d_pixels), stride, 1, enc->out, off, &pieces, hist_total, reuse);
+    const int rc2 = encode_device(enc, plan, contiguous_images(plan, d_pixels, stride), 1, enc->out, off, &pieces, hist_total, reuse);
     enc->coef_tagged = false;
     if (rc2 != JPGB_OK) return rc2;
     timing_end(enc);

@@ -54,6 +54,11 @@ struct StageAParams {
     int n_images;
     int planar;            // 1: pixels = ncomp full-resolution planes of width*height bytes (plane_stride apart)
     unsigned long long plane_stride;
+    unsigned long long row_stride; // bytes between pixel rows (of a plane when planar / channel_planar)
+    // 1: the packed ColorType's pixels come as planes, byte k of a pixel from plane plane_of[k] (plane_stride apart);
+    // the kernels interleave them while staging
+    int channel_planar;
+    int plane_of[4];
     int use_fast;          // 1: stage_a_warp_kernel / stage_a_plane_kernel, 0: stage_a_kernel
     // Coefficient layout (DESIGN.md section 3). mcu_order = 1 (interleaved scan): blocks in the order the scan codes
     // them, block = (mcu * bpu + slot). mcu_order = 0: per component the raster of its TRUE grid (comp_tw x comp_th,

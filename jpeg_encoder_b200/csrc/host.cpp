@@ -604,6 +604,7 @@ void Plan::fill_stage_a(StageAParams &a) const {
     a.planar = planar ? 1 : 0;
     a.plane_stride = (unsigned long long)p.width * p.height;
     if (planar) a.bpp = 1;
+    a.row_stride = (unsigned long long)p.width * a.bpp;
     for (int t = 0; t < 2; ++t)
         for (int i = 0; i < 64; ++i) {
             const int32_t c = q[t].corr[i] * q[t].recip[i];

@@ -158,6 +158,18 @@ __device__ __noinline__ void stage_edge_chunk(uint8_t *dst, const uint8_t *row, 
     }
 }
 
+// The same chunk of packed pixels gathered from channel planes: byte ch of a pixel comes from plane plane_of[ch].
+// `row` is the row's first pixel in plane 0.
+template <int BPP>
+__device__ __noinline__ void stage_planes_chunk(uint8_t *dst, const uint8_t *row, unsigned long long plane_stride, const int *plane_of,
+                                                int cb, int valid_px) {
+    for (int b = 0; b < 16; ++b) {
+        const int byte = cb + b;
+        const int px = byte / BPP, ch = byte - px * BPP;
+        dst[cb + b] = row[(size_t)plane_of[ch] * plane_stride + min(px, valid_px - 1)];
+    }
+}
+
 template <int CT>
 __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ StageAParams p) {
     extern __shared__ __align__(128) uint8_t tile[];
@@ -168,7 +180,7 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
     const int mcu_x0 = tile_x * 32 * p.groups;
     const int px0 = mcu_x0 * 8 * p.hmax, py0 = mcu_y * 8 * p.vmax;
     const uint8_t *src = p.pixels + (size_t)img * p.image_stride;
-    const size_t row_bytes = (size_t)p.width * BPP;
+    const int px_bytes = p.channel_planar ? 1 : BPP; // bytes of one pixel in one input row
 
     // ---- stage the tile: 16-byte chunks, edges replicated (Q4) ----
     const int chunks_per_row = p.tile_pitch / 16;
@@ -181,9 +193,10 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
         const int plane = c / n_chunks, cc = c - plane * n_chunks;
         const int ry = cc / chunks_per_row, cb = (cc - ry * chunks_per_row) * 16;
         const int sy = min(py0 + ry, p.height - 1);
-        const uint8_t *row = src + (size_t)plane * p.plane_stride + (size_t)sy * row_bytes + (size_t)px0 * BPP;
+        const uint8_t *row = src + (size_t)plane * p.plane_stride + (size_t)sy * p.row_stride + (size_t)px0 * px_bytes;
         uint8_t *dst = tile + plane * plane_tile + ry * p.tile_pitch;
-        if (cb + 16 <= valid_bytes && ((reinterpret_cast<uintptr_t>(row + cb) & 15) == 0))
+        if (p.channel_planar) stage_planes_chunk<BPP>(dst, row, p.plane_stride, p.plane_of, cb, valid_px);
+        else if (cb + 16 <= valid_bytes && ((reinterpret_cast<uintptr_t>(row + cb) & 15) == 0))
             *reinterpret_cast<uint4 *>(dst + cb) = __ldg(reinterpret_cast<const uint4 *>(row + cb));
         else stage_edge_chunk<BPP>(dst, row, cb, valid_px);
     }
@@ -406,13 +419,84 @@ __device__ __forceinline__ void load_words(const uint8_t *row, uint32_t (&w)[NW]
     }
 }
 
+// ---- channel-planar tiles ([plane][rows][256]): the same pixel words, interleaved from one word per plane ----
+// Byte t of packed word M is byte (4M + t) % BPP (the channel) of pixel (4M + t) / BPP. It is taken from word
+// pixel / 4 of that channel's plane. A packed word draws on at most four plane words: one PRMT merges the first
+// two, one more each further source.
+struct WordSrc {
+    int n, ch[4], j[4], sel[3];
+};
+template <int BPP>
+__host__ __device__ constexpr WordSrc word_src(int m) {
+    WordSrc r{};
+    int src[4] = {}, byte[4] = {};
+    for (int t = 0; t < 4; ++t) {
+        const int q = (4 * m + t) / BPP, ch = (4 * m + t) % BPP, j = q >> 2;
+        int k = 0;
+        while (k < r.n && !(r.ch[k] == ch && r.j[k] == j)) ++k;
+        if (k == r.n) r.ch[r.n] = ch, r.j[r.n] = j, ++r.n;
+        src[t] = k;
+        byte[t] = q & 3;
+    }
+    for (int t = 0; t < 4; ++t) {
+        r.sel[0] |= (src[t] == 0 ? byte[t] : (src[t] == 1 ? 4 + byte[t] : 0)) << (4 * t);
+        r.sel[1] |= (src[t] == 2 ? 4 + byte[t] : t) << (4 * t);
+        r.sel[2] |= (src[t] == 3 ? 4 + byte[t] : t) << (4 * t);
+    }
+    return r;
+}
+template <int BPP, int M, int NPW>
+__device__ __forceinline__ uint32_t packed_word(const uint32_t (&pw)[BPP][NPW]) {
+    constexpr WordSrc s = word_src<BPP>(M);
+    static_assert(s.j[0] < NPW && s.j[1] < NPW && s.j[2] < NPW && s.j[3] < NPW, "pixels of the block row");
+    uint32_t acc = __byte_perm(pw[s.ch[0]][s.j[0]], pw[s.ch[1]][s.j[1]], s.sel[0]);
+    if constexpr (s.n > 2) acc = __byte_perm(acc, pw[s.ch[2]][s.j[2]], s.sel[1]);
+    if constexpr (s.n > 3) acc = __byte_perm(acc, pw[s.ch[3]][s.j[3]], s.sel[2]);
+    return acc;
+}
+template <int BPP, int SX, int NW, int NPW, int... Ms>
+__device__ __forceinline__ void interleave_words(const uint32_t (&pw)[BPP][NPW], uint32_t (&w)[NW], std::integer_sequence<int, Ms...>) {
+    ((w[Ms] = (BPP == 4 && SX > 1 && Ms % SX) ? 0u : packed_word<BPP, Ms, NPW>(pw)), ...); // the words load_words leaves 0
+}
+// load_words for a channel-planar tile: `row` is the block row's first pixel in tile plane 0, plane offsets in `choff`
+// (byte k of a pixel lies choff[k] further). A block row starts at a multiple of 8 * SX pixels.
+template <int BPP, int SX, int NW>
+__device__ __forceinline__ void load_words_planes(const uint8_t *row, const int *choff, uint32_t (&w)[NW]) {
+    constexpr int NPW = 2 * SX; // words of one plane under the 8 * SX pixels
+    uint32_t pw[BPP][NPW];
+#pragma unroll
+    for (int k = 0; k < BPP; ++k) {
+        if constexpr (SX == 1) {
+            const uint2 a = *reinterpret_cast<const uint2 *>(row + choff[k]);
+            pw[k][0] = a.x;
+            pw[k][1] = a.y;
+        } else {
+#pragma unroll
+            for (int i = 0; i < NPW / 4; ++i) {
+                const uint4 a = reinterpret_cast<const uint4 *>(row + choff[k])[i];
+                pw[k][4 * i] = a.x;
+                pw[k][4 * i + 1] = a.y;
+                pw[k][4 * i + 2] = a.z;
+                pw[k][4 * i + 3] = a.w;
+            }
+        }
+    }
+    interleave_words<BPP, SX, NW, NPW>(pw, w, std::make_integer_sequence<int, NW>{});
+}
+template <int BPP, int SX, bool PL, int NW>
+__device__ __forceinline__ void load_tile_words(const uint8_t *row, const int *choff, uint32_t (&w)[NW]) {
+    if constexpr (PL) load_words_planes<BPP, SX>(row, choff, w);
+    else load_words<BPP, SX>(row, w);
+}
+
 // 8 samples (unshifted, 0..255) of one block row. `row` points at the first pixel of the row in the
 // shared tile; the pixels used are 0, SX, 2*SX, ... (point decimation, encoder.rs:1222-1242).
-template <int CT, int ROLE, int SX>
-__device__ __forceinline__ void load_row(const uint8_t *row, int *s, const ChromaConsts *cc = nullptr) {
+// PL: a channel-planar tile, plane offsets in `choff`.
+template <int CT, int ROLE, int SX, bool PL = false>
+__device__ __forceinline__ void load_row(const uint8_t *row, int *s, const ChromaConsts *cc = nullptr, const int *choff = nullptr) {
     constexpr int NW = row_words<Fmt<CT>::BPP, SX>();
     uint32_t w[NW];
-    load_words<Fmt<CT>::BPP, SX>(row, w);
+    load_tile_words<Fmt<CT>::BPP, SX, PL>(row, choff, w);
     if constexpr (ROLE == ROLE_CBCR) chroma_row<CT, SX, NW>(w, s, *cc, std::make_integer_sequence<int, 8>{});
     else sample_row<CT, ROLE, SX, NW>(w, s, std::make_integer_sequence<int, 8>{});
 }
@@ -430,23 +514,25 @@ template <int BPP, int SX, int NW, int... Is>
 __device__ __forceinline__ void byte_row(const uint32_t (&w)[NW], int *s, unsigned coff, unsigned xorv, std::integer_sequence<int, Is...>) {
     ((s[Is] = byte_at<BPP, SX, Is, NW>(w, coff, xorv)), ...);
 }
-template <int BPP, int SX>
-__device__ __forceinline__ void load_row_bytes(const uint8_t *row, int *s, unsigned coff, unsigned xorv) {
+template <int BPP, int SX, bool PL>
+__device__ __forceinline__ void load_row_bytes(const uint8_t *row, int *s, unsigned coff, unsigned xorv, const int *choff) {
     constexpr int NW = row_words<BPP, SX>();
     uint32_t w[NW];
-    load_words<BPP, SX>(row, w);
+    load_tile_words<BPP, SX, PL>(row, choff, w);
     byte_row<BPP, SX, NW>(w, s, coff, xorv, std::make_integer_sequence<int, 8>{});
 }
-template <int BPP, int SX, int SY>
-__device__ __forceinline__ void load_block_bytes(const uint8_t *base, int pitch, int (&v)[64], unsigned coff, unsigned xorv) {
+template <int BPP, int SX, int SY, bool PL = false>
+__device__ __forceinline__ void load_block_bytes(const uint8_t *base, int pitch, int (&v)[64], unsigned coff, unsigned xorv,
+                                                 const int *choff = nullptr) {
 #pragma unroll
-    for (int y = 0; y < 8; ++y) load_row_bytes<BPP, SX>(base + y * SY * pitch, &v[y * 8], coff, xorv);
+    for (int y = 0; y < 8; ++y) load_row_bytes<BPP, SX, PL>(base + y * SY * pitch, &v[y * 8], coff, xorv, choff);
 }
 
-template <int CT, int ROLE, int SX, int SY>
-__device__ __forceinline__ void load_block(const uint8_t *base, int pitch, int (&v)[64], const ChromaConsts *cc = nullptr) {
+template <int CT, int ROLE, int SX, int SY, bool PL = false>
+__device__ __forceinline__ void load_block(const uint8_t *base, int pitch, int (&v)[64], const ChromaConsts *cc = nullptr,
+                                           const int *choff = nullptr) {
 #pragma unroll
-    for (int y = 0; y < 8; ++y) load_row<CT, ROLE, SX>(base + y * SY * pitch, &v[y * 8], cc);
+    for (int y = 0; y < 8; ++y) load_row<CT, ROLE, SX, PL>(base + y * SY * pitch, &v[y * 8], cc, choff);
 }
 
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
@@ -480,6 +566,13 @@ __device__ __forceinline__ void tma_load_3d(void *smem_dst, const CUtensorMap *m
                  ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(map), "r"((unsigned)__cvta_generic_to_shared(bar)), "r"(x), "r"(y), "r"(z)
                  : "memory");
 }
+// the same for a 4-D box (x in 4-byte elements, y in rows, z = plane, w = image)
+__device__ __forceinline__ void tma_load_4d(void *smem_dst, const CUtensorMap *map, uint64_t *bar, int x, int y, int z, int w) {
+    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
+                 ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(map), "r"((unsigned)__cvta_generic_to_shared(bar)), "r"(x), "r"(y), "r"(z),
+                 "r"(w)
+                 : "memory");
+}
 
 // MCU rows per warp tile: formats whose one-MCU-row tile is small (grayscale: 2 KB, one task) take several
 // rows per tile so that the staging and bookkeeping are amortised over more blocks.
@@ -495,8 +588,11 @@ __host__ __device__ constexpr int warp_tile_mcu_rows() {
 // __syncwarp only, then run its tasks -- the luma (and K) block rows and one chroma task in which
 // lanes 0..15 take Cb and lanes 16..31 Cr when chroma is horizontally decimated. No CTA barrier, no
 // role imbalance between warps; the other resident warps hide a warp's load latency.
+// PL (channel-planar input, p.channel_planar): the tile holds the BPP planes read, [plane][ROWS][256] in the planes'
+// memory order -- the same bytes per tile -- and the row loader interleaves them into the packed pixel words, so the
+// arithmetic behind it is the packed kernel's. Byte k of a pixel comes from tile plane p.plane_of[k].
 // =================================================================================================
-template <int CT, int HS, int VS>
+template <int CT, int HS, int VS, bool PL>
 __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_constant__ StageAParams p,
                                                               const __grid_constant__ CUtensorMap tmap, const int use_tma) {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -507,8 +603,9 @@ __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_const
     constexpr int MR = warp_tile_mcu_rows<CT, HS, VS>(); // MCU rows per warp tile (small tiles take several)
     constexpr int MROWS = 8 * VS;               // pixel rows of one MCU row
     constexpr int ROWS = MROWS * MR;
-    constexpr int PITCH = 256 * BPP;            // 32 full-resolution blocks wide
-    constexpr int TILE_BYTES = PITCH * ROWS;
+    constexpr int PXB = PL ? 1 : BPP;           // bytes of a pixel in one tile row
+    constexpr int PITCH = 256 * PXB;            // 32 full-resolution blocks wide
+    constexpr int TILE_BYTES = 256 * BPP * ROWS;
     constexpr int MCUS = 32 / HS;               // MCUs per warp tile
     // tasks of one warp tile: luma rows, [K rows], then chroma
     constexpr int N_FULL = Fmt<CT>::NFULL * VS;
@@ -538,21 +635,65 @@ __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_const
     const unsigned tiles_per_row = ((unsigned)p.mcu_cols + MCUS - 1) / MCUS;
     const unsigned tile_rows = ((unsigned)p.mcu_rows + MR - 1) / MR;
     const unsigned n_tiles = tiles_per_row * tile_rows * p.n_images;
-    const size_t row_bytes = (size_t)p.width * BPP;
+    const size_t row_stride = p.row_stride;
+    int choff[4] = {0, 0, 0, 0}; // PL: offset of the tile plane that byte k of a pixel comes from
+    if constexpr (PL)
+#pragma unroll
+        for (int k = 0; k < BPP; ++k) choff[k] = p.plane_of[k] * (PITCH * ROWS);
 
     for (unsigned t = warp_global; t < n_tiles; t += n_warps_total) {
         const unsigned tx = t % tiles_per_row, r = t / tiles_per_row;
         const int mcu_y0 = (int)(r % tile_rows) * MR, img = (int)(r / tile_rows);
         const int mcu_x0 = (int)tx * MCUS;
         // ---- stage this warp's rows (cp.async, L2 only); edges replicated (Q4) ----
-        {
+        if constexpr (PL) {
+            const int px0 = mcu_x0 * 8 * HS, py0 = mcu_y0 * MROWS;
+            const uint8_t *src = p.pixels + (size_t)img * p.image_stride + px0; // plane 0
+            const int valid_px = min(256, p.width - px0);
+            const int needed_px = min(256, p.mcu_cols * 8 * HS - px0);
+            __syncwarp(); // all lanes are done reading the previous tile
+            const bool interior = px0 + 256 <= p.width && py0 + ROWS <= p.height && ((row_stride | p.plane_stride) & 15) == 0 &&
+                                  (reinterpret_cast<uintptr_t>(src) & 15) == 0;
+            if (interior && use_tma) { // one 4-D box: 256 px x ROWS rows x BPP planes
+                if (lane == 0) {
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    mbar_expect_tx(bar, TILE_BYTES);
+                    tma_load_4d(tile, &tmap, bar, px0 / 4, py0, 0, img);
+                }
+                mbar_wait(bar, phase);
+                phase ^= 1;
+            } else if (interior) { // half a warp per 256-byte plane row
+#pragma unroll 4
+                for (int i = lane >> 4; i < BPP * ROWS; i += 2) {
+                    const int k = i / ROWS, ry = i - k * ROWS;
+                    cp_async16(tile + i * PITCH + (lane & 15) * 16, src + (size_t)k * p.plane_stride + (size_t)(py0 + ry) * row_stride + (lane & 15) * 16);
+                }
+            } else {
+#pragma unroll 1
+                for (int i = 0; i < BPP * ROWS; ++i) {
+                    const int k = i / ROWS, ry = i - k * ROWS;
+                    const int sy = min(py0 + ry, p.height - 1);
+                    const uint8_t *row = src + (size_t)k * p.plane_stride + (size_t)sy * row_stride;
+                    uint8_t *dst = tile + i * PITCH;
+                    const bool aligned = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
+                    const int cb = lane * 16;
+                    if (cb < needed_px) {
+                        if (aligned && cb + 16 <= valid_px) cp_async16(dst + cb, row + cb);
+                        else stage_edge_chunk<1>(dst, row, cb, valid_px);
+                    }
+                }
+            }
+            cp_async_commit();
+            cp_async_wait<0>();
+            __syncwarp();
+        } else {
             const int px0 = mcu_x0 * 8 * HS, py0 = mcu_y0 * MROWS;
             const uint8_t *src = p.pixels + (size_t)img * p.image_stride;
             const int valid_px = min(256, p.width - px0);
             const int valid_bytes = valid_px * BPP;
             const int needed_bytes = min(256, p.mcu_cols * 8 * HS - px0) * BPP;
             __syncwarp(); // all lanes are done reading the previous tile
-            const bool interior = px0 + 256 <= p.width && py0 + ROWS <= p.height && (row_bytes & 15) == 0 &&
+            const bool interior = px0 + 256 <= p.width && py0 + ROWS <= p.height && (row_stride & 15) == 0 &&
                                   ((reinterpret_cast<uintptr_t>(src) + (size_t)px0 * BPP) & 15) == 0;
             if (interior && use_tma) {
                 // One TMA box per tile (UTMALDG): a single lane issues it, the tensor unit streams the
@@ -566,21 +707,21 @@ __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_const
                 phase ^= 1;
             } else if (interior) {
                 // whole tile inside the image and 16-byte aligned: every lane copies its fixed chunks of each row
-                const uint8_t *g = src + (size_t)py0 * row_bytes + (size_t)px0 * BPP + lane * 16;
+                const uint8_t *g = src + (size_t)py0 * row_stride + (size_t)px0 * BPP + lane * 16;
                 uint8_t *d = tile + lane * 16;
 #pragma unroll 4
                 for (int ry = 0; ry < ROWS; ++ry) {
 #pragma unroll
                     for (int c = 0; c < (PITCH + 511) / 512; ++c)
                         if (c * 512 + 512 <= PITCH || lane * 16 + c * 512 < PITCH) cp_async16(d + c * 512, g + c * 512);
-                    g += row_bytes;
+                    g += row_stride;
                     d += PITCH;
                 }
             } else {
 #pragma unroll 1
                 for (int ry = 0; ry < ROWS; ++ry) {
                     const int sy = min(py0 + ry, p.height - 1);
-                    const uint8_t *row = src + (size_t)sy * row_bytes + (size_t)px0 * BPP;
+                    const uint8_t *row = src + (size_t)sy * row_stride + (size_t)px0 * BPP;
                     uint8_t *dst = tile + ry * PITCH;
                     const bool aligned = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
 #pragma unroll 1
@@ -621,24 +762,24 @@ __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_const
             // blocks of the MCU padding exist only in the MCU-ordered layout (the interleaved scan codes them)
             const int gy = mcu_y + p.mcu_row0; // MCU row inside the whole image (this launch may cover a slice of it)
             if (p.mcu_order ? bx >= p.comp_pw[comp] : (bx >= p.comp_tw[comp] || gy * V + bv >= p.comp_th[comp])) continue;
-            const uint8_t *base = full ? mtile + (bv * 8) * PITCH + bxl * 8 * BPP : mtile + bxl * 8 * HS * BPP;
+            const uint8_t *base = full ? mtile + (bv * 8) * PITCH + bxl * 8 * PXB : mtile + bxl * 8 * HS * PXB;
 
             int v[64];
             if constexpr (CT == JPGB_LUMA) {
                 load_block<CT, ROLE_RAW, 1, 1>(base, PITCH, v);
             } else if constexpr (BYTES) {
                 const unsigned xorv = CT == JPGB_CMYK ? 0xFFu : 0u; // 255 - c, image_buffer.rs:247-256
-                if (full) load_block_bytes<BPP, 1, 1>(base, PITCH, v, (unsigned)comp, xorv);
-                else load_block_bytes<BPP, HS, VS>(base, PITCH, v, (unsigned)comp, xorv);
+                if (full) load_block_bytes<BPP, 1, 1, PL>(base, PITCH, v, (unsigned)comp, xorv, choff);
+                else load_block_bytes<BPP, HS, VS, PL>(base, PITCH, v, (unsigned)comp, xorv, choff);
             } else if constexpr (PAIRED) {
-                if (task >= N_FULL) load_block<CT, ROLE_CBCR, HS, VS>(base, PITCH, v, &cc); // lanes 0..15 Cb, 16..31 Cr
-                else if (comp == 0) load_block<CT, ROLE_Y, 1, 1>(base, PITCH, v);
-                else load_block<CT, ROLE_K, 1, 1>(base, PITCH, v);
+                if (task >= N_FULL) load_block<CT, ROLE_CBCR, HS, VS, PL>(base, PITCH, v, &cc, choff); // lanes 0..15 Cb, 16..31 Cr
+                else if (comp == 0) load_block<CT, ROLE_Y, 1, 1, PL>(base, PITCH, v, nullptr, choff);
+                else load_block<CT, ROLE_K, 1, 1, PL>(base, PITCH, v, nullptr, choff);
             } else {
-                if (comp == 0) load_block<CT, ROLE_Y, 1, 1>(base, PITCH, v);
-                else if (comp == 1) load_block<CT, ROLE_CB, SUB ? HS : 1, SUB ? VS : 1>(base, PITCH, v);
-                else if (NCOMP == 3 || comp == 2) load_block<CT, ROLE_CR, SUB ? HS : 1, SUB ? VS : 1>(base, PITCH, v);
-                else load_block<CT, ROLE_K, 1, 1>(base, PITCH, v);
+                if (comp == 0) load_block<CT, ROLE_Y, 1, 1, PL>(base, PITCH, v, nullptr, choff);
+                else if (comp == 1) load_block<CT, ROLE_CB, SUB ? HS : 1, SUB ? VS : 1, PL>(base, PITCH, v, nullptr, choff);
+                else if (NCOMP == 3 || comp == 2) load_block<CT, ROLE_CR, SUB ? HS : 1, SUB ? VS : 1, PL>(base, PITCH, v, nullptr, choff);
+                else load_block<CT, ROLE_K, 1, 1, PL>(base, PITCH, v, nullptr, choff);
             }
             dct_2d(v);
 
@@ -693,24 +834,24 @@ __global__ void __launch_bounds__(128, 4) stage_a_plane_kernel(const __grid_cons
         const int valid_px = min(PITCH, p.width - px0);
         const int needed_bytes = min(PITCH, needed_total - px0);
         __syncwarp(); // all lanes are done reading the previous tile
-        const bool interior = px0 + PITCH <= p.width && py0 + (ROWS - 1) * SY < p.height && (p.width & 15) == 0 &&
+        const bool interior = px0 + PITCH <= p.width && py0 + (ROWS - 1) * SY < p.height && (p.row_stride & 15) == 0 &&
                               ((reinterpret_cast<uintptr_t>(src) + (size_t)px0) & 15) == 0;
         if (interior) {
-            const uint8_t *g = src + (size_t)py0 * p.width + px0 + lane * 16;
+            const uint8_t *g = src + (size_t)py0 * p.row_stride + px0 + lane * 16;
             uint8_t *d = tile + lane * 16;
 #pragma unroll 4
             for (int ry = 0; ry < ROWS; ++ry) {
 #pragma unroll
                 for (int c = 0; c < (PITCH + 511) / 512; ++c)
                     if (c * 512 + 512 <= PITCH || lane * 16 + c * 512 < PITCH) cp_async16(d + c * 512, g + c * 512);
-                g += (size_t)SY * p.width;
+                g += (size_t)SY * p.row_stride;
                 d += PITCH;
             }
         } else {
 #pragma unroll 1
             for (int ry = 0; ry < ROWS; ++ry) {
                 const int sy = min(py0 + ry * SY, p.height - 1);
-                const uint8_t *row = src + (size_t)sy * p.width + px0;
+                const uint8_t *row = src + (size_t)sy * p.row_stride + px0;
                 uint8_t *dst = tile + ry * PITCH;
                 const bool aligned = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
 #pragma unroll 1
@@ -760,55 +901,83 @@ inline EncodeTiledFn encode_tiled_fn() {
     return fn;
 }
 
+// The image stride a tensor map is given: the caller's, or for a single image one that cannot matter (every box has
+// image coordinate 0). 0: no map (several images at the same address).
+inline unsigned long long tma_image_stride(const StageAParams &p) {
+    if (p.image_stride || p.n_images > 1) return p.image_stride;
+    return (unsigned long long)p.height * p.row_stride;
+}
+
 // Tensor map of the packed pixels as a 3-D tensor of 4-byte elements: (row bytes / 4, rows, images), box =
 // one warp tile. Needs 16-byte aligned base, row pitch and image pitch; otherwise the kernel stages with cp.async.
+// The extent of a row ends at its last pixel: boxes never reach into the pitch.
 inline bool make_pixel_tensor_map(CUtensorMap &map, const StageAParams &p, int bpp, int pitch_bytes, int rows) {
-    const unsigned long long row_bytes = (unsigned long long)p.width * bpp;
+    const unsigned long long row_bytes = (unsigned long long)p.width * bpp, image_stride = tma_image_stride(p);
     if (std::getenv("JPGB_NO_TMA")) return false;
-    if ((reinterpret_cast<uintptr_t>(p.pixels) & 15) || (row_bytes & 15) || (p.image_stride & 15) || p.width < 256 || p.height < rows) return false;
+    if ((reinterpret_cast<uintptr_t>(p.pixels) & 15) || (p.row_stride & 15) || (image_stride & 15) || !image_stride || p.width < 256 ||
+        p.height < rows)
+        return false;
     EncodeTiledFn fn = encode_tiled_fn();
     if (!fn) return false;
     const cuuint64_t dims[3] = {row_bytes / 4, (cuuint64_t)p.height, (cuuint64_t)p.n_images};
-    const cuuint64_t strides[2] = {row_bytes, p.image_stride};
+    const cuuint64_t strides[2] = {p.row_stride, image_stride};
     const cuuint32_t box[3] = {(cuuint32_t)(pitch_bytes / 4), (cuuint32_t)rows, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
     return fn(&map, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t *>(p.pixels), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int CT, int HS, int VS>
+// Channel-planar pixels as a 4-D tensor of 4-byte elements: (width / 4, rows, planes, images), box = one warp tile of
+// the `planes` planes read (the first ones in memory order). Needs width % 16 == 0 and 16-byte aligned base and strides.
+inline bool make_plane_tensor_map(CUtensorMap &map, const StageAParams &p, int planes, int rows) {
+    const unsigned long long image_stride = tma_image_stride(p);
+    if (std::getenv("JPGB_NO_TMA")) return false;
+    if ((reinterpret_cast<uintptr_t>(p.pixels) & 15) || (p.row_stride & 15) || (p.plane_stride & 15) || (image_stride & 15) || !image_stride ||
+        (p.width & 15) || p.width < 256 || p.height < rows)
+        return false;
+    EncodeTiledFn fn = encode_tiled_fn();
+    if (!fn) return false;
+    const cuuint64_t dims[4] = {(cuuint64_t)p.width / 4, (cuuint64_t)p.height, (cuuint64_t)planes, (cuuint64_t)p.n_images};
+    const cuuint64_t strides[3] = {p.row_stride, p.plane_stride, image_stride};
+    const cuuint32_t box[4] = {64, (cuuint32_t)rows, (cuuint32_t)planes, 1};
+    const cuuint32_t estr[4] = {1, 1, 1, 1};
+    return fn(&map, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, const_cast<uint8_t *>(p.pixels), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+              CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+template <int CT, int HS, int VS, bool PL>
 cudaError_t launch_warp_variant(const StageAParams &p, cudaStream_t stream) {
     constexpr int BPP = Fmt<CT>::BPP;
     constexpr int MR = warp_tile_mcu_rows<CT, HS, VS>();
     constexpr int TILE = 256 * BPP * 8 * VS * MR;
     constexpr size_t smem = (size_t)4 * TILE + 4 * sizeof(uint64_t); // 4 warps per CTA: one private tile and one mbarrier each
     unsigned long long grid = 0;
-    const cudaError_t e = resident_ctas<stage_a_warp_kernel<CT, HS, VS>>(128, smem, grid);
+    const cudaError_t e = resident_ctas<stage_a_warp_kernel<CT, HS, VS, PL>>(128, smem, grid);
     if (e != cudaSuccess) return e;
     constexpr int MCUS = 32 / HS;
     const unsigned long long n_tiles = (unsigned long long)((p.mcu_cols + MCUS - 1) / MCUS) * ((p.mcu_rows + MR - 1) / MR) * p.n_images;
     if (grid * 4 > n_tiles) grid = (n_tiles + 3) / 4;
     CUtensorMap tmap;
     std::memset(&tmap, 0, sizeof(tmap));
-    const int use_tma = make_pixel_tensor_map(tmap, p, BPP, 256 * BPP, 8 * VS * MR) ? 1 : 0;
-    stage_a_warp_kernel<CT, HS, VS><<<(unsigned)grid, 128, smem, stream>>>(p, tmap, use_tma);
+    const bool tma = PL ? make_plane_tensor_map(tmap, p, BPP, 8 * VS * MR) : make_pixel_tensor_map(tmap, p, BPP, 256 * BPP, 8 * VS * MR);
+    stage_a_warp_kernel<CT, HS, VS, PL><<<(unsigned)grid, 128, smem, stream>>>(p, tmap, tma ? 1 : 0);
     return cudaGetLastError();
 }
 
 // the warp kernel instantiated for the luma sampling factors (a single component is always sampled 1x1)
-template <int CT>
+template <int CT, bool PL>
 cudaError_t launch_warp(const StageAParams &p, cudaStream_t stream) {
     if constexpr (Fmt<CT>::NCOMP == 1) {
-        return launch_warp_variant<CT, 1, 1>(p, stream);
+        return launch_warp_variant<CT, 1, 1, PL>(p, stream);
     } else {
-        if (p.hmax == 1 && p.vmax == 1) return launch_warp_variant<CT, 1, 1>(p, stream);
-        if (p.hmax == 2 && p.vmax == 1) return launch_warp_variant<CT, 2, 1>(p, stream);
-        if (p.hmax == 1 && p.vmax == 2) return launch_warp_variant<CT, 1, 2>(p, stream);
-        if (p.hmax == 2 && p.vmax == 2) return launch_warp_variant<CT, 2, 2>(p, stream);
-        if (p.hmax == 4 && p.vmax == 1) return launch_warp_variant<CT, 4, 1>(p, stream);
-        if (p.hmax == 4 && p.vmax == 2) return launch_warp_variant<CT, 4, 2>(p, stream);
-        if (p.hmax == 1 && p.vmax == 4) return launch_warp_variant<CT, 1, 4>(p, stream);
-        return launch_warp_variant<CT, 2, 4>(p, stream);
+        if (p.hmax == 1 && p.vmax == 1) return launch_warp_variant<CT, 1, 1, PL>(p, stream);
+        if (p.hmax == 2 && p.vmax == 1) return launch_warp_variant<CT, 2, 1, PL>(p, stream);
+        if (p.hmax == 1 && p.vmax == 2) return launch_warp_variant<CT, 1, 2, PL>(p, stream);
+        if (p.hmax == 2 && p.vmax == 2) return launch_warp_variant<CT, 2, 2, PL>(p, stream);
+        if (p.hmax == 4 && p.vmax == 1) return launch_warp_variant<CT, 4, 1, PL>(p, stream);
+        if (p.hmax == 4 && p.vmax == 2) return launch_warp_variant<CT, 4, 2, PL>(p, stream);
+        if (p.hmax == 1 && p.vmax == 4) return launch_warp_variant<CT, 1, 4, PL>(p, stream);
+        return launch_warp_variant<CT, 2, 4, PL>(p, stream);
     }
 }
 
@@ -879,10 +1048,15 @@ cudaError_t launch_generic(StageAParams p, cudaStream_t stream) {
     return cudaGetLastError();
 }
 
-// packed pixels: the warp kernel, or the generic one when JPGB_FORCE_GENERIC_STAGE_A asks for the cross-check
+// packed pixels: the warp kernel, or the generic one when JPGB_FORCE_GENERIC_STAGE_A asks for the cross-check.
+// Channel-planar pixels take the warp kernel's planar staging, instantiated for Rgb (Bgr, Rgba and Bgra are Rgb with
+// their planes in another order), Cmyk and CmykAsYcck.
 template <int CT>
 cudaError_t launch_packed(const StageAParams &p, cudaStream_t stream) {
-    return p.use_fast ? launch_warp<CT>(p, stream) : launch_generic<CT>(p, stream);
+    if (!p.use_fast) return launch_generic<CT>(p, stream);
+    if (!p.channel_planar) return launch_warp<CT, false>(p, stream);
+    if constexpr (CT == JPGB_RGB || CT == JPGB_CMYK || CT == JPGB_CMYK_AS_YCCK) return launch_warp<CT, true>(p, stream);
+    return cudaErrorInvalidValue;
 }
 
 } // namespace

@@ -156,6 +156,10 @@ class _Strip(C.Structure):
                 ("full_height", C.c_uint16)]
 
 
+class _DeviceImages(C.Structure):
+    _fields_ = [("data", C.c_void_p), ("image_stride", C.c_uint64), ("row_stride", C.c_uint64), ("plane_stride", C.c_uint64)]
+
+
 N_STAGES = 7
 HIST_WORDS = 2 * 2 * 257  # JPGB_HIST_WORDS
 STAGE_NAMES = ("colour_dct_quant", "histogram_tables", "code_chunks_scans", "place_chunks", "stuff_scatter", "h2d", "d2h")
@@ -192,6 +196,9 @@ def load_library():
                                            C.POINTER(vp), C.POINTER(C.c_uint64)]
     l.jpgb_encode_batch_device.argtypes = [vp, C.POINTER(_Params), vp, C.c_size_t, C.c_uint32,
                                            C.POINTER(vp), C.POINTER(C.c_uint64)]
+    l.jpgb_encode_batch_device_strided.argtypes = [vp, C.POINTER(_Params), C.POINTER(_DeviceImages), C.c_uint32,
+                                                   C.POINTER(vp), C.POINTER(C.c_uint64)]
+    l.jpgb_encoder_wait_stream.argtypes = [vp, vp]
     l.jpgb_scan_count.argtypes = [C.POINTER(_Params), C.POINTER(C.c_uint32)]
     l.jpgb_plan_strips.argtypes = [C.POINTER(_Params), C.c_uint32, C.POINTER(_Strip), C.POINTER(C.c_uint32)]
     l.jpgb_encode_strip_device.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Strip), vp, C.POINTER(vp), C.POINTER(C.c_uint64)]
@@ -267,6 +274,13 @@ class Device:
     def last_launch_count(self):
         return int(self.lib.jpgb_encoder_last_launch_count(self.handle))
 
+    def wait_stream(self, stream):
+        """Order this context's stream after the work queued so far on `stream` (a cudaStream_t as an int; 1 is the
+        legacy default stream, 2 the per-thread one). The host does not block."""
+        rc = self.lib.jpgb_encoder_wait_stream(self.handle, C.c_void_p(stream))
+        if rc != 0:
+            raise EncodingError(rc, self.last_error())
+
 
 _default_devices = {}
 
@@ -284,6 +298,52 @@ def _host_view(data):
             a = a.astype(np.uint8)
         return a.reshape(-1)
     return np.frombuffer(data, dtype=np.uint8)
+
+
+def _cuda_array_layout(iface, bpp, channels_first):
+    """The jpgb_device_images of a `__cuda_array_interface__` dict holding uint8 images:
+    (data, n, width, height, image_stride, row_stride, plane_stride). Shapes: (H, W, C) / (N, H, W, C), or with
+    channels_first (C, H, W) / (N, C, H, W); C must be the colour type's bytes per pixel. Raises ValueError for a
+    layout the encoder cannot read in place."""
+    if iface.get("typestr") != "|u1":
+        raise ValueError("uint8 images only (typestr '|u1'), got %r" % (iface.get("typestr"),))
+    if iface.get("mask") is not None:
+        raise ValueError("masked arrays are not supported")
+    shape = tuple(int(d) for d in iface["shape"])
+    if len(shape) not in (3, 4):
+        raise ValueError("expected a 3-D (one image) or 4-D (batch) array, got shape %r" % (shape,))
+    strides = iface.get("strides")
+    if strides is None:  # C-contiguous
+        strides, step = [], 1
+        for d in reversed(shape):
+            strides.insert(0, step)
+            step *= d
+    strides = tuple(int(x) for x in strides)
+    names = ("c", "y", "x") if channels_first else ("y", "x", "c")
+    if len(shape) == 4:
+        names = ("n",) + names
+    for name, st in zip(names, strides):
+        if st < 0:
+            raise ValueError("negative %s stride %d: make the array .contiguous() first" % (name, st))
+    dim = dict(zip(names, shape))
+    stride = dict(zip(names, strides))
+    if dim["c"] != bpp:
+        raise ValueError("the colour type takes %d channels, the array has %d" % (bpp, dim["c"]))
+    if channels_first:
+        if stride["x"] != 1:
+            raise ValueError("x stride %d: channel-planar rows must be contiguous; make the array .contiguous() first" % stride["x"])
+        plane_stride = stride["c"] if bpp > 1 else 0  # one plane is packed Luma
+        if bpp > 1 and plane_stride == 0:
+            raise ValueError("channel stride 0: planes at one address cannot be read; make the array .contiguous() first")
+    else:
+        if stride["c"] != 1:
+            raise ValueError("channel stride %d: channels must be adjacent; make the array .contiguous() first" % stride["c"])
+        if stride["x"] != bpp:
+            raise ValueError("pixel stride %d: pixels must be %d bytes apart; make the array .contiguous() first" % (stride["x"], bpp))
+        plane_stride = 0
+    if dim["x"] > 65535 or dim["y"] > 65535:
+        raise ValueError("image dimensions above 65535 (%d x %d)" % (dim["x"], dim["y"]))
+    return (int(iface["data"][0]), dim.get("n", 1), dim["x"], dim["y"], stride.get("n", 0), stride["y"], plane_stride)
 
 
 class Encoder:
@@ -509,6 +569,31 @@ class Encoder:
         if rc != 0:
             self._raise(rc)
         return d_files.value, list(offs)
+
+    def encode_batch_device_strided(self, d_ptr, n, width, height, color_type, image_stride, row_stride, plane_stride=0):
+        """Device images in any row pitch, packed (plane_stride 0) or channel-planar (jpgb_device_images,
+        include/jpegenc_b200.h): returns (device pointer of the files, offsets[n+1]), like encode_batch_device."""
+        dev = self._dev()
+        p = self._params(width, height, ColorType(color_type))
+        im = _DeviceImages(d_ptr, image_stride, row_stride, plane_stride)
+        d_files = C.c_void_p()
+        offs = (C.c_uint64 * (n + 1))()
+        rc = dev.lib.jpgb_encode_batch_device_strided(dev.handle, C.byref(p), C.byref(im), n, C.byref(d_files), offs)
+        if rc != 0:
+            self._raise(rc)
+        return d_files.value, list(offs)
+
+    def encode_cuda_array(self, arr, color_type, channels_first=False):
+        """Encode uint8 device images where they lie: any object with `__cuda_array_interface__` (a torch CUDA tensor,
+        CuPy, Numba) shaped (H, W, C) / (N, H, W, C), or (C, H, W) / (N, C, H, W) with channels_first. Crops and other
+        views with a row pitch need no copy. When the interface names a stream, the encode waits for it first.
+        Returns (device pointer of the files, offsets[n+1]), like encode_batch_device."""
+        ct = ColorType(color_type)
+        iface = arr.__cuda_array_interface__
+        ptr, n, w, h, image_stride, row_stride, plane_stride = _cuda_array_layout(iface, ct.get_bytes_per_pixel(), channels_first)
+        if iface.get("stream") is not None:
+            self._dev().wait_stream(int(iface["stream"]))
+        return self.encode_batch_device_strided(ptr, n, w, h, ct, image_stride, row_stride, plane_stride)
 
     # -- one large image cut into restart-aligned strips (BASELINE config 5) --
     def scan_count(self, width, height, color_type):
