@@ -100,6 +100,18 @@ inline PlanSig plan_sig(const Plan &plan) {
     s.planar = plan.planar;
     return s;
 }
+// Whose coefficients the context's `coef` holds, set by jpgb_strip_histogram_device and dropped by every write of
+// `coef`: the optimized strip encode that follows on the same strip and pixels does not run the colour+DCT kernel again
+struct CoefTag {
+    bool set = false;
+    PlanSig sig{};
+    const void *pixels = nullptr;
+    uint64_t stride = 0;
+    float ms[2] = {0.f, 0.f}; // with timing on: what the colour+DCT kernel and the histogram of that call took (added to the reusing call's stages)
+    bool matches(const PlanSig &s, const void *px, uint64_t st) const {
+        return set && pixels == px && stride == st && std::memcmp(&s, &sig, sizeof(s)) == 0;
+    }
+};
 struct CapKey {
     PlanSig sig;
     uint64_t raw_bytes;
@@ -193,13 +205,7 @@ struct jpgb_encoder {
     bool have_timing = false;
     uint32_t launches = 0;
     uint32_t last_piece_scans = 0; // scans of the last strip encode (its piece offsets are in piece_off)
-    // whose coefficients `coef` holds (set by jpgb_strip_histogram_device, cleared by every other call that writes `coef`):
-    // the optimized strip encode that follows on the same strip and pixels does not run the colour+DCT kernel again
-    bool coef_tagged = false;
-    PlanSig coef_sig{};
-    const void *coef_pixels = nullptr;
-    uint64_t coef_stride = 0;
-    float coef_ms[2] = {0.f, 0.f}; // with timing on: what the colour+DCT kernel and the histogram of that call took (added to the reusing call's stages)
+    CoefTag coef_tag;
     GraphCache graphs;
     // Capacities are sticky per (settings, batch size): steady-state calls provision exactly what the last successful
     // call settled on, so the launch sequence has identical parameters call after call and is replayed as a CUDA graph.
@@ -254,6 +260,14 @@ void timing_end(jpgb_encoder *enc) {
     enc->have_timing = true;
 }
 
+// Plan::build, with the message of a failure: for a strip, that its settings or geometry do not allow strips
+int build_plan(jpgb_encoder *enc, const jpgb_params &p, Plan &plan, const jpgb_strip *strip = nullptr) {
+    const int rc = plan.build(p, strip);
+    if (rc == JPGB_OK) return rc;
+    if (strip) return fail(enc, rc, "settings or strip geometry do not allow strip encoding (needs restart intervals aligned in every scan)");
+    return fail(enc, rc, rc == JPGB_ERR_ZERO_DIMENSIONS ? "Image dimensions must be non zero" : "invalid parameters");
+}
+
 int validate_and_plan(jpgb_encoder *enc, const jpgb_params *p, size_t len_each, Plan &plan) {
     if (!p) return fail(enc, JPGB_ERR_BAD_PARAMS, "null params");
     if (p->color_type > JPGB_YCCK) return fail(enc, JPGB_ERR_BAD_PARAMS, "bad color_type");
@@ -263,9 +277,7 @@ int validate_and_plan(jpgb_encoder *enc, const jpgb_params *p, size_t len_each, 
         snprintf(m, sizeof(m), "Image data too small for dimensions and color_type: %zu need at least %zu", len_each, required);
         return fail(enc, JPGB_ERR_BAD_IMAGE_DATA, m);
     }
-    const int rc = plan.build(*p);
-    if (rc != JPGB_OK) return fail(enc, rc, rc == JPGB_ERR_ZERO_DIMENSIONS ? "Image dimensions must be non zero" : "invalid parameters");
-    return JPGB_OK;
+    return build_plan(enc, *p, plan);
 }
 
 typedef CUresult (*MemGetAddressRangeFn)(CUdeviceptr *, size_t *, CUdeviceptr);
@@ -561,26 +573,21 @@ jpgb_device_images contiguous_images(const Plan &plan, const void *d_pixels, uin
     return {d_pixels, image_stride, row, plan.planar ? row * plan.p.height : 0};
 }
 
-// Where stage A finds the pixels (jpgb_device_images, include/jpegenc_b200.h). Channel-planar pixels of a packed
-// ColorType are staged by the kernels with byte k of a pixel taken from plane plane_of[k]: Bgr, Rgba and Bgra are the
-// Rgb kernels with their R, G, B planes in that order (the alpha plane is not read).
-void set_pixel_layout(StageAParams &ap, const Plan &plan, const jpgb_device_images &im) {
-    ap.pixels = static_cast<const uint8_t *>(im.data);
-    ap.image_stride = im.image_stride;
-    ap.row_stride = im.row_stride;
-    if (plan.planar) {
-        ap.plane_stride = im.plane_stride;
-    } else if (im.plane_stride && plan.ncomp > 1) {
-        const uint8_t ct = plan.p.color_type;
-        const bool bgr = ct == JPGB_BGR || ct == JPGB_BGRA;
-        ap.channel_planar = 1;
-        ap.plane_stride = im.plane_stride;
-        for (int k = 0; k < 4; ++k) ap.plane_of[k] = (bgr && k < 3) ? 2 - k : k;
-        if (ct == JPGB_BGR || ct == JPGB_RGBA || ct == JPGB_BGRA) {
-            ap.color_type = JPGB_RGB;
-            ap.bpp = 3;
-        }
-    }
+// The context's coefficient buffer for `n` images, about to be written by stage A. The tag is dropped before the
+// buffer is reserved: a failed reserve frees the buffer, and no later call may take it for the tagged coefficients.
+int stage_a_coef(jpgb_encoder *enc, const Plan &plan, uint32_t n, int16_t *&coef) {
+    enc->coef_tag.set = false;
+    CK(enc->coef.reserve(plan.blocks_per_image * n * 128), "alloc coefficients");
+    coef = enc->coef.as<int16_t>();
+    return JPGB_OK;
+}
+
+// Every colour+DCT launch of a context: timed as stage 0 and counted
+int run_stage_a(jpgb_encoder *enc, const StageAParams &ap, uint32_t n) {
+    StageTimer t(enc, 0);
+    CK(launch_stage_a(ap, n, enc->stream), "stage A launch");
+    enc->launches += 1;
+    return JPGB_OK;
 }
 
 // The whole device pipeline for `n` device-resident images. On success the files lie back to back
@@ -597,21 +604,18 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
     const uint64_t n_segs = (uint64_t)plan.segs_per_image * n;
     const uint64_t n_chunks = (uint64_t)plan.chunks_per_image * n;
 
-    CK(enc->coef.reserve(plan.blocks_per_image * n * 128), "alloc coefficients");
-    // ---- stage A (unless the caller has already run it slice by slice behind the upload) ----
+    // ---- stage A (unless the caller has already run it: slice by slice behind the upload, or for a strip histogram) ----
+    int rc;
     if (!coef_ready) {
-        enc->coef_tagged = false;
+        int16_t *coef = nullptr;
+        if ((rc = stage_a_coef(enc, plan, n, coef)) != JPGB_OK) return rc;
         StageAParams ap;
-        plan.fill_stage_a(ap);
-        set_pixel_layout(ap, plan, images);
-        ap.coef = enc->coef.as<int16_t>();
-        StageTimer t(enc, 0);
-        CK(launch_stage_a(ap, n, st), "stage A launch");
-        enc->launches += 1;
+        plan.fill_stage_a(ap, images, coef);
+        if ((rc = run_stage_a(enc, ap, n)) != JPGB_OK) return rc;
     }
 
     HeaderLayout hl;
-    int rc = setup_header(enc, plan, n, given_hist, hl);
+    rc = setup_header(enc, plan, n, given_hist, hl);
     if (rc != JPGB_OK) return rc;
 
     // ---- entropy coding: chunks -> pool, two small prefix sums, placement, stuffing ----
@@ -753,6 +757,59 @@ cudaError_t upload_host(jpgb_encoder *enc, void *d_dst, const uint8_t *src, size
     return cudaSuccess;
 }
 
+// The one file in enc->out -> the context's pinned output buffer h_out
+int download_file(jpgb_encoder *enc, size_t bytes) {
+    CK(enc->h_out.reserve(std::max<size_t>(bytes, 1)), "alloc pinned output");
+    CK(cudaMemcpyAsync(enc->h_out.p, enc->out.p, bytes, cudaMemcpyDeviceToHost, enc->stream), "download file");
+    CK(cudaStreamSynchronize(enc->stream), "download sync");
+    return JPGB_OK;
+}
+
+// One large image: the upload dominates (3 B/pixel over PCIe against ~1 ms of device work), so the image is cut into
+// slices of whole MCU rows and the colour+DCT kernel runs on slice k while slice k + 1 is still on the link.
+// On success the file is h_out[0 .. offsets[1]).
+int encode_host_sliced(jpgb_encoder *enc, const Plan &plan, const uint8_t *pixels, std::vector<uint64_t> &offsets) {
+    const size_t row_bytes = (size_t)plan.p.width * plan.bpp;
+    const size_t stride = (row_bytes * plan.p.height + 255) & ~(size_t)255;
+    const uint32_t mcu_px = 8 * plan.vmax;
+    uint32_t rows_per_slice = (uint32_t)std::max<size_t>(1, (32u << 20) / (row_bytes * mcu_px)); // in MCU rows, ~32 MB
+    rows_per_slice = (rows_per_slice + 3) & ~3u; // whole warp tiles (up to four MCU rows each)
+    const uint32_t n_slices = (plan.mcu_rows + rows_per_slice - 1) / rows_per_slice;
+    CK(enc->pixels.reserve(stride), "alloc pixels");
+    int16_t *coef = nullptr;
+    int rc = stage_a_coef(enc, plan, 1, coef);
+    if (rc != JPGB_OK) return rc;
+    while (enc->ev_slice.size() < n_slices) {
+        cudaEvent_t e;
+        CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming), "create event");
+        enc->ev_slice.push_back(e);
+    }
+    const jpgb_device_images im = contiguous_images(plan, enc->pixels.p, stride);
+    StageAParams ap;
+    plan.fill_stage_a(ap, im, coef);
+    for (uint32_t k = 0; k < n_slices; ++k) { // all uploads are queued first: the link never idles
+        const size_t r0 = (size_t)k * rows_per_slice * mcu_px, r1 = std::min<size_t>(plan.p.height, r0 + (size_t)rows_per_slice * mcu_px);
+        CK(upload_host(enc, enc->pixels.as<uint8_t>() + r0 * row_bytes, pixels + r0 * row_bytes, (r1 - r0) * row_bytes, enc->s_h2d), "upload slice");
+        CK(cudaEventRecord(enc->ev_slice[k], enc->s_h2d), "record slice");
+    }
+    for (uint32_t k = 0; k < n_slices; ++k) {
+        const size_t r0 = (size_t)k * rows_per_slice * mcu_px, r1 = std::min<size_t>(plan.p.height, r0 + (size_t)rows_per_slice * mcu_px);
+        StageAParams sp = ap;
+        sp.pixels = ap.pixels + r0 * row_bytes;
+        sp.height = (int)(r1 - r0);
+        sp.mcu_row0 = (int)(k * rows_per_slice);
+        sp.mcu_rows = (int)std::min<uint32_t>(rows_per_slice, plan.mcu_rows - k * rows_per_slice);
+        CK(cudaStreamWaitEvent(enc->stream, enc->ev_slice[k], 0), "wait slice");
+        rc = run_stage_a(enc, sp, 1);
+        if (rc != JPGB_OK) return rc;
+    }
+    std::vector<uint64_t> off;
+    rc = encode_device(enc, plan, im, 1, enc->out, off, nullptr, nullptr, true);
+    if (rc != JPGB_OK) return rc;
+    offsets = {0, off[1]};
+    return download_file(enc, off[1]);
+}
+
 // Host pixels -> host files for n images, pipelined in chunks over three streams: while chunk c is
 // encoded on the context's stream, chunk c+1 is uploaded (s_h2d) and the files of chunk c-1 are
 // downloaded (s_d2h) into one pinned buffer owned by the context. PCIe moves 3 B/pixel in and the
@@ -770,52 +827,6 @@ int encode_host_pipelined(jpgb_encoder *enc, const Plan &plan, const uint8_t *co
     CK(enc->h_out.reserve(std::max<size_t>(img_bytes * n / 3, 1 << 20)), "alloc pinned output");
     offsets.assign(1, 0);
     cudaStream_t st = enc->stream;
-
-    // One large image: the upload dominates (3 B/pixel over PCIe against ~1 ms of device work), so the image is cut into
-    // slices of whole MCU rows and the colour+DCT kernel runs on slice k while slice k + 1 is still on the link.
-    if (n == 1 && !plan.planar && img_bytes >= (48u << 20)) {
-        const size_t row_bytes = (size_t)plan.p.width * plan.bpp;
-        const uint32_t mcu_px = 8 * plan.vmax;
-        uint32_t rows_per_slice = (uint32_t)std::max<size_t>(1, (32u << 20) / (row_bytes * mcu_px)); // in MCU rows, ~32 MB
-        rows_per_slice = (rows_per_slice + 3) & ~3u; // whole warp tiles (up to four MCU rows each)
-        const uint32_t n_slices = (plan.mcu_rows + rows_per_slice - 1) / rows_per_slice;
-        CK(enc->pixels.reserve(stride), "alloc pixels");
-        CK(enc->coef.reserve(plan.blocks_per_image * 128), "alloc coefficients");
-        enc->coef_tagged = false;
-        while (enc->ev_slice.size() < n_slices) {
-            cudaEvent_t e;
-            CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming), "create event");
-            enc->ev_slice.push_back(e);
-        }
-        StageAParams ap;
-        plan.fill_stage_a(ap);
-        for (uint32_t k = 0; k < n_slices; ++k) { // all uploads are queued first: the link never idles
-            const size_t r0 = (size_t)k * rows_per_slice * mcu_px, r1 = std::min<size_t>(plan.p.height, r0 + (size_t)rows_per_slice * mcu_px);
-            CK(upload_host(enc, enc->pixels.as<uint8_t>() + r0 * row_bytes, pixels[0] + r0 * row_bytes, (r1 - r0) * row_bytes, enc->s_h2d), "upload slice");
-            CK(cudaEventRecord(enc->ev_slice[k], enc->s_h2d), "record slice");
-        }
-        for (uint32_t k = 0; k < n_slices; ++k) {
-            const size_t r0 = (size_t)k * rows_per_slice * mcu_px, r1 = std::min<size_t>(plan.p.height, r0 + (size_t)rows_per_slice * mcu_px);
-            StageAParams sp = ap;
-            sp.pixels = enc->pixels.as<uint8_t>() + r0 * row_bytes;
-            sp.coef = enc->coef.as<int16_t>();
-            sp.image_stride = stride;
-            sp.height = (int)(r1 - r0);
-            sp.mcu_row0 = (int)(k * rows_per_slice);
-            sp.mcu_rows = (int)std::min<uint32_t>(rows_per_slice, plan.mcu_rows - k * rows_per_slice);
-            CK(cudaStreamWaitEvent(st, enc->ev_slice[k], 0), "wait slice");
-            CK(launch_stage_a(sp, 1, st), "stage A launch");
-            enc->launches += 1;
-        }
-        std::vector<uint64_t> off;
-        const int rc = encode_device(enc, plan, contiguous_images(plan, enc->pixels.p, stride), 1, enc->out, off, nullptr, nullptr, true);
-        if (rc != JPGB_OK) return rc;
-        CK(enc->h_out.reserve(std::max<size_t>(off[1], 1 << 20)), "alloc pinned output");
-        CK(cudaMemcpyAsync(enc->h_out.p, enc->out.p, off[1], cudaMemcpyDeviceToHost, st), "download file");
-        CK(cudaStreamSynchronize(st), "download sync");
-        offsets.push_back(off[1]);
-        return JPGB_OK;
-    }
 
     auto upload = [&](uint32_t c) -> cudaError_t {
         DevBuf &px = (c & 1) ? enc->pixels2 : enc->pixels;
@@ -883,7 +894,8 @@ int encode_host_batch(jpgb_encoder *enc, const jpgb_params *p, const uint8_t *co
     enc->timing = false; // per-stage events are per encode_device call; the pipelined path runs several
     timing_begin(enc);
     std::vector<uint64_t> off;
-    rc = encode_host_pipelined(enc, plan, pixels, n, off);
+    const bool one_large = n == 1 && !plan.planar && (size_t)plan.p.width * plan.p.height * plan.bpp >= (48u << 20);
+    rc = one_large ? encode_host_sliced(enc, plan, pixels[0], off) : encode_host_pipelined(enc, plan, pixels, n, off);
     enc->timing = was_timing;
     if (rc != JPGB_OK) return rc;
     if (pinned_api) {
@@ -901,6 +913,29 @@ int encode_host_batch(jpgb_encoder *enc, const jpgb_params *p, const uint8_t *co
         out_lens[i] = sz;
         std::memcpy(outs[i], enc->h_out.as<uint8_t>() + off[i], sz);
     }
+    return JPGB_OK;
+}
+
+// jpgb_encode_batch_device[_strided] after their checks: the files stay in enc->out
+int encode_batch_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images &images, uint32_t n, const void **d_files,
+                        uint64_t *offsets) {
+    timing_begin(enc);
+    std::vector<uint64_t> off;
+    const int rc = encode_device(enc, plan, images, n, enc->out, off);
+    if (rc != JPGB_OK) return rc;
+    timing_end(enc);
+    std::memcpy(offsets, off.data(), (size_t)(n + 1) * 8);
+    *d_files = enc->out.p;
+    return JPGB_OK;
+}
+
+// The strip entries after their own argument checks: the strip's plan, the device, and the strip's pixels (packed
+// rows back to back) at d_pixels
+int plan_strip(jpgb_encoder *enc, const jpgb_params &p, const jpgb_strip &strip, const void *d_pixels, Plan &plan, jpgb_device_images &im) {
+    const int rc = build_plan(enc, p, plan, &strip);
+    if (rc != JPGB_OK) return rc;
+    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    im = contiguous_images(plan, d_pixels, (uint64_t)plan.p.width * plan.p.height * plan.bpp); // p.height: the strip's rows
     return JPGB_OK;
 }
 
@@ -995,8 +1030,8 @@ static int encode_planar_pinned(jpgb_encoder *enc, const jpgb_params *p, const u
     if (plane_len < plane_bytes) return fail(enc, JPGB_ERR_BAD_IMAGE_DATA, "plane shorter than width*height");
     Plan plan;
     plan.planar = true;
-    const int rc = plan.build(*p);
-    if (rc != JPGB_OK) return fail(enc, rc, rc == JPGB_ERR_ZERO_DIMENSIONS ? "Image dimensions must be non zero" : "invalid parameters");
+    int rc = build_plan(enc, *p, plan);
+    if (rc != JPGB_OK) return rc;
     CK(cudaSetDevice(enc->device), "cudaSetDevice");
     timing_begin(enc);
     const size_t stride = (plane_bytes * plan.ncomp + 255) & ~(size_t)255;
@@ -1006,13 +1041,11 @@ static int encode_planar_pinned(jpgb_encoder *enc, const jpgb_params *p, const u
         CK(upload_host(enc, enc->pixels.as<uint8_t>() + plane_bytes * c, planes[c], plane_bytes, enc->stream), "upload plane");
     }
     std::vector<uint64_t> off;
-    const int rc2 = encode_device(enc, plan, contiguous_images(plan, enc->pixels.p, stride), 1, enc->out, off);
-    if (rc2 != JPGB_OK) return rc2;
-    const size_t sz = (size_t)off[1];
-    CK(enc->h_out.reserve(sz ? sz : 1), "alloc pinned output");
-    CK(cudaMemcpyAsync(enc->h_out.p, enc->out.p, sz, cudaMemcpyDeviceToHost, enc->stream), "download file");
-    CK(cudaStreamSynchronize(enc->stream), "download sync");
-    *out_len = sz;
+    rc = encode_device(enc, plan, contiguous_images(plan, enc->pixels.p, stride), 1, enc->out, off);
+    if (rc != JPGB_OK) return rc;
+    rc = download_file(enc, off[1]);
+    if (rc != JPGB_OK) return rc;
+    *out_len = off[1];
     timing_end(enc);
     return JPGB_OK;
 }
@@ -1076,17 +1109,10 @@ int jpgb_encode_batch_device(jpgb_encoder *enc, const jpgb_params *p, const void
     if (!enc) return JPGB_ERR_BAD_PARAMS;
     if (!d_pixels || !d_files || !offsets || n == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
     Plan plan;
-    int rc = validate_and_plan(enc, p, image_stride, plan);
+    const int rc = validate_and_plan(enc, p, image_stride, plan);
     if (rc != JPGB_OK) return rc;
     CK(cudaSetDevice(enc->device), "cudaSetDevice");
-    timing_begin(enc);
-    std::vector<uint64_t> off;
-    rc = encode_device(enc, plan, contiguous_images(plan, d_pixels, image_stride), n, enc->out, off);
-    if (rc != JPGB_OK) return rc;
-    timing_end(enc);
-    std::memcpy(offsets, off.data(), (size_t)(n + 1) * 8);
-    *d_files = enc->out.p;
-    return JPGB_OK;
+    return encode_batch_device(enc, plan, contiguous_images(plan, d_pixels, image_stride), n, d_files, offsets);
 }
 
 int jpgb_encode_batch_device_strided(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_images *images, uint32_t n,
@@ -1101,14 +1127,7 @@ int jpgb_encode_batch_device_strided(jpgb_encoder *enc, const jpgb_params *p, co
     if (rc != JPGB_OK) return rc;
     // Ycbcr and Ycck planes are the ImageBuffer planes: samples taken verbatim, one plane per component
     plan.planar = images->plane_stride != 0 && (p->color_type == JPGB_YCBCR || p->color_type == JPGB_YCCK);
-    timing_begin(enc);
-    std::vector<uint64_t> off;
-    rc = encode_device(enc, plan, *images, n, enc->out, off);
-    if (rc != JPGB_OK) return rc;
-    timing_end(enc);
-    std::memcpy(offsets, off.data(), (size_t)(n + 1) * 8);
-    *d_files = enc->out.p;
-    return JPGB_OK;
+    return encode_batch_device(enc, plan, *images, n, d_files, offsets);
 }
 
 int jpgb_encoder_wait_stream(jpgb_encoder *enc, void *stream) {
@@ -1172,24 +1191,19 @@ static int encode_strip(jpgb_encoder *enc, const jpgb_params *p, const jpgb_stri
     if ((p->optimize_huffman != 0) != (hist_total != nullptr))
         return fail(enc, JPGB_ERR_BAD_PARAMS, "optimized tables with strips take the whole image's histogram (jpgb_encode_strip_device_optimized); other settings take none");
     Plan plan;
-    const int rc = plan.build(*p, strip);
-    if (rc != JPGB_OK) return fail(enc, rc, "settings or strip geometry do not allow strip encoding (needs restart intervals aligned in every scan)");
-    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    jpgb_device_images im;
+    int rc = plan_strip(enc, *p, *strip, d_pixels, plan, im);
+    if (rc != JPGB_OK) return rc;
     timing_begin(enc);
+    const bool reuse = hist_total && enc->coef_tag.matches(plan_sig(plan), d_pixels, im.image_stride);
+    enc->coef_tag.set = false; // a tag is used at most once
     std::vector<uint64_t> off, pieces;
-    const size_t stride = (size_t)p->width * strip->rows * bytes_per_pixel(p->color_type);
-    bool reuse = false;
-    if (hist_total && enc->coef_tagged && enc->coef_pixels == d_pixels && enc->coef_stride == uint64_t(stride)) {
-        const PlanSig sig = plan_sig(plan);
-        reuse = std::memcmp(&sig, &enc->coef_sig, sizeof(sig)) == 0;
-    }
-    const int rc2 = encode_device(enc, plan, contiguous_images(plan, d_pixels, stride), 1, enc->out, off, &pieces, hist_total, reuse);
-    enc->coef_tagged = false;
-    if (rc2 != JPGB_OK) return rc2;
+    rc = encode_device(enc, plan, im, 1, enc->out, off, &pieces, hist_total, reuse);
+    if (rc != JPGB_OK) return rc;
     timing_end(enc);
     if (reuse && enc->timing) { // the stages that ran in the histogram call belong to this strip's encode
-        enc->last_ms[0] += enc->coef_ms[0];
-        enc->last_ms[1] += enc->coef_ms[1];
+        enc->last_ms[0] += enc->coef_tag.ms[0];
+        enc->last_ms[1] += enc->coef_tag.ms[1];
     }
     std::memcpy(piece_offsets, pieces.data(), pieces.size() * 8);
     *d_bytes = enc->out.p;
@@ -1213,32 +1227,29 @@ int jpgb_strip_histogram_device(jpgb_encoder *enc, const jpgb_params *p, const j
     if (!p || !strip || !d_pixels || !hist || !edge_dc) return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
     if (p->color_type > JPGB_YCCK || !p->optimize_huffman) return fail(enc, JPGB_ERR_BAD_PARAMS, "strip histograms belong to optimized Huffman tables");
     Plan plan;
-    const int rc = plan.build(*p, strip);
-    if (rc != JPGB_OK) return fail(enc, rc, "settings or strip geometry do not allow strip encoding (needs restart intervals aligned in every scan)");
-    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    jpgb_device_images im;
+    int rc = plan_strip(enc, *p, *strip, d_pixels, plan, im);
+    if (rc != JPGB_OK) return rc;
     cudaStream_t st = enc->stream;
     DevPlan hp;
     plan.fill_device_plan(hp);
+    int16_t *coef = nullptr;
+    rc = stage_a_coef(enc, plan, 1, coef);
+    if (rc != JPGB_OK) return rc;
     StageAParams ap;
-    plan.fill_stage_a(ap);
-    CK(enc->coef.reserve(plan.blocks_per_image * 128), "alloc coefficients");
-    ap.pixels = static_cast<const uint8_t *>(d_pixels);
-    ap.coef = enc->coef.as<int16_t>();
-    ap.image_stride = (size_t)p->width * strip->rows * bytes_per_pixel(p->color_type);
+    plan.fill_stage_a(ap, im, coef);
     timing_begin(enc);
-    {
-        StageTimer t(enc, 0);
-        CK(launch_stage_a(ap, 1, st), "stage A launch");
-    }
+    rc = run_stage_a(enc, ap, 1);
+    if (rc != JPGB_OK) return rc;
     const size_t hist_bytes = JPGB_HIST_WORDS * 4;
     CK(enc->hist.reserve(hist_bytes), "alloc histogram");
     CK(enc->h_hist.reserve(hist_bytes + 16), "alloc histogram (host)");
     {
         StageTimer t(enc, 1);
         CK(cudaMemsetAsync(enc->hist.p, 0, hist_bytes, st), "clear histogram");
-        CK(launch_histogram(hp, enc->coef.as<int16_t>(), 1, enc->hist.as<uint32_t>(), st), "histogram launch");
+        CK(launch_histogram(hp, coef, 1, enc->hist.as<uint32_t>(), st), "histogram launch");
     }
-    enc->launches = 2;
+    enc->launches += 1;
     CK(cudaMemcpyAsync(enc->h_hist.p, enc->hist.p, hist_bytes, cudaMemcpyDeviceToHost, st), "download histogram");
     // DC of the first and of the last block of every component's true grid (the histogram chains DC differences
     // across the whole image without restart resets, encoder.rs:1086-1200: the neighbours need them)
@@ -1246,19 +1257,14 @@ int jpgb_strip_histogram_device(jpgb_encoder *enc, const jpgb_params *p, const j
     std::memset(edge, 0, 16);
     for (int c = 0; c < plan.ncomp; ++c) {
         const uint64_t first = plan.block_off[c], last = plan.block_off[c] + (uint64_t)plan.true_w[c] * plan.true_h[c] - 1; // raster of the true grid
-        CK(cudaMemcpyAsync(edge + c, enc->coef.as<int16_t>() + first * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
-        CK(cudaMemcpyAsync(edge + 4 + c, enc->coef.as<int16_t>() + last * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
+        CK(cudaMemcpyAsync(edge + c, coef + first * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
+        CK(cudaMemcpyAsync(edge + 4 + c, coef + last * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
     }
     CK(cudaStreamSynchronize(st), "histogram sync");
     std::memcpy(hist, enc->h_hist.p, hist_bytes);
     std::memcpy(edge_dc, edge, 16);
-    enc->coef_sig = plan_sig(plan);
-    enc->coef_pixels = d_pixels;
-    enc->coef_stride = uint64_t(ap.image_stride);
-    enc->coef_tagged = true;
     timing_end(enc);
-    enc->coef_ms[0] = enc->timing ? enc->last_ms[0] : 0.f;
-    enc->coef_ms[1] = enc->timing ? enc->last_ms[1] : 0.f;
+    enc->coef_tag = {true, plan_sig(plan), d_pixels, im.image_stride, {enc->timing ? enc->last_ms[0] : 0.f, enc->timing ? enc->last_ms[1] : 0.f}};
     return JPGB_OK;
 }
 
@@ -1388,14 +1394,9 @@ int jpgb_stage_a_device(jpgb_encoder *enc, const jpgb_params *p, const void *d_p
     if (rc != JPGB_OK) return rc;
     CK(cudaSetDevice(enc->device), "cudaSetDevice");
     StageAParams ap;
-    plan.fill_stage_a(ap);
-    ap.pixels = static_cast<const uint8_t *>(d_pixels);
-    ap.coef = static_cast<int16_t *>(d_coef);
-    ap.image_stride = image_stride;
+    plan.fill_stage_a(ap, contiguous_images(plan, d_pixels, image_stride), static_cast<int16_t *>(d_coef));
     enc->launches = 0;
-    CK(launch_stage_a(ap, n, enc->stream), "stage A launch");
-    enc->launches = 1;
-    return JPGB_OK;
+    return run_stage_a(enc, ap, n);
 }
 
 void jpgb_encoder_set_timing(jpgb_encoder *enc, int enabled) {

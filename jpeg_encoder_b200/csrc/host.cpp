@@ -573,8 +573,11 @@ void Plan::fill_device_plan(DevPlan &d) const {
     }
 }
 
-void Plan::fill_stage_a(StageAParams &a) const {
+void Plan::fill_stage_a(StageAParams &a, const jpgb_device_images &im, int16_t *coef) const {
     std::memset(&a, 0, sizeof(a));
+    a.pixels = static_cast<const uint8_t *>(im.data);
+    a.coef = coef;
+    a.image_stride = im.image_stride;
     a.blocks_per_image = blocks_per_image;
     a.width = p.width;
     a.height = p.height;
@@ -602,9 +605,24 @@ void Plan::fill_stage_a(StageAParams &a) const {
     const char *fg = std::getenv("JPGB_FORCE_GENERIC_STAGE_A");
     a.use_fast = !(fg && fg[0] == '1');
     a.planar = planar ? 1 : 0;
-    a.plane_stride = (unsigned long long)p.width * p.height;
-    if (planar) a.bpp = 1;
-    a.row_stride = (unsigned long long)p.width * a.bpp;
+    a.row_stride = im.row_stride;
+    // Channel-planar pixels of a packed ColorType are staged by the kernels with byte k of a pixel taken from plane
+    // plane_of[k]: Bgr, Rgba and Bgra are the Rgb kernels with their R, G, B planes in that order (the alpha plane is
+    // not read). Packed pixels leave plane_stride 0: no kernel reads it for them.
+    if (planar) {
+        a.bpp = 1;
+        a.plane_stride = im.plane_stride;
+    } else if (im.plane_stride && ncomp > 1) {
+        const uint8_t ct = p.color_type;
+        const bool bgr = ct == JPGB_BGR || ct == JPGB_BGRA;
+        a.channel_planar = 1;
+        a.plane_stride = im.plane_stride;
+        for (int k = 0; k < 4; ++k) a.plane_of[k] = (bgr && k < 3) ? 2 - k : k;
+        if (ct == JPGB_BGR || ct == JPGB_RGBA || ct == JPGB_BGRA) {
+            a.color_type = JPGB_RGB;
+            a.bpp = 3;
+        }
+    }
     for (int t = 0; t < 2; ++t)
         for (int i = 0; i < 64; ++i) {
             const int32_t c = q[t].corr[i] * q[t].recip[i];

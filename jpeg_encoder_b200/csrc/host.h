@@ -91,7 +91,8 @@ struct Plan {
     // SOF, DQT x2, DHT x2|4, [DRI] (Encoder::write_frame_header, src/encoder.rs:633-667)
     void frame_header(const HuffTable huff[2][2], std::vector<uint8_t> &out) const;
     void fill_device_plan(DevPlan &d) const;
-    void fill_stage_a(StageAParams &a) const;
+    // The colour+DCT launch of pixels laid out as `im` describes, writing the coefficients to `coef`
+    void fill_stage_a(StageAParams &a, const jpgb_device_images &im, int16_t *coef) const;
 };
 
 void default_huffman_tables(HuffTable huff[2][2]); // Annex K.3, src/huffman.rs:14-64
