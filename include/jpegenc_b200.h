@@ -238,6 +238,46 @@ int jpgb_last_piece_offsets_device(jpgb_encoder *enc, const uint64_t **d_offsets
 int jpgb_gather_place_pieces(jpgb_encoder *enc, void *d_target, size_t target_capacity, const uint64_t *d_table, uint32_t world,
                              uint32_t rank, uint64_t *d_total);
 
+/* ---- one large image in strips without restart intervals ------------------------------------------
+ * With restart_interval == 0 (Encoder::new's default, src/encoder.rs:239-275) a scan is one bit-contiguous stream: the
+ * DC predictor never resets and nothing is byte aligned between the first and the last bit of a scan. Strips of whole
+ * MCU rows are still coded on their own GPUs; the file bytes are the same as those of the whole image:
+ *  1. every strip: jpgb_contiguous_strip_prepare_device runs stage A (and, with optimized tables, the strip histogram,
+ *     as jpgb_strip_histogram_device does) and returns edge_dc[0..3] / edge_dc[4..7], the DC of the first / last block
+ *     of each component in the order the scans code them (MCU order when interleaved, the raster of the component's
+ *     true grid otherwise; jpgb_coef_layout_for);
+ *  2. the caller all-gathers the edge_dc arrays in strip order (n_strips * 8 values); with optimized tables it also
+ *     sums the histograms and merges them with jpgb_merge_strip_histograms -> hist_total;
+ *  3. every strip: jpgb_encode_contiguous_strip_device codes its part of every scan, the first DC difference of each
+ *     component taken against the last block of that component in the strip in front (strip 0: against 0). A piece is a
+ *     bare bit string: no header, SOS, pad bits, 0xFF stuffing or EOI. The pieces lie in context memory (*d_bits),
+ *     piece k at sum over j < k of its pieces' bytes rounded up to 16; jpgb_last_piece_bits_device gives their bit
+ *     lengths (n_scans u64, device memory) for an all-gather into a world x n_scans table in rank order;
+ *  4. every strip: jpgb_join_place_bits stores its pieces at their bit positions in a gather target (jpgb_gather_target_
+ *     create / _open; rank 0's memory). The target holds a side table of 2 * world * n_scans 16-byte entries (rounded
+ *     up to 128 bytes), then the joined stream: per scan its lead (the file header for scan 0, its SOS otherwise) and
+ *     the pieces of strips 0..n-1 back to back at bit granularity. A rank stores the 32-bit words wholly inside its
+ *     piece; the words it shares with a neighbour go to its own side-table entries. No atomics cross GPUs. Nothing is
+ *     written when the stream would not fit in `capacity` bytes;
+ *  5. rank 0, after a barrier that orders every rank's placement before it: jpgb_join_finish_device writes the header
+ *     (its DHT segments from hist_total when optimized), the SOS leads, pad bits and EOI, ORs in the side table, and
+ *     stuffs 0xFF: the file is in context memory, *d_file[0 .. *len).
+ * `p` is the whole image's settings throughout (p->height = the whole image's height), and restart_interval must be 0.
+ * The strip calls take the strip's pixels (packed rows back to back) at d_pixels. Steps 1 and 3 on the same context,
+ * strip and pixel pointer (the pixels untouched in between) run the colour+DCT kernel once. */
+int jpgb_plan_contiguous_strips(const jpgb_params *p, uint32_t max_strips, jpgb_strip *strips, uint32_t *n_strips); /* host only;
+                               equal-as-possible strips of whole MCU rows, never more than MCU rows; BAD_PARAMS unless restart 0 */
+int jpgb_contiguous_strip_prepare_device(jpgb_encoder *enc, const jpgb_params *p, const jpgb_strip *strip, const void *d_pixels,
+                                         uint32_t *hist /* JPGB_HIST_WORDS; NULL unless optimize_huffman */, int16_t edge_dc[8]);
+int jpgb_encode_contiguous_strip_device(jpgb_encoder *enc, const jpgb_params *p, const jpgb_strip *strip, const void *d_pixels,
+                                        const int16_t *edge_dc_table /* n_strips * 8, strip order */,
+                                        const uint32_t *hist_total /* NULL unless optimize_huffman */, const void **d_bits);
+int jpgb_last_piece_bits_device(jpgb_encoder *enc, const uint64_t **d_bits_table, uint32_t *n_scans);
+int jpgb_join_place_bits(jpgb_encoder *enc, void *d_target, size_t capacity, const uint64_t *d_bit_table /* world * n_scans */, uint32_t world,
+                         uint32_t rank);
+int jpgb_join_finish_device(jpgb_encoder *enc, const jpgb_params *p, void *d_target, size_t capacity, const uint64_t *d_bit_table, uint32_t world,
+                            const uint32_t *hist_total /* NULL unless optimize_huffman */, const void **d_file, uint64_t *len);
+
 /* Copy `n` bytes of context-owned (or any) device memory to host memory; synchronous on the context's stream. */
 int jpgb_download(jpgb_encoder *enc, const void *d_src, size_t n, void *host_dst);
 

@@ -72,7 +72,7 @@ using PinnedBuf = Buf<true>;
 struct PlanSig {
     jpgb_params p;
     jpgb_strip strip;
-    uint32_t is_strip, planar;
+    uint32_t is_strip, planar, contiguous, join_world;
 };
 inline PlanSig plan_sig(const Plan &plan) {
     PlanSig s;
@@ -98,6 +98,8 @@ inline PlanSig plan_sig(const Plan &plan) {
     }
     s.is_strip = plan.is_strip;
     s.planar = plan.planar;
+    s.contiguous = plan.contiguous;
+    s.join_world = plan.join_world;
     return s;
 }
 // Whose coefficients the context's `coef` holds, set by jpgb_strip_histogram_device and dropped by every write of
@@ -124,7 +126,7 @@ struct Caps { uint64_t ustream, out, pool_units; };
 // What a captured launch sequence bakes in (graph_key), word by word: no padding of the caller's structs takes part
 struct GraphKey {
     PlanSig sig;
-    uint64_t words[39];
+    uint64_t words[41];
 };
 
 // Replay of the launch sequence behind stage A as a CUDA graph (same settings, batch size and buffers)
@@ -186,11 +188,11 @@ struct jpgb_encoder {
     bool own_stream = false;
     std::string err;
     DevBuf pixels, coef, huff, hdr, hdr_len, scratch, pool, chunk_bits, chunk_pool, chunk_bitpos, seglen, segpos, ustream, ffcount, ffpos,
-        out, scan_tmp, hist, piece_off, out2, pixels2, status, hdr_parts;
+        out, scan_tmp, hist, piece_off, out2, pixels2, status, hdr_parts, piece_bits;
     std::vector<uint8_t> last_tables; // what the device currently holds
     double ucap_ratio = 0; // unstuffed-stream bytes to provision per raw pixel byte, learnt from earlier calls
     double pool_ratio = 0; // the same for the chunk pool (code bytes incl. per-chunk alignment)
-    PinnedBuf h_small, h_hist, h_tables, h_pieces, h_out, h_stage[2];
+    PinnedBuf h_small, h_hist, h_tables, h_pieces, h_out, h_stage[2], h_pred;
     cudaEvent_t ev_stage[2] = {};
     bool stage_busy[2] = {};
     CopyPool copy_pool;
@@ -205,6 +207,10 @@ struct jpgb_encoder {
     bool have_timing = false;
     uint32_t launches = 0;
     uint32_t last_piece_scans = 0; // scans of the last strip encode (its piece offsets are in piece_off)
+    // the last encode was a strip without restart intervals: its pieces are in `ustream`, their bits in `piece_bits`, and
+    // join_leads holds the lead bytes in front of each scan's data in the joined stream
+    uint32_t last_bit_scans = 0;
+    JoinLeads join_leads{};
     CoefTag coef_tag;
     GraphCache graphs;
     // Capacities are sticky per (settings, batch size): steady-state calls provision exactly what the last successful
@@ -264,6 +270,7 @@ void timing_end(jpgb_encoder *enc) {
 int build_plan(jpgb_encoder *enc, const jpgb_params &p, Plan &plan, const jpgb_strip *strip = nullptr) {
     const int rc = plan.build(p, strip);
     if (rc == JPGB_OK) return rc;
+    if (strip && plan.contiguous) return fail(enc, rc, "settings or strip geometry do not allow contiguous strips (needs restart_interval 0 and strips of whole MCU rows)");
     if (strip) return fail(enc, rc, "settings or strip geometry do not allow strip encoding (needs restart intervals aligned in every scan)");
     return fail(enc, rc, rc == JPGB_ERR_ZERO_DIMENSIONS ? "Image dimensions must be non zero" : "invalid parameters");
 }
@@ -479,13 +486,24 @@ void settle_caps(jpgb_encoder *enc, const CapKey &ck, const Caps &c, uint64_t ub
 }
 
 // What one attempt's launch sequence runs: the optimized tables (first attempt only; with given_hist from the caller's
-// histogram), the coder (else only the tail is repeated), the JPGB_POISON_STREAM hook, the read-back of strip pieces
-struct SequenceFlags { bool tables, given_hist, coder, poison, pieces; };
+// histogram), the coder (else only the tail is repeated), the JPGB_POISON_STREAM hook, the read-back of strip pieces,
+// the upload of the DC predictors of a contiguous strip (enc->h_pred)
+struct SequenceFlags { bool tables, given_hist, coder, poison, pieces, dc_pred; };
+
+// The root of a contiguous-strip join (jpgb_join_finish_device): instead of coding coefficients, the sequence takes the
+// pieces every strip has stored into the gather target
+struct JoinInput {
+    uint8_t *stream;                 // the joined unstuffed stream, behind the side table
+    uint64_t stream_cap;             // bytes, a multiple of kStuffChunk
+    const JoinSideWord *side;
+    const unsigned long long *table; // world x n_scans piece bits, rank order
+    uint32_t world;
+};
 
 // Everything behind stage A, for one attempt: tables, coding and positions, placement, stuffing, and the copy of the
 // file offsets and status words to enc->h_small. Every launch counts itself in enc->launches.
 int enqueue_sequence(jpgb_encoder *enc, const Plan &plan, const DevPlan &hp, const EntropyBuffers &b, uint32_t n, const CoderLaunch &coder,
-                     const HeaderLayout &hl, const SequenceFlags &f) {
+                     const HeaderLayout &hl, const SequenceFlags &f, const JoinInput *join) {
     cudaStream_t st = enc->stream;
     const uint64_t n_chunks = (uint64_t)plan.chunks_per_image * n, n_segs = b.n_segs_total, n_pieces = b.ustream_cap / kStuffChunk;
     const StatusBlock sb = status_block(n, b.ustream_cap);
@@ -493,6 +511,8 @@ int enqueue_sequence(jpgb_encoder *enc, const Plan &plan, const DevPlan &hp, con
     // status words of the coder and of the table build (only the words the tail writes when only the tail is repeated)
     if (f.coder) {
         CK(cudaMemsetAsync(b.status, 0, 2 * kStatusWords * 8 + sb.mask_bytes, st), "clear status and raw mask");
+        // read at replay time (a graph memcpy node reads the pinned source when it runs): no stale predictor is baked in
+        if (f.dc_pred) CK(cudaMemcpyAsync(b.status + kStatDcPred, enc->h_pred.p, 8, cudaMemcpyHostToDevice, st), "upload DC predictors");
     } else { // the pool cursor and the table status are not read again (grow_caps)
         CK(cudaMemsetAsync(b.status, 0, (kStatScanError + 1) * 8, st), "clear status");
         CK(cudaMemsetAsync(b.raw_mask, 0, sb.mask_bytes, st), "clear raw mask");
@@ -510,7 +530,12 @@ int enqueue_sequence(jpgb_encoder *enc, const Plan &plan, const DevPlan &hp, con
            "table build launch");
         enc->launches += 1;
     }
-    if (f.coder) {
+    if (f.coder && join) { // the ranks' piece sizes are the chunk sizes: positions, segment lengths and positions in one launch
+        StageTimer t(enc, 2);
+        CK(launch_join_chunks(b, join->table, join->world, (unsigned)plan.scans.size(), st), "join table launch");
+        CK(launch_positions(b, hp, n, true, st), "positions launch");
+        enc->launches += 2;
+    } else if (f.coder) {
         StageTimer t(enc, 2);
         CK(launch_encode_chunks(b, hp, n, coder, st), "coding launch");
         enc->launches += 1;
@@ -531,8 +556,15 @@ int enqueue_sequence(jpgb_encoder *enc, const Plan &plan, const DevPlan &hp, con
         // test hook: the stream starts out as all ones, so a byte that the kernels neither store nor zero shows in the output
         if (f.poison) CK(cudaMemsetAsync(b.ustream, 0xFF, b.ustream_cap + 64, st), "poison stream");
         CK(launch_segment_leads(b, hp, n, st), "segment lead launch");
-        CK(launch_place_chunks(b, hp, n, st), "placement launch");
+        if (join) CK(launch_join_merge(b, hp, join->side, join->world, st), "join merge launch");
+        else CK(launch_place_chunks(b, hp, n, st), "placement launch");
         enc->launches += 2;
+    }
+    if (plan.contiguous) { // bare pieces: no stuffing; their bit lengths stay on the device for the all-gather
+        CK(launch_piece_bits(b, hp, enc->piece_bits.as<unsigned long long>(), st), "piece bits launch");
+        enc->launches += 1;
+        CK(cudaMemcpyAsync(enc->h_small.p, b.file_off, sb.readback_bytes(), cudaMemcpyDeviceToHost, st), "read status");
+        return JPGB_OK;
     }
     {
         StageTimer t(enc, 4);
@@ -559,9 +591,11 @@ GraphKey graph_key(const jpgb_encoder *enc, const PlanSig &sig, const EntropyBuf
         (uint64_t)b.ffpos, (uint64_t)b.out, (uint64_t)b.file_off, (uint64_t)b.scan_tmp, b.ustream_cap, b.out_cap, b.n_segs_total,
         (uint64_t)b.status, b.scan_tmp_bytes,
         coder.grid, coder.smem, coder.scratch_bytes, n,
-        (uint64_t)f.tables | (uint64_t)f.given_hist << 1 | (uint64_t)f.coder << 2 | (uint64_t)f.poison << 3 | (uint64_t)f.pieces << 4,
+        (uint64_t)f.tables | (uint64_t)f.given_hist << 1 | (uint64_t)f.coder << 2 | (uint64_t)f.poison << 3 | (uint64_t)f.pieces << 4 |
+            (uint64_t)f.dc_pred << 5,
         hl.head_len, hl.tail_len, (uint64_t)hl.n_tables,
-        (uint64_t)enc->hist.p, (uint64_t)enc->hdr_parts.p, (uint64_t)enc->piece_off.p, (uint64_t)enc->h_small.p, (uint64_t)enc->h_pieces.p}};
+        (uint64_t)enc->hist.p, (uint64_t)enc->hdr_parts.p, (uint64_t)enc->piece_off.p, (uint64_t)enc->h_small.p, (uint64_t)enc->h_pieces.p,
+        (uint64_t)enc->h_pred.p, (uint64_t)enc->piece_bits.p}};
     std::memcpy(&k.sig, &sig, sizeof(sig));
     return k;
 }
@@ -594,19 +628,22 @@ int run_stage_a(jpgb_encoder *enc, const StageAParams &ap, uint32_t n) {
 // in `out` and `offsets` (host, n + 1) delimits them.
 // `given_hist` (strips with optimized tables): the symbol histogram of the *whole* image, [table][dc|ac][257],
 // used instead of the one of these pixels.
+// A contiguous strip (plan.contiguous) leaves its bare pieces in enc->ustream and their bits in enc->piece_bits, and no
+// file. `join` (the root of a join, plan.join_world > 0): the file is made from the pieces in the gather target.
 int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images &images, uint32_t n, DevBuf &out,
                   std::vector<uint64_t> &offsets, std::vector<uint64_t> *piece_offsets = nullptr, const uint32_t *given_hist = nullptr,
-                  bool coef_ready = false) {
+                  bool coef_ready = false, const JoinInput *join = nullptr) {
     cudaStream_t st = enc->stream;
     DevPlan hp;
     plan.fill_device_plan(hp);
+    enc->last_bit_scans = 0; // every call overwrites the stream that holds the bare pieces
 
     const uint64_t n_segs = (uint64_t)plan.segs_per_image * n;
     const uint64_t n_chunks = (uint64_t)plan.chunks_per_image * n;
 
     // ---- stage A (unless the caller has already run it: slice by slice behind the upload, or for a strip histogram) ----
     int rc;
-    if (!coef_ready) {
+    if (!coef_ready && !join) {
         int16_t *coef = nullptr;
         if ((rc = stage_a_coef(enc, plan, n, coef)) != JPGB_OK) return rc;
         StageAParams ap;
@@ -625,8 +662,11 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
     CK(enc->seglen.reserve(n_segs * 4), "alloc seglen");
     CK(enc->segpos.reserve((n_segs + 1) * 8), "alloc segpos");
     CoderLaunch coder{};
-    CK(coder_launch_config(hp, n, coder), "coder configuration");
-    CK(enc->scratch.reserve(coder.scratch_bytes), "alloc coder scratch");
+    if (!join) {
+        CK(coder_launch_config(hp, n, coder), "coder configuration");
+        CK(enc->scratch.reserve(coder.scratch_bytes), "alloc coder scratch");
+    }
+    if (plan.contiguous) CK(enc->piece_bits.reserve(plan.scans.size() * 8), "alloc piece bits");
     CK(enc->h_small.reserve(status_block(n, 0).readback_bytes()), "alloc readback");
     if (piece_offsets) {
         CK(enc->piece_off.reserve((plan.scans.size() + 1) * 8), "alloc piece offsets");
@@ -658,19 +698,19 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
     uint64_t ubytes = 0, total = 0, pool_used = 0;
     bool coded = false;
     for (int attempt = 0;; ++attempt) {
-        caps.ustream = (caps.ustream + kStuffChunk - 1) / kStuffChunk * kStuffChunk;
+        caps.ustream = join ? join->stream_cap : (caps.ustream + kStuffChunk - 1) / kStuffChunk * kStuffChunk;
         const uint64_t n_pieces = caps.ustream / kStuffChunk;
         const StatusBlock sb = status_block(n, caps.ustream);
-        CK(enc->ustream.reserve(caps.ustream + 64), "alloc unstuffed stream");
+        if (!join) CK(enc->ustream.reserve(caps.ustream + 64), "alloc unstuffed stream");
         CK(enc->status.reserve(sb.bytes()), "alloc status and raw mask");
         CK(enc->ffcount.reserve((n_pieces + 1) * 4), "alloc ff counts");
         CK(enc->ffpos.reserve((n_pieces + 2) * 8), "alloc ff positions");
         CK(enc->scan_tmp.reserve(scan_tmp_bytes(std::max<uint64_t>(n_pieces, std::max(n_chunks, n_segs)))), "alloc scan scratch");
-        CK(enc->pool.reserve(caps.pool_units * 16), "alloc chunk pool");
-        CK(out.reserve(caps.out + 64), "alloc output");
+        if (!join) CK(enc->pool.reserve(caps.pool_units * 16), "alloc chunk pool");
+        if (!plan.contiguous) CK(out.reserve(caps.out + 64), "alloc output");
         b.pool = enc->pool.as<uint32_t>();
         b.pool_cap = caps.pool_units;
-        b.ustream = enc->ustream.as<uint8_t>();
+        b.ustream = join ? join->stream : enc->ustream.as<uint8_t>();
         b.file_off = sb.file_off(enc->status.p);
         b.status = sb.status(enc->status.p);
         b.raw_mask = sb.raw_mask(enc->status.p);
@@ -680,13 +720,14 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
         b.out = out.as<uint8_t>();
         b.ustream_cap = caps.ustream;
         b.out_cap = caps.out;
-        const SequenceFlags f{plan.p.optimize_huffman != 0 && attempt == 0, given_hist != nullptr, !coded, poison_env && poison_env[0] == '1',
-                              piece_offsets != nullptr};
-        auto enqueue = [&] { return enqueue_sequence(enc, plan, hp, b, n, coder, hl, f); };
+        // (the poison hook would wipe the ranks' pieces in a join target)
+        const SequenceFlags f{plan.p.optimize_huffman != 0 && attempt == 0, given_hist != nullptr, !coded, !join && poison_env && poison_env[0] == '1',
+                              piece_offsets != nullptr, plan.contiguous};
+        auto enqueue = [&] { return enqueue_sequence(enc, plan, hp, b, n, coder, hl, f, join); };
         // Everything behind stage A is one fixed launch sequence per (settings, batch size, buffers): captured once,
         // replayed afterwards (a dozen launches cost ~10 us each from the host; a 1080p frame needs 70 us of kernels).
         bool replayed = false;
-        if (attempt == 0 && enc->graphs.ok && !enc->timing)
+        if (attempt == 0 && enc->graphs.ok && !enc->timing && !join)
             CK(enc->graphs.replay(graph_key(enc, ck.sig, b, n, coder, hl, f), st, enc->launches, enqueue, replayed), "graph launch");
         if (!replayed) {
             rc = enqueue();
@@ -696,6 +737,7 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
         const unsigned long long *status = sb.status(enc->h_small.p);
         if (status[kStatScanError]) return fail(enc, JPGB_ERR_CUDA, "internal: prefix-sum look-back timed out");
         if (status[kStatFlags] & kFlagSegment4G) return fail(enc, JPGB_ERR_BAD_PARAMS, "a scan segment exceeds 4 GiB (use a restart interval)");
+        if (join && (status[kStatFlags] & kFlagStream)) return fail(enc, JPGB_ERR_BAD_PARAMS, "the joined stream does not fit in the gather target");
         if (f.tables && (sb.table_status(enc->h_small.p)[kStatFlags] & kFlagHuffmanLong))
             return fail(enc, JPGB_ERR_HUFFMAN, "an optimized Huffman code does not fit (longer than 32 bits, or code plus value bits beyond 31)");
         ubytes = status[kStatUnstuffed];
@@ -710,6 +752,10 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
         grow_caps(caps, status, pool_used);
     }
     settle_caps(enc, ck, caps, ubytes, total, pool_used, n_chunks);
+    if (plan.contiguous) {
+        enc->last_bit_scans = (uint32_t)plan.scans.size();
+        return JPGB_OK;
+    }
     if (piece_offsets) {
         piece_offsets->assign(enc->h_pieces.as<uint64_t>(), enc->h_pieces.as<uint64_t>() + plan.scans.size() + 1);
         enc->last_piece_scans = (uint32_t)plan.scans.size();
@@ -939,6 +985,105 @@ int plan_strip(jpgb_encoder *enc, const jpgb_params &p, const jpgb_strip &strip,
     return JPGB_OK;
 }
 
+// At most max_strips equal-as-possible strips of whole groups of `step` MCU rows (the last group may be short)
+uint32_t cut_strips(const Plan &plan, uint64_t step, uint32_t max_strips, jpgb_strip *strips) {
+    const uint64_t groups = (plan.mcu_rows + step - 1) / step;
+    uint32_t n = (uint32_t)std::min<uint64_t>(max_strips, groups);
+    if (n == 0) n = 1;
+    const uint32_t rows_per_mcu = 8 * plan.vmax;
+    uint64_t g0 = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        const uint64_t g1 = groups * (i + 1) / n;
+        const uint64_t r0 = g0 * step * rows_per_mcu, r1 = std::min<uint64_t>(g1 * step * rows_per_mcu, plan.p.height);
+        strips[i].strip_index = i;
+        strips[i].n_strips = n;
+        strips[i].first_row = (uint16_t)r0;
+        strips[i].rows = (uint16_t)(r1 - r0);
+        strips[i].full_height = plan.p.height;
+        g0 = g1;
+    }
+    return n;
+}
+
+// Stage A of a strip into the context's coefficients, tagged for the encode that follows; with `hist`, the strip's
+// symbol histogram (DC chain started at 0). edge_dc[c] / edge_dc[4 + c]: DC of the first / last block of component c
+// in the strip's coefficient layout, which is the order its scans code the blocks (MCU order when interleaved, the
+// raster of the true grid otherwise): the neighbours' DC chains continue from them.
+int strip_prepare(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images &im, uint32_t *hist, int16_t edge_dc[8]) {
+    cudaStream_t st = enc->stream;
+    DevPlan hp;
+    plan.fill_device_plan(hp);
+    int16_t *coef = nullptr;
+    int rc = stage_a_coef(enc, plan, 1, coef);
+    if (rc != JPGB_OK) return rc;
+    StageAParams ap;
+    plan.fill_stage_a(ap, im, coef);
+    timing_begin(enc);
+    rc = run_stage_a(enc, ap, 1);
+    if (rc != JPGB_OK) return rc;
+    const size_t hist_bytes = JPGB_HIST_WORDS * 4;
+    CK(enc->h_hist.reserve(hist_bytes + 16), "alloc histogram (host)");
+    if (hist) {
+        CK(enc->hist.reserve(hist_bytes), "alloc histogram");
+        StageTimer t(enc, 1);
+        CK(cudaMemsetAsync(enc->hist.p, 0, hist_bytes, st), "clear histogram");
+        CK(launch_histogram(hp, coef, 1, enc->hist.as<uint32_t>(), st), "histogram launch");
+        enc->launches += 1;
+        CK(cudaMemcpyAsync(enc->h_hist.p, enc->hist.p, hist_bytes, cudaMemcpyDeviceToHost, st), "download histogram");
+    }
+    int16_t *edge = reinterpret_cast<int16_t *>(enc->h_hist.as<uint8_t>() + hist_bytes);
+    std::memset(edge, 0, 16);
+    for (int c = 0; c < plan.ncomp; ++c) {
+        uint64_t first = plan.block_off[c], last = plan.block_off[c] + (uint64_t)plan.true_w[c] * plan.true_h[c] - 1; // raster of the true grid
+        if (plan.mode == Mode::Interleaved) { // block of (MCU m, slot s) = m * blocks_per_mcu + s
+            first = plan.slot_base[c];
+            last = ((uint64_t)plan.mcu_cols * plan.mcu_rows - 1) * plan.bpu_interleaved + plan.slot_base[c] + plan.comps[c].h * plan.comps[c].v - 1;
+        }
+        CK(cudaMemcpyAsync(edge + c, coef + first * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
+        CK(cudaMemcpyAsync(edge + 4 + c, coef + last * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
+    }
+    CK(cudaStreamSynchronize(st), "strip stage A sync");
+    if (hist) std::memcpy(hist, enc->h_hist.p, hist_bytes);
+    std::memcpy(edge_dc, edge, 16);
+    timing_end(enc);
+    enc->coef_tag = {true, plan_sig(plan), im.data, im.image_stride, {enc->timing ? enc->last_ms[0] : 0.f, enc->timing ? enc->last_ms[1] : 0.f}};
+    return JPGB_OK;
+}
+
+// Bytes in front of each scan's data in the joined stream, as the root will write them: the file header with the
+// default tables or with the tables of `hist_total` (Annex K.2, built here as the root builds them on the device), SOS.
+int join_leads_for(jpgb_encoder *enc, const Plan &plan, const uint32_t *hist_total, JoinLeads &leads) {
+    HuffTable tables[2][2];
+    if (!hist_total) {
+        default_huffman_tables(tables);
+    } else {
+        const uint8_t none[16] = {0};
+        const int n_tables = plan.ncomp >= 3 ? 2 : 1;
+        for (int t = 0; t < 2; ++t)
+            for (int cls = 0; cls < 2; ++cls) {
+                tables[t][cls].set(none, nullptr, 0);
+                uint32_t freq[257];
+                std::memcpy(freq, hist_total + (size_t)(t * 2 + cls) * 257, sizeof(freq));
+                freq[256] = 1; // the reserved code point (src/encoder.rs:1092-1095)
+                if (t < n_tables && !tables[t][cls].set_optimized(freq))
+                    return fail(enc, JPGB_ERR_HUFFMAN, "an optimized Huffman code does not fit (longer than 32 bits)");
+            }
+    }
+    std::vector<uint8_t> h = plan.prefix;
+    plan.frame_header(tables, h);
+    leads.n_scans = (unsigned)plan.scans.size();
+    for (size_t k = 0; k < plan.scans.size(); ++k) leads.lead[k] = (unsigned)(plan.scans[k].sos.size() + (k == 0 ? h.size() : 0));
+    return JPGB_OK;
+}
+
+// The contiguous-strip entries after their null checks: the strip's plan (restart_interval 0) and pixels
+int plan_contiguous_strip(jpgb_encoder *enc, const jpgb_params &p, const jpgb_strip &strip, const void *d_pixels, Plan &plan,
+                          jpgb_device_images &im) {
+    if (p.color_type > JPGB_YCCK) return fail(enc, JPGB_ERR_BAD_PARAMS, "bad color_type");
+    plan.contiguous = true;
+    return plan_strip(enc, p, strip, d_pixels, plan, im);
+}
+
 } // namespace
 
 extern "C" {
@@ -1164,22 +1309,17 @@ int jpgb_plan_strips(const jpgb_params *p, uint32_t max_strips, jpgb_strip *stri
         const uint64_t need = R / gcd(R, upr);
         step = step / gcd(step, need) * need;
     }
-    const uint64_t groups = (plan.mcu_rows + step - 1) / step; // groups of `step` MCU rows (the last may be short)
-    uint32_t n = (uint32_t)std::min<uint64_t>(max_strips, groups);
-    if (n == 0) n = 1;
-    const uint32_t rows_per_mcu = 8 * plan.vmax;
-    uint64_t g0 = 0;
-    for (uint32_t i = 0; i < n; ++i) {
-        const uint64_t g1 = groups * (i + 1) / n;
-        const uint64_t r0 = g0 * step * rows_per_mcu, r1 = std::min<uint64_t>(g1 * step * rows_per_mcu, p->height);
-        strips[i].strip_index = i;
-        strips[i].n_strips = n;
-        strips[i].first_row = (uint16_t)r0;
-        strips[i].rows = (uint16_t)(r1 - r0);
-        strips[i].full_height = p->height;
-        g0 = g1;
-    }
-    *n_strips = n;
+    *n_strips = cut_strips(plan, step, max_strips, strips);
+    return JPGB_OK;
+}
+
+int jpgb_plan_contiguous_strips(const jpgb_params *p, uint32_t max_strips, jpgb_strip *strips, uint32_t *n_strips) {
+    if (!p || !strips || !n_strips || max_strips == 0) return JPGB_ERR_BAD_PARAMS;
+    Plan plan;
+    const int rc = plan.build(*p);
+    if (rc != JPGB_OK) return rc;
+    if (p->restart_interval != 0) return JPGB_ERR_BAD_PARAMS;
+    *n_strips = cut_strips(plan, 1, max_strips, strips);
     return JPGB_OK;
 }
 
@@ -1228,44 +1368,9 @@ int jpgb_strip_histogram_device(jpgb_encoder *enc, const jpgb_params *p, const j
     if (p->color_type > JPGB_YCCK || !p->optimize_huffman) return fail(enc, JPGB_ERR_BAD_PARAMS, "strip histograms belong to optimized Huffman tables");
     Plan plan;
     jpgb_device_images im;
-    int rc = plan_strip(enc, *p, *strip, d_pixels, plan, im);
+    const int rc = plan_strip(enc, *p, *strip, d_pixels, plan, im);
     if (rc != JPGB_OK) return rc;
-    cudaStream_t st = enc->stream;
-    DevPlan hp;
-    plan.fill_device_plan(hp);
-    int16_t *coef = nullptr;
-    rc = stage_a_coef(enc, plan, 1, coef);
-    if (rc != JPGB_OK) return rc;
-    StageAParams ap;
-    plan.fill_stage_a(ap, im, coef);
-    timing_begin(enc);
-    rc = run_stage_a(enc, ap, 1);
-    if (rc != JPGB_OK) return rc;
-    const size_t hist_bytes = JPGB_HIST_WORDS * 4;
-    CK(enc->hist.reserve(hist_bytes), "alloc histogram");
-    CK(enc->h_hist.reserve(hist_bytes + 16), "alloc histogram (host)");
-    {
-        StageTimer t(enc, 1);
-        CK(cudaMemsetAsync(enc->hist.p, 0, hist_bytes, st), "clear histogram");
-        CK(launch_histogram(hp, coef, 1, enc->hist.as<uint32_t>(), st), "histogram launch");
-    }
-    enc->launches += 1;
-    CK(cudaMemcpyAsync(enc->h_hist.p, enc->hist.p, hist_bytes, cudaMemcpyDeviceToHost, st), "download histogram");
-    // DC of the first and of the last block of every component's true grid (the histogram chains DC differences
-    // across the whole image without restart resets, encoder.rs:1086-1200: the neighbours need them)
-    int16_t *edge = reinterpret_cast<int16_t *>(enc->h_hist.as<uint8_t>() + hist_bytes);
-    std::memset(edge, 0, 16);
-    for (int c = 0; c < plan.ncomp; ++c) {
-        const uint64_t first = plan.block_off[c], last = plan.block_off[c] + (uint64_t)plan.true_w[c] * plan.true_h[c] - 1; // raster of the true grid
-        CK(cudaMemcpyAsync(edge + c, coef + first * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
-        CK(cudaMemcpyAsync(edge + 4 + c, coef + last * 64, 2, cudaMemcpyDeviceToHost, st), "read edge DC");
-    }
-    CK(cudaStreamSynchronize(st), "histogram sync");
-    std::memcpy(hist, enc->h_hist.p, hist_bytes);
-    std::memcpy(edge_dc, edge, 16);
-    timing_end(enc);
-    enc->coef_tag = {true, plan_sig(plan), d_pixels, im.image_stride, {enc->timing ? enc->last_ms[0] : 0.f, enc->timing ? enc->last_ms[1] : 0.f}};
-    return JPGB_OK;
+    return strip_prepare(enc, plan, im, hist, edge_dc);
 }
 
 int jpgb_merge_strip_histograms(const jpgb_params *p, uint32_t n_strips, const uint32_t hist_sum[JPGB_HIST_WORDS], const int16_t *edge_dc,
@@ -1348,6 +1453,100 @@ int jpgb_gather_place_pieces(jpgb_encoder *enc, void *d_target, size_t target_ca
     CK(launch_place_pieces(enc->out.as<uint8_t>(), static_cast<uint8_t *>(d_target), target_capacity, reinterpret_cast<const unsigned long long *>(d_table),
                            world, rank, enc->last_piece_scans, reinterpret_cast<unsigned long long *>(d_total), enc->stream),
        "piece placement launch");
+    return JPGB_OK;
+}
+
+int jpgb_contiguous_strip_prepare_device(jpgb_encoder *enc, const jpgb_params *p, const jpgb_strip *strip, const void *d_pixels,
+                                         uint32_t *hist, int16_t edge_dc[8]) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    if (!p || !strip || !d_pixels || !edge_dc) return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
+    if ((p->optimize_huffman != 0) != (hist != nullptr))
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "optimized tables take a strip histogram buffer; other settings take none");
+    Plan plan;
+    jpgb_device_images im;
+    const int rc = plan_contiguous_strip(enc, *p, *strip, d_pixels, plan, im);
+    if (rc != JPGB_OK) return rc;
+    return strip_prepare(enc, plan, im, hist, edge_dc);
+}
+
+int jpgb_encode_contiguous_strip_device(jpgb_encoder *enc, const jpgb_params *p, const jpgb_strip *strip, const void *d_pixels,
+                                        const int16_t *edge_dc_table, const uint32_t *hist_total, const void **d_bits) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    if (!p || !strip || !d_pixels || !edge_dc_table || !d_bits) return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
+    if ((p->optimize_huffman != 0) != (hist_total != nullptr))
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "optimized tables take the whole image's histogram; other settings take none");
+    Plan plan;
+    jpgb_device_images im;
+    int rc = plan_contiguous_strip(enc, *p, *strip, d_pixels, plan, im);
+    if (rc != JPGB_OK) return rc;
+    JoinLeads leads;
+    rc = join_leads_for(enc, plan, hist_total, leads);
+    if (rc != JPGB_OK) return rc;
+    // the first DC difference of each component is taken against the last block of that component in the strip in front
+    uint64_t pred = 0;
+    if (strip->strip_index > 0)
+        for (int c = 0; c < plan.ncomp; ++c) pred |= (uint64_t)(uint16_t)edge_dc_table[(strip->strip_index - 1) * 8 + 4 + c] << (16 * c);
+    CK(enc->h_pred.reserve(8), "alloc DC predictors (host)");
+    std::memcpy(enc->h_pred.p, &pred, 8); // the context's stream is idle: every encode call ends with a synchronise
+    timing_begin(enc);
+    const bool reuse = enc->coef_tag.matches(plan_sig(plan), d_pixels, im.image_stride);
+    enc->coef_tag.set = false; // a tag is used at most once
+    std::vector<uint64_t> off;
+    rc = encode_device(enc, plan, im, 1, enc->out, off, nullptr, hist_total, reuse);
+    if (rc != JPGB_OK) return rc;
+    timing_end(enc);
+    if (reuse && enc->timing) { // the stages that ran in the prepare call belong to this strip's encode
+        enc->last_ms[0] += enc->coef_tag.ms[0];
+        enc->last_ms[1] += enc->coef_tag.ms[1];
+    }
+    enc->join_leads = leads;
+    *d_bits = enc->ustream.p;
+    return JPGB_OK;
+}
+
+int jpgb_last_piece_bits_device(jpgb_encoder *enc, const uint64_t **d_bits_table, uint32_t *n_scans) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    if (!d_bits_table || !n_scans || enc->last_bit_scans == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "no contiguous strip has been encoded on this context");
+    *d_bits_table = enc->piece_bits.as<uint64_t>();
+    *n_scans = enc->last_bit_scans;
+    return JPGB_OK;
+}
+
+int jpgb_join_place_bits(jpgb_encoder *enc, void *d_target, size_t capacity, const uint64_t *d_bit_table, uint32_t world, uint32_t rank) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    if (!d_target || !d_bit_table || world == 0 || rank >= world || enc->last_bit_scans == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "bad join arguments");
+    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    CK(launch_join_place(enc->ustream.as<uint8_t>(), static_cast<uint8_t *>(d_target), capacity, reinterpret_cast<const unsigned long long *>(d_bit_table),
+                         world, rank, enc->join_leads, enc->stream),
+       "join placement launch");
+    return JPGB_OK;
+}
+
+int jpgb_join_finish_device(jpgb_encoder *enc, const jpgb_params *p, void *d_target, size_t capacity, const uint64_t *d_bit_table, uint32_t world,
+                            const uint32_t *hist_total, const void **d_file, uint64_t *len) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    if (!p || !d_target || !d_bit_table || !d_file || !len || world == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
+    if (p->color_type > JPGB_YCCK) return fail(enc, JPGB_ERR_BAD_PARAMS, "bad color_type");
+    if ((p->optimize_huffman != 0) != (hist_total != nullptr))
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "optimized tables take the whole image's histogram; other settings take none");
+    if (p->restart_interval != 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "contiguous strips have no restart intervals");
+    Plan plan;
+    int rc = build_plan(enc, *p, plan);
+    if (rc != JPGB_OK) return rc;
+    plan.join(world);
+    const uint64_t side = join_side_bytes(world, (unsigned)plan.scans.size());
+    if (capacity < side + kStuffChunk) return fail(enc, JPGB_ERR_BAD_PARAMS, "the gather target is too small for the join");
+    uint8_t *target = static_cast<uint8_t *>(d_target);
+    const JoinInput join{target + side, (capacity - side) / kStuffChunk * kStuffChunk, reinterpret_cast<const JoinSideWord *>(target),
+                         reinterpret_cast<const unsigned long long *>(d_bit_table), world};
+    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    timing_begin(enc);
+    std::vector<uint64_t> off;
+    rc = encode_device(enc, plan, contiguous_images(plan, nullptr, 0), 1, enc->out, off, nullptr, hist_total, true, &join);
+    if (rc != JPGB_OK) return rc;
+    timing_end(enc);
+    *d_file = enc->out.p;
+    *len = off[1];
     return JPGB_OK;
 }
 

@@ -107,6 +107,9 @@ struct DevPlan {
     unsigned segs_per_image, chunks_per_image, items_per_image;
     FastDiv div_items;      // by items_per_image (tickets below 2^32; beyond that the kernel divides in 64 bits)
     int has_eoi;            // 0 for every strip but the last
+    // 1: a strip without restart intervals. Its part of each scan is a bare bit string: no lead, no pad bits, no EOI,
+    // and the scan's segment is rounded up to 16 bytes so that the next one starts on a 128-bit word
+    int bare;
     int8_t slot_comp[kMaxSlots];
     uint8_t slot_back[kMaxSlots];   // interleaved: distance (in blocks of the MCU-ordered buffer) to the DC predecessor
     uint8_t slot_first[kMaxSlots];  // 1: first block of its component inside the MCU (predictor resets at restarts)

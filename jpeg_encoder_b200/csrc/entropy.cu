@@ -186,7 +186,9 @@ struct CoderSmem {
     static constexpr int oAc = kCoefBytes + (FULL ? 0 : kAsmWordsProg * 4);
     static constexpr int oDc = oAc + 2048;  // AC tables: 2 x 256 packed words
     static constexpr int oSlot = oDc + 256; // DC tables: 2 x 16 x {code << size, length}
-    static constexpr int oBin = oSlot + 128; // per MCU slot: table | distance to the DC predecessor << 8 | first of its component << 16
+    static constexpr int oBin = oSlot + 128; // per MCU slot: table | distance to the DC predecessor << 8 | first of its component << 16 | component << 24;
+                                             // words kMaxSlots .. + 3: each component's DC predictor at the start of a segment (kStatDcPred)
+    static_assert(kMaxSlots + 4 <= 32, "the DC predictors follow the slot words");
     static constexpr int oNb = oBin + 256;
     static constexpr int oOrder = oNb + T * 4;
     static constexpr int oWsum = oOrder + T * 2;
@@ -233,7 +235,10 @@ __global__ void __launch_bounds__(T, coder_min_ctas(T, FULL)) encode_chunks_kern
     uint32_t *scratch = b.scratch + (size_t)blockIdx.x * (T * kSlotWords);
     long long tab_img = -1; // whose Huffman tables the shared copy holds
     for (int i = tid; i < 64; i += T) bin[i] = 0;
-    if (tid < kMaxSlots) slot_tab[tid] = (unsigned)P.comp_tbl[P.slot_comp[tid]] | (unsigned)P.slot_back[tid] << 8 | (unsigned)P.slot_first[tid] << 16;
+    if (tid < kMaxSlots)
+        slot_tab[tid] = (unsigned)P.comp_tbl[P.slot_comp[tid]] | (unsigned)P.slot_back[tid] << 8 | (unsigned)P.slot_first[tid] << 16 |
+                        (unsigned)(uint8_t)P.slot_comp[tid] << 24;
+    else if (tid < kMaxSlots + 4) slot_tab[tid] = (unsigned)(int)(int16_t)(b.status[kStatDcPred] >> (16 * (tid - kMaxSlots)));
     // Work items are handed out by a ticket counter. Thread 0 runs one chunk ahead: while the CTA codes chunk i it
     // requests the ticket of chunk i + 2 and works out where chunk i + 1 lies, so neither the round trip of the
     // atomic nor the arithmetic is ever waited for.
@@ -347,12 +352,14 @@ __global__ void __launch_bounds__(T, coder_min_ctas(T, FULL)) encode_chunks_kern
             const unsigned v_in_seg = it.v_in_seg0 + tid;
             unsigned unit = v_in_seg, slot = 0;
             if (G.bpu > 1) divmod(v_in_seg, G.div_bpu, unit, slot);
-            const unsigned sinfo = G.comp < 0 ? slot_tab[slot] : ((unsigned)P.comp_tbl[G.comp] | 0x10100u);
+            const unsigned sinfo = G.comp < 0 ? slot_tab[slot] : ((unsigned)P.comp_tbl[G.comp] | 0x10100u | (unsigned)G.comp << 24);
             tbl = sinfo & 0xFF;
             const int back = (sinfo >> 8) & 0xFF;
-            const bool first_of_comp = (sinfo >> 16) != 0;
-            int prev = 0;
+            const bool first_of_comp = (sinfo >> 16) & 1;
+            int prev;
             if (!(unit == 0 && first_of_comp)) prev = tid >= back ? (int)coef[(tid - back) * kStageStride] : (int)__ldg(src_blocks + ((long long)tid - back) * 64);
+            else prev = (int)slot_tab[kMaxSlots + (sinfo >> 24)]; // 0, or the strip in front's last DC
+
             dcdiff = (int)(int16_t)(coef[tid * kStageStride] - prev);
         }
 
@@ -515,27 +522,10 @@ __global__ void __launch_bounds__(T, coder_min_ctas(T, FULL)) encode_chunks_kern
 // (writer.rs:424-452) or RSTn (encoder.rs:748-752: marker index = restarts % 8).
 __device__ __forceinline__ unsigned lead_len(const EntropyBuffers &b, const DevPlan &P, unsigned long long img, int k,
                                              unsigned seg_in_scan) {
+    if (P.bare) return 0;
     if (P.scans[k].rst_base + seg_in_scan > 0) return 2; // RSTn (for a strip: also before its first segment)
     if (k > 0) return P.scans[k].sos_len;
     return b.hdr_len[b.huff_per_image ? img : 0];
-}
-
-__global__ void __launch_bounds__(256) segment_len_kernel(const __grid_constant__ EntropyBuffers b, const __grid_constant__ DevPlan P, unsigned long long n_segs) {
-    const unsigned long long g = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= n_segs) return;
-    const unsigned long long img = g / P.segs_per_image;
-    const unsigned s = (unsigned)(g - img * P.segs_per_image);
-    const int k = find_scan_by_seg(P, s);
-    const DevScan &S = P.scans[k];
-    const unsigned i = s - S.seg_base;
-    const unsigned cps = P.groups[k % P.n_groups].cps;
-    // the segment's chunks are consecutive; the chunk after its last one starts the next segment (or scan, or image)
-    const unsigned long long c0 = img * P.chunks_per_image + S.chunk_base + (unsigned long long)i * cps;
-    const unsigned long long bits = b.chunk_bitpos[c0 + cps] - b.chunk_bitpos[c0];
-    const unsigned tail = (s == P.segs_per_image - 1 && P.has_eoi) ? 2u : 0u; // EOI, encoder.rs:564
-    const unsigned long long bytes = lead_len(b, P, img, k, i) + ((bits + 7) >> 3) + tail;
-    if (bytes > 0xFFFFFFFFull) atomicOr(b.status + kStatFlags, kFlagSegment4G); // seglen is 32-bit: reported, never wrapped silently
-    b.seglen[g] = (unsigned)bytes;
 }
 
 // bytes of local segment g (lead + data + EOI); the caller raises kFlagSegment4G beyond 4 GiB
@@ -546,10 +536,20 @@ __device__ __forceinline__ unsigned long long segment_bytes(const EntropyBuffers
     const DevScan &S = P.scans[k];
     const unsigned i = s - S.seg_base;
     const unsigned cps = P.groups[k % P.n_groups].cps;
+    // the segment's chunks are consecutive; the chunk after its last one starts the next segment (or scan, or image)
     const unsigned long long c0 = img * P.chunks_per_image + S.chunk_base + (unsigned long long)i * cps;
     const unsigned long long bits = b.chunk_bitpos[c0 + cps] - b.chunk_bitpos[c0];
-    const unsigned tail = (s == P.segs_per_image - 1 && P.has_eoi) ? 2u : 0u;
+    if (P.bare) return (bits + 127) >> 7 << 4;
+    const unsigned tail = (s == P.segs_per_image - 1 && P.has_eoi) ? 2u : 0u; // EOI, encoder.rs:564
     return lead_len(b, P, img, k, i) + ((bits + 7) >> 3) + tail;
+}
+
+__global__ void __launch_bounds__(256) segment_len_kernel(const __grid_constant__ EntropyBuffers b, const __grid_constant__ DevPlan P, unsigned long long n_segs) {
+    const unsigned long long g = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= n_segs) return;
+    const unsigned long long bytes = segment_bytes(b, P, g);
+    if (bytes > 0xFFFFFFFFull) atomicOr(b.status + kStatFlags, kFlagSegment4G); // seglen is 32-bit: reported, never wrapped silently
+    b.seglen[g] = (unsigned)bytes;
 }
 
 // exclusive prefix over the 1024 threads of a CTA (sm: 33 words); `total` = the CTA's sum
@@ -665,7 +665,7 @@ __global__ void __launch_bounds__(128) segment_lead_kernel(const __grid_constant
                 for (unsigned long long x = lo; x < hi; ++x) b.ustream[x] = 0;
         }
     }
-    if (slice != 0) return;
+    if (slice != 0 || P.bare) return;
     if (S.rst_base + i > 0) {
         if (lane == 0) {
             put_raw(b, pos, 0xFF);
@@ -691,6 +691,16 @@ __global__ void __launch_bounds__(128) segment_lead_kernel(const __grid_constant
         const unsigned long long end = b.segpos[g + 1];
         put_raw(b, end - 2, 0xFF);
         put_raw(b, end - 1, 0xD9);
+    }
+}
+
+// finalize_bit_buffer (writer.rs:138-145): ones behind the segment's last bit up to the byte boundary
+__device__ __forceinline__ void put_pad(uint32_t *stream, unsigned long long data_byte, unsigned long long seg_bits) {
+    const unsigned pad = (unsigned)(-(long long)seg_bits) & 7u;
+    if (pad) {
+        const unsigned long long pbit = data_byte * 8 + seg_bits;
+        const unsigned s2 = (unsigned)(pbit & 31); // pad never crosses a byte, hence never a word
+        atomicOr(stream + (pbit >> 5), __byte_perm(((1u << pad) - 1u) << (32 - s2 - pad), 0, 0x0123));
     }
 }
 
@@ -726,15 +736,7 @@ __global__ void __launch_bounds__(256) place_chunks_kernel(const __grid_constant
                 const unsigned long long data_byte = b.segpos[img * P.segs_per_image + S.seg_base + seg] + lead_len(b, P, img, k, seg);
                 my_bitpos = data_byte * 8 + (b.chunk_bitpos[c] - seg_first);
                 if (my_bits) my_pool = b.chunk_pool[c];
-                if (q == 0) { // pad with ones up to the byte boundary behind the segment's last bit
-                    const unsigned long long seg_bits = b.chunk_bitpos[c + G.cps] - seg_first;
-                    const unsigned pad = (unsigned)(-(long long)seg_bits) & 7u;
-                    if (pad) {
-                        const unsigned long long pbit = data_byte * 8 + seg_bits;
-                        const unsigned s2 = (unsigned)(pbit & 31); // pad never crosses a byte, hence never a word
-                        atomicOr(stream + (pbit >> 5), __byte_perm(((1u << pad) - 1u) << (32 - s2 - pad), 0, 0x0123));
-                    }
-                }
+                if (q == 0 && !P.bare) put_pad(stream, data_byte, b.chunk_bitpos[c + G.cps] - seg_first);
             }
         }
         unsigned todo = __ballot_sync(0xffffffffu, my_bits != 0);
@@ -773,6 +775,44 @@ __global__ void __launch_bounds__(256) place_chunks_kernel(const __grid_constant
                 }
             }
         }
+    }
+}
+
+// ---- strips without restart intervals -----------------------------------------------------------
+// A bare strip (one image, one segment per scan): the bits of its piece of every scan
+__global__ void __launch_bounds__(256) piece_bits_kernel(const __grid_constant__ EntropyBuffers b, const __grid_constant__ DevPlan P,
+                                                         unsigned long long *bits) {
+    for (int k = threadIdx.x; k < P.n_scans; k += blockDim.x) {
+        const unsigned c1 = k + 1 < P.n_scans ? P.scans[k + 1].chunk_base : P.chunks_per_image;
+        bits[k] = b.chunk_bitpos[c1] - b.chunk_bitpos[P.scans[k].chunk_base];
+    }
+}
+
+// The root of a join: chunk k * world + r of its plan is rank r's piece of scan k (table: world x n_scans, rank order)
+__global__ void __launch_bounds__(256) join_chunks_kernel(const EntropyBuffers b, const unsigned long long *__restrict__ table, unsigned world,
+                                                          unsigned n_scans) {
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= world * n_scans) return;
+    const unsigned k = i / world, r = i - k * world;
+    const unsigned long long bits = table[(unsigned long long)r * n_scans + k];
+    if (bits > 0xFFFFFFFFull) atomicOr(b.status + kStatFlags, kFlagSegment4G); // chunk sizes are 32-bit
+    b.chunk_bits[i] = (uint32_t)bits;
+}
+
+// The root of a join, once every rank's stores have landed and segment_lead_kernel has written the leads and zeroed the
+// shared words: the pad bits behind every scan and the ranks' side words
+__global__ void __launch_bounds__(256) join_merge_kernel(const __grid_constant__ EntropyBuffers b, const __grid_constant__ DevPlan P,
+                                                         const JoinSideWord *__restrict__ side, unsigned world) {
+    if (!stream_fits(b)) return;
+    uint32_t *stream = reinterpret_cast<uint32_t *>(b.ustream);
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < (unsigned)P.n_scans) {
+        const unsigned long long c0 = P.scans[i].chunk_base;
+        put_pad(stream, b.segpos[i] + lead_len(b, P, 0, (int)i, 0), b.chunk_bitpos[c0 + world] - b.chunk_bitpos[c0]);
+    }
+    if (i < 2 * world * (unsigned)P.n_scans) {
+        const JoinSideWord sw = side[i];
+        if (sw.word < b.ustream_cap / 4) atomicOr(stream + sw.word, sw.value);
     }
 }
 
@@ -1130,6 +1170,18 @@ cudaError_t launch_place_chunks(const EntropyBuffers &b, const DevPlan &hp, uint
     while (per_warp < 32 && nc / (per_warp * 2) >= 16384) per_warp *= 2;
     const unsigned long long ctas = (nc + 8ull * per_warp - 1) / (8ull * per_warp); // grid-stride beyond 64 K CTAs
     place_chunks_kernel<<<(unsigned)(ctas < 65536 ? (ctas ? ctas : 1) : 65536), 256, 0, s>>>(b, hp, nc, per_warp);
+    return cudaGetLastError();
+}
+cudaError_t launch_piece_bits(const EntropyBuffers &b, const DevPlan &hp, unsigned long long *bits, cudaStream_t s) {
+    piece_bits_kernel<<<1, 256, 0, s>>>(b, hp, bits);
+    return cudaGetLastError();
+}
+cudaError_t launch_join_chunks(const EntropyBuffers &b, const unsigned long long *table, unsigned world, unsigned n_scans, cudaStream_t s) {
+    join_chunks_kernel<<<grid_for((unsigned long long)world * n_scans, 256), 256, 0, s>>>(b, table, world, n_scans);
+    return cudaGetLastError();
+}
+cudaError_t launch_join_merge(const EntropyBuffers &b, const DevPlan &hp, const JoinSideWord *side, unsigned world, cudaStream_t s) {
+    join_merge_kernel<<<grid_for(2ull * world * hp.n_scans, 256), 256, 0, s>>>(b, hp, side, world);
     return cudaGetLastError();
 }
 cudaError_t launch_count_ff(const EntropyBuffers &b, cudaStream_t s) {

@@ -52,7 +52,99 @@ __global__ void __launch_bounds__(256) place_pieces_kernel(const uint8_t *__rest
     }
 }
 
+__device__ __forceinline__ unsigned long long warp_sum64(unsigned long long v) {
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+    return v;
+}
+
+// Strips without restart intervals. table[r * n + k] = bits of rank r's piece of scan k. The target holds the side table
+// (join_side_bytes) and then the root's unstuffed stream: per scan its lead, the pieces of ranks 0..world-1 back to back
+// at bit granularity, pad bits up to the byte; EOI at the end. Piece k of this rank lies in `src` at the sum of its
+// earlier pieces rounded up to 16 bytes each. Every rank derives the same positions from the same table.
+__global__ void __launch_bounds__(256) join_place_kernel(const uint8_t *__restrict__ src, uint8_t *target, unsigned long long target_cap,
+                                                         const unsigned long long *__restrict__ table, unsigned world, unsigned rank,
+                                                         const __grid_constant__ JoinLeads L) {
+    __shared__ unsigned long long at_sh[4];
+    const unsigned n = L.n_scans;
+    const unsigned long long side_bytes = join_side_bytes(world, n);
+    uint32_t *stream = reinterpret_cast<uint32_t *>(target + side_bytes);
+    JoinSideWord *side = reinterpret_cast<JoinSideWord *>(target);
+    const int lane = threadIdx.x & 31;
+    for (unsigned k = blockIdx.y; k < n; k += gridDim.y) {
+        if (threadIdx.x < 32) { // where the piece comes from and goes to, and whether the stream fits
+            unsigned long long s0 = 0, before = 0, all = 0, in_front = 0;
+            for (unsigned j = lane; j < n; j += 32) {
+                unsigned long long t = 0;
+                for (unsigned r = 0; r < world; ++r) {
+                    const unsigned long long v = table[(unsigned long long)r * n + j];
+                    t += v;
+                    if (j == k && r < rank) before += v;
+                }
+                const unsigned long long bytes = L.lead[j] + ((t + 7) >> 3);
+                all += bytes;
+                if (j < k) in_front += bytes, s0 += (table[(unsigned long long)rank * n + j] + 127) >> 7 << 4;
+            }
+            s0 = warp_sum64(s0), before = warp_sum64(before), all = warp_sum64(all), in_front = warp_sum64(in_front);
+            if (lane == 0) {
+                at_sh[0] = s0;
+                at_sh[1] = (in_front + L.lead[k]) * 8 + before;
+                at_sh[2] = side_bytes + all + 2 <= target_cap; // + EOI
+            }
+        }
+        __syncthreads();
+        const unsigned long long s0 = at_sh[0], B = at_sh[1], bits = table[(unsigned long long)rank * n + k];
+        const bool fits = at_sh[2] != 0;
+        __syncthreads(); // at_sh is rewritten for the next scan
+        const uint32_t *sw = reinterpret_cast<const uint32_t *>(src + s0);
+        const unsigned long long nw = (bits + 31) >> 5;
+        const unsigned sft = (unsigned)(B & 31), tail_bits = (unsigned)(bits & 31);
+        // source word i as a big-endian number, zero outside the piece
+        auto word = [&](long long i) -> uint32_t {
+            if (i < 0 || (unsigned long long)i >= nw) return 0u;
+            uint32_t v = __byte_perm(__ldg(sw + i), 0, 0x0123);
+            if ((unsigned long long)i == nw - 1 && tail_bits) v &= ~0u << (32 - tail_bits);
+            return v;
+        };
+        const unsigned long long dw0 = B >> 5;
+        // destination word d in memory byte order
+        auto dst_word = [&](unsigned long long d) -> uint32_t {
+            const long long i = (long long)(d - dw0);
+            const uint32_t v = sft ? __funnelshift_r(word(i), word(i - 1), sft) : word(i);
+            return __byte_perm(v, 0, 0x0123);
+        };
+        const unsigned long long o0 = (B + 31) >> 5, o1 = (B + bits) >> 5; // words wholly inside the piece: [o0, o1)
+        if (fits && o0 < o1) {
+            const unsigned long long a0 = (o0 + 3) & ~3ull, a1 = o1 & ~3ull;
+            const unsigned long long tid = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x, stride = (unsigned long long)gridDim.x * blockDim.x;
+            if (a0 < a1) { // aligned 128-bit peer stores for the body, single words at the two ends
+                for (unsigned long long q = a0 + tid * 4; q < a1; q += stride * 4)
+                    *reinterpret_cast<uint4 *>(stream + q) = make_uint4(dst_word(q), dst_word(q + 1), dst_word(q + 2), dst_word(q + 3));
+                if (tid < a0 - o0) stream[o0 + tid] = dst_word(o0 + tid);
+                if (tid < o1 - a1) stream[a1 + tid] = dst_word(a1 + tid);
+            } else if (tid < o1 - o0) {
+                stream[o0 + tid] = dst_word(o0 + tid);
+            }
+        }
+        if (blockIdx.x == 0 && threadIdx.x == 0) { // the shared words: the one holding the first bit and the one holding the last
+            const unsigned long long head = (fits && bits && sft) ? dw0 : ~0ull;
+            unsigned long long tail = (fits && bits && ((B + bits) & 31)) ? (B + bits - 1) >> 5 : ~0ull;
+            if (tail == head) tail = ~0ull;
+            JoinSideWord *slot = side + ((unsigned long long)k * world + rank) * 2;
+            slot[0] = {head, head != ~0ull ? dst_word(head) : 0u, 0u};
+            slot[1] = {tail, tail != ~0ull ? dst_word(tail) : 0u, 0u};
+        }
+    }
+}
+
 } // namespace
+
+cudaError_t launch_join_place(const uint8_t *src, uint8_t *target, unsigned long long target_cap, const unsigned long long *table, unsigned world,
+                              unsigned rank, const JoinLeads &leads, cudaStream_t stream) {
+    dim3 grid(148, leads.n_scans < 64 ? leads.n_scans : 64);
+    join_place_kernel<<<grid, 256, 0, stream>>>(src, target, target_cap, table, world, rank, leads);
+    return cudaGetLastError();
+}
 
 cudaError_t launch_place_pieces(const uint8_t *src, uint8_t *dst, unsigned long long dst_cap, const unsigned long long *table, unsigned world,
                                 unsigned rank, unsigned n_scans, unsigned long long *total_out, cudaStream_t stream) {

@@ -380,12 +380,13 @@ int Plan::build(const jpgb_params &params, const jpgb_strip *st) {
         }
     }
     if (is_strip) {
-        if (!p.restart_interval) return JPGB_ERR_BAD_PARAMS;
+        if ((p.restart_interval == 0) != contiguous) return JPGB_ERR_BAD_PARAMS;
         if (strip.n_strips == 0 || strip.strip_index >= strip.n_strips || strip.rows == 0) return JPGB_ERR_BAD_PARAMS;
         if (strip.first_row % (8 * vmax) != 0 || (uint32_t)strip.first_row + strip.rows > strip.full_height) return JPGB_ERR_BAD_PARAMS;
         if (strip.strip_index + 1 < strip.n_strips && strip.rows % (8 * vmax) != 0) return JPGB_ERR_BAD_PARAMS;
         const uint32_t mcu_row0 = strip.first_row / (8 * vmax);
         for (Scan &s : scans) {
+            if (contiguous) break;
             const uint64_t first_unit = s.comp < 0 ? (uint64_t)mcu_row0 * mcu_cols : (uint64_t)mcu_row0 * comps[s.comp].v * true_w[s.comp];
             if (first_unit % p.restart_interval != 0) return JPGB_ERR_BAD_PARAMS;
             s.rst_base = (uint32_t)(first_unit / p.restart_interval);
@@ -472,6 +473,13 @@ int Plan::build(const jpgb_params &params, const jpgb_strip *st) {
     return JPGB_OK;
 }
 
+void Plan::join(uint32_t world) {
+    join_world = world;
+    for (size_t k = 0; k < scans.size(); ++k) scans[k].chunk_base = (uint32_t)(k * world);
+    for (uint32_t g = 0; g < n_groups; ++g) groups[g].cps = world;
+    chunks_per_image = (uint32_t)scans.size() * world;
+}
+
 void Plan::frame_header(const HuffTable huff[2][2], std::vector<uint8_t> &o) const {
     put_marker(o, p.progressive_scans ? 0xC2 : 0xC0); // writer.rs:390-422
     put16(o, 2 + 1 + 2 + 2 + 1 + ncomp * 3);
@@ -522,7 +530,8 @@ void Plan::fill_device_plan(DevPlan &d) const {
     d.chunks_per_image = chunks_per_image;
     d.items_per_image = items_per_image;
     d.div_items = make_fastdiv(items_per_image);
-    d.has_eoi = !is_strip || strip.strip_index + 1 == strip.n_strips;
+    d.has_eoi = !is_strip || (!contiguous && strip.strip_index + 1 == strip.n_strips);
+    d.bare = contiguous;
     int n = 0;
     for (int c = 0; c < ncomp; ++c) {
         d.comp_tbl[c] = comps[c].dc_table;

@@ -86,8 +86,15 @@ struct Plan {
     // strip mode (strip != nullptr): geometry of the strip, header of the whole image
     bool planar = false; // ImageBuffer path: one plane per component, samples taken verbatim
     bool is_strip = false;
+    // set before build: a strip of an image without restart intervals (restart_interval must be 0). Its scans are coded
+    // against the DC values of the strip in front and come out as bare bit strings (DevPlan::bare)
+    bool contiguous = false;
+    uint32_t join_world = 0; // join(): the pieces of that many strips make up every scan
     jpgb_strip strip{};
     int build(const jpgb_params &params, const jpgb_strip *strip = nullptr); // returns JPGB_* code
+    // The whole image's plan (restart 0) as the root of a contiguous-strip join sees it: scan k is one segment made of
+    // `world` chunks, chunk r holding strip r's piece of the scan
+    void join(uint32_t world);
     // SOF, DQT x2, DHT x2|4, [DRI] (Encoder::write_frame_header, src/encoder.rs:633-667)
     void frame_header(const HuffTable huff[2][2], std::vector<uint8_t> &out) const;
     void fill_device_plan(DevPlan &d) const;

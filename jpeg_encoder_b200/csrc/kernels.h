@@ -84,6 +84,9 @@ constexpr int kStatusWords = 8;
 // Words of a status part: unstuffed bytes, 0xFF bytes of the coded data, flags, look-back scan error, work-item ticket
 // of the coding kernel, pool cursor (16-byte units; it counts every request, also beyond the capacity).
 constexpr int kStatUnstuffed = 0, kStatDataFF = 1, kStatFlags = 2, kStatScanError = 3, kStatTicket = 4, kStatPoolCursor = 5;
+// Word kStatDcPred: the DC predictor of the first block of each component (four i16, component c in bits 16c..16c+15).
+// Cleared with the rest of the status; a strip without restart intervals writes the last DCs of the strip in front.
+constexpr int kStatDcPred = 6;
 // Flag bits: overflow of the unstuffed stream, the output, the chunk pool; a scan segment over 4 GiB; an optimized
 // Huffman code that does not fit (longer than 32 bits, or code plus value bits beyond 31; table-build part)
 constexpr unsigned long long kFlagStream = 1, kFlagOut = 2, kFlagPool = 4, kFlagSegment4G = 8, kFlagHuffmanLong = 16;
@@ -139,6 +142,34 @@ cudaError_t launch_build_single_tables(const uint32_t *hist, uint32_t n, int ac,
 // gather.cu -- a rank's pieces stored at their place in the assembled file (possibly in a peer GPU's memory)
 cudaError_t launch_place_pieces(const uint8_t *src, uint8_t *dst, unsigned long long dst_cap, const unsigned long long *table, unsigned world,
                                 unsigned rank, unsigned n_scans, unsigned long long *total_out, cudaStream_t stream);
+
+// ---- strips without restart intervals: bit-string pieces joined on the root ----
+// A rank's piece of a scan starts and ends inside 32-bit words of the root's unstuffed stream that it shares with its
+// neighbours. It stores the words wholly inside the piece; each shared word goes to the rank's own slot of a side table
+// at the front of the gather target (stream word index, the piece's bits of it in memory byte order, zero elsewhere;
+// word ~0: no such word), and the root ORs them in.
+struct JoinSideWord {
+    unsigned long long word;
+    uint32_t value, unused;
+};
+// Bytes of the side table: two words per (scan, rank), rounded up to 128 bytes. The unstuffed stream follows it.
+__host__ __device__ inline unsigned long long join_side_bytes(unsigned world, unsigned n_scans) {
+    return ((unsigned long long)world * n_scans * 2 * sizeof(JoinSideWord) + 127) & ~127ull;
+}
+// Bytes in front of each scan's data in the root's unstuffed stream: the file header (scan 0) or the scan's SOS
+struct JoinLeads {
+    unsigned n_scans;
+    unsigned lead[kMaxScans];
+};
+// entropy.cu -- a bare strip: bits of its piece of every scan (n_scans u64); the root: the all-gathered table
+// (world x n_scans bit lengths, rank order) as the chunk sizes of its join plan, then pad bits and the side words
+cudaError_t launch_piece_bits(const EntropyBuffers &b, const DevPlan &hplan, unsigned long long *bits, cudaStream_t stream);
+cudaError_t launch_join_chunks(const EntropyBuffers &b, const unsigned long long *table, unsigned world, unsigned n_scans, cudaStream_t stream);
+cudaError_t launch_join_merge(const EntropyBuffers &b, const DevPlan &hplan, const JoinSideWord *side, unsigned world, cudaStream_t stream);
+// gather.cu -- this rank's pieces (in `src`, each scan's starting on a 16-byte boundary) stored at their bit positions
+// in the stream of the gather target; nothing is written when the stream would not fit in `target_cap` bytes
+cudaError_t launch_join_place(const uint8_t *src, uint8_t *target, unsigned long long target_cap, const unsigned long long *table, unsigned world,
+                              unsigned rank, const JoinLeads &leads, cudaStream_t stream);
 
 // scan.cu -- device-wide exclusive prefix sum of u32 into u64; out has n + 1 entries (out[n] = total)
 size_t scan_tmp_bytes(uint64_t n);

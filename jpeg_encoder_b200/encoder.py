@@ -206,6 +206,14 @@ def load_library():
                                                      C.POINTER(C.c_uint64)]
     l.jpgb_strip_histogram_device.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Strip), vp, C.POINTER(C.c_uint32), C.POINTER(C.c_int16)]
     l.jpgb_merge_strip_histograms.argtypes = [C.POINTER(_Params), C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(C.c_int16), C.POINTER(C.c_uint32)]
+    l.jpgb_plan_contiguous_strips.argtypes = [C.POINTER(_Params), C.c_uint32, C.POINTER(_Strip), C.POINTER(C.c_uint32)]
+    l.jpgb_contiguous_strip_prepare_device.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Strip), vp, C.POINTER(C.c_uint32), C.POINTER(C.c_int16)]
+    l.jpgb_encode_contiguous_strip_device.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Strip), vp, C.POINTER(C.c_int16), C.POINTER(C.c_uint32),
+                                                      C.POINTER(vp)]
+    l.jpgb_last_piece_bits_device.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_uint32)]
+    l.jpgb_join_place_bits.argtypes = [vp, vp, C.c_size_t, vp, C.c_uint32, C.c_uint32]
+    l.jpgb_join_finish_device.argtypes = [vp, C.POINTER(_Params), vp, C.c_size_t, vp, C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(vp),
+                                          C.POINTER(C.c_uint64)]
     l.jpgb_download.argtypes = [vp, vp, C.c_size_t, vp]
     l.jpgb_gather_target_create.argtypes = [vp, C.c_size_t, C.POINTER(vp), u8p]
     l.jpgb_gather_target_open.argtypes = [vp, u8p, C.POINTER(vp)]
@@ -657,6 +665,73 @@ class Encoder:
         if rc != 0:
             raise EncodingError(rc)
         return list(out)
+
+    # -- one large image in strips without restart intervals (include/jpegenc_b200.h) --
+    def plan_contiguous_strips(self, width, height, color_type, max_strips):
+        """[(first_row, rows)] for at most max_strips strips of whole MCU rows (never more than MCU rows). Needs
+        restart interval 0; raises EncodingError(BadParams) otherwise. Host only."""
+        p = self._params(width, height, ColorType(color_type))
+        arr = (_Strip * max_strips)()
+        n = C.c_uint32()
+        rc = load_library().jpgb_plan_contiguous_strips(C.byref(p), max_strips, arr, C.byref(n))
+        if rc != 0:
+            raise EncodingError(rc, "contiguous strips need restart interval 0")
+        return [(arr[i].first_row, arr[i].rows) for i in range(n.value)]
+
+    def contiguous_strip_prepare_device(self, d_pixels, strip_index, n_strips, first_row, rows, width, full_height, color_type):
+        """Step 1: stage A of the strip. Returns (hist[HIST_WORDS] or None without optimized tables, edge_dc[8])."""
+        dev = self._dev()
+        p = self._params(width, full_height, ColorType(color_type))
+        st = _Strip(strip_index, n_strips, first_row, rows, full_height)
+        hist = (C.c_uint32 * HIST_WORDS)() if self._optimize_huffman_table else None
+        edge = (C.c_int16 * 8)()
+        rc = dev.lib.jpgb_contiguous_strip_prepare_device(dev.handle, C.byref(p), C.byref(st), C.c_void_p(d_pixels), hist, edge)
+        if rc != 0:
+            self._raise(rc)
+        return (list(hist) if hist is not None else None), list(edge)
+
+    def encode_contiguous_strip_device(self, d_pixels, strip_index, n_strips, first_row, rows, width, full_height, color_type, edge_dc_table,
+                                       hist_total=None):
+        """Step 3: code the strip's bare pieces against the edge DCs of every strip (n_strips * 8, strip order). Returns the
+        device pointer of the pieces; their bit lengths are left on the device (piece_bits_device)."""
+        dev = self._dev()
+        p = self._params(width, full_height, ColorType(color_type))
+        st = _Strip(strip_index, n_strips, first_row, rows, full_height)
+        ed = (C.c_int16 * len(edge_dc_table))(*[int(x) for x in edge_dc_table])
+        h = (C.c_uint32 * HIST_WORDS)(*[int(x) for x in hist_total]) if hist_total is not None else None
+        d_bits = C.c_void_p()
+        rc = dev.lib.jpgb_encode_contiguous_strip_device(dev.handle, C.byref(p), C.byref(st), C.c_void_p(d_pixels), ed, h, C.byref(d_bits))
+        if rc != 0:
+            self._raise(rc)
+        return d_bits.value
+
+    def piece_bits_device(self):
+        """(device pointer, n_scans): the bit lengths (u64) of the last contiguous strip's pieces."""
+        dev = self._dev()
+        ptr, n = C.c_void_p(), C.c_uint32()
+        rc = dev.lib.jpgb_last_piece_bits_device(dev.handle, C.byref(ptr), C.byref(n))
+        if rc != 0:
+            self._raise(rc)
+        return ptr.value, n.value
+
+    def join_place_bits(self, d_target, capacity, d_bit_table, world, rank):
+        """Step 4: store the last contiguous strip's pieces at their bit positions in the gather target. Asynchronous."""
+        dev = self._dev()
+        rc = dev.lib.jpgb_join_place_bits(dev.handle, C.c_void_p(d_target), capacity, C.c_void_p(d_bit_table), world, rank)
+        if rc != 0:
+            self._raise(rc)
+
+    def join_finish_device(self, d_target, capacity, d_bit_table, world, width, height, color_type, hist_total=None):
+        """Step 5, rank 0: the whole file from the joined pieces. Returns (device pointer of the file, its length)."""
+        dev = self._dev()
+        p = self._params(width, height, ColorType(color_type))
+        h = (C.c_uint32 * HIST_WORDS)(*[int(x) for x in hist_total]) if hist_total is not None else None
+        d_file, n = C.c_void_p(), C.c_uint64()
+        rc = dev.lib.jpgb_join_finish_device(dev.handle, C.byref(p), C.c_void_p(d_target), capacity, C.c_void_p(d_bit_table), world, h,
+                                             C.byref(d_file), C.byref(n))
+        if rc != 0:
+            self._raise(rc)
+        return d_file.value, n.value
 
     def build_header(self, width, height, color_type):
         """SOI .. first SOS as the host planner writes them (default Huffman tables). No GPU needed."""

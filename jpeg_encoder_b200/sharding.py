@@ -6,6 +6,10 @@
   per-scan byte pieces to rank 0 (sizes first, then one grouped batch of variable-length sends over
   NCCL/NVLink), where they are concatenated scan-major. With optimized Huffman tables the strips
   first all-reduce their symbol histograms (the tables describe the whole image).
+* Without restart intervals a scan is one bit string. Strips of whole MCU rows still code on their own ranks: they
+  all-gather the DC values at their edges, code their pieces against the strip in front, and store the pieces at
+  their bit positions in rank 0's buffer (PeerGather.gather_bits); rank 0 adds leads, pad bits and EOI and stuffs 0xFF
+  once over the joined stream (PeerGather.finish_bits).
 
 The exchange functions work on whatever device the tensors live on: NCCL with CUDA tensors on the
 B200 box, gloo with CPU tensors in the world_size-2 CPU tests.
@@ -43,11 +47,51 @@ def exchange_strip_histograms(hist, edge_dc, device, group=None):
     the strip edges are all-gathered in rank order. Returns (hist_sum list, edge_dc list of world * 8)."""
     h = torch.tensor(hist, dtype=torch.int64, device=device)  # NCCL has no u32 sum; counts fit easily
     dist.all_reduce(h, op=dist.ReduceOp.SUM, group=group)
+    return h.cpu().tolist(), exchange_edge_dc(edge_dc, device, group)
+
+
+def exchange_edge_dc(edge_dc, device, group=None):
+    """Strips without restart intervals: all-gather the strips' edge_dc arrays (8 values each) in rank order."""
     e = torch.tensor(edge_dc, dtype=torch.int32, device=device)
     world = dist.get_world_size(group)
     table = torch.empty(world * 8, dtype=torch.int32, device=device)
     dist.all_gather_into_tensor(table, e, group=group)
-    return h.cpu().tolist(), table.cpu().tolist()
+    return table.cpu().tolist()
+
+
+def join_destinations(table, leads):
+    """Strips without restart intervals. table[r][k] = bits of rank r's piece of scan k, leads[k] = bytes in front of scan
+    k's data (the header for scan 0, its SOS otherwise). Returns (dest, src, total): dest[r][k] = bit position of the
+    piece in the joined stream, src[r][k] = byte offset of the piece in rank r's own buffer (each piece rounded up to 16
+    bytes), total = bytes of the joined stream with pad bits and EOI. The arithmetic of csrc/gather.cu, restated."""
+    world, n = len(table), len(table[0])
+    dest = [[0] * n for _ in range(world)]
+    src = [[0] * n for _ in range(world)]
+    at = 0
+    for k in range(n):
+        at += leads[k]
+        bit = at * 8
+        for r in range(world):
+            dest[r][k] = bit
+            bit += table[r][k]
+            if k + 1 < n:
+                src[r][k + 1] = src[r][k] + (table[r][k] + 127) // 128 * 16
+        at = (bit + 7) // 8
+    return dest, src, at + 2
+
+
+def join_words(dest_bit, bits):
+    """The 32-bit words of the joined stream a piece at [dest_bit, dest_bit + bits) touches: (owned, shared), owned the
+    range of words wholly inside the piece (stored by the rank), shared the words it shares with a neighbour (sent
+    through the side table and ORed in by rank 0)."""
+    end = dest_bit + bits
+    owned = range((dest_bit + 31) // 32, end // 32)
+    shared = []
+    if bits and dest_bit % 32:
+        shared.append(dest_bit // 32)
+    if bits and end % 32 and (end - 1) // 32 not in shared:
+        shared.append((end - 1) // 32)
+    return owned, shared
 
 
 def piece_destinations(table):
@@ -106,15 +150,7 @@ class PeerGather:
         rc = self.dev.lib.jpgb_last_piece_offsets_device(self.dev.handle, C.byref(d_offs), C.byref(n_scans))
         if rc != 0:
             raise RuntimeError("jpgb_last_piece_offsets_device: %s" % self.dev.last_error())
-        n = n_scans.value + 1
-        if self.n_table != n:
-            self.table = torch.empty(self.world * n, dtype=torch.int64, device=self.tdev)
-            self.n_table = n
-        mine = _device_view(d_offs.value, n, self.tdev)
-        if self.world > 1:
-            dist.all_gather_into_tensor(self.table, mine, group=self.group)
-        else:
-            self.table.copy_(mine)
+        self._all_gather_table(d_offs.value, n_scans.value + 1)
         rc = self.dev.lib.jpgb_gather_place_pieces(self.dev.handle, C.c_void_p(self.target), self.capacity, C.c_void_p(self.table.data_ptr()),
                                                    self.world, self.rank, C.c_void_p(self.total.data_ptr()))
         if rc != 0:
@@ -132,6 +168,31 @@ class PeerGather:
         if total > self.capacity:
             raise RuntimeError("gather target too small: %d > %d" % (total, self.capacity))
         return _device_view(self.target, total, self.tdev, "|u1") if self.rank == 0 else None
+
+    def _all_gather_table(self, d_ptr, n):
+        if self.n_table != n:
+            self.table = torch.empty(self.world * n, dtype=torch.int64, device=self.tdev)
+            self.n_table = n
+        mine = _device_view(d_ptr, n, self.tdev)
+        if self.world > 1:
+            dist.all_gather_into_tensor(self.table, mine, group=self.group)
+        else:
+            self.table.copy_(mine)
+
+    def gather_bits(self, encoder):
+        """Bit-join mode (strips without restart intervals): call right after encoder.encode_contiguous_strip_device on
+        this rank. One all-gather of the pieces' bit lengths (device tensors), then this rank's kernel stores its pieces
+        at their bit positions in rank 0's buffer. Asynchronous; follow with barrier(), then finish_bits() on rank 0."""
+        d_bits, n_scans = encoder.piece_bits_device()
+        self._all_gather_table(d_bits, n_scans)
+        encoder.join_place_bits(self.target, self.capacity, self.table.data_ptr(), self.world, self.rank)
+
+    def finish_bits(self, encoder, width, height, color_type, hist_total=None):
+        """Rank 0, after barrier(): leads, pad bits, EOI, the shared words, 0xFF stuffing. Returns the file as a uint8
+        device tensor (a view of the encoder context's output, valid until its next call)."""
+        d_file, n = encoder.join_finish_device(self.target, self.capacity, self.table.data_ptr(), self.world, width, height, color_type,
+                                               hist_total=hist_total)
+        return _device_view(d_file, n, self.tdev, "|u1")
 
     def close(self):
         if self.target:
