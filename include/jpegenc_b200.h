@@ -164,6 +164,40 @@ typedef struct jpgb_device_images {
 int jpgb_encode_batch_device_strided(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_images *images,
                                      uint32_t n, const void **d_files, uint64_t *offsets);
 
+/* ---- device images of wider samples: float32, float16, bfloat16 and uint16 (model outputs, raw and medical data) ----
+ * Element types of jpgb_sample_format.type, all little-endian. (0 is uint8, which takes jpgb_encode_batch_device_strided.) */
+enum { JPGB_SAMPLE_U16 = 1, JPGB_SAMPLE_F16 = 2, JPGB_SAMPLE_BF16 = 3, JPGB_SAMPLE_F32 = 4 };
+typedef struct jpgb_sample_format {
+    uint32_t type;        /* JPGB_SAMPLE_* */
+    float scale, offset;  /* finite */
+} jpgb_sample_format;
+
+/* jpgb_encode_batch_device_strided for images whose samples are elements of fmt->type. The layout and the output mean
+ * what they mean there; every stride stays in bytes, and sample ch of pixel (x, y) is one element of the type
+ * (es = 2 or 4 bytes) at
+ *   packed (plane_stride == 0): data + i*image_stride + y*row_stride + (x*bpp + ch)*es
+ *   planar (plane_stride > 0):  data + i*image_stride + ch*plane_stride + y*row_stride + x*es
+ * Each element x read becomes the 8-bit sample
+ *   y = fadd_rn(fmul_rn(float(x), scale), offset)    two separately rounded fp32 operations, never a fused multiply-add
+ *   sample = NaN(y) ? 0 : clamp(rint(y), 0, 255)     rint rounds half to even: 0.5 -> 0, 2.5 -> 2, 254.5 -> 254
+ * (float(x) is exact for every type), and that sample takes the uint8 colour path unchanged: the files are byte-identical
+ * to jpgb_encode_batch_device's for the converted image handed over packed. value_range (lo, hi) maps to
+ * scale = float(255 / (hi - lo)), offset = float(-lo * 255 / (hi - lo)), each computed in double and rounded once.
+ * Colour types: Luma, Rgb, Bgr, Rgba, Bgra. The alpha element is never converted, and never read when planar.
+ * Rejected before anything is enqueued (no launch), in this order, with JPGB_ERR_BAD_PARAMS unless noted:
+ *   null arguments (fmt included) or n == 0;
+ *   what jpgb_encode_batch_device rejects in `p` (same codes), except the BadImageData length check;
+ *   fmt->type 0 (uint8: use jpgb_encode_batch_device_strided) or not a JPGB_SAMPLE_* value;
+ *   color_type Ycbcr, Cmyk, CmykAsYcck or Ycck;
+ *   a scale or offset that is infinite or NaN;
+ *   data, row_stride, plane_stride or image_stride not a multiple of es;
+ *   then the layout checks of jpgb_encode_batch_device_strided in their order, counted in elements: a row is
+ *   width*bpp*es bytes packed and width*es planar, and the last byte read is
+ *     (n-1)*image_stride + (height-1)*row_stride + width*bpp*es - 1                       (packed)
+ *     (n-1)*image_stride + c_max*plane_stride + (height-1)*row_stride + width*es - 1      (planar) */
+int jpgb_encode_batch_device_samples(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_images *images,
+                                     const jpgb_sample_format *fmt, uint32_t n, const void **d_files, uint64_t *offsets);
+
 /* Order the context's stream after all work queued so far on `stream` (an event wait; the host does not block).
  * stream may be cudaStreamLegacy (1) or cudaStreamPerThread (2); the context's own stream is a no-op. Use it when
  * the pixels of the next encode are produced on a stream of the caller's. */

@@ -4,4 +4,4 @@ Package contents: csrc/ (CUDA kernels + C ABI + host planner), encoder.py (ctype
 reference's `Encoder`), build.py (nvcc build of libjpegenc_b200.so). No CPU fallback exists.
 """
 from .encoder import (ColorType, Device, Encoder, EncodingError, JpegColorType, PixelDensity, PixelDensityUnit,  # noqa: F401
-                      QuantizationTableType, SamplingFactor, default_device, load_library)
+                      QuantizationTableType, SampleType, SamplingFactor, default_device, load_library, sample_scale_offset)

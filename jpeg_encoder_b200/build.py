@@ -23,7 +23,7 @@ def _stale():
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    deps = sources() + glob.glob(os.path.join(CSRC, "*.h")) + glob.glob(os.path.join(PKG, "..", "include", "*.h"))
+    deps = sources() + glob.glob(os.path.join(CSRC, "*.h")) + glob.glob(os.path.join(CSRC, "*.inc")) + glob.glob(os.path.join(PKG, "..", "include", "*.h"))
     return any(os.path.getmtime(d) > t for d in deps)
 
 

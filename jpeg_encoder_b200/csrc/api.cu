@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <climits>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -298,19 +299,20 @@ MemGetAddressRangeFn mem_get_address_range_fn() {
     return fn;
 }
 
-// The checks of jpgb_encode_batch_device_strided on the layout, in the order the header lists them. Nothing is enqueued
-// before they pass, so no kernel reads a byte outside the allocation that holds `data`.
-int check_device_images(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images &im, uint32_t n) {
+// The checks of jpgb_encode_batch_device_strided on the layout, in the order the header lists them, for samples of `es`
+// bytes (jpgb_encode_batch_device_samples). Nothing is enqueued before they pass, so no kernel reads a byte outside the
+// allocation that holds `data`.
+int check_device_images(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images &im, uint32_t n, uint64_t es = 1) {
     const uint64_t w = plan.p.width, h = plan.p.height;
     const bool planes = im.plane_stride != 0;
-    const uint64_t row_bytes = planes ? w : w * (uint64_t)plan.bpp; // bytes of a row read (of one plane)
+    const uint64_t row_bytes = (planes ? w : w * (uint64_t)plan.bpp) * es; // bytes of a row read (of one plane)
     char m[192];
     if (im.row_stride < row_bytes) {
         snprintf(m, sizeof(m), "row_stride %llu is shorter than a row (%llu bytes)", (unsigned long long)im.row_stride, (unsigned long long)row_bytes);
         return fail(enc, JPGB_ERR_BAD_PARAMS, m);
     }
-    if (planes && im.plane_stride < w) {
-        snprintf(m, sizeof(m), "plane_stride %llu is shorter than a row (%llu bytes)", (unsigned long long)im.plane_stride, (unsigned long long)w);
+    if (planes && im.plane_stride < w * es) {
+        snprintf(m, sizeof(m), "plane_stride %llu is shorter than a row (%llu bytes)", (unsigned long long)im.plane_stride, (unsigned long long)(w * es));
         return fail(enc, JPGB_ERR_BAD_PARAMS, m);
     }
     // the last byte read: (n-1)*image_stride + c_max*plane_stride + (h-1)*row_stride + row_bytes - 1 (alpha is not read)
@@ -616,10 +618,10 @@ int stage_a_coef(jpgb_encoder *enc, const Plan &plan, uint32_t n, int16_t *&coef
     return JPGB_OK;
 }
 
-// Every colour+DCT launch of a context: timed as stage 0 and counted
-int run_stage_a(jpgb_encoder *enc, const StageAParams &ap, uint32_t n) {
+// Every colour+DCT launch of a context: timed as stage 0 and counted. `fmt`: the pixels' element type (type 0: uint8)
+int run_stage_a(jpgb_encoder *enc, const StageAParams &ap, uint32_t n, const jpgb_sample_format &fmt = {}) {
     StageTimer t(enc, 0);
-    CK(launch_stage_a(ap, n, enc->stream), "stage A launch");
+    CK(launch_stage_a(ap, n, fmt, enc->stream), "stage A launch");
     enc->launches += 1;
     return JPGB_OK;
 }
@@ -648,7 +650,7 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
         if ((rc = stage_a_coef(enc, plan, n, coef)) != JPGB_OK) return rc;
         StageAParams ap;
         plan.fill_stage_a(ap, images, coef);
-        if ((rc = run_stage_a(enc, ap, n)) != JPGB_OK) return rc;
+        if ((rc = run_stage_a(enc, ap, n, plan.sample)) != JPGB_OK) return rc;
     }
 
     HeaderLayout hl;
@@ -1272,6 +1274,32 @@ int jpgb_encode_batch_device_strided(jpgb_encoder *enc, const jpgb_params *p, co
     if (rc != JPGB_OK) return rc;
     // Ycbcr and Ycck planes are the ImageBuffer planes: samples taken verbatim, one plane per component
     plan.planar = images->plane_stride != 0 && (p->color_type == JPGB_YCBCR || p->color_type == JPGB_YCCK);
+    return encode_batch_device(enc, plan, *images, n, d_files, offsets);
+}
+
+int jpgb_encode_batch_device_samples(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_images *images,
+                                     const jpgb_sample_format *fmt, uint32_t n, const void **d_files, uint64_t *offsets) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    enc->launches = 0; // a rejected call reports no launches
+    if (!images || !images->data || !fmt || !d_files || !offsets || n == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
+    Plan plan;
+    int rc = validate_and_plan(enc, p, SIZE_MAX, plan); // a strided layout has no length to check
+    if (rc != JPGB_OK) return rc;
+    if (fmt->type == 0) return fail(enc, JPGB_ERR_BAD_PARAMS, "sample type 0 is uint8: use jpgb_encode_batch_device_strided");
+    if (fmt->type > JPGB_SAMPLE_F32) return fail(enc, JPGB_ERR_BAD_PARAMS, "unknown sample type");
+    const uint8_t ct = p->color_type;
+    if (ct != JPGB_LUMA && ct != JPGB_RGB && ct != JPGB_BGR && ct != JPGB_RGBA && ct != JPGB_BGRA)
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "sample types other than uint8 take Luma, Rgb, Bgr, Rgba and Bgra only");
+    if (!std::isfinite(fmt->scale) || !std::isfinite(fmt->offset)) return fail(enc, JPGB_ERR_BAD_PARAMS, "scale and offset must be finite");
+    const uint64_t es = fmt->type == JPGB_SAMPLE_F32 ? 4 : 2;
+    if (((uint64_t)(uintptr_t)images->data | images->row_stride | images->plane_stride | images->image_stride) % es != 0) {
+        char m[128];
+        snprintf(m, sizeof(m), "data and strides must be multiples of the element size (%llu bytes)", (unsigned long long)es);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    rc = check_device_images(enc, plan, *images, n, es);
+    if (rc != JPGB_OK) return rc;
+    plan.sample = *fmt;
     return encode_batch_device(enc, plan, *images, n, d_files, offsets);
 }
 

@@ -40,8 +40,9 @@ cudaError_t resident_ctas(int threads, size_t smem, unsigned long long &ctas) {
     return cudaSuccess;
 }
 
-// stage_a.cu -- colour + decimate + level shift + fDCT + quantize -> zig-zag i16 coefficients
-cudaError_t launch_stage_a(const StageAParams &p, uint32_t n_images, cudaStream_t stream);
+// stage_a.cu -- colour + decimate + level shift + fDCT + quantize -> zig-zag i16 coefficients. `fmt`: the element
+// type of the pixels (type 0: uint8), converted to 8-bit samples while staging
+cudaError_t launch_stage_a(const StageAParams &p, uint32_t n_images, const jpgb_sample_format &fmt, cudaStream_t stream);
 
 // Huffman code tables as the kernels see them: [image][table 0|1][class dc|ac][256] of (size<<16)|code
 constexpr size_t kHuffWordsPerImage = 2 * 2 * 256;

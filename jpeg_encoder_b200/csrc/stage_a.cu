@@ -18,6 +18,7 @@
 //
 // All arithmetic is 32-bit integer; tensor cores are not used (the DCT must be bit-exact).
 #include <cuda.h>
+#include <cuda_fp16.h>
 
 #include <algorithm>
 #include <cstdlib>
@@ -170,8 +171,128 @@ __device__ __noinline__ void stage_planes_chunk(uint8_t *dst, const uint8_t *row
     }
 }
 
-template <int CT>
-__global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ StageAParams p) {
+// ---- samples of a wider element type (jpgb_sample_format), turned into the 8-bit samples of the tile while staging ----
+// Colour types that take them: Luma and the RGB family (Bgr, Rgba and Bgra planes are Rgb planes in another order)
+__host__ __device__ constexpr bool converts(int ct) {
+    return ct == JPGB_LUMA || ct == JPGB_RGB || ct == JPGB_BGR || ct == JPGB_RGBA || ct == JPGB_BGRA;
+}
+__host__ __device__ constexpr int element_size(int type) { return type == JPGB_SAMPLE_F32 ? 4 : 2; }
+
+// The conversion of jpgb_encode_batch_device_samples: y = fadd_rn(fmul_rn(x, scale), offset) -- the intrinsics keep
+// nvcc from contracting them into an FMA -- then NaN -> 0, else clamp(rint(y), 0, 255). cvt.rni.sat.u8.f32 is that last
+// step: round to nearest even, saturate to 0..255, NaN to 0. The result is read through its low byte only.
+__device__ __forceinline__ uint32_t to_sample(float x, const jpgb_sample_format &f) {
+    const float y = __fadd_rn(__fmul_rn(x, f.scale), f.offset);
+    uint32_t r;
+    asm("cvt.rni.sat.u8.f32 %0, %1;" : "=r"(r) : "f"(y));
+    return r;
+}
+// element `bits` (the low 16 bits for the 16-bit types) of type T widened to fp32: exact for every type
+template <int T>
+__device__ __forceinline__ float widen(uint32_t bits) {
+    if constexpr (T == JPGB_SAMPLE_U16) return (float)(bits & 0xFFFFu);
+    else if constexpr (T == JPGB_SAMPLE_F16) return __half2float(__ushort_as_half((unsigned short)bits));
+    else if constexpr (T == JPGB_SAMPLE_BF16) return __uint_as_float(bits << 16);
+    else return __uint_as_float(bits);
+}
+__device__ __forceinline__ float load_element(const uint8_t *src, int type) {
+    if (type == JPGB_SAMPLE_F32) return widen<JPGB_SAMPLE_F32>(__ldg(reinterpret_cast<const unsigned *>(src)));
+    const uint32_t b = __ldg(reinterpret_cast<const unsigned short *>(src));
+    if (type == JPGB_SAMPLE_U16) return widen<JPGB_SAMPLE_U16>(b);
+    if (type == JPGB_SAMPLE_F16) return widen<JPGB_SAMPLE_F16>(b);
+    return widen<JPGB_SAMPLE_BF16>(b);
+}
+
+// The converting counterpart of stage_edge_chunk / stage_planes_chunk, element by element: tile bytes e0 .. e0 + n - 1 of
+// a row whose pixels have `pxe` samples, the row's last valid pixel replicated (Q4). Sample ch of pixel px lies at
+// row + (px * pxe + ch) * es, or with `plane_of` at row + plane_of[ch] * plane_stride + px * es. A fourth (alpha) sample
+// of packed pixels is not read: its tile byte is 0. Cold path (image edges, rows not 16-byte aligned), kept out of line.
+__device__ __noinline__ void stage_convert_edge(uint8_t *dst, const uint8_t *row, int e0, int n, int pxe, int valid_px,
+                                                const jpgb_sample_format f, const int *plane_of, unsigned long long plane_stride) {
+    const int es = element_size((int)f.type);
+    for (int e = e0; e < e0 + n; ++e) {
+        const int px = e / pxe, ch = e - px * pxe, sx = min(px, valid_px - 1);
+        uint32_t s = 0;
+        if (plane_of) s = to_sample(load_element(row + (size_t)plane_of[ch] * plane_stride + (size_t)sx * es, (int)f.type), f);
+        else if (!(pxe == 4 && ch == 3)) s = to_sample(load_element(row + ((size_t)sx * pxe + ch) * es, (int)f.type), f);
+        dst[e] = (uint8_t)s;
+    }
+}
+
+// 8 consecutive elements of type T at a 16-byte aligned address -> their 8 tile bytes. ALPHA: packed 4-sample pixels
+// (the unit starts on a pixel); their alpha sample is not converted and its byte is 0.
+template <int T>
+__device__ __forceinline__ void load_unit(const uint8_t *g, uint4 (&a)[2]) {
+    a[0] = __ldg(reinterpret_cast<const uint4 *>(g));
+    if constexpr (element_size(T) == 4) a[1] = __ldg(reinterpret_cast<const uint4 *>(g) + 1);
+}
+template <int T, bool ALPHA>
+__device__ __forceinline__ uint2 convert_unit(const uint4 (&a)[2], const jpgb_sample_format &f) {
+    const uint32_t w[8] = {a[0].x, a[0].y, a[0].z, a[0].w, a[1].x, a[1].y, a[1].z, a[1].w};
+    uint32_t s[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const uint32_t bits = element_size(T) == 4 ? w[j] : (j & 1 ? w[j >> 1] >> 16 : w[j >> 1]);
+        s[j] = (ALPHA && (j & 3) == 3) ? 0u : to_sample(widen<T>(bits), f);
+    }
+    auto pack4 = [](uint32_t b0, uint32_t b1, uint32_t b2, uint32_t b3) {
+        return __byte_perm(__byte_perm(b0, b1, 0x0040), __byte_perm(b2, b3, 0x0040), 0x5410);
+    };
+    return make_uint2(pack4(s[0], s[1], s[2], s[3]), pack4(s[4], s[5], s[6], s[7]));
+}
+
+// A warp tile of LINES lines of 256 * PXB samples (packed rows, or ROWS rows of each plane read) converted into the u8
+// tile, line i at tile + i * PITCH. Line i is row min(py0 + i % ROWS, height - 1) of plane i / ROWS, from
+// src = image + px0 * PXB * es (+ plane * plane_stride). Interior tiles: every lane converts its 8-element units with
+// 16-byte loads, U units (U or 2U loads) in flight. Elsewhere a unit inside the row's valid samples takes the same
+// path when the row is 16-byte aligned, and stage_convert_edge otherwise.
+template <int T, int PXB, int ROWS, int LINES, bool ALPHA>
+__device__ __forceinline__ void stage_convert_tile(uint8_t *tile, const uint8_t *src, const StageAParams &p, const jpgb_sample_format &f,
+                                                   int py0, int valid_px, int needed_px, bool interior, int lane) {
+    constexpr int ES = element_size(T), UPL = 32 * PXB, PITCH = 256 * PXB, U = 4;
+    const size_t row_stride = p.row_stride;
+    if (interior) {
+        static_assert((LINES * PXB) % U == 0, "whole batches of units per lane");
+#pragma unroll 1
+        for (int u0 = lane; u0 < LINES * UPL; u0 += 32 * U) {
+            uint4 a[U][2];
+#pragma unroll
+            for (int j = 0; j < U; ++j) {
+                const int u = u0 + 32 * j, i = u / UPL, k = i / ROWS, ry = i - k * ROWS;
+                load_unit<T>(src + (size_t)k * p.plane_stride + (size_t)(py0 + ry) * row_stride + (size_t)(u - i * UPL) * 8 * ES, a[j]);
+            }
+#pragma unroll
+            for (int j = 0; j < U; ++j) {
+                const int u = u0 + 32 * j, i = u / UPL;
+                *reinterpret_cast<uint2 *>(tile + i * PITCH + (u - i * UPL) * 8) = convert_unit<T, ALPHA>(a[j], f);
+            }
+        }
+        return;
+    }
+    const int valid = valid_px * PXB, needed = needed_px * PXB;
+#pragma unroll 1
+    for (int i = 0; i < LINES; ++i) {
+        const int k = i / ROWS, ry = i - k * ROWS;
+        const uint8_t *row = src + (size_t)k * p.plane_stride + (size_t)min(py0 + ry, p.height - 1) * row_stride;
+        uint8_t *dst = tile + i * PITCH;
+        const bool aligned = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
+#pragma unroll 1
+        for (int e0 = lane * 8; e0 < needed; e0 += 32 * 8) {
+            if (aligned && e0 + 8 <= valid) {
+                uint4 a[2];
+                load_unit<T>(row + (size_t)e0 * ES, a);
+                *reinterpret_cast<uint2 *>(dst + e0) = convert_unit<T, ALPHA>(a, f);
+            } else {
+                stage_convert_edge(dst, row, e0, 8, PXB, valid_px, f, nullptr, 0);
+            }
+        }
+    }
+}
+
+// The generic kernel's body: a CTA tile of `groups` x 32 MCUs x one MCU row. CONV: the samples are elements of
+// fmt.type, converted while staging.
+template <int CT, bool CONV>
+__device__ __forceinline__ void generic_tile(const StageAParams &p, const jpgb_sample_format &fmt) {
     extern __shared__ __align__(128) uint8_t tile[];
     constexpr int BPP = (CT == JPGB_LUMA || CT == kPlanar) ? 1 : ((CT == JPGB_RGB || CT == JPGB_BGR || CT == JPGB_YCBCR) ? 3 : 4);
     constexpr bool PLANAR = CT == kPlanar;
@@ -180,7 +301,7 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
     const int mcu_x0 = tile_x * 32 * p.groups;
     const int px0 = mcu_x0 * 8 * p.hmax, py0 = mcu_y * 8 * p.vmax;
     const uint8_t *src = p.pixels + (size_t)img * p.image_stride;
-    const int px_bytes = p.channel_planar ? 1 : BPP; // bytes of one pixel in one input row
+    const int px_bytes = (p.channel_planar ? 1 : BPP) * (CONV ? element_size((int)fmt.type) : 1); // of one pixel in one input row
 
     // ---- stage the tile: 16-byte chunks, edges replicated (Q4) ----
     const int chunks_per_row = p.tile_pitch / 16;
@@ -195,7 +316,8 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
         const int sy = min(py0 + ry, p.height - 1);
         const uint8_t *row = src + (size_t)plane * p.plane_stride + (size_t)sy * p.row_stride + (size_t)px0 * px_bytes;
         uint8_t *dst = tile + plane * plane_tile + ry * p.tile_pitch;
-        if (p.channel_planar) stage_planes_chunk<BPP>(dst, row, p.plane_stride, p.plane_of, cb, valid_px);
+        if (CONV) stage_convert_edge(dst, row, cb, 16, BPP, valid_px, fmt, p.channel_planar ? p.plane_of : nullptr, p.plane_stride);
+        else if (p.channel_planar) stage_planes_chunk<BPP>(dst, row, p.plane_stride, p.plane_of, cb, valid_px);
         else if (cb + 16 <= valid_bytes && ((reinterpret_cast<uintptr_t>(row + cb) & 15) == 0))
             *reinterpret_cast<uint4 *>(dst + cb) = __ldg(reinterpret_cast<const uint4 *>(row + cb));
         else stage_edge_chunk<BPP>(dst, row, cb, valid_px);
@@ -237,6 +359,15 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
         if (p.comp_qt[comp] == 0) quantize_store256<0>(p, v, dst);
         else quantize_store256<1>(p, v, dst);
     }
+}
+
+template <int CT>
+__global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ StageAParams p) {
+    generic_tile<CT, false>(p, jpgb_sample_format{});
+}
+template <int CT>
+__global__ void __launch_bounds__(256) stage_a_convert_kernel(const __grid_constant__ StageAParams p, const __grid_constant__ jpgb_sample_format fmt) {
+    generic_tile<CT, true>(p, fmt);
 }
 
 
@@ -592,209 +723,23 @@ __host__ __device__ constexpr int warp_tile_mcu_rows() {
 // memory order -- the same bytes per tile -- and the row loader interleaves them into the packed pixel words, so the
 // arithmetic behind it is the packed kernel's. Byte k of a pixel comes from tile plane p.plane_of[k].
 // =================================================================================================
+// The body is shared as text (stage_a_warp_body.inc) rather than through an inline function: with the parameters
+// passed to a function, the compiler schedules the uint8 kernels' instructions differently.
 template <int CT, int HS, int VS, bool PL>
 __global__ void __launch_bounds__(128, 4) stage_a_warp_kernel(const __grid_constant__ StageAParams p,
                                                               const __grid_constant__ CUtensorMap tmap, const int use_tma) {
-    extern __shared__ __align__(128) uint8_t smem[];
-    constexpr int BPP = Fmt<CT>::BPP;
-    constexpr bool SUB = HS * VS > 1;
-    constexpr int NCOMP = Fmt<CT>::NCOMP;
-    constexpr bool BYTES = Fmt<CT>::BYTES;
-    constexpr int MR = warp_tile_mcu_rows<CT, HS, VS>(); // MCU rows per warp tile (small tiles take several)
-    constexpr int MROWS = 8 * VS;               // pixel rows of one MCU row
-    constexpr int ROWS = MROWS * MR;
-    constexpr int PXB = PL ? 1 : BPP;           // bytes of a pixel in one tile row
-    constexpr int PITCH = 256 * PXB;            // 32 full-resolution blocks wide
-    constexpr int TILE_BYTES = 256 * BPP * ROWS;
-    constexpr int MCUS = 32 / HS;               // MCUs per warp tile
-    // tasks of one warp tile: luma rows, [K rows], then chroma
-    constexpr int N_FULL = Fmt<CT>::NFULL * VS;
-    // when chroma is horizontally decimated a 1x1 component has only 32 / HS blocks per tile: HS of them share a task
-    constexpr bool PAIRED = SUB && HS >= 2;
-    constexpr int LPC = 32 / HS; // lanes (blocks) per component in a shared task
-    constexpr int N_CHROMA = PAIRED ? (Fmt<CT>::NSUB + HS - 1) / HS : Fmt<CT>::NSUB;
-    constexpr int N_TASKS_ROW = N_FULL + N_CHROMA;
-    constexpr int N_TASKS = N_TASKS_ROW * MR;
-
-    const int lane = threadIdx.x & 31;
-    ChromaConsts cc{};
-    if constexpr (PAIRED && !BYTES && NCOMP > 1) cc = chroma_consts<CT>(((lane / LPC) & 1) != 0);
-    const unsigned warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const unsigned n_warps_total = (gridDim.x * blockDim.x) >> 5;
-    uint8_t *tile = smem + (threadIdx.x >> 5) * TILE_BYTES;
-    // one mbarrier per warp behind the four tiles: TMA signals the bytes of this warp's tile on it
-    uint64_t *bar = reinterpret_cast<uint64_t *>(smem + 4 * TILE_BYTES) + (threadIdx.x >> 5);
-    unsigned phase = 0;
-    if (use_tma) {
-        if (lane == 0) {
-            mbar_init(bar, 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncwarp();
-    }
-    const unsigned tiles_per_row = ((unsigned)p.mcu_cols + MCUS - 1) / MCUS;
-    const unsigned tile_rows = ((unsigned)p.mcu_rows + MR - 1) / MR;
-    const unsigned n_tiles = tiles_per_row * tile_rows * p.n_images;
-    const size_t row_stride = p.row_stride;
-    int choff[4] = {0, 0, 0, 0}; // PL: offset of the tile plane that byte k of a pixel comes from
-    if constexpr (PL)
-#pragma unroll
-        for (int k = 0; k < BPP; ++k) choff[k] = p.plane_of[k] * (PITCH * ROWS);
-
-    for (unsigned t = warp_global; t < n_tiles; t += n_warps_total) {
-        const unsigned tx = t % tiles_per_row, r = t / tiles_per_row;
-        const int mcu_y0 = (int)(r % tile_rows) * MR, img = (int)(r / tile_rows);
-        const int mcu_x0 = (int)tx * MCUS;
-        // ---- stage this warp's rows (cp.async, L2 only); edges replicated (Q4) ----
-        if constexpr (PL) {
-            const int px0 = mcu_x0 * 8 * HS, py0 = mcu_y0 * MROWS;
-            const uint8_t *src = p.pixels + (size_t)img * p.image_stride + px0; // plane 0
-            const int valid_px = min(256, p.width - px0);
-            const int needed_px = min(256, p.mcu_cols * 8 * HS - px0);
-            __syncwarp(); // all lanes are done reading the previous tile
-            const bool interior = px0 + 256 <= p.width && py0 + ROWS <= p.height && ((row_stride | p.plane_stride) & 15) == 0 &&
-                                  (reinterpret_cast<uintptr_t>(src) & 15) == 0;
-            if (interior && use_tma) { // one 4-D box: 256 px x ROWS rows x BPP planes
-                if (lane == 0) {
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    mbar_expect_tx(bar, TILE_BYTES);
-                    tma_load_4d(tile, &tmap, bar, px0 / 4, py0, 0, img);
-                }
-                mbar_wait(bar, phase);
-                phase ^= 1;
-            } else if (interior) { // half a warp per 256-byte plane row
-#pragma unroll 4
-                for (int i = lane >> 4; i < BPP * ROWS; i += 2) {
-                    const int k = i / ROWS, ry = i - k * ROWS;
-                    cp_async16(tile + i * PITCH + (lane & 15) * 16, src + (size_t)k * p.plane_stride + (size_t)(py0 + ry) * row_stride + (lane & 15) * 16);
-                }
-            } else {
-#pragma unroll 1
-                for (int i = 0; i < BPP * ROWS; ++i) {
-                    const int k = i / ROWS, ry = i - k * ROWS;
-                    const int sy = min(py0 + ry, p.height - 1);
-                    const uint8_t *row = src + (size_t)k * p.plane_stride + (size_t)sy * row_stride;
-                    uint8_t *dst = tile + i * PITCH;
-                    const bool aligned = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
-                    const int cb = lane * 16;
-                    if (cb < needed_px) {
-                        if (aligned && cb + 16 <= valid_px) cp_async16(dst + cb, row + cb);
-                        else stage_edge_chunk<1>(dst, row, cb, valid_px);
-                    }
-                }
-            }
-            cp_async_commit();
-            cp_async_wait<0>();
-            __syncwarp();
-        } else {
-            const int px0 = mcu_x0 * 8 * HS, py0 = mcu_y0 * MROWS;
-            const uint8_t *src = p.pixels + (size_t)img * p.image_stride;
-            const int valid_px = min(256, p.width - px0);
-            const int valid_bytes = valid_px * BPP;
-            const int needed_bytes = min(256, p.mcu_cols * 8 * HS - px0) * BPP;
-            __syncwarp(); // all lanes are done reading the previous tile
-            const bool interior = px0 + 256 <= p.width && py0 + ROWS <= p.height && (row_stride & 15) == 0 &&
-                                  ((reinterpret_cast<uintptr_t>(src) + (size_t)px0 * BPP) & 15) == 0;
-            if (interior && use_tma) {
-                // One TMA box per tile (UTMALDG): a single lane issues it, the tensor unit streams the
-                // 256-pixel x ROWS box into this warp's tile and signals the byte count on the warp's mbarrier.
-                if (lane == 0) {
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // earlier generic-proxy accesses of the tile
-                    mbar_expect_tx(bar, TILE_BYTES);
-                    tma_load_3d(tile, &tmap, bar, px0 * BPP / 4, py0, img);
-                }
-                mbar_wait(bar, phase);
-                phase ^= 1;
-            } else if (interior) {
-                // whole tile inside the image and 16-byte aligned: every lane copies its fixed chunks of each row
-                const uint8_t *g = src + (size_t)py0 * row_stride + (size_t)px0 * BPP + lane * 16;
-                uint8_t *d = tile + lane * 16;
-#pragma unroll 4
-                for (int ry = 0; ry < ROWS; ++ry) {
-#pragma unroll
-                    for (int c = 0; c < (PITCH + 511) / 512; ++c)
-                        if (c * 512 + 512 <= PITCH || lane * 16 + c * 512 < PITCH) cp_async16(d + c * 512, g + c * 512);
-                    g += row_stride;
-                    d += PITCH;
-                }
-            } else {
-#pragma unroll 1
-                for (int ry = 0; ry < ROWS; ++ry) {
-                    const int sy = min(py0 + ry, p.height - 1);
-                    const uint8_t *row = src + (size_t)sy * row_stride + (size_t)px0 * BPP;
-                    uint8_t *dst = tile + ry * PITCH;
-                    const bool aligned = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
-#pragma unroll 1
-                    for (int cb = lane * 16; cb < needed_bytes; cb += 32 * 16) {
-                        if (aligned && cb + 16 <= valid_bytes) cp_async16(dst + cb, row + cb);
-                        else stage_edge_chunk<BPP>(dst, row, cb, valid_px); // cold: right edge / unaligned rows
-                    }
-                }
-            }
-            cp_async_commit();
-            cp_async_wait<0>();
-            __syncwarp();
-        }
-        // ---- tasks ----
-#pragma unroll 1
-        for (int task_all = 0; task_all < N_TASKS; ++task_all) {
-            const int mr = MR == 1 ? 0 : task_all / N_TASKS_ROW, task = MR == 1 ? task_all : task_all - mr * N_TASKS_ROW;
-            const int mcu_y = mcu_y0 + mr;
-            if (mcu_y >= p.mcu_rows) break;
-            const uint8_t *mtile = tile + mr * MROWS * PITCH; // this MCU row's pixel rows inside the tile
-            int comp, bv = 0, bxl = lane; // component, block row inside the MCU row, block column inside the tile
-            bool full = true;
-            if (task < N_FULL) {
-                comp = Fmt<CT>::full_comp(task >= VS ? 1 : 0);
-                bv = task >= VS ? task - VS : task;
-            } else if (PAIRED) {
-                const int ci = HS * (task - N_FULL) + lane / LPC;
-                if (ci >= Fmt<CT>::NSUB) continue; // fewer 1x1 components than the task has room for: those lanes rest
-                comp = Fmt<CT>::sub_comp(ci);
-                bxl = lane % LPC;
-                full = false;
-            } else {
-                comp = Fmt<CT>::sub_comp(task - N_FULL);
-                full = !SUB;
-            }
-            const int H = full ? HS : 1, V = full ? VS : 1;
-            const int bx = mcu_x0 * H + bxl;
-            // blocks of the MCU padding exist only in the MCU-ordered layout (the interleaved scan codes them)
-            const int gy = mcu_y + p.mcu_row0; // MCU row inside the whole image (this launch may cover a slice of it)
-            if (p.mcu_order ? bx >= p.comp_pw[comp] : (bx >= p.comp_tw[comp] || gy * V + bv >= p.comp_th[comp])) continue;
-            const uint8_t *base = full ? mtile + (bv * 8) * PITCH + bxl * 8 * PXB : mtile + bxl * 8 * HS * PXB;
-
-            int v[64];
-            if constexpr (CT == JPGB_LUMA) {
-                load_block<CT, ROLE_RAW, 1, 1>(base, PITCH, v);
-            } else if constexpr (BYTES) {
-                const unsigned xorv = CT == JPGB_CMYK ? 0xFFu : 0u; // 255 - c, image_buffer.rs:247-256
-                if (full) load_block_bytes<BPP, 1, 1, PL>(base, PITCH, v, (unsigned)comp, xorv, choff);
-                else load_block_bytes<BPP, HS, VS, PL>(base, PITCH, v, (unsigned)comp, xorv, choff);
-            } else if constexpr (PAIRED) {
-                if (task >= N_FULL) load_block<CT, ROLE_CBCR, HS, VS, PL>(base, PITCH, v, &cc, choff); // lanes 0..15 Cb, 16..31 Cr
-                else if (comp == 0) load_block<CT, ROLE_Y, 1, 1, PL>(base, PITCH, v, nullptr, choff);
-                else load_block<CT, ROLE_K, 1, 1, PL>(base, PITCH, v, nullptr, choff);
-            } else {
-                if (comp == 0) load_block<CT, ROLE_Y, 1, 1, PL>(base, PITCH, v, nullptr, choff);
-                else if (comp == 1) load_block<CT, ROLE_CB, SUB ? HS : 1, SUB ? VS : 1, PL>(base, PITCH, v, nullptr, choff);
-                else if (NCOMP == 3 || comp == 2) load_block<CT, ROLE_CR, SUB ? HS : 1, SUB ? VS : 1, PL>(base, PITCH, v, nullptr, choff);
-                else load_block<CT, ROLE_K, 1, 1, PL>(base, PITCH, v, nullptr, choff);
-            }
-            dct_2d(v);
-
-            size_t blk = (size_t)img * p.blocks_per_image;
-            if (p.mcu_order) { // H, V are 1 or 2 here: bx = mcu_x * H + bh
-                const int mcu_x = H == 2 ? bx >> 1 : bx, bh = H == 2 ? bx & 1 : 0;
-                blk += ((size_t)gy * p.mcu_cols + mcu_x) * p.bpu + p.slot_base[comp] + bv * H + bh;
-            } else {
-                blk += p.comp_off[comp] + (size_t)(gy * V + bv) * p.comp_tw[comp] + bx;
-            }
-            int16_t *dst = p.coef + blk * 64;
-            if (p.comp_qt[comp] == 0) quantize_store256<0>(p, v, dst);
-            else quantize_store256<1>(p, v, dst);
-        }
-    }
+    constexpr bool CONV = false;
+    [[maybe_unused]] const jpgb_sample_format fmt{};
+#include "stage_a_warp_body.inc"
+}
+// CONV: the samples are elements of fmt.type, converted while staging; no TMA (tmap and use_tma are placeholders)
+template <int CT, int HS, int VS, bool PL>
+__global__ void __launch_bounds__(128, 4) stage_a_warp_convert_kernel(const __grid_constant__ StageAParams p,
+                                                                      const __grid_constant__ jpgb_sample_format fmt) {
+    constexpr bool CONV = true;
+    [[maybe_unused]] const CUtensorMap tmap{};
+    const int use_tma = 0;
+#include "stage_a_warp_body.inc"
 }
 
 // =================================================================================================
@@ -945,39 +890,56 @@ inline bool make_plane_tensor_map(CUtensorMap &map, const StageAParams &p, int p
               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// Grid of a persistent warp-kernel launch: the CTAs that fit at once, but no more than the warp tiles need
+template <auto Kernel, int CT, int HS, int VS>
+cudaError_t warp_grid(const StageAParams &p, size_t smem, unsigned &grid) {
+    constexpr int MR = warp_tile_mcu_rows<CT, HS, VS>(), MCUS = 32 / HS;
+    unsigned long long ctas = 0;
+    const cudaError_t e = resident_ctas<Kernel>(128, smem, ctas);
+    if (e != cudaSuccess) return e;
+    const unsigned long long n_tiles = (unsigned long long)((p.mcu_cols + MCUS - 1) / MCUS) * ((p.mcu_rows + MR - 1) / MR) * p.n_images;
+    if (ctas * 4 > n_tiles) ctas = (n_tiles + 3) / 4;
+    grid = (unsigned)ctas;
+    return cudaSuccess;
+}
+
 template <int CT, int HS, int VS, bool PL>
-cudaError_t launch_warp_variant(const StageAParams &p, cudaStream_t stream) {
+cudaError_t launch_warp_variant(const StageAParams &p, const jpgb_sample_format &fmt, cudaStream_t stream) {
     constexpr int BPP = Fmt<CT>::BPP;
     constexpr int MR = warp_tile_mcu_rows<CT, HS, VS>();
     constexpr int TILE = 256 * BPP * 8 * VS * MR;
     constexpr size_t smem = (size_t)4 * TILE + 4 * sizeof(uint64_t); // 4 warps per CTA: one private tile and one mbarrier each
-    unsigned long long grid = 0;
-    const cudaError_t e = resident_ctas<stage_a_warp_kernel<CT, HS, VS, PL>>(128, smem, grid);
-    if (e != cudaSuccess) return e;
-    constexpr int MCUS = 32 / HS;
-    const unsigned long long n_tiles = (unsigned long long)((p.mcu_cols + MCUS - 1) / MCUS) * ((p.mcu_rows + MR - 1) / MR) * p.n_images;
-    if (grid * 4 > n_tiles) grid = (n_tiles + 3) / 4;
+    unsigned grid = 0;
+    cudaError_t e;
+    if constexpr (converts(CT)) {
+        if (fmt.type) {
+            if ((e = warp_grid<stage_a_warp_convert_kernel<CT, HS, VS, PL>, CT, HS, VS>(p, smem, grid)) != cudaSuccess) return e;
+            stage_a_warp_convert_kernel<CT, HS, VS, PL><<<grid, 128, smem, stream>>>(p, fmt);
+            return cudaGetLastError();
+        }
+    }
+    if ((e = warp_grid<stage_a_warp_kernel<CT, HS, VS, PL>, CT, HS, VS>(p, smem, grid)) != cudaSuccess) return e;
     CUtensorMap tmap;
     std::memset(&tmap, 0, sizeof(tmap));
     const bool tma = PL ? make_plane_tensor_map(tmap, p, BPP, 8 * VS * MR) : make_pixel_tensor_map(tmap, p, BPP, 256 * BPP, 8 * VS * MR);
-    stage_a_warp_kernel<CT, HS, VS, PL><<<(unsigned)grid, 128, smem, stream>>>(p, tmap, tma ? 1 : 0);
+    stage_a_warp_kernel<CT, HS, VS, PL><<<grid, 128, smem, stream>>>(p, tmap, tma ? 1 : 0);
     return cudaGetLastError();
 }
 
 // the warp kernel instantiated for the luma sampling factors (a single component is always sampled 1x1)
 template <int CT, bool PL>
-cudaError_t launch_warp(const StageAParams &p, cudaStream_t stream) {
+cudaError_t launch_warp(const StageAParams &p, const jpgb_sample_format &fmt, cudaStream_t stream) {
     if constexpr (Fmt<CT>::NCOMP == 1) {
-        return launch_warp_variant<CT, 1, 1, PL>(p, stream);
+        return launch_warp_variant<CT, 1, 1, PL>(p, fmt, stream);
     } else {
-        if (p.hmax == 1 && p.vmax == 1) return launch_warp_variant<CT, 1, 1, PL>(p, stream);
-        if (p.hmax == 2 && p.vmax == 1) return launch_warp_variant<CT, 2, 1, PL>(p, stream);
-        if (p.hmax == 1 && p.vmax == 2) return launch_warp_variant<CT, 1, 2, PL>(p, stream);
-        if (p.hmax == 2 && p.vmax == 2) return launch_warp_variant<CT, 2, 2, PL>(p, stream);
-        if (p.hmax == 4 && p.vmax == 1) return launch_warp_variant<CT, 4, 1, PL>(p, stream);
-        if (p.hmax == 4 && p.vmax == 2) return launch_warp_variant<CT, 4, 2, PL>(p, stream);
-        if (p.hmax == 1 && p.vmax == 4) return launch_warp_variant<CT, 1, 4, PL>(p, stream);
-        return launch_warp_variant<CT, 2, 4, PL>(p, stream);
+        if (p.hmax == 1 && p.vmax == 1) return launch_warp_variant<CT, 1, 1, PL>(p, fmt, stream);
+        if (p.hmax == 2 && p.vmax == 1) return launch_warp_variant<CT, 2, 1, PL>(p, fmt, stream);
+        if (p.hmax == 1 && p.vmax == 2) return launch_warp_variant<CT, 1, 2, PL>(p, fmt, stream);
+        if (p.hmax == 2 && p.vmax == 2) return launch_warp_variant<CT, 2, 2, PL>(p, fmt, stream);
+        if (p.hmax == 4 && p.vmax == 1) return launch_warp_variant<CT, 4, 1, PL>(p, fmt, stream);
+        if (p.hmax == 4 && p.vmax == 2) return launch_warp_variant<CT, 4, 2, PL>(p, fmt, stream);
+        if (p.hmax == 1 && p.vmax == 4) return launch_warp_variant<CT, 1, 4, PL>(p, fmt, stream);
+        return launch_warp_variant<CT, 2, 4, PL>(p, fmt, stream);
     }
 }
 
@@ -1013,7 +975,7 @@ cudaError_t launch_planes(const StageAParams &p, cudaStream_t stream) {
 // The generic kernel's CTA tile: `groups` x 32 MCUs wide, one MCU row high, ~24 KB of pixels in shared memory. A warp
 // task is one block position of the MCU (component, v, h) in one group.
 template <int CT>
-cudaError_t launch_generic(StageAParams p, cudaStream_t stream) {
+cudaError_t launch_generic(StageAParams p, const jpgb_sample_format &fmt, cudaStream_t stream) {
     const int group_bytes = 32 * 8 * p.hmax * 8 * p.vmax * (p.planar ? p.ncomp : p.bpp);
     const int g = std::min({std::max(1, 24576 / group_bytes), 8, (p.mcu_cols + 31) / 32});
     p.groups = g;
@@ -1032,7 +994,9 @@ cudaError_t launch_generic(StageAParams p, cudaStream_t stream) {
     p.tasks_per_group = n;
     const size_t smem = (size_t)p.tile_pitch * p.tile_h_px * (p.planar ? p.ncomp : 1);
     if (smem > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(stage_a_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(stage_a_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if constexpr (converts(CT))
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(stage_a_convert_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
     const int warps = std::min(g * n, 8);
@@ -1043,38 +1007,49 @@ cudaError_t launch_generic(StageAParams p, cudaStream_t stream) {
         q.pixels = p.pixels + (size_t)i0 * p.image_stride;
         q.coef = p.coef + (size_t)i0 * p.blocks_per_image * 64;
         q.n_images = (int)std::min(n_images - i0, 65535u);
-        stage_a_kernel<CT><<<dim3(p.tiles_per_row, p.mcu_rows, q.n_images), warps * 32, smem, stream>>>(q);
+        const dim3 grid(p.tiles_per_row, p.mcu_rows, q.n_images);
+        if constexpr (converts(CT))
+            if (fmt.type) {
+                stage_a_convert_kernel<CT><<<grid, warps * 32, smem, stream>>>(q, fmt);
+                continue;
+            }
+        stage_a_kernel<CT><<<grid, warps * 32, smem, stream>>>(q);
     }
     return cudaGetLastError();
 }
 
 // packed pixels: the warp kernel, or the generic one when JPGB_FORCE_GENERIC_STAGE_A asks for the cross-check.
 // Channel-planar pixels take the warp kernel's planar staging, instantiated for Rgb (Bgr, Rgba and Bgra are Rgb with
-// their planes in another order), Cmyk and CmykAsYcck.
+// their planes in another order), Cmyk and CmykAsYcck. Samples of a wider type: the converting kernels, instantiated
+// for the colour types that take them (converts()).
 template <int CT>
-cudaError_t launch_packed(const StageAParams &p, cudaStream_t stream) {
-    if (!p.use_fast) return launch_generic<CT>(p, stream);
-    if (!p.channel_planar) return launch_warp<CT, false>(p, stream);
-    if constexpr (CT == JPGB_RGB || CT == JPGB_CMYK || CT == JPGB_CMYK_AS_YCCK) return launch_warp<CT, true>(p, stream);
+cudaError_t launch_packed(const StageAParams &p, const jpgb_sample_format &fmt, cudaStream_t stream) {
+    if (fmt.type && !converts(CT)) return cudaErrorInvalidValue;
+    if (!p.use_fast) return launch_generic<CT>(p, fmt, stream);
+    if (!p.channel_planar) return launch_warp<CT, false>(p, fmt, stream);
+    if constexpr (CT == JPGB_RGB || CT == JPGB_CMYK || CT == JPGB_CMYK_AS_YCCK) return launch_warp<CT, true>(p, fmt, stream);
     return cudaErrorInvalidValue;
 }
 
 } // namespace
 
-cudaError_t launch_stage_a(const StageAParams &p_in, uint32_t n_images, cudaStream_t stream) {
+cudaError_t launch_stage_a(const StageAParams &p_in, uint32_t n_images, const jpgb_sample_format &fmt, cudaStream_t stream) {
     StageAParams p = p_in;
     p.n_images = (int)n_images;
-    if (p.planar) return p.use_fast ? launch_planes(p, stream) : launch_generic<kPlanar>(p, stream);
+    if (p.planar) {
+        if (fmt.type) return cudaErrorInvalidValue;
+        return p.use_fast ? launch_planes(p, stream) : launch_generic<kPlanar>(p, fmt, stream);
+    }
     switch (p.color_type) {
-    case JPGB_LUMA: return launch_packed<JPGB_LUMA>(p, stream);
-    case JPGB_RGB: return launch_packed<JPGB_RGB>(p, stream);
-    case JPGB_RGBA: return launch_packed<JPGB_RGBA>(p, stream);
-    case JPGB_BGR: return launch_packed<JPGB_BGR>(p, stream);
-    case JPGB_BGRA: return launch_packed<JPGB_BGRA>(p, stream);
-    case JPGB_CMYK_AS_YCCK: return launch_packed<JPGB_CMYK_AS_YCCK>(p, stream);
-    case JPGB_YCBCR: return launch_packed<JPGB_YCBCR>(p, stream);
-    case JPGB_YCCK: return launch_packed<JPGB_YCCK>(p, stream);
-    case JPGB_CMYK: return launch_packed<JPGB_CMYK>(p, stream);
+    case JPGB_LUMA: return launch_packed<JPGB_LUMA>(p, fmt, stream);
+    case JPGB_RGB: return launch_packed<JPGB_RGB>(p, fmt, stream);
+    case JPGB_RGBA: return launch_packed<JPGB_RGBA>(p, fmt, stream);
+    case JPGB_BGR: return launch_packed<JPGB_BGR>(p, fmt, stream);
+    case JPGB_BGRA: return launch_packed<JPGB_BGRA>(p, fmt, stream);
+    case JPGB_CMYK_AS_YCCK: return launch_packed<JPGB_CMYK_AS_YCCK>(p, fmt, stream);
+    case JPGB_YCBCR: return launch_packed<JPGB_YCBCR>(p, fmt, stream);
+    case JPGB_YCCK: return launch_packed<JPGB_YCCK>(p, fmt, stream);
+    case JPGB_CMYK: return launch_packed<JPGB_CMYK>(p, fmt, stream);
     default: return cudaErrorInvalidValue;
     }
 }

@@ -160,6 +160,38 @@ class _DeviceImages(C.Structure):
     _fields_ = [("data", C.c_void_p), ("image_stride", C.c_uint64), ("row_stride", C.c_uint64), ("plane_stride", C.c_uint64)]
 
 
+class SampleType(enum.IntEnum):
+    """Element types of device images other than uint8 (JPGB_SAMPLE_*, include/jpegenc_b200.h)."""
+    U16 = 1
+    F16 = 2
+    BF16 = 3
+    F32 = 4
+
+    @property
+    def element_size(self):
+        return 4 if self == SampleType.F32 else 2
+
+
+class _SampleFormat(C.Structure):
+    _fields_ = [("type", C.c_uint32), ("scale", C.c_float), ("offset", C.c_float)]
+
+
+def sample_scale_offset(sample_type, value_range=None):
+    """(scale, offset) of jpgb_sample_format for `value_range` = (lo, hi), the values that map to 0 and 255:
+    scale = f32(255 / (hi - lo)), offset = f32(-lo * 255 / (hi - lo)), each computed in float64 and rounded once.
+    Default ranges: (0, 1) for the float types, (0, 65535) for U16."""
+    st = SampleType(sample_type)
+    lo, hi = value_range if value_range is not None else ((0.0, 65535.0) if st == SampleType.U16 else (0.0, 1.0))
+    lo, hi = float(lo), float(hi)
+    if not (np.isfinite(lo) and np.isfinite(hi)) or hi == lo:
+        raise ValueError("value_range must be two different finite numbers, got %r" % ((lo, hi),))
+    with np.errstate(over="ignore"):
+        scale, offset = np.float32(255.0 / (hi - lo)), np.float32(-lo * 255.0 / (hi - lo))
+    if not (np.isfinite(scale) and np.isfinite(offset)):
+        raise ValueError("value_range %r gives a scale or offset beyond float32" % ((lo, hi),))
+    return float(scale), float(offset)
+
+
 N_STAGES = 7
 HIST_WORDS = 2 * 2 * 257  # JPGB_HIST_WORDS
 STAGE_NAMES = ("colour_dct_quant", "histogram_tables", "code_chunks_scans", "place_chunks", "stuff_scatter", "h2d", "d2h")
@@ -197,6 +229,8 @@ def load_library():
     l.jpgb_encode_batch_device.argtypes = [vp, C.POINTER(_Params), vp, C.c_size_t, C.c_uint32,
                                            C.POINTER(vp), C.POINTER(C.c_uint64)]
     l.jpgb_encode_batch_device_strided.argtypes = [vp, C.POINTER(_Params), C.POINTER(_DeviceImages), C.c_uint32,
+                                                   C.POINTER(vp), C.POINTER(C.c_uint64)]
+    l.jpgb_encode_batch_device_samples.argtypes = [vp, C.POINTER(_Params), C.POINTER(_DeviceImages), C.POINTER(_SampleFormat), C.c_uint32,
                                                    C.POINTER(vp), C.POINTER(C.c_uint64)]
     l.jpgb_encoder_wait_stream.argtypes = [vp, vp]
     l.jpgb_scan_count.argtypes = [C.POINTER(_Params), C.POINTER(C.c_uint32)]
@@ -315,6 +349,43 @@ def _cuda_array_layout(iface, bpp, channels_first):
     layout the encoder cannot read in place."""
     if iface.get("typestr") != "|u1":
         raise ValueError("uint8 images only (typestr '|u1'), got %r" % (iface.get("typestr"),))
+    return _strided_layout(iface, bpp, channels_first, 1)
+
+
+# typestrs of the element types encode_cuda_samples reads; torch reports bfloat16 as the ambiguous '<V2'
+_SAMPLE_TYPESTRS = {"<u2": SampleType.U16, "<f2": SampleType.F16, "<f4": SampleType.F32}
+
+
+def _cuda_samples_layout(iface, bpp, channels_first, sample_type=None, is_bf16=False):
+    """_cuda_array_layout for images of a wider element type: (SampleType, data, n, width, height, image_stride,
+    row_stride, plane_stride), strides in bytes. '<V2' is bfloat16 when `sample_type` says so or `is_bf16` (a torch
+    bfloat16 tensor). Raises ValueError for another typestr, and for data or strides that are not multiples of the
+    element size."""
+    ts = iface.get("typestr")
+    want = SampleType[sample_type.upper()] if isinstance(sample_type, str) else (None if sample_type is None else SampleType(sample_type))
+    if ts in _SAMPLE_TYPESTRS:
+        st = _SAMPLE_TYPESTRS[ts]
+        if want is not None and want != st:
+            raise ValueError("typestr %r is %s, not the requested %s" % (ts, st.name, want.name))
+    elif ts == "<V2" and (want == SampleType.BF16 or (want is None and is_bf16)):
+        st = SampleType.BF16
+    elif ts == "<V2":
+        raise ValueError("typestr '<V2' is ambiguous: pass sample_type='bf16' for bfloat16 data")
+    elif ts == "|u1":
+        raise ValueError("uint8 images take encode_cuda_array")
+    else:
+        raise ValueError("sample types float32 ('<f4'), float16 ('<f2'), bfloat16 ('<V2') and uint16 ('<u2') only, got %r" % (ts,))
+    es = st.element_size
+    layout = _strided_layout(iface, bpp, channels_first, es)
+    ptr, n, w, h, image_stride, row_stride, plane_stride = layout
+    for name, v in (("data", ptr), ("image stride", image_stride), ("row stride", row_stride), ("plane stride", plane_stride)):
+        if v % es:
+            raise ValueError("%s %d is not a multiple of the element size (%d bytes)" % (name, v, es))
+    return (st,) + layout
+
+
+def _strided_layout(iface, bpp, channels_first, es):
+    """The shape and stride logic of _cuda_array_layout for elements of `es` bytes (strides stay in bytes)."""
     if iface.get("mask") is not None:
         raise ValueError("masked arrays are not supported")
     shape = tuple(int(d) for d in iface["shape"])
@@ -322,7 +393,7 @@ def _cuda_array_layout(iface, bpp, channels_first):
         raise ValueError("expected a 3-D (one image) or 4-D (batch) array, got shape %r" % (shape,))
     strides = iface.get("strides")
     if strides is None:  # C-contiguous
-        strides, step = [], 1
+        strides, step = [], es
         for d in reversed(shape):
             strides.insert(0, step)
             step *= d
@@ -338,16 +409,16 @@ def _cuda_array_layout(iface, bpp, channels_first):
     if dim["c"] != bpp:
         raise ValueError("the colour type takes %d channels, the array has %d" % (bpp, dim["c"]))
     if channels_first:
-        if stride["x"] != 1:
+        if stride["x"] != es:
             raise ValueError("x stride %d: channel-planar rows must be contiguous; make the array .contiguous() first" % stride["x"])
         plane_stride = stride["c"] if bpp > 1 else 0  # one plane is packed Luma
         if bpp > 1 and plane_stride == 0:
             raise ValueError("channel stride 0: planes at one address cannot be read; make the array .contiguous() first")
     else:
-        if stride["c"] != 1:
+        if stride["c"] != es:
             raise ValueError("channel stride %d: channels must be adjacent; make the array .contiguous() first" % stride["c"])
-        if stride["x"] != bpp:
-            raise ValueError("pixel stride %d: pixels must be %d bytes apart; make the array .contiguous() first" % (stride["x"], bpp))
+        if stride["x"] != bpp * es:
+            raise ValueError("pixel stride %d: pixels must be %d bytes apart; make the array .contiguous() first" % (stride["x"], bpp * es))
         plane_stride = 0
     if dim["x"] > 65535 or dim["y"] > 65535:
         raise ValueError("image dimensions above 65535 (%d x %d)" % (dim["x"], dim["y"]))
@@ -602,6 +673,36 @@ class Encoder:
         if iface.get("stream") is not None:
             self._dev().wait_stream(int(iface["stream"]))
         return self.encode_batch_device_strided(ptr, n, w, h, ct, image_stride, row_stride, plane_stride)
+
+    def encode_batch_device_samples(self, d_ptr, n, width, height, color_type, sample_type, image_stride, row_stride, plane_stride=0,
+                                    value_range=None):
+        """encode_batch_device_strided for samples of a wider element type (SampleType; strides in bytes): each element
+        becomes clamp(rint(x * scale + offset), 0, 255), NaN 0, with (scale, offset) from `value_range`
+        (sample_scale_offset). Returns (device pointer of the files, offsets[n+1])."""
+        dev = self._dev()
+        st = SampleType(sample_type)
+        p = self._params(width, height, ColorType(color_type))
+        im = _DeviceImages(d_ptr, image_stride, row_stride, plane_stride)
+        fmt = _SampleFormat(int(st), *sample_scale_offset(st, value_range))
+        d_files = C.c_void_p()
+        offs = (C.c_uint64 * (n + 1))()
+        rc = dev.lib.jpgb_encode_batch_device_samples(dev.handle, C.byref(p), C.byref(im), C.byref(fmt), n, C.byref(d_files), offs)
+        if rc != 0:
+            self._raise(rc)
+        return d_files.value, list(offs)
+
+    def encode_cuda_samples(self, arr, color_type, channels_first=False, value_range=None, sample_type=None):
+        """encode_cuda_array for float32, float16, bfloat16 and uint16 device images (typestr '<f4', '<f2', '<u2'; '<V2'
+        is bfloat16 for a torch bfloat16 tensor or with sample_type='bf16'). `value_range` = (lo, hi) maps lo to 0 and
+        hi to 255; default (0, 1), or (0, 65535) for uint16. Returns (device pointer of the files, offsets[n+1])."""
+        ct = ColorType(color_type)
+        iface = arr.__cuda_array_interface__
+        is_bf16 = type(arr).__module__.startswith("torch") and str(getattr(arr, "dtype", "")) == "torch.bfloat16"
+        st, ptr, n, w, h, image_stride, row_stride, plane_stride = _cuda_samples_layout(iface, ct.get_bytes_per_pixel(), channels_first,
+                                                                                       sample_type, is_bf16)
+        if iface.get("stream") is not None:
+            self._dev().wait_stream(int(iface["stream"]))
+        return self.encode_batch_device_samples(ptr, n, w, h, ct, st, image_stride, row_stride, plane_stride, value_range)
 
     # -- one large image cut into restart-aligned strips (BASELINE config 5) --
     def scan_count(self, width, height, color_type):
