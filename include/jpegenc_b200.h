@@ -198,6 +198,44 @@ typedef struct jpgb_sample_format {
 int jpgb_encode_batch_device_samples(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_images *images,
                                      const jpgb_sample_format *fmt, uint32_t n, const void **d_files, uint64_t *offsets);
 
+/* ---- YCbCr frames with subsampled chroma, as video decoders hand them out (I420, I422, I444, NV12, NV21, NV16) ----
+ * A luma plane and two chroma planes, each read where it lies. With cw = ceil(width / c_h) and ch = ceil(height / c_v),
+ * pixel (x, y) of image i is
+ *   Y  = y [i*y_image_stride + y*y_row_stride + x]
+ *   Cb = cb[i*c_image_stride + (y / c_v)*c_row_stride + (x / c_h)*c_sample_stride]
+ *   Cr = cr[i*c_image_stride + (y / c_v)*c_row_stride + (x / c_h)*c_sample_stride]
+ * that is, the full-resolution image whose chroma repeats every plane sample c_h x c_v times (nearest neighbour). The
+ * file is byte-identical to jpgb_encode_batch_device's for that image handed over packed as JPGB_YCBCR. The JPEG
+ * sampling factor is p->sampling, whatever the planes' subsampling: I420 at F_1_1 is upsampled, I444 at F_2_2 decimated,
+ * both by point sampling as every path of the encoder does.
+ * Samples are taken verbatim as full-range (JFIF) YCbCr: limited-range ("video range") samples are not expanded, and
+ * BT.709 samples are not converted to the BT.601 matrix of JFIF. */
+typedef struct jpgb_device_ycbcr {
+    const void *y, *cb, *cr;   /* image 0's first sample of each plane (NV12: cr = cb + 1; NV21: cb = cr + 1) */
+    uint64_t y_image_stride, y_row_stride;   /* bytes; an image stride of 0: every image is the same frame */
+    uint64_t c_image_stride, c_row_stride;   /* bytes, shared by Cb and Cr */
+    uint32_t c_sample_stride;  /* bytes between horizontally adjacent chroma samples: 1 planar, 2 interleaved */
+    uint8_t c_h, c_v;          /* luma samples per chroma sample across / down: 1 or 2 (I420 / NV12: 2, 2; I422 / NV16: 2, 1) */
+} jpgb_device_ycbcr;
+
+/* Encode n frames laid out as `frames` describes. Output and lifetime as for jpgb_encode_batch_device_strided.
+ * Rejected before anything is enqueued (no launch), in this order, with JPGB_ERR_BAD_PARAMS unless noted:
+ *   null arguments (frames, y, cb or cr included) or n == 0;
+ *   what jpgb_encode_batch_device rejects in `p` (same codes), except the BadImageData length check;
+ *   color_type other than Ycbcr;
+ *   c_h or c_v not 1 or 2; c_sample_stride not 1 or 2;
+ *   y_row_stride < width; c_row_stride < (cw - 1)*c_sample_stride + 1;
+ *   an extent beyond 64-bit addresses;
+ *   then for y, cb and cr in turn: not device or managed memory usable on the context's device, or a last byte read
+ *   outside the allocation that holds it. The last bytes read are
+ *     y:      (n-1)*y_image_stride + (height-1)*y_row_stride + width - 1
+ *     cb, cr: (n-1)*c_image_stride + (ch-1)*c_row_stride + (cw-1)*c_sample_stride
+ * Interleaved chroma is read in whole byte pairs up to the channel's last sample, so the kernels may read the other
+ * channel's bytes of a pair, never a byte past the last sample. A channel at an odd address is read from the byte in
+ * front of it; that byte lies in the same allocation, because allocations start at aligned addresses. */
+int jpgb_encode_batch_device_ycbcr(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_ycbcr *frames, uint32_t n,
+                                   const void **d_files, uint64_t *offsets);
+
 /* Order the context's stream after all work queued so far on `stream` (an event wait; the host does not block).
  * stream may be cudaStreamLegacy (1) or cudaStreamPerThread (2); the context's own stream is a no-op. Use it when
  * the pixels of the next encode are produced on a stream of the caller's. */

@@ -299,6 +299,53 @@ MemGetAddressRangeFn mem_get_address_range_fn() {
     return fn;
 }
 
+// One plane of device memory a call reads: n images image_stride apart, each `rows` rows of `row_bytes` bytes
+// row_stride apart, starting `offset` bytes behind `data` (a further plane of a channel-planar image)
+struct DevicePlane {
+    const void *data;
+    uint64_t image_stride, offset, rows, row_stride, row_bytes;
+};
+
+// The offset from plane.data of the last byte read, (n-1)*image_stride + offset + (rows-1)*row_stride + row_bytes - 1.
+// false: it, or data plus it, lies beyond 64-bit addresses.
+bool last_byte_read(const DevicePlane &pl, uint32_t n, uint64_t &last) {
+    uint64_t t = 0;
+    bool over = __builtin_mul_overflow((uint64_t)(n - 1), pl.image_stride, &last);
+    over |= __builtin_add_overflow(last, pl.offset, &last);
+    over |= __builtin_mul_overflow(pl.rows - 1, pl.row_stride, &t) || __builtin_add_overflow(last, t, &last);
+    over |= __builtin_add_overflow(last, pl.row_bytes - 1, &last);
+    over |= __builtin_add_overflow((uint64_t)(uintptr_t)pl.data, last, &t);
+    return !over;
+}
+
+// `data` (called `name` in the messages) is device or managed memory of the context's device, and the allocation that
+// holds it covers the bytes from data to data + last
+int check_device_range(jpgb_encoder *enc, const void *data, uint64_t last, const char *name) {
+    char m[192];
+    CK(cudaSetDevice(enc->device), "cudaSetDevice");
+    cudaPointerAttributes attr{};
+    const bool known = cudaPointerGetAttributes(&attr, data) == cudaSuccess;
+    cudaGetLastError();
+    if (!known || !(attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == enc->device))) {
+        snprintf(m, sizeof(m), "%s is not device or managed memory of the context's device", name);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    MemGetAddressRangeFn range = mem_get_address_range_fn();
+    CUdeviceptr base = 0;
+    size_t size = 0;
+    if (!range || range(&base, &size, (CUdeviceptr)(uintptr_t)data) != CUDA_SUCCESS) {
+        snprintf(m, sizeof(m), "no allocation is found at %s", name);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    const uint64_t end = (uint64_t)(uintptr_t)data + last; // the last byte read
+    if (end >= (uint64_t)base + size) {
+        snprintf(m, sizeof(m), "the described pixels end %llu bytes past the end of the allocation that holds %s",
+                 (unsigned long long)(end + 1 - ((uint64_t)base + size)), name);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    return JPGB_OK;
+}
+
 // The checks of jpgb_encode_batch_device_strided on the layout, in the order the header lists them, for samples of `es`
 // bytes (jpgb_encode_batch_device_samples). Nothing is enqueued before they pass, so no kernel reads a byte outside the
 // allocation that holds `data`.
@@ -318,29 +365,47 @@ int check_device_images(jpgb_encoder *enc, const Plan &plan, const jpgb_device_i
     // the last byte read: (n-1)*image_stride + c_max*plane_stride + (h-1)*row_stride + row_bytes - 1 (alpha is not read)
     const uint8_t ct = plan.p.color_type;
     const uint64_t c_max = !planes ? 0 : (ct == JPGB_LUMA ? 0 : (plan.bpp == 3 || ct == JPGB_RGBA || ct == JPGB_BGRA) ? 2 : 3);
-    uint64_t last = 0, t = 0;
-    bool over = __builtin_mul_overflow((uint64_t)(n - 1), im.image_stride, &last);
-    over |= __builtin_mul_overflow(c_max, im.plane_stride, &t) || __builtin_add_overflow(last, t, &last);
-    over |= __builtin_mul_overflow(h - 1, im.row_stride, &t) || __builtin_add_overflow(last, t, &last);
-    over |= __builtin_add_overflow(last, row_bytes - 1, &last);
-    over |= __builtin_add_overflow((uint64_t)(uintptr_t)im.data, last, &t);
-    if (over) return fail(enc, JPGB_ERR_BAD_PARAMS, "the described pixels extend beyond 64-bit addresses");
-    CK(cudaSetDevice(enc->device), "cudaSetDevice");
-    cudaPointerAttributes attr{};
-    const bool known = cudaPointerGetAttributes(&attr, im.data) == cudaSuccess;
-    cudaGetLastError();
-    if (!known || !(attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == enc->device)))
-        return fail(enc, JPGB_ERR_BAD_PARAMS, "data is not device or managed memory of the context's device");
-    MemGetAddressRangeFn range = mem_get_address_range_fn();
-    CUdeviceptr base = 0;
-    size_t size = 0;
-    if (!range || range(&base, &size, (CUdeviceptr)(uintptr_t)im.data) != CUDA_SUCCESS)
-        return fail(enc, JPGB_ERR_BAD_PARAMS, "no allocation is found at data");
-    const uint64_t end = (uint64_t)(uintptr_t)im.data + last; // the last byte read
-    if (end >= (uint64_t)base + size) {
-        snprintf(m, sizeof(m), "the described pixels end %llu bytes past the end of the allocation that holds data",
-                 (unsigned long long)(end + 1 - ((uint64_t)base + size)));
+    uint64_t offset = 0, last = 0;
+    const bool over = __builtin_mul_overflow(c_max, im.plane_stride, &offset);
+    if (over || !last_byte_read({im.data, im.image_stride, offset, h, im.row_stride, row_bytes}, n, last))
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "the described pixels extend beyond 64-bit addresses");
+    return check_device_range(enc, im.data, last, "data");
+}
+
+// The checks of jpgb_encode_batch_device_ycbcr on the frame layout, in the order the header lists them
+int check_device_ycbcr(jpgb_encoder *enc, const Plan &plan, const jpgb_device_ycbcr &f, uint32_t n) {
+    const uint64_t w = plan.p.width, h = plan.p.height;
+    char m[192];
+    if ((f.c_h != 1 && f.c_h != 2) || (f.c_v != 1 && f.c_v != 2)) {
+        snprintf(m, sizeof(m), "chroma subsampling c_h = %u, c_v = %u: each must be 1 or 2", f.c_h, f.c_v);
         return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    if (f.c_sample_stride != 1 && f.c_sample_stride != 2) {
+        snprintf(m, sizeof(m), "c_sample_stride %u: chroma samples must be 1 (planar) or 2 (interleaved) bytes apart", f.c_sample_stride);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    const uint64_t cw = (w + f.c_h - 1) / f.c_h, ch = (h + f.c_v - 1) / f.c_v, c_row = (cw - 1) * f.c_sample_stride + 1;
+    if (f.y_row_stride < w) {
+        snprintf(m, sizeof(m), "y_row_stride %llu is shorter than a row (%llu bytes)", (unsigned long long)f.y_row_stride, (unsigned long long)w);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    if (f.c_row_stride < c_row) {
+        snprintf(m, sizeof(m), "c_row_stride %llu is shorter than a chroma row (%llu bytes)", (unsigned long long)f.c_row_stride,
+                 (unsigned long long)c_row);
+        return fail(enc, JPGB_ERR_BAD_PARAMS, m);
+    }
+    const DevicePlane planes[3] = {{f.y, f.y_image_stride, 0, h, f.y_row_stride, w},
+                                   {f.cb, f.c_image_stride, 0, ch, f.c_row_stride, c_row},
+                                   {f.cr, f.c_image_stride, 0, ch, f.c_row_stride, c_row}};
+    uint64_t last[3];
+    for (int c = 0; c < 3; ++c)
+        if (!last_byte_read(planes[c], n, last[c])) return fail(enc, JPGB_ERR_BAD_PARAMS, "the described pixels extend beyond 64-bit addresses");
+    const char *names[3] = {"y", "cb", "cr"};
+    // An interleaved channel at an odd address is staged from the byte in front of it, the first of its pair. That byte
+    // lies in the same allocation: allocations start at aligned addresses, so an odd address is never their first byte.
+    for (int c = 0; c < 3; ++c) {
+        const int rc = check_device_range(enc, planes[c].data, last[c], names[c]);
+        if (rc != JPGB_OK) return rc;
     }
     return JPGB_OK;
 }
@@ -618,10 +683,12 @@ int stage_a_coef(jpgb_encoder *enc, const Plan &plan, uint32_t n, int16_t *&coef
     return JPGB_OK;
 }
 
-// Every colour+DCT launch of a context: timed as stage 0 and counted. `fmt`: the pixels' element type (type 0: uint8)
-int run_stage_a(jpgb_encoder *enc, const StageAParams &ap, uint32_t n, const jpgb_sample_format &fmt = {}) {
+// Every colour+DCT launch of a context: timed as stage 0 and counted. `fmt`: the pixels' element type (type 0: uint8).
+// `frame`: the pixels are the subsampled planes of a jpgb_device_ycbcr
+int run_stage_a(jpgb_encoder *enc, const StageAParams &ap, uint32_t n, const jpgb_sample_format &fmt = {}, const jpgb_device_ycbcr *frame = nullptr) {
     StageTimer t(enc, 0);
-    CK(launch_stage_a(ap, n, fmt, enc->stream), "stage A launch");
+    if (frame) CK(launch_stage_a_frames(ap, n, *frame, enc->stream), "stage A launch");
+    else CK(launch_stage_a(ap, n, fmt, enc->stream), "stage A launch");
     enc->launches += 1;
     return JPGB_OK;
 }
@@ -650,7 +717,7 @@ int encode_device(jpgb_encoder *enc, const Plan &plan, const jpgb_device_images 
         if ((rc = stage_a_coef(enc, plan, n, coef)) != JPGB_OK) return rc;
         StageAParams ap;
         plan.fill_stage_a(ap, images, coef);
-        if ((rc = run_stage_a(enc, ap, n, plan.sample)) != JPGB_OK) return rc;
+        if ((rc = run_stage_a(enc, ap, n, plan.sample, plan.frame.y ? &plan.frame : nullptr)) != JPGB_OK) return rc;
     }
 
     HeaderLayout hl;
@@ -1301,6 +1368,25 @@ int jpgb_encode_batch_device_samples(jpgb_encoder *enc, const jpgb_params *p, co
     if (rc != JPGB_OK) return rc;
     plan.sample = *fmt;
     return encode_batch_device(enc, plan, *images, n, d_files, offsets);
+}
+
+int jpgb_encode_batch_device_ycbcr(jpgb_encoder *enc, const jpgb_params *p, const jpgb_device_ycbcr *frames, uint32_t n,
+                                   const void **d_files, uint64_t *offsets) {
+    if (!enc) return JPGB_ERR_BAD_PARAMS;
+    enc->launches = 0; // a rejected call reports no launches
+    if (!frames || !frames->y || !frames->cb || !frames->cr || !d_files || !offsets || n == 0)
+        return fail(enc, JPGB_ERR_BAD_PARAMS, "null argument");
+    Plan plan;
+    int rc = validate_and_plan(enc, p, SIZE_MAX, plan); // a strided layout has no length to check
+    if (rc != JPGB_OK) return rc;
+    if (p->color_type != JPGB_YCBCR) return fail(enc, JPGB_ERR_BAD_PARAMS, "YCbCr frames take color_type Ycbcr");
+    rc = check_device_ycbcr(enc, plan, *frames, n);
+    if (rc != JPGB_OK) return rc;
+    // the planes of the ImageBuffer path, read by stage A at their own resolution; the luma plane stands for them
+    plan.planar = true;
+    plan.frame = *frames;
+    const jpgb_device_images luma{frames->y, frames->y_image_stride, frames->y_row_stride, 0};
+    return encode_batch_device(enc, plan, luma, n, d_files, offsets);
 }
 
 int jpgb_encoder_wait_stream(jpgb_encoder *enc, void *stream) {

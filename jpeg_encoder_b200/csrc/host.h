@@ -86,6 +86,7 @@ struct Plan {
     // strip mode (strip != nullptr): geometry of the strip, header of the whole image
     bool planar = false; // ImageBuffer path: one plane per component, samples taken verbatim
     jpgb_sample_format sample{}; // element type of device pixels (type 0: uint8); stage A converts the others while staging
+    jpgb_device_ycbcr frame{};   // y != nullptr: the planes of subsampled YCbCr frames, which stage A reads (planar is set)
     bool is_strip = false;
     // set before build: a strip of an image without restart intervals (restart_interval must be 0). Its scans are coded
     // against the DC values of the strip in front and come out as bare bit strings (DevPlan::bare)

@@ -43,6 +43,9 @@ cudaError_t resident_ctas(int threads, size_t smem, unsigned long long &ctas) {
 // stage_a.cu -- colour + decimate + level shift + fDCT + quantize -> zig-zag i16 coefficients. `fmt`: the element
 // type of the pixels (type 0: uint8), converted to 8-bit samples while staging
 cudaError_t launch_stage_a(const StageAParams &p, uint32_t n_images, const jpgb_sample_format &fmt, cudaStream_t stream);
+// The same for the subsampled planes of `frame` (p: a planar Ycbcr plan). The block geometry and coefficient
+// destinations come from p, the samples from the frame's planes.
+cudaError_t launch_stage_a_frames(const StageAParams &p, uint32_t n_images, const jpgb_device_ycbcr &frame, cudaStream_t stream);
 
 // Huffman code tables as the kernels see them: [image][table 0|1][class dc|ac][256] of (size<<16)|code
 constexpr size_t kHuffWordsPerImage = 2 * 2 * 256;

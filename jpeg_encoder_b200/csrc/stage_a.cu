@@ -290,9 +290,10 @@ __device__ __forceinline__ void stage_convert_tile(uint8_t *tile, const uint8_t 
 }
 
 // The generic kernel's body: a CTA tile of `groups` x 32 MCUs x one MCU row. CONV: the samples are elements of
-// fmt.type, converted while staging.
-template <int CT, bool CONV>
-__device__ __forceinline__ void generic_tile(const StageAParams &p, const jpgb_sample_format &fmt) {
+// fmt.type, converted while staging. FRAME (CT == kPlanar): the planes are those of `frame`, subsampled, staged
+// upsampled to full resolution with byte loads.
+template <int CT, bool CONV, bool FRAME = false>
+__device__ __forceinline__ void generic_tile(const StageAParams &p, const jpgb_sample_format &fmt, const jpgb_device_ycbcr &frame = {}) {
     extern __shared__ __align__(128) uint8_t tile[];
     constexpr int BPP = (CT == JPGB_LUMA || CT == kPlanar) ? 1 : ((CT == JPGB_RGB || CT == JPGB_BGR || CT == JPGB_YCBCR) ? 3 : 4);
     constexpr bool PLANAR = CT == kPlanar;
@@ -316,6 +317,14 @@ __device__ __forceinline__ void generic_tile(const StageAParams &p, const jpgb_s
         const int sy = min(py0 + ry, p.height - 1);
         const uint8_t *row = src + (size_t)plane * p.plane_stride + (size_t)sy * p.row_stride + (size_t)px0 * px_bytes;
         uint8_t *dst = tile + plane * plane_tile + ry * p.tile_pitch;
+        if constexpr (FRAME) { // the mapping of jpgb_device_ycbcr restated: plane row sy / c_v, column (px / c_h) * c_sample_stride
+            const int sh = plane ? frame.c_h : 1, sv = plane ? frame.c_v : 1, ss = plane ? (int)frame.c_sample_stride : 1;
+            const uint8_t *fr = static_cast<const uint8_t *>(plane == 0 ? frame.y : (plane == 1 ? frame.cb : frame.cr)) +
+                                (size_t)img * (plane ? frame.c_image_stride : frame.y_image_stride) +
+                                (size_t)(sy / sv) * (plane ? frame.c_row_stride : frame.y_row_stride);
+            for (int b = 0; b < 16; ++b) dst[cb + b] = fr[(size_t)((px0 + min(cb + b, valid_px - 1)) / sh) * ss];
+            continue;
+        }
         if (CONV) stage_convert_edge(dst, row, cb, 16, BPP, valid_px, fmt, p.channel_planar ? p.plane_of : nullptr, p.plane_stride);
         else if (p.channel_planar) stage_planes_chunk<BPP>(dst, row, p.plane_stride, p.plane_of, cb, valid_px);
         else if (cb + 16 <= valid_bytes && ((reinterpret_cast<uintptr_t>(row + cb) & 15) == 0))
@@ -368,6 +377,11 @@ __global__ void __launch_bounds__(256) stage_a_kernel(const __grid_constant__ St
 template <int CT>
 __global__ void __launch_bounds__(256) stage_a_convert_kernel(const __grid_constant__ StageAParams p, const __grid_constant__ jpgb_sample_format fmt) {
     generic_tile<CT, true>(p, fmt);
+}
+// the cross-check of jpgb_encode_batch_device_ycbcr (JPGB_FORCE_GENERIC_STAGE_A=1)
+__global__ void __launch_bounds__(256) stage_a_frame_generic_kernel(const __grid_constant__ StageAParams p,
+                                                                    const __grid_constant__ jpgb_device_ycbcr frame) {
+    generic_tile<kPlanar, false, true>(p, jpgb_sample_format{}, frame);
 }
 
 
@@ -833,6 +847,159 @@ __global__ void __launch_bounds__(128, 4) stage_a_plane_kernel(const __grid_cons
     }
 }
 
+// =================================================================================================
+// Subsampled YCbCr frames (jpgb_encode_batch_device_ycbcr): one launch per component, each reading its own plane.
+// A frame means the full-resolution image whose chroma repeats every plane sample c_h x c_v times. Its block sample at
+// full-resolution column X = bx*8*sx + k*sx (sx: the component's decimation) reads column min(X, w-1), which is plane
+// column min(X / c_h, cw - 1): the plane is read at its own resolution and clamped at its own edge, rows alike.
+// With sx >= c_h and sy >= c_v and one byte per sample, that is stage_a_plane_kernel<sx / c_h, sy / c_v> on the plane
+// (its launch's pixels, width and height describe the plane). stage_a_frame_kernel covers the rest:
+//   NX, NY: the step between block samples in half plane samples (1, 2, 4, 8). Step 1 (sx = 1 < c_h = 2): each plane
+//           sample feeds two block samples; block sample k reads plane sample (k * NX) / 2 of the block's span.
+//   BPP:    bytes between horizontally adjacent samples (2: interleaved Cb/Cr). The channel read is byte `coff` of a
+//           pair; p.pixels is the pair's first byte, so the edge clamp lands on the same channel's last sample.
+//           n_comp = 2 (Cb and Cr in the two bytes of the same pairs, NV12 / NV21): one launch codes components comp and
+//           comp + 1, the second from byte coff ^ 1, so the interleaved plane is staged once for both.
+// A warp tile is 32 blocks x MR block rows; only the plane rows the blocks read are staged (cp.async).
+// =================================================================================================
+template <int NX, int NY, int BPP>
+struct FrameTile {
+    static constexpr int SPAN = 4 * NX;             // plane samples under a block row
+    static constexpr int PITCH = 32 * SPAN * BPP;   // bytes of a staged row
+    static constexpr int R = NY == 1 ? 4 : 8;       // plane rows under a block
+    static constexpr int YSTEP = NY == 1 ? 1 : NY / 2;
+    static constexpr int FIT = 8192 / (PITCH * R);  // block rows in about 8 KB
+    static constexpr int MR = FIT < 1 ? 1 : (FIT > 8 ? 8 : FIT);
+    static constexpr int ROWS = R * MR, TILE_BYTES = PITCH * ROWS;
+};
+
+// One 16-byte chunk of a staged frame row, byte by byte, the row's last valid sample of each channel replicated.
+// coff >= 0: only byte coff of a pair is read, and the pair's other byte gets that channel's sample too (it is never
+// read); coff < 0: both channels. Cold path, kept out of line.
+template <int BPP>
+__device__ __noinline__ void stage_frame_edge_chunk(uint8_t *dst, const uint8_t *row, int cb, int valid_px, int coff) {
+    for (int b = 0; b < 16; ++b) dst[cb + b] = row[(coff < 0 ? (cb + b) % BPP : coff) + min((cb + b) / BPP, valid_px - 1) * BPP];
+}
+
+template <int NX, int BPP, int I, int NW>
+__device__ __forceinline__ int frame_sample_at(const uint32_t (&w)[NW], unsigned coff) {
+    constexpr int O = (I * NX / 2) * BPP;
+    return (int)__byte_perm(w[O >> 2], 0, 0x4440 + (O & 3) + (BPP == 1 ? 0u : coff));
+}
+template <int NX, int BPP, int NW, int... Is>
+__device__ __forceinline__ void frame_row(const uint32_t (&w)[NW], int *s, unsigned coff, std::integer_sequence<int, Is...>) {
+    ((s[Is] = frame_sample_at<NX, BPP, Is, NW>(w, coff)), ...);
+}
+// the 8 samples of a block row: the words under its 4 * NX samples (row: 4 * NX * BPP-byte aligned), then the bytes
+template <int NX, int BPP>
+__device__ __forceinline__ void load_frame_row(const uint8_t *row, int *s, unsigned coff) {
+    constexpr int NW = NX * BPP;
+    uint32_t w[NW];
+    if constexpr (NW % 4 == 0) {
+#pragma unroll
+        for (int i = 0; i < NW / 4; ++i) {
+            const uint4 a = reinterpret_cast<const uint4 *>(row)[i];
+            w[4 * i] = a.x;
+            w[4 * i + 1] = a.y;
+            w[4 * i + 2] = a.z;
+            w[4 * i + 3] = a.w;
+        }
+    } else if constexpr (NW == 2) {
+        const uint2 a = *reinterpret_cast<const uint2 *>(row);
+        w[0] = a.x;
+        w[1] = a.y;
+    } else {
+        w[0] = *reinterpret_cast<const uint32_t *>(row);
+    }
+    frame_row<NX, BPP, NW>(w, s, coff, std::make_integer_sequence<int, 8>{});
+}
+
+template <int NX, int NY, int BPP>
+__global__ void __launch_bounds__(128, 4) stage_a_frame_kernel(const __grid_constant__ StageAParams p, const int comp, const int coff,
+                                                                       const int n_comp) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    using T = FrameTile<NX, NY, BPP>;
+    constexpr int SPAN = T::SPAN, PITCH = T::PITCH, R = T::R, YSTEP = T::YSTEP, MR = T::MR, ROWS = T::ROWS;
+    const int lane = threadIdx.x & 31;
+    const unsigned warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const unsigned n_warps_total = (gridDim.x * blockDim.x) >> 5;
+    uint8_t *tile = smem + (threadIdx.x >> 5) * T::TILE_BYTES;
+    const int H = p.comp_h[comp], V = p.comp_v[comp];
+    const int tw = p.mcu_order ? p.comp_pw[comp] : p.comp_tw[comp];
+    const int th = p.mcu_order ? p.mcu_rows * V : min(p.mcu_rows * V, p.comp_th[comp] - p.mcu_row0 * V);
+    if (th <= 0) return;
+    const unsigned tiles_per_row = ((unsigned)tw + 31) / 32, tile_rows = ((unsigned)th + MR - 1) / MR;
+    const unsigned n_tiles = tiles_per_row * tile_rows * p.n_images;
+    const int needed_total = tw * SPAN * BPP; // bytes of a row the blocks read (beyond the plane: its last sample repeated)
+
+    for (unsigned t = warp_global; t < n_tiles; t += n_warps_total) {
+        const unsigned tx = t % tiles_per_row, r = t / tiles_per_row;
+        const int by0 = (int)(r % tile_rows) * MR, img = (int)(r / tile_rows);
+        const int bx0 = (int)tx * 32;
+        const int px0 = bx0 * SPAN, py0 = by0 * 4 * NY; // in plane samples and rows
+        const uint8_t *src = p.pixels + (size_t)img * p.image_stride + (size_t)px0 * BPP;
+        const int valid_px = p.width - px0;                     // > 0: a tile starts inside the image
+        const int valid_bytes = n_comp == 2 ? valid_px * BPP : coff + (valid_px - 1) * BPP + 1; // up to the channel's last sample
+        const int needed_bytes = min(PITCH, needed_total - px0 * BPP);
+        __syncwarp(); // all lanes are done reading the previous tile
+        const bool interior = PITCH <= valid_bytes && py0 + (ROWS - 1) * YSTEP < p.height && (p.row_stride & 15) == 0 &&
+                              (reinterpret_cast<uintptr_t>(src) & 15) == 0;
+        if (interior) {
+            const uint8_t *g = src + (size_t)py0 * p.row_stride + lane * 16;
+            uint8_t *d = tile + lane * 16;
+#pragma unroll 4
+            for (int ry = 0; ry < ROWS; ++ry) {
+#pragma unroll
+                for (int c = 0; c < (PITCH + 511) / 512; ++c)
+                    if (c * 512 + 512 <= PITCH || lane * 16 + c * 512 < PITCH) cp_async16(d + c * 512, g + c * 512);
+                g += (size_t)YSTEP * p.row_stride;
+                d += PITCH;
+            }
+        } else {
+#pragma unroll 1
+            for (int ry = 0; ry < ROWS; ++ry) {
+                const uint8_t *row = src + (size_t)min(py0 + ry * YSTEP, p.height - 1) * p.row_stride;
+                uint8_t *dst = tile + ry * PITCH;
+                const bool aligned = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
+#pragma unroll 1
+                for (int cb = lane * 16; cb < needed_bytes; cb += 32 * 16) {
+                    if (aligned && cb + 16 <= valid_bytes) cp_async16(dst + cb, row + cb);
+                    else stage_frame_edge_chunk<BPP>(dst, row, cb, valid_px, n_comp == 2 ? -1 : coff);
+                }
+            }
+        }
+        cp_async_commit();
+        cp_async_wait<0>();
+        __syncwarp();
+#pragma unroll 1
+        for (int mr = 0; mr < MR; ++mr) {
+            const int by = by0 + mr, bx = bx0 + lane;
+            if (by >= th) break;
+            if (bx >= tw) continue;
+            const uint8_t *base = tile + mr * R * PITCH + lane * SPAN * BPP;
+            const int gby = by + p.mcu_row0 * V; // block row inside the whole image
+#pragma unroll 1
+            for (int k = 0; k < (BPP == 2 ? n_comp : 1); ++k) { // the components share their sampling factors
+                const int c = comp + k;
+                int v[64];
+#pragma unroll
+                for (int y = 0; y < 8; ++y) load_frame_row<NX, BPP>(base + (NY == 1 ? y / 2 : y) * PITCH, &v[y * 8], (unsigned)(coff ^ k));
+                dct_2d(v);
+                size_t blk = (size_t)img * p.blocks_per_image;
+                if (p.mcu_order) {
+                    const int mcu_x = bx / H, bh = bx - mcu_x * H, gy = gby / V, bv = gby - gy * V;
+                    blk += ((size_t)gy * p.mcu_cols + mcu_x) * p.bpu + p.slot_base[c] + bv * H + bh;
+                } else {
+                    blk += p.comp_off[c] + (size_t)gby * p.comp_tw[c] + bx;
+                }
+                int16_t *dst = p.coef + blk * 64;
+                if (p.comp_qt[c] == 0) quantize_store256<0>(p, v, dst);
+                else quantize_store256<1>(p, v, dst);
+            }
+        }
+    }
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -972,10 +1139,69 @@ cudaError_t launch_planes(const StageAParams &p, cudaStream_t stream) {
     return cudaSuccess;
 }
 
+template <int NX, int NY, int BPP>
+cudaError_t launch_frame_variant(const StageAParams &p, int comp, int coff, int n_comp, cudaStream_t stream) {
+    using T = FrameTile<NX, NY, BPP>;
+    constexpr size_t smem = (size_t)4 * T::TILE_BYTES;
+    unsigned long long grid = 0;
+    const cudaError_t e = resident_ctas<stage_a_frame_kernel<NX, NY, BPP>>(128, smem, grid);
+    if (e != cudaSuccess) return e;
+    const int tw = p.mcu_order ? p.comp_pw[comp] : p.comp_tw[comp], th = p.mcu_rows * p.comp_v[comp];
+    const unsigned long long n_tiles = (unsigned long long)((tw + 31) / 32) * ((th + T::MR - 1) / T::MR) * p.n_images;
+    if (grid * 4 > n_tiles) grid = (n_tiles + 3) / 4;
+    stage_a_frame_kernel<NX, NY, BPP><<<(unsigned)grid, 128, smem, stream>>>(p, comp, coff, n_comp);
+    return cudaGetLastError();
+}
+
+// subsampled YCbCr frames: one launch per component, each with its own plane as p.pixels, width, height, row_stride
+// and image_stride; the block geometry and coefficient destinations stay the image's. Cb and Cr in the two bytes of the
+// same pairs (NV12, NV21) share one launch: the interleaved plane is read once.
+cudaError_t launch_frames(const StageAParams &p, const jpgb_device_ycbcr &f, cudaStream_t stream) {
+    const uint8_t *cb = static_cast<const uint8_t *>(f.cb), *cr = static_cast<const uint8_t *>(f.cr);
+    const bool pairs = f.c_sample_stride == 2 && (cr == cb + 1 || cb == cr + 1);
+    for (int c = 0; c < 3; c += (c == 1 && pairs) ? 2 : 1) {
+        const int ch = c ? f.c_h : 1, cv = c ? f.c_v : 1, bpp = c ? (int)f.c_sample_stride : 1;
+        const int n_comp = (c == 1 && pairs) ? 2 : 1;
+        const uint8_t *plane = c == 0 ? static_cast<const uint8_t *>(f.y) : (c == 1 ? cb : cr);
+        const int coff = n_comp == 2 ? (cb > cr ? 1 : 0) : (bpp == 2 ? (int)(reinterpret_cast<uintptr_t>(plane) & 1) : 0); // the channel's byte in its pair
+        StageAParams q = p;
+        q.pixels = plane - coff;
+        q.width = (p.width + ch - 1) / ch;
+        q.height = (p.height + cv - 1) / cv;
+        q.row_stride = c ? f.c_row_stride : f.y_row_stride;
+        q.image_stride = c ? f.c_image_stride : f.y_image_stride;
+        q.plane_stride = 0;
+        const int nx = 2 * (p.hmax / p.comp_h[c]) / ch, ny = 2 * (p.vmax / p.comp_v[c]) / cv; // steps in half samples
+        cudaError_t e = cudaErrorInvalidValue;
+        if (bpp == 1 && nx >= 2 && ny >= 2) {
+#define JPGB_PLANE(X, Y) \
+    if (nx == 2 * X && ny == 2 * Y) e = launch_plane_variant<X, Y>(q, c, stream);
+            JPGB_PLANE(1, 1) JPGB_PLANE(2, 1) JPGB_PLANE(1, 2) JPGB_PLANE(2, 2)
+            JPGB_PLANE(4, 1) JPGB_PLANE(4, 2) JPGB_PLANE(1, 4) JPGB_PLANE(2, 4) JPGB_PLANE(4, 4)
+#undef JPGB_PLANE
+        } else {
+#define JPGB_FRAME(X, Y, B) \
+    if (nx == X && ny == Y && bpp == B) e = launch_frame_variant<X, Y, B>(q, c, coff, n_comp, stream);
+            // one byte per sample: only the steps of half a sample
+            JPGB_FRAME(1, 1, 1) JPGB_FRAME(1, 2, 1) JPGB_FRAME(1, 4, 1) JPGB_FRAME(1, 8, 1)
+            JPGB_FRAME(2, 1, 1) JPGB_FRAME(4, 1, 1) JPGB_FRAME(8, 1, 1)
+            // interleaved: every step the 8 JPEG samplings and the 4 chroma subsamplings give
+            JPGB_FRAME(1, 1, 2) JPGB_FRAME(1, 2, 2) JPGB_FRAME(1, 4, 2) JPGB_FRAME(1, 8, 2)
+            JPGB_FRAME(2, 1, 2) JPGB_FRAME(2, 2, 2) JPGB_FRAME(2, 4, 2) JPGB_FRAME(2, 8, 2)
+            JPGB_FRAME(4, 1, 2) JPGB_FRAME(4, 2, 2) JPGB_FRAME(4, 4, 2) JPGB_FRAME(4, 8, 2)
+            JPGB_FRAME(8, 1, 2) JPGB_FRAME(8, 2, 2) JPGB_FRAME(8, 4, 2)
+#undef JPGB_FRAME
+        }
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 // The generic kernel's CTA tile: `groups` x 32 MCUs wide, one MCU row high, ~24 KB of pixels in shared memory. A warp
-// task is one block position of the MCU (component, v, h) in one group.
+// task is one block position of the MCU (component, v, h) in one group. `frame`: the planes of a subsampled YCbCr
+// frame batch (CT == kPlanar)
 template <int CT>
-cudaError_t launch_generic(StageAParams p, const jpgb_sample_format &fmt, cudaStream_t stream) {
+cudaError_t launch_generic(StageAParams p, const jpgb_sample_format &fmt, cudaStream_t stream, const jpgb_device_ycbcr *frame = nullptr) {
     const int group_bytes = 32 * 8 * p.hmax * 8 * p.vmax * (p.planar ? p.ncomp : p.bpp);
     const int g = std::min({std::max(1, 24576 / group_bytes), 8, (p.mcu_cols + 31) / 32});
     p.groups = g;
@@ -997,6 +1223,7 @@ cudaError_t launch_generic(StageAParams p, const jpgb_sample_format &fmt, cudaSt
         cudaError_t e = cudaFuncSetAttribute(stage_a_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if constexpr (converts(CT))
             if (e == cudaSuccess) e = cudaFuncSetAttribute(stage_a_convert_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (frame && e == cudaSuccess) e = cudaFuncSetAttribute(stage_a_frame_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
     const int warps = std::min(g * n, 8);
@@ -1008,6 +1235,14 @@ cudaError_t launch_generic(StageAParams p, const jpgb_sample_format &fmt, cudaSt
         q.coef = p.coef + (size_t)i0 * p.blocks_per_image * 64;
         q.n_images = (int)std::min(n_images - i0, 65535u);
         const dim3 grid(p.tiles_per_row, p.mcu_rows, q.n_images);
+        if (frame) {
+            jpgb_device_ycbcr f = *frame;
+            f.y = static_cast<const uint8_t *>(f.y) + (size_t)i0 * f.y_image_stride;
+            f.cb = static_cast<const uint8_t *>(f.cb) + (size_t)i0 * f.c_image_stride;
+            f.cr = static_cast<const uint8_t *>(f.cr) + (size_t)i0 * f.c_image_stride;
+            stage_a_frame_generic_kernel<<<grid, warps * 32, smem, stream>>>(q, f);
+            continue;
+        }
         if constexpr (converts(CT))
             if (fmt.type) {
                 stage_a_convert_kernel<CT><<<grid, warps * 32, smem, stream>>>(q, fmt);
@@ -1052,6 +1287,13 @@ cudaError_t launch_stage_a(const StageAParams &p_in, uint32_t n_images, const jp
     case JPGB_CMYK: return launch_packed<JPGB_CMYK>(p, fmt, stream);
     default: return cudaErrorInvalidValue;
     }
+}
+
+cudaError_t launch_stage_a_frames(const StageAParams &p_in, uint32_t n_images, const jpgb_device_ycbcr &frame, cudaStream_t stream) {
+    StageAParams p = p_in;
+    p.n_images = (int)n_images;
+    if (!p.planar || p.ncomp != 3) return cudaErrorInvalidValue;
+    return p.use_fast ? launch_frames(p, frame, stream) : launch_generic<kPlanar>(p, jpgb_sample_format{}, stream, &frame);
 }
 
 } // namespace jpgb

@@ -160,6 +160,12 @@ class _DeviceImages(C.Structure):
     _fields_ = [("data", C.c_void_p), ("image_stride", C.c_uint64), ("row_stride", C.c_uint64), ("plane_stride", C.c_uint64)]
 
 
+class _DeviceYcbcr(C.Structure):
+    _fields_ = [("y", C.c_void_p), ("cb", C.c_void_p), ("cr", C.c_void_p), ("y_image_stride", C.c_uint64), ("y_row_stride", C.c_uint64),
+                ("c_image_stride", C.c_uint64), ("c_row_stride", C.c_uint64), ("c_sample_stride", C.c_uint32), ("c_h", C.c_uint8),
+                ("c_v", C.c_uint8)]
+
+
 class SampleType(enum.IntEnum):
     """Element types of device images other than uint8 (JPGB_SAMPLE_*, include/jpegenc_b200.h)."""
     U16 = 1
@@ -232,6 +238,8 @@ def load_library():
                                                    C.POINTER(vp), C.POINTER(C.c_uint64)]
     l.jpgb_encode_batch_device_samples.argtypes = [vp, C.POINTER(_Params), C.POINTER(_DeviceImages), C.POINTER(_SampleFormat), C.c_uint32,
                                                    C.POINTER(vp), C.POINTER(C.c_uint64)]
+    l.jpgb_encode_batch_device_ycbcr.argtypes = [vp, C.POINTER(_Params), C.POINTER(_DeviceYcbcr), C.c_uint32, C.POINTER(vp),
+                                                 C.POINTER(C.c_uint64)]
     l.jpgb_encoder_wait_stream.argtypes = [vp, vp]
     l.jpgb_scan_count.argtypes = [C.POINTER(_Params), C.POINTER(C.c_uint32)]
     l.jpgb_plan_strips.argtypes = [C.POINTER(_Params), C.c_uint32, C.POINTER(_Strip), C.POINTER(C.c_uint32)]
@@ -384,28 +392,36 @@ def _cuda_samples_layout(iface, bpp, channels_first, sample_type=None, is_bf16=F
     return (st,) + layout
 
 
-def _strided_layout(iface, bpp, channels_first, es):
-    """The shape and stride logic of _cuda_array_layout for elements of `es` bytes (strides stay in bytes)."""
+def _shape_strides(iface, es, ndims, what):
+    """Shape and byte strides of an interface dict of `es`-byte elements with one of the dimension counts `ndims`
+    (C-contiguous when it gives no strides)."""
     if iface.get("mask") is not None:
         raise ValueError("masked arrays are not supported")
     shape = tuple(int(d) for d in iface["shape"])
-    if len(shape) not in (3, 4):
-        raise ValueError("expected a 3-D (one image) or 4-D (batch) array, got shape %r" % (shape,))
+    if len(shape) not in ndims:
+        raise ValueError("expected %s, got shape %r" % (what, shape))
     strides = iface.get("strides")
     if strides is None:  # C-contiguous
         strides, step = [], es
         for d in reversed(shape):
             strides.insert(0, step)
             step *= d
-    strides = tuple(int(x) for x in strides)
-    names = ("c", "y", "x") if channels_first else ("y", "x", "c")
-    if len(shape) == 4:
-        names = ("n",) + names
+    return shape, tuple(int(x) for x in strides)
+
+
+def _named(shape, strides, names):
+    """{name: extent} and {name: stride} of the dimensions, the leading ones named first; negative strides rejected"""
+    names = names[len(names) - len(shape):]
     for name, st in zip(names, strides):
         if st < 0:
             raise ValueError("negative %s stride %d: make the array .contiguous() first" % (name, st))
-    dim = dict(zip(names, shape))
-    stride = dict(zip(names, strides))
+    return dict(zip(names, shape)), dict(zip(names, strides))
+
+
+def _strided_layout(iface, bpp, channels_first, es):
+    """The shape and stride logic of _cuda_array_layout for elements of `es` bytes (strides stay in bytes)."""
+    shape, strides = _shape_strides(iface, es, (3, 4), "a 3-D (one image) or 4-D (batch) array")
+    dim, stride = _named(shape, strides, ("n", "c", "y", "x") if channels_first else ("n", "y", "x", "c"))
     if dim["c"] != bpp:
         raise ValueError("the colour type takes %d channels, the array has %d" % (bpp, dim["c"]))
     if channels_first:
@@ -423,6 +439,51 @@ def _strided_layout(iface, bpp, channels_first, es):
     if dim["x"] > 65535 or dim["y"] > 65535:
         raise ValueError("image dimensions above 65535 (%d x %d)" % (dim["x"], dim["y"]))
     return (int(iface["data"][0]), dim.get("n", 1), dim["x"], dim["y"], stride.get("n", 0), stride["y"], plane_stride)
+
+
+def _subsampling(full, sub, axis):
+    """Luma samples per chroma sample along `axis`: 1 when the chroma plane is as long as the luma plane, 2 when it is
+    ceil(full / 2) long (a length of 1 reads the same either way and is 1)."""
+    if sub == full:
+        return 1
+    if sub == (full + 1) // 2:
+        return 2
+    raise ValueError("chroma %s %d fits no subsampling of luma %s %d: it must be %d (1:1) or %d (2:1)"
+                     % (axis, sub, axis, full, full, (full + 1) // 2))
+
+
+def _cuda_ycbcr_layout(y_iface, cb_iface, cr_iface):
+    """The jpgb_device_ycbcr of three `__cuda_array_interface__` dicts: y (N, H, W) / (H, W) uint8 and cb, cr
+    (N, ch, cw) / (ch, cw) uint8 views with the same strides, x stride 1 (planar) or 2 (interleaved). Returns
+    (y, cb, cr, n, width, height, y_image_stride, y_row_stride, c_image_stride, c_row_stride, c_sample_stride, c_h, c_v).
+    Raises ValueError for a layout the encoder cannot read in place."""
+    for name, iface in (("y", y_iface), ("cb", cb_iface), ("cr", cr_iface)):
+        if iface.get("typestr") != "|u1":
+            raise ValueError("uint8 planes only (typestr '|u1'), %s has %r" % (name, iface.get("typestr")))
+    what = "a 2-D (one frame) or 3-D (batch) plane"
+    ys, yst = _shape_strides(y_iface, 1, (2, 3), what)
+    cs, cst = _shape_strides(cb_iface, 1, (2, 3), what)
+    rs, rst = _shape_strides(cr_iface, 1, (2, 3), what)
+    if not (len(ys) == len(cs) == len(rs)):
+        raise ValueError("y, cb and cr must all be batches or all single frames, got shapes %r, %r, %r" % (ys, cs, rs))
+    if cs != rs:
+        raise ValueError("cb and cr shapes differ: %r and %r" % (cs, rs))
+    if cst != rst:
+        raise ValueError("cb and cr strides differ: %r and %r" % (cst, rst))
+    ydim, ystride = _named(ys, yst, ("n", "y", "x"))
+    cdim, cstride = _named(cs, cst, ("n", "y", "x"))
+    if ydim.get("n", 1) != cdim.get("n", 1):
+        raise ValueError("y holds %d frames, cb and cr %d" % (ydim["n"], cdim["n"]))
+    if ystride["x"] != 1:
+        raise ValueError("y x stride %d: luma rows must be contiguous; make the array .contiguous() first" % ystride["x"])
+    if cstride["x"] not in (1, 2):
+        raise ValueError("chroma x stride %d: chroma samples must be 1 (planar) or 2 (interleaved) bytes apart" % cstride["x"])
+    w, h = ydim["x"], ydim["y"]
+    if w > 65535 or h > 65535:
+        raise ValueError("image dimensions above 65535 (%d x %d)" % (w, h))
+    c_h, c_v = _subsampling(w, cdim["x"], "width"), _subsampling(h, cdim["y"], "height")
+    return (int(y_iface["data"][0]), int(cb_iface["data"][0]), int(cr_iface["data"][0]), ydim.get("n", 1), w, h,
+            ystride.get("n", 0), ystride["y"], cstride.get("n", 0), cstride["y"], cstride["x"], c_h, c_v)
 
 
 class Encoder:
@@ -703,6 +764,40 @@ class Encoder:
         if iface.get("stream") is not None:
             self._dev().wait_stream(int(iface["stream"]))
         return self.encode_batch_device_samples(ptr, n, w, h, ct, st, image_stride, row_stride, plane_stride, value_range)
+
+    def encode_batch_device_ycbcr(self, y, cb, cr, n, width, height, y_image_stride, y_row_stride, c_image_stride, c_row_stride,
+                                  c_sample_stride, c_h, c_v):
+        """YCbCr frames with subsampled chroma (jpgb_device_ycbcr, include/jpegenc_b200.h): device pointers of image 0's
+        first Y, Cb and Cr sample, strides in bytes. Chroma sample (x // c_h, y // c_v) stands for the pixels it covers.
+        Returns (device pointer of the files, offsets[n+1]), like encode_batch_device."""
+        dev = self._dev()
+        p = self._params(width, height, ColorType.Ycbcr)
+        f = _DeviceYcbcr(y, cb, cr, y_image_stride, y_row_stride, c_image_stride, c_row_stride, c_sample_stride, c_h, c_v)
+        d_files = C.c_void_p()
+        offs = (C.c_uint64 * (n + 1))()
+        rc = dev.lib.jpgb_encode_batch_device_ycbcr(dev.handle, C.byref(p), C.byref(f), n, C.byref(d_files), offs)
+        if rc != 0:
+            self._raise(rc)
+        return d_files.value, list(offs)
+
+    def encode_cuda_ycbcr(self, y, cb, cr):
+        """Encode YCbCr video frames where they lie (I420, I422, I444, NV12, NV21, NV16): `__cuda_array_interface__`
+        objects (torch CUDA tensors). y is (N, H, W) or (H, W) uint8; cb and cr are (N, ch, cw) or (ch, cw) uint8 views
+        with the same strides and an x stride of 1 (planar) or 2 (interleaved). The subsampling follows from the shapes:
+        cw == W is 1:1 across, cw == ceil(W / 2) is 2:1, and rows alike. The JPEG sampling is the encoder's own.
+        Samples are taken as full-range YCbCr, verbatim. An NV12 frame buffer f of shape (H * 3 // 2, W):
+
+            y = f[:H]
+            uv = f[H:].view(H // 2, W // 2, 2)
+            enc.encode_cuda_ycbcr(y, uv[..., 0], uv[..., 1])      # NV21: uv[..., 1], uv[..., 0]
+
+        When an interface names a stream, the encode waits for it first. Returns (device pointer of the files,
+        offsets[n+1]), like encode_batch_device."""
+        ifaces = [a.__cuda_array_interface__ for a in (y, cb, cr)]
+        lay = _cuda_ycbcr_layout(*ifaces)
+        for s in sorted({int(i["stream"]) for i in ifaces if i.get("stream") is not None}):
+            self._dev().wait_stream(s)
+        return self.encode_batch_device_ycbcr(*lay)
 
     # -- one large image cut into restart-aligned strips (BASELINE config 5) --
     def scan_count(self, width, height, color_type):
